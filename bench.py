@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- stereo frames/s of the ORB front-end (extract L+R + stereo match, 2000 features) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--frames F] [--transport nccl|peer] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--frames F] [--transport nccl|peer] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (pyramid+blur, FAST, quadtree, orientation+BRIEF, stereo match) over the synthetic
 4541-frame KITTI-00-length stereo sequence (BASELINE.json configs[2]; per frame it is configs[0]), sharded by frame over the
@@ -547,6 +547,43 @@ def bench_other_configs(args, api, torch, stream, local_rank, with_oracle):
     return out
 
 
+DUMP_FRAMES = 32  # frames per sampled output: about 30 MB of .npy files in all at 2000 features
+
+
+def dump_outputs(out_dir, ctx, torch, d_rec, n_local, res, F):
+    """Write what the last timed step returned as float32 / float64 .npy files: the per-frame records of a fixed, seeded
+    sample of this rank's frames, the gathered left descriptors of a seeded sample of the sequence's frames and the gathered
+    keypoint counts of every frame.  Entries past a frame's keypoint count are not part of the result and are written as 0."""
+    from orb_slam2_ros2_b200 import api
+
+    os.makedirs(out_dir, exist_ok=True)
+    N = ctx.n_features
+    rng = np.random.default_rng(0)
+    out = {}
+    idx = np.sort(rng.choice(n_local, min(n_local, DUMP_FRAMES), replace=False))
+    rec = d_rec[torch.from_numpy(idx).cuda()].cpu().numpy().view(ctx.record_dtype())[:, 0]
+    out["frames"] = idx.astype(np.float64)  # rank 0's block starts at frame 0
+    for side in ("left", "right"):
+        n = rec["n_" + side]
+        keep = np.arange(N)[None, :] < n[:, None]
+        kps = rec["kps_" + side]
+        out["n_" + side] = n.astype(np.float64)
+        out["kps_" + side] = np.where(keep[..., None], np.stack([kps[f].astype(np.float32) for f in api.KP_DTYPE.names], -1), 0)
+        out["desc_" + side] = np.where(keep[..., None], rec["desc_" + side], 0).astype(np.float32)
+        if side == "left":
+            out["u_right"], out["depth"] = np.where(keep, rec["u_right"], 0.0), np.where(keep, rec["depth"], 0.0)
+    out["n_matches"] = rec["n_matches"].astype(np.float64)
+    g_n = ctx.read_device(res.gathered_n, (F,), np.int32)
+    g_idx = np.sort(rng.choice(F, min(F, DUMP_FRAMES), replace=False))
+    g_desc = torch.as_tensor(CudaArray(res.gathered_desc, (res.world * res.block, N, 32), "|u1"), device="cuda")
+    keep = np.arange(N)[None, :] < g_n[g_idx][:, None]
+    out["gathered_n"] = g_n.astype(np.float64)
+    out["gathered_frames"] = g_idx.astype(np.float64)
+    out["gathered_desc"] = np.where(keep[..., None], g_desc[torch.from_numpy(g_idx).cuda()].cpu().numpy(), 0).astype(np.float32)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_gpu_arm(args):
     import torch
     import torch.distributed as dist
@@ -656,6 +693,8 @@ def run_gpu_arm(args):
     ms = e0.elapsed_time(e1)
     launches = ctx.launch_count - launches0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx, torch, d_rec, n_local, last["res"], F)
     t = torch.tensor([ms], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -892,7 +931,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-matchers", action="store_true", help="skip the secondary tracking-matcher / serialisation / bag-of-words measurements")
     ap.add_argument("--no-configs", action="store_true", help="skip the secondary BASELINE configurations (TUM RGB-D, 1080p, latency sweep)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step (a seeded sample of frames) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference_arm(args)

@@ -40,6 +40,14 @@ def main():
         np.savez_compressed(os.path.join(OUT, "kitti_stereo_seed0_d17.npz"), seed=0, disparity=17, left_sha=sha(left), right_sha=sha(right),
                             kl=r["kl"], dl=r["dl"], kr=r["kr"], dr=r["dr"], u_right=r["u_right"], depth=r["depth"], n_matches=r["n_matches"],
                             pyr_sha=np.array([sha(l) for l in info["levels"]]))
+        # 1b. TUM-shaped stereo pair, 1000 features (test_gpu_parity.py::test_stereo_matches_the_compiled_reference)
+        c = synth.TUM
+        left, right = synth.synth_stereo_pair(c["height"], c["width"], 3, 17)
+        O.ref_reset()
+        O.ref_set_camera(c["fx"], c["fy"], c["cx"], c["cy"], c["bl"], None)
+        r = O.ref_stereo(left, right, tp, 1000, 8, 1.2)
+        np.savez_compressed(os.path.join(OUT, "tum_stereo_seed3_d17.npz"), seed=3, disparity=17, left_sha=sha(left), right_sha=sha(right),
+                            kl=r["kl"], dl=r["dl"], kr=r["kr"], dr=r["dr"], u_right=r["u_right"], depth=r["depth"], n_matches=r["n_matches"])
         # 2. small stereo pair used by smoke-sized tests: 320x240, 500 features, 4 levels
         left, right = synth.synth_stereo_pair(240, 320, 0, 9)
         O.ref_reset()

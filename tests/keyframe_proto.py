@@ -1,6 +1,6 @@
 """The orbslam2.KeyFrameData schema (reference: proto/Keyframe.proto:1-70) restated as a dynamically built descriptor for
-the python protobuf runtime (this image has no protoc).  test_serialize.py checks the restatement against the reference's
-.proto text when /root/reference is present, and uses the runtime's own serializer / parser as the wire-format oracle."""
+the python protobuf runtime (no protoc needed).  test_serialize.py checks the restatement against a digest of the
+reference's .proto text as parse_proto_text reads it, and uses the runtime's own serializer / parser as the wire-format oracle."""
 import re
 
 from google.protobuf import descriptor_pb2, descriptor_pool, message_factory
