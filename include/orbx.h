@@ -250,6 +250,27 @@ typedef struct orbx_sequence_result {
  * max_batch device slots in chunks on the pipeline streams (H2D of one chunk, kernels of another, D2H of a third overlap). */
 int orbx_sequence_stereo(orbx_ctx *ctx, orbx_comm *comm, int64_t n_frames_total, const orbx_sequence_io *io, orbx_sequence_result *out);
 
+/* Offline map export: the same call, and in addition every frame of this rank's block as the orbslam2.KeyFrameData record
+ * of a keyframe made from it (orbx_serialize_keyframe_bow, src/KeyFrame.cc:553-647,585-599).  After a chunk's records are
+ * packed, three kernels run on its stream: the bag-of-words descent and assembly (VirtualFrame::computeBow,
+ * include/ORB_SLAM2/Frame.h:224-231) and the serialiser.  Keyframe records stay on their rank; the descriptor gather is
+ * unchanged.  Host outputs leave the device in one copy per chunk (and one copy of `sizes` at the end).  The BoW results
+ * are not kept resident: orbx_search_by_bow still returns ORBX_ERR_STATE afterwards.  Write a KeyFrameList with
+ * orbx_keyframe_list_head (rank 0 only, next_id = id0 + n_frames_total) and orbx_keyframe_list_entry_prefix. */
+typedef struct orbx_keyframe_io {
+  const struct orbx_vocab *vocab; /* NULL: fields 10 / 11 present but empty, as orbx_serialize_keyframe (must belong to this context) */
+  int32_t levelsup;        /* 4 = VirtualFrame::computeBow (include/ORB_SLAM2/Frame.h:224-231) */
+  int32_t with_map_points;
+  uint64_t id0;            /* the record of GLOBAL frame f carries id id0 + f */
+  const float *pose_rt;    /* [n_local][12] Tcw (R row-major, t) in the same memory as `out`, or NULL = identity */
+  int32_t on_device;       /* where out / sizes / pose_rt live */
+  uint8_t *out;            /* [n_local][stride], this rank's block; 16-byte aligned */
+  size_t stride;           /* >= orbx_serialized_capacity_bow (vocab) / orbx_serialized_capacity (no vocab), multiple of 16 */
+  int64_t *sizes;          /* [n_local] bytes of each record */
+} orbx_keyframe_io;
+int orbx_sequence_stereo_keyframes(orbx_ctx *ctx, orbx_comm *comm, int64_t n_frames_total, const orbx_sequence_io *io,
+                                   const orbx_keyframe_io *kf, orbx_sequence_result *out);
+
 /* ---- tracking-side Hamming matchers (SURVEY.md section 8(f) rank 2) -------------------------------------- */
 /* One query of VirtualFrame::findFeaturesInArea (src/Frame.cc:286-311): the keypoint `kp` (position in undistorted
  * image coordinates + octave), the radius BEFORE its multiplication by getScaledFactor2(kp.octave), and the inclusive
@@ -311,6 +332,28 @@ int orbx_serialize_keyframe_text(orbx_ctx *ctx, int frame, uint64_t id, const fl
  * 4-byte aligned), its size in d_sizes[f]. */
 int orbx_serialize_keyframes_device(orbx_ctx *ctx, int n_frames, uint64_t id0, const float *d_pose_rt,
                                     int with_map_points, uint8_t *d_out, size_t frame_stride, int64_t *d_sizes);
+
+/* The same record for a keyframe whose bag of words has been computed (src/KeyFrame.cc:553-647, fields 10 / 11 filled from
+ * mBowVec / mFeatVec at :585-599): bow_vector = 10 { map<uint32, double> words = 1 } with one entry per word in ascending
+ * word id (std::map order), key and value always written; feature_vector = 11 { repeated FeatureNode nodes = 1 } with the
+ * nodes in ascending id, each { node_id = 1 (left out when 0), packed feature_ids = 2 in ascending feature index }.
+ * The BoW of the frame(s) must be resident from orbx_bow_transform* on the same call's frames (as for orbx_search_by_bow):
+ * ORBX_ERR_STATE otherwise.  Everything else is as orbx_serialize_keyframe / orbx_serialize_keyframes_device, with the
+ * larger bound orbx_serialized_capacity_bow (multiple of 16). */
+int64_t orbx_serialized_capacity_bow(const orbx_ctx *ctx);
+int orbx_serialize_keyframe_bow(orbx_ctx *ctx, int frame, uint64_t id, const float *pose_rt /* [12] or NULL */,
+                                int with_map_points, uint8_t *out, size_t cap, int64_t *n_bytes);
+int orbx_serialize_keyframes_bow_device(orbx_ctx *ctx, int n_frames, uint64_t id0, const float *d_pose_rt,
+                                        int with_map_points, uint8_t *d_out, size_t frame_stride, int64_t *d_sizes);
+
+/* KeyFrameList { uint64 next_id = 1; repeated float scale_factors = 2; repeated KeyFrameData keyframes = 3 }
+ * (proto/Keyframe.proto:66-70, writer src/Map.cc:205-224), written piecewise: the head (next_id, left out when 0, and the
+ * context's level scale factors, packed), then for every record the prefix 0x1A varint(record_bytes) and the record.
+ * A sharded export stays ONE list: rank 0 writes head + entries, every other rank entries only; the per-rank outputs
+ * concatenated in rank order parse as a single KeyFrameList.  *n_bytes is set even when cap is too small. */
+int orbx_keyframe_list_head(const orbx_ctx *ctx, uint64_t next_id, uint8_t *out, size_t cap, int64_t *n_bytes);
+/* writes the entry prefix of a record of record_bytes bytes; returns its length (<= 11) or ORBX_ERR_INVALID_ARG */
+int orbx_keyframe_list_entry_prefix(int64_t record_bytes, uint8_t *out /* [11] */);
 
 /* ---- bag-of-words transform (SURVEY.md section 8(f) rank 3) ----------------------------------------------- */
 /* A DBoW3::Vocabulary (the reference loads one in src/System.cc:93) resident on the context's device.  Records follow

@@ -21,16 +21,6 @@
 
 using namespace orbx;
 
-// DBoW3 vocabulary tree resident on one device
-struct orbx_vocab
-{
-  int device = 0;
-  int k = 0, L = 0, n_nodes = 0, n_words = 0;
-  int *child_start = nullptr, *child_ids = nullptr, *word = nullptr;
-  uint8_t *desc = nullptr;
-  double *weight = nullptr;
-};
-
 namespace
 {
 
@@ -479,6 +469,36 @@ int fail(orbx_ctx *c, int code, const std::string &msg)
   return code;
 }
 
+int bow_buffers(orbx_ctx *c)
+{
+  if (c->bow_ready) return ORBX_OK;
+  const size_t F = (size_t)c->cfg.max_batch, N = (size_t)c->cfg.n_features;
+  if (N > 65535) return fail(c, ORBX_ERR_CAPACITY, "the bag-of-words kernels index features with 16 bits");
+  int rc;
+  BowArgs &b = c->bow;
+  if ((rc = dev_alloc(c, &b.f_word, F * N))) return rc;
+  if ((rc = dev_alloc(c, &b.f_nid, F * N))) return rc;
+  if ((rc = dev_alloc(c, &b.f_weight, F * N))) return rc;
+  if ((rc = dev_alloc(c, &b.bow_ids, F * N))) return rc;
+  if ((rc = dev_alloc(c, &b.bow_vals, F * N))) return rc;
+  if ((rc = dev_alloc(c, &b.n_bow, F))) return rc;
+  if ((rc = dev_alloc(c, &b.fv_nodes, F * N))) return rc;
+  if ((rc = dev_alloc(c, &b.fv_start, F * (N + 1)))) return rc;
+  if ((rc = dev_alloc(c, &b.fv_feats, F * N))) return rc;
+  if ((rc = dev_alloc(c, &b.n_fv, F))) return rc;
+  if (bow_configure((int)N) != 0) return fail(c, ORBX_ERR_CUDA, "cannot reserve shared memory for the bag-of-words sort");
+  c->bow_ready = true;
+  return ORBX_OK;
+}
+
+BowArgs bow_args(const orbx_ctx *c, const orbx_vocab *v, int levelsup)
+{
+  BowArgs a = c->bow;
+  a.child_start = v->child_start, a.child_ids = v->child_ids, a.v_desc = v->desc, a.v_weight = v->weight, a.v_word = v->word;
+  a.L = v->L, a.levelsup = levelsup, a.image_stride = c->last_stereo ? 2 : 1;
+  return a;
+}
+
 // Params whose per-image buffers start at image `img0` (and per-frame buffers at frame `frame0`)
 Params params_at(const orbx_ctx *c, int img0, int frame0)
 {
@@ -881,6 +901,8 @@ extern "C"
     destroy_self_comm(c);
     if (c->rec_staging) cudaFree(c->rec_staging);
     if (c->h_rec1) cudaFreeHost(c->h_rec1);
+    if (c->kf_staging) cudaFree(c->kf_staging);
+    if (c->kf_sizes) cudaFree(c->kf_sizes);
     delete c;
   }
 
@@ -1441,30 +1463,57 @@ extern "C"
     return (int64_t)((128 + (size_t)c->cfg.n_features * (28 + 4 + 4 + 36 + 10) + 15) & ~(size_t)15);
   }
 
-  int orbx_serialize_keyframes_device(orbx_ctx *c, int n_frames, uint64_t id0, const float *d_pose_rt, int with_map_points, uint8_t *d_out,
-                                      size_t frame_stride, int64_t *d_sizes)
+  int64_t orbx_serialized_capacity_bow(const orbx_ctx *c)
+  {
+    if (!c) return 0;
+    // + per keypoint at most one BowVector entry (<= 17) and one FeatureNode (<= 13 + 3 per feature id), + two field headers
+    return (int64_t)((128 + 12 + (size_t)c->cfg.n_features * (28 + 4 + 4 + 36 + 10 + 17 + 13 + 3) + 15) & ~(size_t)15);
+  }
+
+  static bool bow_resident(const orbx_ctx *c, int n_frames) { return c->bow_epoch == c->frame_epoch && n_frames <= c->bow_frames; }
+
+  static int serialize_frames_device(orbx_ctx *c, int n_frames, uint64_t id0, const float *d_pose_rt, int with_map_points, uint8_t *d_out,
+                                     size_t frame_stride, int64_t *d_sizes, bool bow)
   {
     if (!c || n_frames < 1 || !d_out || !d_sizes) return ORBX_ERR_INVALID_ARG;
     if (((size_t)d_out & 3) || (frame_stride & 3)) return fail(c, ORBX_ERR_INVALID_ARG, "output buffer and stride must be 4-byte aligned");
+    if (bow && (int64_t)frame_stride < orbx_serialized_capacity_bow(c))
+      return fail(c, ORBX_ERR_CAPACITY, "frame_stride is smaller than orbx_serialized_capacity_bow()");
     if ((int64_t)frame_stride < orbx_serialized_capacity(c)) return fail(c, ORBX_ERR_CAPACITY, "frame_stride is smaller than orbx_serialized_capacity()");
     if (n_frames > c->last_frames) return fail(c, ORBX_ERR_STATE, "more frames than the last stereo / RGB-D call processed");
+    if (bow && !bow_resident(c, n_frames)) return fail(c, ORBX_ERR_STATE, "call orbx_bow_transform* for these frames first (their BoW must be resident)");
     ORBX_CUDA(c, cudaSetDevice(c->device));
     SerArgs a{};
     a.out = d_out, a.stride = frame_stride, a.sizes = (long long *)d_sizes, a.id0 = id0, a.pose = d_pose_rt, a.with_map_points = with_map_points;
     a.image_stride = c->last_stereo ? 2 : 1;
     a.max_u = c->max_u, a.max_v = c->max_v, a.min_u = c->min_u, a.min_v = c->min_v;
+    if (bow) ser_bow_inputs(a, c->bow, 0, (size_t)c->cfg.n_features);
     launch_serialize(c->p, a, n_frames, c->stream);
     ++c->launches;
     ORBX_CUDA(c, cudaGetLastError());
     return ORBX_OK;
   }
 
-  int orbx_serialize_keyframe(orbx_ctx *c, int frame, uint64_t id, const float *pose_rt, int with_map_points, uint8_t *out, size_t cap, int64_t *n_bytes)
+  int orbx_serialize_keyframes_device(orbx_ctx *c, int n_frames, uint64_t id0, const float *d_pose_rt, int with_map_points, uint8_t *d_out,
+                                      size_t frame_stride, int64_t *d_sizes)
+  {
+    return serialize_frames_device(c, n_frames, id0, d_pose_rt, with_map_points, d_out, frame_stride, d_sizes, false);
+  }
+
+  int orbx_serialize_keyframes_bow_device(orbx_ctx *c, int n_frames, uint64_t id0, const float *d_pose_rt, int with_map_points, uint8_t *d_out,
+                                          size_t frame_stride, int64_t *d_sizes)
+  {
+    return serialize_frames_device(c, n_frames, id0, d_pose_rt, with_map_points, d_out, frame_stride, d_sizes, true);
+  }
+
+  static int serialize_frame(orbx_ctx *c, int frame, uint64_t id, const float *pose_rt, int with_map_points, uint8_t *out, size_t cap, int64_t *n_bytes,
+                             bool bow)
   {
     if (!c || frame < 0 || !out || !n_bytes) return ORBX_ERR_INVALID_ARG;
     if (frame >= c->last_frames) return fail(c, ORBX_ERR_STATE, "no frame with that index has been processed by a stereo / RGB-D call");
+    if (bow && !bow_resident(c, frame + 1)) return fail(c, ORBX_ERR_STATE, "call orbx_bow_transform for this frame first (its BoW must be resident)");
     ORBX_CUDA(c, cudaSetDevice(c->device));
-    const size_t rec = (size_t)orbx_serialized_capacity(c);
+    const size_t rec = (size_t)(bow ? orbx_serialized_capacity_bow(c) : orbx_serialized_capacity(c));
     uint8_t *base = nullptr;
     int rc = match_scratch(c, rec + 256, &base);
     if (rc) return rc;
@@ -1478,6 +1527,7 @@ extern "C"
     a.image_stride = c->last_stereo ? 2 : 1;
     a.max_u = c->max_u, a.max_v = c->max_v, a.min_u = c->min_u, a.min_v = c->min_v;
     const Params p = params_at(c, frame * a.image_stride, frame); // the single CTA (block 0) works on `frame`
+    if (bow) ser_bow_inputs(a, c->bow, (size_t)frame, (size_t)c->cfg.n_features);
     launch_serialize(p, a, 1, s);
     ++c->launches;
     ORBX_CUDA(c, cudaGetLastError());
@@ -1488,6 +1538,47 @@ extern "C"
     if ((size_t)sz > cap) return fail(c, ORBX_ERR_CAPACITY, "output buffer too small for the record (see *n_bytes)");
     ORBX_CUDA(c, cudaMemcpy(out, base, (size_t)sz, cudaMemcpyDeviceToHost));
     return ORBX_OK;
+  }
+
+  int orbx_serialize_keyframe(orbx_ctx *c, int frame, uint64_t id, const float *pose_rt, int with_map_points, uint8_t *out, size_t cap, int64_t *n_bytes)
+  {
+    return serialize_frame(c, frame, id, pose_rt, with_map_points, out, cap, n_bytes, false);
+  }
+
+  int orbx_serialize_keyframe_bow(orbx_ctx *c, int frame, uint64_t id, const float *pose_rt, int with_map_points, uint8_t *out, size_t cap,
+                                  int64_t *n_bytes)
+  {
+    return serialize_frame(c, frame, id, pose_rt, with_map_points, out, cap, n_bytes, true);
+  }
+
+  int orbx_keyframe_list_head(const orbx_ctx *c, uint64_t next_id, uint8_t *out, size_t cap, int64_t *n_bytes)
+  {
+    if (!c || !out || !n_bytes) return ORBX_ERR_INVALID_ARG;
+    uint8_t buf[16 + 4 * kMaxLevels];
+    size_t n = 0;
+    auto varint = [&](uint64_t v) {
+      while (v >= 0x80u) buf[n++] = (uint8_t)(v | 0x80u), v >>= 7;
+      buf[n++] = (uint8_t)v;
+    };
+    if (next_id) buf[n++] = 0x08, varint(next_id); // uint64 next_id = 1 (proto3: left out when 0)
+    buf[n++] = 0x12;                                // repeated float scale_factors = 2, packed
+    varint(4u * (uint64_t)c->levels.size());
+    for (const Level &L : c->levels) std::memcpy(buf + n, &L.sf, 4), n += 4;
+    *n_bytes = (int64_t)n;
+    if (n > cap) return ORBX_ERR_CAPACITY;
+    std::memcpy(out, buf, n);
+    return ORBX_OK;
+  }
+
+  int orbx_keyframe_list_entry_prefix(int64_t record_bytes, uint8_t *out)
+  {
+    if (!out || record_bytes < 0) return ORBX_ERR_INVALID_ARG;
+    int n = 0;
+    uint64_t v = (uint64_t)record_bytes;
+    out[n++] = 0x1A; // repeated KeyFrameData keyframes = 3
+    while (v >= 0x80u) out[n++] = (uint8_t)(v | 0x80u), v >>= 7;
+    out[n++] = (uint8_t)v;
+    return n;
   }
 
   int orbx_serialize_keyframe_text(orbx_ctx *c, int frame, uint64_t id, const float *pose_rt, int with_map_points, int with_scale_header, uint64_t next_id,
@@ -1601,7 +1692,7 @@ extern "C"
     std::memcpy(w.data() + 1, weight, (size_t)n_records * sizeof(double));
     ORBX_CUDA(c, cudaSetDevice(c->device));
     orbx_vocab *v = new orbx_vocab();
-    v->device = c->device, v->k = k, v->L = L, v->n_nodes = n, v->n_words = n_words;
+    v->ctx = c, v->device = c->device, v->k = k, v->L = L, v->n_nodes = n, v->n_words = n_words;
     auto up = [&](auto **dst, const auto &src) -> cudaError_t {
       cudaError_t e = cudaMalloc((void **)dst, src.size() * sizeof(src[0]) + 64);
       if (e != cudaSuccess) return e;
@@ -1674,28 +1765,6 @@ extern "C"
     return ORBX_OK;
   }
 
-  static int bow_buffers(orbx_ctx *c)
-  {
-    if (c->bow_ready) return ORBX_OK;
-    const size_t F = (size_t)c->cfg.max_batch, N = (size_t)c->cfg.n_features;
-    if (N > 65535) return fail(c, ORBX_ERR_CAPACITY, "the bag-of-words kernels index features with 16 bits");
-    int rc;
-    BowArgs &b = c->bow;
-    if ((rc = dev_alloc(c, &b.f_word, F * N))) return rc;
-    if ((rc = dev_alloc(c, &b.f_nid, F * N))) return rc;
-    if ((rc = dev_alloc(c, &b.f_weight, F * N))) return rc;
-    if ((rc = dev_alloc(c, &b.bow_ids, F * N))) return rc;
-    if ((rc = dev_alloc(c, &b.bow_vals, F * N))) return rc;
-    if ((rc = dev_alloc(c, &b.n_bow, F))) return rc;
-    if ((rc = dev_alloc(c, &b.fv_nodes, F * N))) return rc;
-    if ((rc = dev_alloc(c, &b.fv_start, F * (N + 1)))) return rc;
-    if ((rc = dev_alloc(c, &b.fv_feats, F * N))) return rc;
-    if ((rc = dev_alloc(c, &b.n_fv, F))) return rc;
-    if (bow_configure((int)N) != 0) return fail(c, ORBX_ERR_CUDA, "cannot reserve shared memory for the bag-of-words sort");
-    c->bow_ready = true;
-    return ORBX_OK;
-  }
-
   int orbx_bow_transform_batch_device(orbx_ctx *c, const orbx_vocab *v, int n_frames, int levelsup, orbx_device_bow *out)
   {
     if (!c || !v || n_frames < 1 || !out) return ORBX_ERR_INVALID_ARG;
@@ -1704,9 +1773,7 @@ extern "C"
     ORBX_CUDA(c, cudaSetDevice(c->device));
     int rc = bow_buffers(c);
     if (rc) return rc;
-    BowArgs a = c->bow;
-    a.child_start = v->child_start, a.child_ids = v->child_ids, a.v_desc = v->desc, a.v_weight = v->weight, a.v_word = v->word;
-    a.L = v->L, a.levelsup = levelsup, a.image_stride = c->last_stereo ? 2 : 1;
+    const BowArgs a = bow_args(c, v, levelsup);
     launch_bow_descend(c->p, a, n_frames, c->stream);
     launch_bow_assemble(c->p, a, n_frames, c->stream);
     c->launches += 2;

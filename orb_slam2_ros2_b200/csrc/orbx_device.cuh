@@ -199,6 +199,10 @@ struct SerArgs
   int with_map_points;
   int image_stride;
   float max_u, max_v, min_u, min_v;
+  // optional BowVector / FeatureVector of the launch's frames in the layout of BowArgs (per frame: n_features entries,
+  // fv_start n_features + 1); null = fields 10 / 11 present but empty
+  const int *bow_ids, *n_bow, *fv_nodes, *fv_start, *fv_feats, *n_fv;
+  const double *bow_vals;
 };
 
 // bag-of-words transform (orbx_bow.cu)
@@ -218,6 +222,14 @@ struct BowArgs
   double *bow_vals;
   int *fv_nodes, *fv_start /* [frame][n_features + 1] */, *fv_feats, *n_fv;
 };
+
+// the BoW results of frame `frame0` onwards as serialiser inputs
+inline void ser_bow_inputs(SerArgs &s, const BowArgs &b, size_t frame0, size_t n_features)
+{
+  s.bow_ids = b.bow_ids + frame0 * n_features, s.bow_vals = b.bow_vals + frame0 * n_features, s.n_bow = b.n_bow + frame0;
+  s.fv_nodes = b.fv_nodes + frame0 * n_features, s.fv_start = b.fv_start + frame0 * (n_features + 1), s.fv_feats = b.fv_feats + frame0 * n_features;
+  s.n_fv = b.n_fv + frame0;
+}
 
 // launchers (orbx_kernels.cu / orbx_match.cu / orbx_serialize.cu / orbx_bow.cu); every call enqueues exactly one kernel on `s` (launch_pyramid: two)
 constexpr int kPyramidLaunches = 2;

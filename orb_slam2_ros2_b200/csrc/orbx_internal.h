@@ -62,6 +62,23 @@ struct orbx_ctx
   uint64_t frame_epoch = 0;   // bumped by every call that produces frames
   uint64_t bow_epoch = ~0ull; // frame_epoch at the last bag-of-words call
   int bow_frames = 0;         // frames covered by that call
+  // keyframe records of sequences (orbx_sequence_stereo_keyframes): per-slot staging of records + poses for host outputs,
+  // and the sizes of a whole block (copied to the host once at the end)
+  uint8_t *kf_staging = nullptr;
+  size_t kf_staging_bytes = 0;
+  int64_t *kf_sizes = nullptr;
+  size_t kf_sizes_count = 0;
+};
+
+// DBoW3 vocabulary tree resident on one device
+struct orbx_vocab
+{
+  const orbx_ctx *ctx = nullptr; // the context that created it
+  int device = 0;
+  int k = 0, L = 0, n_nodes = 0, n_words = 0;
+  int *child_start = nullptr, *child_ids = nullptr, *word = nullptr;
+  uint8_t *desc = nullptr;
+  double *weight = nullptr;
 };
 
 namespace orbx
@@ -81,6 +98,10 @@ int pack_frame_records(orbx_ctx *c, cudaStream_t s, int d0, int nf, uint8_t *d_r
 int ensure_record_staging(orbx_ctx *c, size_t rec_stride);
 // frees the gathered arrays a context keeps for single-rank sequence calls
 void destroy_self_comm(orbx_ctx *c);
+// allocates the context's bag-of-words result buffers (max_batch frames) on first use
+int bow_buffers(orbx_ctx *c);
+// c->bow with the vocabulary's tree, ready for launch_bow_descend / launch_bow_assemble
+BowArgs bow_args(const orbx_ctx *c, const orbx_vocab *v, int levelsup);
 
 } // namespace orbx
 

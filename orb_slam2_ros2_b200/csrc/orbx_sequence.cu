@@ -11,6 +11,9 @@
 //   peer   the pack kernel that assembles the records stores the descriptors straight into every rank's gathered array
 //          through peer pointers (same process: cudaDeviceEnablePeerAccess; other processes: CUDA IPC handles) -- the
 //          gather is fused into the kernel that produces the data and rides NVLink as plain stores
+// For an offline map export (orbx_sequence_stereo_keyframes) every chunk also runs, after its pack kernel, the
+// bag-of-words descent and assembly and the serialiser on its own slots, so that each frame additionally leaves the
+// device as the KeyFrameData record of a keyframe made from it; those records stay on their rank.
 #include <dlfcn.h>
 
 #include <algorithm>
@@ -215,6 +218,76 @@ int ensure_record_staging_impl(orbx_ctx *c, size_t rec_stride)
   return ORBX_OK;
 }
 
+// host-side keyframe outputs: per slot `stride` bytes of record + 12 floats of pose; the sizes of a whole block
+int ensure_keyframe_staging(orbx_ctx *c, size_t stride, int64_t n_local)
+{
+  const size_t want = (size_t)c->cfg.max_batch * (stride + 12 * sizeof(float));
+  const size_t n_sizes = (size_t)std::max<int64_t>(1, n_local);
+  if ((c->kf_staging && c->kf_staging_bytes < want) || (c->kf_sizes && c->kf_sizes_count < n_sizes)) ORBX_CUDA(c, cudaDeviceSynchronize());
+  if (c->kf_staging && c->kf_staging_bytes < want)
+  {
+    cudaFree(c->kf_staging);
+    c->kf_staging = nullptr;
+  }
+  if (!c->kf_staging)
+  {
+    ORBX_CUDA(c, cudaMalloc((void **)&c->kf_staging, want));
+    c->kf_staging_bytes = want;
+  }
+  if (c->kf_sizes && c->kf_sizes_count < n_sizes)
+  {
+    cudaFree(c->kf_sizes);
+    c->kf_sizes = nullptr;
+  }
+  if (!c->kf_sizes)
+  {
+    ORBX_CUDA(c, cudaMalloc((void **)&c->kf_sizes, n_sizes * sizeof(int64_t)));
+    c->kf_sizes_count = n_sizes;
+  }
+  return ORBX_OK;
+}
+
+// keyframe records of the chunk in device slots [d0, d0 + nf) = local frames [f0, f0 + nf), on the chunk's stream after its
+// pack kernel: bag-of-words descent + assembly into the slots' BoW buffers (with a vocabulary), then the serialiser
+int keyframe_chunk(orbx_ctx *c, const orbx_keyframe_io *kio, const Params &p, cudaStream_t s, size_t d0, int64_t f0, int nf, int64_t lo)
+{
+  const size_t N = (size_t)c->cfg.n_features, ks = kio->stride;
+  const bool host = !kio->on_device;
+  uint8_t *stage = host ? c->kf_staging + d0 * ks : nullptr;
+  float *stage_pose = host ? reinterpret_cast<float *>(c->kf_staging + (size_t)c->cfg.max_batch * ks) + d0 * 12 : nullptr;
+  SerArgs sa{};
+  sa.out = host ? stage : kio->out + (size_t)f0 * ks;
+  sa.stride = ks;
+  sa.sizes = (long long *)(host ? c->kf_sizes : kio->sizes) + f0;
+  sa.id0 = kio->id0 + (uint64_t)(lo + f0);
+  sa.pose = nullptr;
+  if (kio->pose_rt)
+  {
+    if (host) ORBX_CUDA(c, cudaMemcpyAsync(stage_pose, kio->pose_rt + (size_t)f0 * 12, (size_t)nf * 12 * sizeof(float), cudaMemcpyHostToDevice, s));
+    sa.pose = host ? stage_pose : kio->pose_rt + (size_t)f0 * 12;
+  }
+  sa.with_map_points = kio->with_map_points;
+  sa.image_stride = 2;
+  sa.max_u = c->max_u, sa.max_v = c->max_v, sa.min_u = c->min_u, sa.min_v = c->min_v;
+  if (kio->vocab)
+  {
+    BowArgs ba = bow_args(c, kio->vocab, kio->levelsup);
+    ba.image_stride = 2;
+    ba.f_word += d0 * N, ba.f_nid += d0 * N, ba.f_weight += d0 * N; // the slots' own frames of the max_batch-frame buffers
+    ba.bow_ids += d0 * N, ba.bow_vals += d0 * N, ba.n_bow += d0;
+    ba.fv_nodes += d0 * N, ba.fv_start += d0 * (N + 1), ba.fv_feats += d0 * N, ba.n_fv += d0;
+    launch_bow_descend(p, ba, nf, s);
+    launch_bow_assemble(p, ba, nf, s);
+    c->launches += 2;
+    ser_bow_inputs(sa, ba, 0, N);
+  }
+  launch_serialize(p, sa, nf, s);
+  ++c->launches;
+  ORBX_CUDA(c, cudaGetLastError());
+  if (host) ORBX_CUDA(c, cudaMemcpyAsync(kio->out + (size_t)f0 * ks, stage, ks * nf, cudaMemcpyDeviceToHost, s));
+  return ORBX_OK;
+}
+
 void comm_free(orbx_comm *m)
 {
   if (!m) return;
@@ -400,8 +473,15 @@ extern "C"
 
   int orbx_sequence_stereo(orbx_ctx *c, orbx_comm *m, int64_t n_frames_total, const orbx_sequence_io *io, orbx_sequence_result *res)
   {
+    return orbx_sequence_stereo_keyframes(c, m, n_frames_total, io, nullptr, res);
+  }
+
+  int orbx_sequence_stereo_keyframes(orbx_ctx *c, orbx_comm *m, int64_t n_frames_total, const orbx_sequence_io *io, const orbx_keyframe_io *kio,
+                                     orbx_sequence_result *res)
+  {
     if (!c || !io || n_frames_total < 0 || !io->left || !io->right) return ORBX_ERR_INVALID_ARG;
     if (m && m->ctx != c) return fail(c, ORBX_ERR_INVALID_ARG, "communicator belongs to another context");
+    if (kio && kio->vocab && kio->vocab->ctx != c) return fail(c, ORBX_ERR_INVALID_ARG, "vocabulary belongs to another context");
     ORBX_CUDA(c, cudaSetDevice(c->device));
     if (!m)
     { // single rank: the context keeps its own gathered arrays
@@ -444,6 +524,18 @@ extern "C"
     const size_t W = (size_t)c->cfg.width, H = (size_t)c->cfg.height, N = (size_t)c->cfg.n_features;
     const size_t stride = io->stride, frame_stride = io->frame_stride;
     if (stride < W || frame_stride < stride * (H - 1) + W) return fail(c, ORBX_ERR_INVALID_ARG, "stride / frame_stride smaller than the image");
+    const bool kf_bow = kio && kio->vocab, kf_host = kio && !kio->on_device;
+    if (kio)
+    {
+      if (n_local > 0 && (!kio->out || !kio->sizes)) return fail(c, ORBX_ERR_INVALID_ARG, "keyframe io needs `out` and `sizes`");
+      if ((kio->stride & 15) || ((size_t)kio->out & 15))
+        return fail(c, ORBX_ERR_INVALID_ARG, "keyframe records must be 16-byte aligned with a stride that is a multiple of 16");
+      if ((int64_t)kio->stride < (kf_bow ? orbx_serialized_capacity_bow(c) : orbx_serialized_capacity(c)))
+        return fail(c, ORBX_ERR_CAPACITY, kf_bow ? "keyframe stride is smaller than orbx_serialized_capacity_bow()" : "keyframe stride is smaller than orbx_serialized_capacity()");
+      int rc = kf_bow ? bow_buffers(c) : ORBX_OK;
+      if (!rc && kf_host) rc = ensure_keyframe_staging(c, kio->stride, n_local);
+      if (rc) return rc;
+    }
 
     // inputs from the host are staged per slot exactly as in orbx_stereo_batch (one linear copy per side when rows are dense)
     size_t fs = c->in_pitch * H, dstride = c->in_pitch;
@@ -550,6 +642,11 @@ extern "C"
       ++c->launches;
       ORBX_CUDA(c, cudaGetLastError());
       if (rec_host) ORBX_CUDA(c, cudaMemcpyAsync((uint8_t *)io->records + (size_t)f0 * rs, c->rec_staging + d0 * rs, rs * nf, cudaMemcpyDeviceToHost, s));
+      if (kio)
+      {
+        rc = keyframe_chunk(c, kio, p, s, d0, f0, nf, lo);
+        if (rc) return rc;
+      }
       const int64_t done = f0 + nf;
       while (next_piece < n_pieces && done >= std::min<int64_t>(n_local, (next_piece + 1) * piece))
       {
@@ -571,6 +668,7 @@ extern "C"
         ORBX_NCCL(c, nccl().AllReduce(m->d_flag, m->d_flag + 1, 1, kNcclInt32, kNcclSum, m->nccl_comm, m->comm_stream));
       ORBX_CUDA(c, cudaStreamSynchronize(m->comm_stream));
     }
+    if (kf_host && n_local > 0) ORBX_CUDA(c, cudaMemcpy(kio->sizes, c->kf_sizes, (size_t)n_local * sizeof(int64_t), cudaMemcpyDeviceToHost));
     if (io->gathered_desc_host) ORBX_CUDA(c, cudaMemcpy(io->gathered_desc_host, m->g.desc(), (size_t)F * N * 32, cudaMemcpyDeviceToHost));
     if (io->gathered_n_host) ORBX_CUDA(c, cudaMemcpy(io->gathered_n_host, m->g.n(), (size_t)F * 4, cudaMemcpyDeviceToHost));
 

@@ -5,9 +5,12 @@
 // from a fresh frame, straight from the device-resident results: one CTA per frame, so that only the finished records
 // cross PCIe.  Layout of a record (fields in number order, as every protobuf serializer emits them):
 //   1 id | 2-5 max_u max_v min_u min_v | 6 keypoints[] | 7 right_u (packed) | 8 depths (packed) | 9 descriptors[] |
-//   10 bow_vector (present, empty) | 11 feature_vector (present, empty) | 12 pose | 16 map_points (packed, -1 each)
+//   10 bow_vector | 11 feature_vector | 12 pose | 16 map_points (packed, -1 each)
 // proto3 scalars whose bit pattern is zero are not written.  Keypoint entries have variable size (block scan for their
 // offsets, byte stores); everything behind them is fixed-stride and written as aligned words assembled byte by byte.
+// Fields 10 / 11 are present and empty unless the launch carries the frames' BoW results (SerArgs::bow_ids ...), as
+// KeyFrame::serializeToProtobuf fills them from mBowVec / mFeatVec (src/KeyFrame.cc:585-599): then they are byte-stored
+// entries at offsets from closed forms (sorted ids -> varint sizes by binary search) and a block scan over the nodes.
 #include "orbx_device.cuh"
 
 namespace orbx
@@ -76,11 +79,52 @@ __device__ __forceinline__ int keypoint_entry(const orbx_keypoint &k, uint8_t *m
   return l;
 }
 
+__device__ __forceinline__ int varint_len(unsigned long long v)
+{
+  int n = 1;
+  while (v >= 0x80ull) v >>= 7, ++n;
+  return n;
+}
+
+// first index in the ascending a[lo, hi) whose value is >= v
+__device__ __forceinline__ int lower_bound_int(const int *a, int lo, int hi, int v)
+{
+  while (lo < hi)
+  {
+    const int mid = (lo + hi) >> 1;
+    if (a[mid] < v) lo = mid + 1;
+    else hi = mid;
+  }
+  return lo;
+}
+
+// FeatureVector.FeatureNode j: 0A len [08 node_id, left out when 0] 12 plen <packed varint feature ids>.  Feature ids
+// ascend inside a node and are < 2^16, so plen = count + (count >= 128) + (count >= 16384) from two binary searches.
+struct FvNode
+{
+  int s, e, lb1, lb2; // features [s, e); the first >= 128 / >= 16384
+  int node, plen, inner, len;
+};
+__device__ __forceinline__ FvNode fv_node(const int *fv_nodes, const int *fv_start, const int *fv_feats, int j)
+{
+  FvNode d;
+  d.s = fv_start[j], d.e = fv_start[j + 1];
+  d.lb1 = lower_bound_int(fv_feats, d.s, d.e, 1 << 7);
+  d.lb2 = lower_bound_int(fv_feats, d.lb1, d.e, 1 << 14);
+  d.node = fv_nodes[j];
+  d.plen = (d.e - d.s) + (d.e - d.lb1) + (d.e - d.lb2);
+  d.inner = (d.node ? 1 + varint_len((unsigned)d.node) : 0) + 1 + varint_len((unsigned)d.plen) + d.plen;
+  d.len = 1 + varint_len((unsigned)d.inner) + d.inner;
+  return d;
+}
+
 __global__ void __launch_bounds__(kSerThreads) serialize_kernel(const Params p, const SerArgs a)
 {
   __shared__ uint8_t s_head[40], s_tail[64], s_pk[3][12]; // s_pk: the length-delimited headers of fields 7, 8, 16
   __shared__ int s_warp[kSerThreads / 32];
   __shared__ int s_len[4]; // head, tail, and the header lengths of the packed fields
+  __shared__ int s_lb[4];  // BowVector: first entry whose word id needs 2, 3, 4, 5 varint bytes
+  __shared__ int s_fv[5][kSerThreads]; // FeatureVector chunk: s, e, lb1, lb2 and payload offset of each node
   const int frame = blockIdx.x, tid = threadIdx.x;
   const int img = frame * a.image_stride;
   const int n = p.n_kps[img];
@@ -136,11 +180,38 @@ __global__ void __launch_bounds__(kSerThreads) serialize_kernel(const Params p, 
     base += total;
   }
 
-  // everything behind the keypoints is a function of the byte position
+  // fields 10 and 11 with content: sizes first (their headers precede them), from closed forms and one block reduction
+  const bool bow = a.bow_ids != nullptr;
+  const size_t fo = (size_t)frame * p.n_features;
+  const int *bow_ids = bow ? a.bow_ids + fo : nullptr, *fv_nodes = bow ? a.fv_nodes + fo : nullptr, *fv_feats = bow ? a.fv_feats + fo : nullptr;
+  const int *fv_start = bow ? a.fv_start + (size_t)frame * (p.n_features + 1) : nullptr;
+  int n_bow = 0, n_fv = 0;
+  long long sz_bow = 0, sz_fv = 0;
+  if (bow)
+  {
+    n_bow = a.n_bow[frame], n_fv = a.n_fv[frame];
+    // entry k = 0A len 08 <varint id> 11 <double>: 12 + varint_len(id) bytes; ids ascend, so the bytes before entry k are
+    // 13 k + sum over t of max(0, k - s_lb[t])
+    if (tid < 4) s_lb[tid] = lower_bound_int(bow_ids, 0, n_bow, 1 << (7 * (tid + 1)));
+    int mine = 0;
+    for (int j = tid; j < n_fv; j += kSerThreads) mine += fv_node(fv_nodes, fv_start, fv_feats, j).len;
+    int fv_total;
+    block_exclusive_scan_ser(mine, fv_total, s_warp); // its barriers also publish s_lb
+    sz_bow = 13ll * n_bow;
+    for (int t = 0; t < 4; ++t) sz_bow += n_bow - s_lb[t];
+    sz_fv = fv_total;
+  }
+
+  // everything behind the keypoints except the BoW sections is a function of the byte position
   const long long off_ru = base;
   const long long sec_pk = n ? (long long)PH + 4ll * n : 0;            // fields 7 and 8 (absent when empty)
   const long long off_dp = off_ru + sec_pk, off_desc = off_dp + sec_pk;
-  const long long off_tail = off_desc + 36ll * n, off_mp = off_tail + T;
+  const long long off_bow = off_desc + 36ll * n;
+  const long long off_bow_e = off_bow + 1 + varint_len((unsigned long long)sz_bow), off_fv = off_bow_e + sz_bow;
+  const long long off_fv_e = off_fv + 1 + varint_len((unsigned long long)sz_fv);
+  // without BoW inputs s_tail starts with the empty fields 10 / 11; with them it starts at the pose
+  const int tail_skip = bow ? 4 : 0;
+  const long long off_tail = bow ? off_fv_e + sz_fv : off_bow, off_mp = off_tail + T - tail_skip;
   const long long total = off_mp + ((a.with_map_points && n) ? (long long)MH + 10ll * n : 0);
   auto byte_at = [&](long long pos) -> uint32_t {
     if (pos < off_desc)
@@ -159,25 +230,89 @@ __global__ void __launch_bounds__(kSerThreads) serialize_kernel(const Params p, 
       if (r < 4) return (0x200A224Au >> (8 * r)) & 0xffu; // 0x4A, 34, 0x0A, 32
       return desc[e * 32 + (r - 4)];
     }
-    if (pos < off_mp) return s_tail[pos - off_tail];
+    if (pos < off_mp) return s_tail[tail_skip + (pos - off_tail)];
     const long long q = pos - off_mp;
     if (q < MH) return s_pk[2][q];
     return ((q - MH) % 10 == 9) ? 0x01u : 0xffu; // int64 -1 as a 10-byte varint
   };
-  const long long w0 = off_ru >> 2, w1 = (total + 3) >> 2; // aligned output words (out and stride are 4-byte aligned)
-  for (long long w = w0 + tid; w < w1; w += kSerThreads)
+  // aligned output words of [lo, hi) (out and stride are 4-byte aligned); bytes of the edge words outside the range belong
+  // to the byte-stored sections
+  auto write_words = [&](long long lo, long long hi) {
+    const long long w0 = lo >> 2, w1 = (hi + 3) >> 2;
+    for (long long w = w0 + tid; w < w1; w += kSerThreads)
+    {
+      const long long pos = w << 2;
+      if (pos >= lo && pos + 4 <= hi)
+      {
+        const uint32_t v = byte_at(pos) | (byte_at(pos + 1) << 8) | (byte_at(pos + 2) << 16) | (byte_at(pos + 3) << 24);
+        *reinterpret_cast<uint32_t *>(out + pos) = v;
+      }
+      else
+      {
+        for (int k = 0; k < 4; ++k)
+          if (pos + k >= lo && pos + k < hi) out[pos + k] = (uint8_t)byte_at(pos + k);
+      }
+    }
+  };
+  if (!bow)
   {
-    const long long pos = w << 2;
-    if (pos >= off_ru && pos + 4 <= total)
+    write_words(off_ru, total);
+    if (tid == 0) a.sizes[frame] = total;
+    return;
+  }
+  write_words(off_ru, off_bow);
+  write_words(off_tail, total);
+
+  // field 10 BowVector { map<uint32, double> words = 1 }: entries in ascending word id (std::map order), key and value
+  // always written
+  if (tid == 0)
+  {
+    out[off_bow] = 0x52, put_varint(out + off_bow + 1, (unsigned long long)sz_bow);
+    out[off_fv] = 0x5A, put_varint(out + off_fv + 1, (unsigned long long)sz_fv);
+  }
+  const double *bow_vals = a.bow_vals + fo;
+  for (int k = tid; k < n_bow; k += kSerThreads)
+  {
+    long long pos = off_bow_e + 13ll * k;
+    for (int t = 0; t < 4; ++t) pos += max(0, k - s_lb[t]);
+    uint8_t *o = out + pos;
+    const unsigned id = (unsigned)bow_ids[k];
+    o[0] = 0x0A, o[1] = (uint8_t)(10 + varint_len(id)), o[2] = 0x08;
+    int l = 3 + put_varint(o + 3, id);
+    o[l++] = 0x11;
+    const unsigned long long v = (unsigned long long)__double_as_longlong(bow_vals[k]);
+    for (int b = 0; b < 8; ++b) o[l + b] = (uint8_t)(v >> (8 * b));
+  }
+
+  // field 11 FeatureVector { repeated FeatureNode nodes = 1 }: nodes in ascending id; node headers by one thread per node
+  // at block-scan offsets, then the packed feature ids by one warp per node at closed-form offsets
+  const int lane = tid & 31, wid = tid >> 5;
+  long long fbase = off_fv_e;
+  for (int j0 = 0; j0 < n_fv; j0 += kSerThreads)
+  {
+    const int j = j0 + tid, cnt = min(kSerThreads, n_fv - j0);
+    FvNode d{};
+    if (j < n_fv) d = fv_node(fv_nodes, fv_start, fv_feats, j);
+    int chunk_total;
+    const int off = block_exclusive_scan_ser(j < n_fv ? d.len : 0, chunk_total, s_warp);
+    if (j < n_fv)
     {
-      const uint32_t v = byte_at(pos) | (byte_at(pos + 1) << 8) | (byte_at(pos + 2) << 16) | (byte_at(pos + 3) << 24);
-      *reinterpret_cast<uint32_t *>(out + pos) = v;
+      uint8_t *o = out + fbase + off;
+      int q = 0;
+      o[q++] = 0x0A, q += put_varint(o + q, (unsigned)d.inner);
+      if (d.node) o[q++] = 0x08, q += put_varint(o + q, (unsigned)d.node);
+      o[q++] = 0x12, q += put_varint(o + q, (unsigned)d.plen);
+      s_fv[0][tid] = d.s, s_fv[1][tid] = d.e, s_fv[2][tid] = d.lb1, s_fv[3][tid] = d.lb2, s_fv[4][tid] = (int)(fbase + off + q);
     }
-    else
+    __syncthreads();
+    for (int q = wid; q < cnt; q += kSerThreads / 32)
     {
-      for (int k = 0; k < 4; ++k)
-        if (pos + k >= off_ru && pos + k < total) out[pos + k] = (uint8_t)byte_at(pos + k);
+      const int s = s_fv[0][q], e = s_fv[1][q], lb1 = s_fv[2][q], lb2 = s_fv[3][q], pay = s_fv[4][q];
+      for (int t = s + lane; t < e; t += 32)
+        put_varint(out + pay + (t - s) + max(0, t - lb1) + max(0, t - lb2), (unsigned)fv_feats[t]);
     }
+    fbase += chunk_total;
+    __syncthreads(); // s_fv is reused by the next chunk
   }
   if (tid == 0) a.sizes[frame] = total;
 }
