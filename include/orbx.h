@@ -132,7 +132,8 @@ int orbx_get_grid(orbx_ctx *ctx, int frame, int32_t *cell_start, int32_t *entrie
 /* A sequence of n_frames stereo pairs (ANY length) from HOST memory; pinned memory makes the copies asynchronous.  The
  * frames stream through the context's max_batch device slots in chunks, so that the H2D copy of one chunk, the kernels of
  * another and the D2H copy of a third overlap.
- * left/right: frame f at base + f * frame_stride bytes, rows `stride` bytes apart.  Outputs are fixed-stride arrays:
+ * left/right: frame f at base + f * frame_stride bytes, rows `stride` bytes apart (stride >= width and frame_stride >=
+ * stride * (height - 1) + width, else ORBX_ERR_INVALID_ARG).  Outputs are fixed-stride arrays:
  * kps_*[f * n_features + i], desc_*[(f * n_features + i) * 32], u_right/depth[f * n_features + i], n_*[f].
  * Returns after all results have landed in the output arrays. */
 int orbx_stereo_batch(orbx_ctx *ctx, int n_frames, const uint8_t *left, const uint8_t *right, size_t stride,

@@ -527,6 +527,23 @@ Params params_at(const orbx_ctx *c, int img0, int frame0)
   return p;
 }
 
+// records the frames now resident in the device slots (what frame-level consumers may read) and bumps frame_epoch
+static void set_resident(orbx_ctx *c, int images, int frames, int stereo)
+{
+  c->last_images = images;
+  c->last_frames = frames;
+  c->last_stereo = stereo;
+  ++c->frame_epoch;
+}
+
+// the pipeline streams wait for the work enqueued so far on the context's stream
+static int fork_pipes(orbx_ctx *c)
+{
+  ORBX_CUDA(c, cudaEventRecord(c->fork_ev, c->stream));
+  for (int i = 0; i < c->kPipe; ++i) ORBX_CUDA(c, cudaStreamWaitEvent(c->pipe[i], c->fork_ev, 0));
+  return ORBX_OK;
+}
+
 // NVTX range around the enqueue of one stage (host side; profilers correlate the launches inside it)
 struct NvtxRange
 {
@@ -534,42 +551,71 @@ struct NvtxRange
   ~NvtxRange() { nvtxRangePop(); }
 };
 
-// the kernels of a stereo batch for device slots [frame0, frame0 + nf) on stream s
-int run_stereo_range(orbx_ctx *c, cudaStream_t s, int frame0, int nf, const uint8_t *d_left, const uint8_t *d_right, size_t stride, size_t frame_stride)
+// ORBExtractor ctor + extract for n_images device-resident images on stream s; with `ev`, ev[0 .. 5] are recorded at the
+// boundaries of the first five stages of orbx_stage_name
+static int run_extract(orbx_ctx *c, const Params &p, int n_images, cudaStream_t s, cudaEvent_t *ev = nullptr)
 {
-  Params p = params_at(c, 2 * frame0, frame0);
+  if (ev) ORBX_CUDA(c, cudaEventRecord(ev[0], s));
+  {
+    NvtxRange q("orbx:pyramid_blur");
+    launch_pyramid_level0(p, n_images, s);
+    if (ev) ORBX_CUDA(c, cudaEventRecord(ev[1], s));
+    launch_pyramid_levels(p, c->maps_src, n_images, s);
+  }
+  if (ev) ORBX_CUDA(c, cudaEventRecord(ev[2], s));
+  {
+    NvtxRange q("orbx:fast_cells");
+    launch_fast(p, c->maps, n_images, s);
+  }
+  if (ev) ORBX_CUDA(c, cudaEventRecord(ev[3], s));
+  {
+    NvtxRange q("orbx:quadtree");
+    launch_quadtree(p, n_images, c->qt_smem, s);
+  }
+  if (ev) ORBX_CUDA(c, cudaEventRecord(ev[4], s));
+  {
+    NvtxRange q("orbx:orient_brief");
+    launch_orient_brief(p, c->maps_blur, n_images, s);
+  }
+  if (ev) ORBX_CUDA(c, cudaEventRecord(ev[5], s));
+  c->launches += 5;
+  ORBX_CUDA(c, cudaGetLastError());
+  return ORBX_OK;
+}
+
+// the Params of a stereo batch whose first frame is device slot d0, reading its images at d_left / d_right
+static Params stereo_params(const orbx_ctx *c, int d0, const uint8_t *d_left, const uint8_t *d_right, size_t stride, size_t frame_stride)
+{
+  Params p = params_at(c, 2 * d0, d0);
   p.stereo = 1;
   p.in_left = d_left;
   p.in_right = d_right;
   p.in_stride = stride;
   p.in_frame_stride = frame_stride;
+  return p;
+}
+
+// the kernels of a stereo batch for device slots [frame0, frame0 + nf) on stream s (inputs: frame 0 of the range at d_left /
+// d_right); with `ev`, ev[0 .. ORBX_N_STAGES] are recorded on s at the stage boundaries of orbx_stage_name
+static int run_stereo_range(orbx_ctx *c, cudaStream_t s, int frame0, int nf, const uint8_t *d_left, const uint8_t *d_right, size_t stride, size_t frame_stride,
+                            cudaEvent_t *ev = nullptr)
+{
+  const Params p = stereo_params(c, frame0, d_left, d_right, stride, frame_stride);
   NvtxRange r("orbx:stereo_range");
   ORBX_CUDA(c, cudaMemsetAsync(p.n_matches, 0, (size_t)nf * sizeof(int), s));
-  {
-    NvtxRange q("orbx:pyramid_blur");
-    launch_pyramid(p, c->maps_src, 2 * nf, s);
-  }
-  {
-    NvtxRange q("orbx:fast_cells");
-    launch_fast(p, c->maps, 2 * nf, s);
-  }
-  {
-    NvtxRange q("orbx:quadtree");
-    launch_quadtree(p, 2 * nf, c->qt_smem, s);
-  }
-  {
-    NvtxRange q("orbx:orient_brief");
-    launch_orient_brief(p, c->maps_blur, 2 * nf, s);
-  }
+  int rc = run_extract(c, p, 2 * nf, s, ev);
+  if (rc) return rc;
   {
     NvtxRange q("orbx:frame_index"); // createRowIndexDB of the right keypoints + initGrid of the left ones, one launch
     launch_frame_index(p, nf, 2, true, s);
   }
+  if (ev) ORBX_CUDA(c, cudaEventRecord(ev[6], s));
   {
     NvtxRange q("orbx:stereo_match");
     launch_stereo(p, nf, s);
   }
-  c->launches += 5 + kPyramidLaunches;
+  if (ev) ORBX_CUDA(c, cudaEventRecord(ev[7], s));
+  c->launches += 2;
   ORBX_CUDA(c, cudaGetLastError());
   return ORBX_OK;
 }
@@ -583,7 +629,8 @@ static void drop_graph(orbx_ctx *c)
   c->graph1_pyr = nullptr;
 }
 
-int run_stereo_single(orbx_ctx *c, cudaStream_t s, const uint8_t *d_left, const uint8_t *d_right, size_t stride, size_t frame_stride)
+// one stereo frame in device slot 0: a single graph launch when the context's graph is enabled and `s` can be captured
+static int run_stereo_single(orbx_ctx *c, cudaStream_t s, const uint8_t *d_left, const uint8_t *d_right, size_t stride, size_t frame_stride)
 {
   // the legacy / per-thread default streams cannot be captured
   const bool can = c->use_graph && s != nullptr && s != cudaStreamLegacy && s != cudaStreamPerThread;
@@ -632,12 +679,7 @@ int run_stereo_single(orbx_ctx *c, cudaStream_t s, const uint8_t *d_left, const 
     // only the pyramid kernel reads the caller's images: patch that node's Params in the instantiated graph
     cudaKernelNodeParams kp;
     ORBX_CUDA(c, cudaGraphKernelNodeGetParams(c->graph1_pyr, &kp));
-    Params p = params_at(c, 0, 0);
-    p.stereo = 1;
-    p.in_left = d_left;
-    p.in_right = d_right;
-    p.in_stride = stride;
-    p.in_frame_stride = frame_stride;
+    Params p = stereo_params(c, 0, d_left, d_right, stride, frame_stride);
     void *args[1] = {&p};
     kp.kernelParams = args;
     kp.extra = nullptr;
@@ -646,6 +688,61 @@ int run_stereo_single(orbx_ctx *c, cudaStream_t s, const uint8_t *d_left, const 
   }
   ORBX_CUDA(c, cudaGraphLaunch(c->graph1_exec, s));
   c->launches += c->graph1_kernels;
+  return ORBX_OK;
+}
+
+int run_stereo_chunks(orbx_ctx *c, int64_t n_frames, const uint8_t *left, size_t left_stride, const uint8_t *right, size_t right_stride, size_t frame_stride,
+                      bool on_device, bool piped, const ChunkOut &out)
+{
+  const size_t W = (size_t)c->cfg.width, H = (size_t)c->cfg.height;
+  if (std::min(left_stride, right_stride) < W || frame_stride < std::max(left_stride, right_stride) * (H - 1) + W)
+    return fail(c, ORBX_ERR_INVALID_ARG, "stride / frame_stride smaller than the image");
+  // Densely stacked rows that fit the staging pitch are copied as ONE linear transfer per side and read on the device
+  // with the caller's stride (the kernels gather bytes, so rows need no alignment); 2-D pitched copies of odd-width
+  // rows run at a fraction of the PCIe rate.
+  const bool linear = left_stride == right_stride && frame_stride == left_stride * H && left_stride <= c->in_pitch;
+  const size_t fs = linear ? frame_stride : c->in_pitch * H, dstride = linear ? left_stride : c->in_pitch;
+  uint8_t *dl = c->d_in, *dr = c->d_in + (size_t)c->cfg.max_batch * c->in_pitch * H;
+  // A slot is always driven by the same pipeline stream, so reusing it is ordered by that stream while the H2D copy of one
+  // chunk, the kernels of another and the D2H copy of a third overlap across streams.
+  const int chunk = c->chunk(), n_slots = std::max(1, c->cfg.max_batch / chunk);
+  if (piped)
+  {
+    int rc = fork_pipes(c);
+    if (rc) return rc;
+  }
+  int k = 0;
+  for (int64_t f0 = 0; f0 < n_frames; f0 += chunk, ++k)
+  {
+    const int nf = (int)std::min<int64_t>(chunk, n_frames - f0);
+    const int slot = k % n_slots, d0 = slot * chunk;
+    cudaStream_t s = piped ? c->pipe[slot % c->kPipe] : c->stream;
+    const uint8_t *in_l = left + (size_t)f0 * frame_stride, *in_r = right + (size_t)f0 * frame_stride;
+    size_t in_stride = left_stride, in_fs = frame_stride;
+    if (!on_device)
+    { // device inputs are read in place: only the intermediate buffers cycle through the slots
+      uint8_t *sl = dl + (size_t)d0 * fs, *sr = dr + (size_t)d0 * fs;
+      if (linear)
+      {
+        ORBX_CUDA(c, cudaMemcpyAsync(sl, in_l, fs * nf, cudaMemcpyHostToDevice, s));
+        ORBX_CUDA(c, cudaMemcpyAsync(sr, in_r, fs * nf, cudaMemcpyHostToDevice, s));
+      }
+      else
+        for (int f = 0; f < nf; ++f)
+        {
+          ORBX_CUDA(c, cudaMemcpy2DAsync(sl + f * fs, c->in_pitch, in_l + f * frame_stride, left_stride, W, H, cudaMemcpyHostToDevice, s));
+          ORBX_CUDA(c, cudaMemcpy2DAsync(sr + f * fs, c->in_pitch, in_r + f * frame_stride, right_stride, W, H, cudaMemcpyHostToDevice, s));
+        }
+      in_l = sl, in_r = sr, in_stride = dstride, in_fs = fs;
+    }
+    // a single frame on the context's stream is the latency path
+    int rc = n_frames == 1 && !piped ? run_stereo_single(c, s, in_l, in_r, in_stride, in_fs) : run_stereo_range(c, s, d0, nf, in_l, in_r, in_stride, in_fs);
+    if (!rc) rc = out(s, d0, f0, nf);
+    if (rc) return rc;
+  }
+  // introspection (get_pyramid / get_grid) refers to the device slots, i.e. to the frames of the last pass over them
+  const int resident = (int)std::min<int64_t>(n_frames, (int64_t)n_slots * chunk);
+  set_resident(c, 2 * resident, resident, 1);
   return ORBX_OK;
 }
 
@@ -695,18 +792,6 @@ int build_level_maps(orbx_ctx *c)
     if (r != CUDA_SUCCESS) return fail(c, ORBX_ERR_CUDA, "cuTensorMapEncodeTiled (blur) failed for level " + std::to_string(l));
   }
   c->p.img0 = 0;
-  return ORBX_OK;
-}
-
-// ORBExtractor ctor + extract for n_images device-resident images
-int run_extract(orbx_ctx *c, const Params &p, int n_images)
-{
-  launch_pyramid(p, c->maps_src, n_images, c->stream);
-  launch_fast(p, c->maps, n_images, c->stream);
-  launch_quadtree(p, n_images, c->qt_smem, c->stream);
-  launch_orient_brief(p, c->maps_blur, n_images, c->stream);
-  c->launches += 3 + kPyramidLaunches;
-  ORBX_CUDA(c, cudaGetLastError());
   return ORBX_OK;
 }
 
@@ -967,12 +1052,9 @@ extern "C"
     p.in_right = nullptr;
     p.in_stride = stride;
     p.in_frame_stride = frame_stride;
-    int rc = run_extract(c, p, n_images);
+    int rc = run_extract(c, p, n_images, c->stream);
     if (rc) return rc;
-    c->last_images = n_images;
-    ++c->frame_epoch;
-    c->last_stereo = 0;
-    c->last_frames = 0; // extract-only images carry no grid / uRight / depth: frame-level consumers must fail with ORBX_ERR_STATE
+    set_resident(c, n_images, 0, 0); // extract-only images carry no grid / uRight / depth: frame-level consumers must fail with ORBX_ERR_STATE
     fill_results(c, n_images, 0, out);
     return ORBX_OK;
   }
@@ -996,14 +1078,15 @@ extern "C"
     else
     {
       // Fork the batch into chunks on the pipeline streams and join back into the caller's stream: the latency-bound
-      // quadtree launches of one chunk then overlap the issue-bound FAST / pyramid launches of the others.
-      ORBX_CUDA(c, cudaEventRecord(c->fork_ev, c->stream));
-      for (int i = 0; i < c->kPipe; ++i) ORBX_CUDA(c, cudaStreamWaitEvent(c->pipe[i], c->fork_ev, 0));
+      // quadtree launches of one chunk then overlap the issue-bound FAST / pyramid launches of the others.  Every frame
+      // keeps its own slot (slot = frame), so all of them stay resident.
+      int rc = fork_pipes(c);
+      if (rc) return rc;
       int k = 0;
       for (int f0 = 0; f0 < n_frames; f0 += c->kChunk, ++k)
       {
-        int rc = run_stereo_range(c, c->pipe[k % c->kPipe], f0, std::min(c->kChunk, n_frames - f0), d_left + (size_t)f0 * frame_stride,
-                                  d_right + (size_t)f0 * frame_stride, stride, frame_stride);
+        rc = run_stereo_range(c, c->pipe[k % c->kPipe], f0, std::min(c->kChunk, n_frames - f0), d_left + (size_t)f0 * frame_stride,
+                              d_right + (size_t)f0 * frame_stride, stride, frame_stride);
         if (rc) return rc;
       }
       for (int i = 0; i < c->kPipe; ++i)
@@ -1012,10 +1095,7 @@ extern "C"
         ORBX_CUDA(c, cudaStreamWaitEvent(c->stream, c->join_ev[i], 0));
       }
     }
-    c->last_images = 2 * n_frames;
-    ++c->frame_epoch;
-    c->last_stereo = 1;
-    c->last_frames = n_frames;
+    set_resident(c, 2 * n_frames, n_frames, 1);
     fill_results(c, 2 * n_frames, n_frames, out);
     return ORBX_OK;
   }
@@ -1032,40 +1112,15 @@ extern "C"
     if (!c || !d_left || !d_right || n_frames < 1 || !stage_ms) return ORBX_ERR_INVALID_ARG;
     if (n_frames > c->cfg.max_batch) return fail(c, ORBX_ERR_CAPACITY, "n_frames > max_batch");
     ORBX_CUDA(c, cudaSetDevice(c->device));
-    Params p = c->p;
-    p.stereo = 1;
-    p.in_left = d_left;
-    p.in_right = d_right;
-    p.in_stride = stride;
-    p.in_frame_stride = frame_stride;
     cudaEvent_t ev[ORBX_N_STAGES + 1];
     for (auto &e : ev) ORBX_CUDA(c, cudaEventCreate(&e));
-    const int ni = 2 * n_frames;
-    ORBX_CUDA(c, cudaMemsetAsync(p.n_matches, 0, (size_t)n_frames * sizeof(int), c->stream));
-    ORBX_CUDA(c, cudaEventRecord(ev[0], c->stream));
-    launch_pyramid_level0(p, ni, c->stream);
-    ORBX_CUDA(c, cudaEventRecord(ev[1], c->stream));
-    launch_pyramid_levels(p, c->maps_src, ni, c->stream);
-    ORBX_CUDA(c, cudaEventRecord(ev[2], c->stream));
-    launch_fast(p, c->maps, ni, c->stream);
-    ORBX_CUDA(c, cudaEventRecord(ev[3], c->stream));
-    launch_quadtree(p, ni, c->qt_smem, c->stream);
-    ORBX_CUDA(c, cudaEventRecord(ev[4], c->stream));
-    launch_orient_brief(p, c->maps_blur, ni, c->stream);
-    ORBX_CUDA(c, cudaEventRecord(ev[5], c->stream));
-    launch_frame_index(p, n_frames, 2, true, c->stream);
-    ORBX_CUDA(c, cudaEventRecord(ev[6], c->stream));
-    launch_stereo(p, n_frames, c->stream);
-    ORBX_CUDA(c, cudaEventRecord(ev[7], c->stream));
-    c->launches += 5 + kPyramidLaunches;
-    ORBX_CUDA(c, cudaGetLastError());
+    // one launch per kernel over all n_frames on the context's stream (not the chunked fork of orbx_stereo_batch_device)
+    int rc = run_stereo_range(c, c->stream, 0, n_frames, d_left, d_right, stride, frame_stride, ev);
+    if (rc) return rc;
     ORBX_CUDA(c, cudaStreamSynchronize(c->stream));
     for (int i = 0; i < ORBX_N_STAGES; ++i) ORBX_CUDA(c, cudaEventElapsedTime(&stage_ms[i], ev[i], ev[i + 1]));
     for (auto &e : ev) cudaEventDestroy(e);
-    c->last_images = ni;
-    ++c->frame_epoch;
-    c->last_stereo = 1;
-    c->last_frames = n_frames;
+    set_resident(c, 2 * n_frames, n_frames, 1);
     return ORBX_OK;
   }
 
@@ -1084,123 +1139,71 @@ extern "C"
     p.depth_stride = depth_stride_bytes;
     p.depth_frame_stride = depth_frame_stride_bytes;
     p.depth_type = depth_type;
-    int rc = run_extract(c, p, n_frames);
+    int rc = run_extract(c, p, n_frames, c->stream);
     if (rc) return rc;
     ORBX_CUDA(c, cudaMemsetAsync(p.n_matches, 0, (size_t)n_frames * sizeof(int), c->stream));
     launch_rgbd(p, n_frames, c->stream);
     launch_frame_index(p, n_frames, 1, false, c->stream);
     c->launches += 2;
     ORBX_CUDA(c, cudaGetLastError());
-    c->last_images = n_frames;
-    ++c->frame_epoch;
-    c->last_stereo = 0;
-    c->last_frames = n_frames;
+    set_resident(c, n_frames, n_frames, 0);
     fill_results(c, n_frames, n_frames, out);
     return ORBX_OK;
   }
 
   // ---------------------------------------------------------------------------------------------------------------
+  // Latency path (the reference's one-frame-at-a-time call): both images staged into slot 0, ONE graph launch, the frame's
+  // results packed into one record on the device and brought back in ONE copy (instead of nine), then handed out from
+  // pinned memory.
+  static int stereo_frame_host(orbx_ctx *c, const uint8_t *left, size_t left_stride, const uint8_t *right, size_t right_stride, size_t frame_stride,
+                               orbx_keypoint *kps_left, uint8_t *desc_left, int32_t *n_left, orbx_keypoint *kps_right, uint8_t *desc_right,
+                               int32_t *n_right, double *u_right, double *depth, int32_t *n_matches)
+  {
+    ORBX_CUDA(c, cudaSetDevice(c->device));
+    orbx_record_layout lay;
+    orbx_record_layout_get(c, &lay);
+    const size_t rs = (size_t)lay.record_bytes;
+    int rc = ensure_record_staging(c, rs);
+    if (rc) return rc;
+    if (!c->h_rec1) ORBX_CUDA(c, cudaHostAlloc((void **)&c->h_rec1, rs, cudaHostAllocDefault));
+    rc = run_stereo_chunks(c, 1, left, left_stride, right, right_stride, frame_stride, false, false, [&](cudaStream_t s, int, int64_t, int) -> int {
+      const int prc = pack_frame_records(c, s, 0, 1, c->rec_staging, rs);
+      if (prc) return prc;
+      ORBX_CUDA(c, cudaMemcpyAsync(c->h_rec1, c->rec_staging, rs, cudaMemcpyDeviceToHost, s));
+      return ORBX_OK;
+    });
+    if (rc) return rc;
+    ORBX_CUDA(c, cudaStreamSynchronize(c->stream));
+    const int32_t *hdr = reinterpret_cast<const int32_t *>(c->h_rec1);
+    const size_t nl = (size_t)hdr[0], nr = (size_t)hdr[1];
+    if (kps_left) std::memcpy(kps_left, c->h_rec1 + lay.off_kps_left, nl * sizeof(orbx_keypoint));
+    if (desc_left) std::memcpy(desc_left, c->h_rec1 + lay.off_desc_left, nl * 32);
+    if (n_left) *n_left = hdr[0];
+    if (kps_right) std::memcpy(kps_right, c->h_rec1 + lay.off_kps_right, nr * sizeof(orbx_keypoint));
+    if (desc_right) std::memcpy(desc_right, c->h_rec1 + lay.off_desc_right, nr * 32);
+    if (n_right) *n_right = hdr[1];
+    if (u_right) std::memcpy(u_right, c->h_rec1 + lay.off_u_right, nl * 8);
+    if (depth) std::memcpy(depth, c->h_rec1 + lay.off_depth, nl * 8);
+    if (n_matches) *n_matches = hdr[2];
+    return ORBX_OK;
+  }
+
   int orbx_stereo_batch(orbx_ctx *c, int n_frames, const uint8_t *left, const uint8_t *right, size_t stride, size_t frame_stride, orbx_keypoint *kps_left,
                         uint8_t *desc_left, int32_t *n_left, orbx_keypoint *kps_right, uint8_t *desc_right, int32_t *n_right, double *u_right,
                         double *depth, int32_t *n_matches)
   {
     if (!c || !left || !right || n_frames < 1) return ORBX_ERR_INVALID_ARG;
-    ORBX_CUDA(c, cudaSetDevice(c->device));
-    const size_t W = (size_t)c->cfg.width, H = (size_t)c->cfg.height, N = (size_t)c->cfg.n_features;
-    size_t fs = c->in_pitch * H, dstride = c->in_pitch;
-    uint8_t *dl = c->d_in, *dr = c->d_in + (size_t)c->cfg.max_batch * c->in_pitch * H;
-    const Params &p = c->p;
-    const size_t kb = N * sizeof(orbx_keypoint), db = N * 32;
     if (n_frames == 1)
-    {
-      // Latency path (the reference's one-frame-at-a-time call): both images up, ONE graph launch, the frame's results packed
-      // into one record on the device and brought back in ONE copy (instead of nine), then handed out from pinned memory.
-      orbx_record_layout lay;
-      orbx_record_layout_get(c, &lay);
-      const size_t rs = (size_t)lay.record_bytes;
-      int rc = ensure_record_staging(c, rs);
-      if (rc) return rc;
-      if (!c->h_rec1) ORBX_CUDA(c, cudaHostAlloc((void **)&c->h_rec1, rs, cudaHostAllocDefault));
-      cudaStream_t s = c->stream;
-      const bool dense = frame_stride == stride * H && stride >= W && stride <= c->in_pitch;
-      if (dense)
-      {
-        ORBX_CUDA(c, cudaMemcpyAsync(dl, left, stride * H, cudaMemcpyHostToDevice, s));
-        ORBX_CUDA(c, cudaMemcpyAsync(dr, right, stride * H, cudaMemcpyHostToDevice, s));
-      }
-      else
-      {
-        ORBX_CUDA(c, cudaMemcpy2DAsync(dl, c->in_pitch, left, stride, W, H, cudaMemcpyHostToDevice, s));
-        ORBX_CUDA(c, cudaMemcpy2DAsync(dr, c->in_pitch, right, stride, W, H, cudaMemcpyHostToDevice, s));
-      }
-      rc = run_stereo_single(c, s, dl, dr, dense ? stride : c->in_pitch, dense ? stride * H : c->in_pitch * H);
-      if (rc) return rc;
-      rc = pack_frame_records(c, s, 0, 1, c->rec_staging, rs);
-      if (rc) return rc;
-      ORBX_CUDA(c, cudaMemcpyAsync(c->h_rec1, c->rec_staging, rs, cudaMemcpyDeviceToHost, s));
-      ORBX_CUDA(c, cudaStreamSynchronize(s));
-      const int32_t *hdr = reinterpret_cast<const int32_t *>(c->h_rec1);
-      const size_t nl = (size_t)hdr[0], nr = (size_t)hdr[1];
-      if (kps_left) std::memcpy(kps_left, c->h_rec1 + lay.off_kps_left, nl * sizeof(orbx_keypoint));
-      if (desc_left) std::memcpy(desc_left, c->h_rec1 + lay.off_desc_left, nl * 32);
-      if (n_left) *n_left = hdr[0];
-      if (kps_right) std::memcpy(kps_right, c->h_rec1 + lay.off_kps_right, nr * sizeof(orbx_keypoint));
-      if (desc_right) std::memcpy(desc_right, c->h_rec1 + lay.off_desc_right, nr * 32);
-      if (n_right) *n_right = hdr[1];
-      if (u_right) std::memcpy(u_right, c->h_rec1 + lay.off_u_right, nl * 8);
-      if (depth) std::memcpy(depth, c->h_rec1 + lay.off_depth, nl * 8);
-      if (n_matches) *n_matches = hdr[2];
-      c->last_frames = 1;
-      c->last_images = 2;
-      ++c->frame_epoch;
-      c->last_stereo = 1;
-      return ORBX_OK;
-    }
-    // Densely stacked rows that fit the staging pitch are copied as ONE linear transfer per side and read on the device
-    // with the caller's stride (the kernels gather bytes, so rows need no alignment); 2-D pitched copies of odd-width
-    // rows run at a fraction of the PCIe rate.
-    const bool linear = frame_stride == stride * H && stride >= W && stride <= c->in_pitch;
-    if (linear)
-    {
-      fs = frame_stride;
-      dstride = stride;
-    }
-    // The sequence streams through the context's max_batch device slots in chunks: chunk k lives in slot k % n_slots, and a
-    // slot is always driven by the same pipeline stream, so reusing it is ordered by that stream while the H2D copy of one
-    // chunk, the kernels of another and the D2H copy of a third overlap across streams.  A sequence that fits one chunk runs
-    // on the context's stream (single-frame latency path).
-    const int chunk = std::min(c->kChunk, c->cfg.max_batch);
-    const int n_slots = std::max(1, c->cfg.max_batch / chunk);
-    const bool piped = n_frames > chunk;
-    if (piped)
-    {
-      ORBX_CUDA(c, cudaEventRecord(c->fork_ev, c->stream));
-      for (int i = 0; i < c->kPipe; ++i) ORBX_CUDA(c, cudaStreamWaitEvent(c->pipe[i], c->fork_ev, 0));
-    }
-    int k = 0;
-    for (int f0 = 0; f0 < n_frames; f0 += chunk, ++k)
-    {
-      const int nf = std::min(chunk, n_frames - f0);
-      const int slot = k % n_slots;
-      const size_t d0 = (size_t)slot * chunk; // first device frame of the slot
-      cudaStream_t s = piped ? c->pipe[slot % c->kPipe] : c->stream;
-      if (linear)
-      {
-        ORBX_CUDA(c, cudaMemcpyAsync(dl + d0 * fs, left + f0 * frame_stride, fs * nf, cudaMemcpyHostToDevice, s));
-        ORBX_CUDA(c, cudaMemcpyAsync(dr + d0 * fs, right + f0 * frame_stride, fs * nf, cudaMemcpyHostToDevice, s));
-      }
-      else
-      {
-        for (int f = 0; f < nf; ++f)
-        {
-          ORBX_CUDA(c, cudaMemcpy2DAsync(dl + (d0 + f) * fs, c->in_pitch, left + (f0 + f) * frame_stride, stride, W, H, cudaMemcpyHostToDevice, s));
-          ORBX_CUDA(c, cudaMemcpy2DAsync(dr + (d0 + f) * fs, c->in_pitch, right + (f0 + f) * frame_stride, stride, W, H, cudaMemcpyHostToDevice, s));
-        }
-      }
-      int rc = (n_frames == 1) ? run_stereo_single(c, s, dl, dr, dstride, fs) : run_stereo_range(c, s, (int)d0, nf, dl + d0 * fs, dr + d0 * fs, dstride, fs);
-      if (rc) return rc;
+      return stereo_frame_host(c, left, stride, right, stride, frame_stride, kps_left, desc_left, n_left, kps_right, desc_right, n_right, u_right, depth,
+                               n_matches);
+    ORBX_CUDA(c, cudaSetDevice(c->device));
+    const size_t N = (size_t)c->cfg.n_features, kb = N * sizeof(orbx_keypoint), db = N * 32;
+    const Params &p = c->p;
+    // a batch that fits one chunk runs on the context's stream
+    const bool piped = n_frames > c->chunk();
+    int rc = run_stereo_chunks(c, n_frames, left, stride, right, stride, frame_stride, false, piped, [&](cudaStream_t s, int d0, int64_t f0, int nf) -> int {
       // results: left = even images, right = odd images -> one strided 2-D copy per array
-      const size_t i0 = 2 * d0;
+      const size_t i0 = 2 * (size_t)d0;
       if (kps_left) ORBX_CUDA(c, cudaMemcpy2DAsync(kps_left + f0 * N, kb, p.kps_und + i0 * N, 2 * kb, kb, nf, cudaMemcpyDeviceToHost, s));
       if (kps_right) ORBX_CUDA(c, cudaMemcpy2DAsync(kps_right + f0 * N, kb, p.kps + (i0 + 1) * N, 2 * kb, kb, nf, cudaMemcpyDeviceToHost, s));
       if (desc_left) ORBX_CUDA(c, cudaMemcpy2DAsync(desc_left + f0 * db, db, p.desc + i0 * db, 2 * db, db, nf, cudaMemcpyDeviceToHost, s));
@@ -1210,16 +1213,13 @@ extern "C"
       if (u_right) ORBX_CUDA(c, cudaMemcpyAsync(u_right + f0 * N, p.u_right + d0 * N, N * 8 * nf, cudaMemcpyDeviceToHost, s));
       if (depth) ORBX_CUDA(c, cudaMemcpyAsync(depth + f0 * N, p.depth + d0 * N, N * 8 * nf, cudaMemcpyDeviceToHost, s));
       if (n_matches) ORBX_CUDA(c, cudaMemcpyAsync(n_matches + f0, p.n_matches + d0, 4 * (size_t)nf, cudaMemcpyDeviceToHost, s));
-    }
+      return ORBX_OK;
+    });
+    if (rc) return rc;
     if (piped)
       for (int i = 0; i < c->kPipe; ++i) ORBX_CUDA(c, cudaStreamSynchronize(c->pipe[i]));
     else
       ORBX_CUDA(c, cudaStreamSynchronize(c->stream));
-    // introspection (get_pyramid / get_grid) refers to the device slots, i.e. to the frames of the last pass over them
-    c->last_frames = std::min(n_frames, n_slots * chunk);
-    c->last_images = 2 * c->last_frames;
-    ++c->frame_epoch;
-    c->last_stereo = 1;
     return ORBX_OK;
   }
 
@@ -1228,30 +1228,8 @@ extern "C"
                         int32_t *n_matches)
   {
     if (!c || !left || !right) return ORBX_ERR_INVALID_ARG;
-    if (left_stride == right_stride)
-      return orbx_stereo_batch(c, 1, left, right, left_stride, left_stride * (size_t)c->cfg.height, kps_left, desc_left, n_left, kps_right, desc_right, n_right,
-                               u_right, depth, n_matches);
-    // different row strides: stage the two images separately, then run the device path
-    ORBX_CUDA(c, cudaSetDevice(c->device));
-    const size_t W = (size_t)c->cfg.width, H = (size_t)c->cfg.height, N = (size_t)c->cfg.n_features;
-    const size_t fs = c->in_pitch * H;
-    uint8_t *dl = c->d_in, *dr = c->d_in + (size_t)c->cfg.max_batch * fs;
-    ORBX_CUDA(c, cudaMemcpy2DAsync(dl, c->in_pitch, left, left_stride, W, H, cudaMemcpyHostToDevice, c->stream));
-    ORBX_CUDA(c, cudaMemcpy2DAsync(dr, c->in_pitch, right, right_stride, W, H, cudaMemcpyHostToDevice, c->stream));
-    int rc = orbx_stereo_batch_device(c, 1, dl, dr, c->in_pitch, fs, nullptr);
-    if (rc) return rc;
-    const Params &p = c->p;
-    if (kps_left) ORBX_CUDA(c, cudaMemcpyAsync(kps_left, p.kps_und, N * sizeof(orbx_keypoint), cudaMemcpyDeviceToHost, c->stream));
-    if (kps_right) ORBX_CUDA(c, cudaMemcpyAsync(kps_right, p.kps + N, N * sizeof(orbx_keypoint), cudaMemcpyDeviceToHost, c->stream));
-    if (desc_left) ORBX_CUDA(c, cudaMemcpyAsync(desc_left, p.desc, N * 32, cudaMemcpyDeviceToHost, c->stream));
-    if (desc_right) ORBX_CUDA(c, cudaMemcpyAsync(desc_right, p.desc + N * 32, N * 32, cudaMemcpyDeviceToHost, c->stream));
-    if (n_left) ORBX_CUDA(c, cudaMemcpyAsync(n_left, p.n_kps, 4, cudaMemcpyDeviceToHost, c->stream));
-    if (n_right) ORBX_CUDA(c, cudaMemcpyAsync(n_right, p.n_kps + 1, 4, cudaMemcpyDeviceToHost, c->stream));
-    if (u_right) ORBX_CUDA(c, cudaMemcpyAsync(u_right, p.u_right, N * 8, cudaMemcpyDeviceToHost, c->stream));
-    if (depth) ORBX_CUDA(c, cudaMemcpyAsync(depth, p.depth, N * 8, cudaMemcpyDeviceToHost, c->stream));
-    if (n_matches) ORBX_CUDA(c, cudaMemcpyAsync(n_matches, p.n_matches, 4, cudaMemcpyDeviceToHost, c->stream));
-    ORBX_CUDA(c, cudaStreamSynchronize(c->stream));
-    return ORBX_OK;
+    return stereo_frame_host(c, left, left_stride, right, right_stride, std::max(left_stride, right_stride) * (size_t)c->cfg.height, kps_left, desc_left,
+                             n_left, kps_right, desc_right, n_right, u_right, depth, n_matches);
   }
 
   int orbx_extract(orbx_ctx *c, const uint8_t *image, size_t stride, orbx_keypoint *kps, uint8_t *desc, int32_t *n)
@@ -1954,9 +1932,8 @@ extern "C"
     c->launches += 1;
     ORBX_CUDA(c, cudaGetLastError());
     ORBX_CUDA(c, cudaStreamSynchronize(c->stream));
-    c->last_images = std::max(c->last_images, 1);
-    c->last_frames = 0; // image 0 was overwritten: the frame-level results of an earlier call no longer match it
-    ++c->frame_epoch;
+    // image 0 was overwritten: the frame-level results of an earlier call no longer match it
+    set_resident(c, std::max(c->last_images, 1), 0, c->last_stereo);
     return ORBX_OK;
   }
 

@@ -231,10 +231,8 @@ inline void ser_bow_inputs(SerArgs &s, const BowArgs &b, size_t frame0, size_t n
   s.n_fv = b.n_fv + frame0;
 }
 
-// launchers (orbx_kernels.cu / orbx_match.cu / orbx_serialize.cu / orbx_bow.cu); every call enqueues exactly one kernel on `s` (launch_pyramid: two)
-constexpr int kPyramidLaunches = 2;
+// launchers (orbx_kernels.cu / orbx_match.cu / orbx_serialize.cu / orbx_bow.cu); every call enqueues exactly one kernel on `s`
 constexpr int kPyrBoxBytesHost = 18 * 1024; // = kPyrBoxBytes of orbx_kernels.cu: shared-memory bytes a level's source box may take
-void launch_pyramid(const Params &p, const LevelMaps &src_maps, int n_images, cudaStream_t s); // kPyramidLaunches kernels: level 0, then the resized levels
 void launch_pyramid_level0(const Params &p, int n_images, cudaStream_t s);
 void launch_pyramid_levels(const Params &p, const LevelMaps &src_maps, int n_images, cudaStream_t s);
 const void *pyramid_kernel_symbol(); // host handle of the level-0 pyramid kernel, the only reader of the caller's images (to find its node in a captured graph)

@@ -1,6 +1,7 @@
 // orbx_internal.h -- host-side state shared by the translation units behind the C ABI (orbx_api.cu, orbx_sequence.cu).
 #pragma once
 
+#include <functional>
 #include <string>
 #include <vector>
 
@@ -37,6 +38,7 @@ struct orbx_ctx
   static constexpr int kPipeMax = 8;
   int kPipe = 8;  // streams (tunable for experiments: ORBX_PIPE); 8 x 8 frames measured best on B200
   int kChunk = 8; // frames per chunk (ORBX_CHUNK)
+  int chunk() const { return kChunk < cfg.max_batch ? kChunk : cfg.max_batch; } // frames per chunk of this context's slots
   cudaStream_t pipe[kPipeMax] = {};
   cudaEvent_t fork_ev = nullptr;
   cudaEvent_t join_ev[kPipeMax] = {};
@@ -88,11 +90,15 @@ namespace orbx
 int fail(orbx_ctx *c, int code, const std::string &msg);
 // Params whose per-image buffers start at image `img0` (and per-frame buffers at frame `frame0`)
 Params params_at(const orbx_ctx *c, int img0, int frame0);
-// the kernels of a stereo batch for device slots [frame0, frame0 + nf) on stream s (inputs: frame 0 of the range at d_left / d_right)
-int run_stereo_range(orbx_ctx *c, cudaStream_t s, int frame0, int nf, const uint8_t *d_left, const uint8_t *d_right, size_t stride, size_t frame_stride);
-
-// one stereo frame in device slot 0: a single graph launch when the context's graph is enabled and `s` can be captured
-int run_stereo_single(orbx_ctx *c, cudaStream_t s, const uint8_t *d_left, const uint8_t *d_right, size_t stride, size_t frame_stride);
+// Stereo input of n_frames frames (host memory, or device memory with `on_device`) streamed through the device slots in
+// chunks of c->chunk() frames.  Chunk k lives in slot k % n_slots and, with `piped`, runs on stream pipe[slot % kPipe]
+// after a fork from the context's stream; otherwise everything runs on the context's stream.  Per chunk: host frames are
+// staged into the slot, the kernels are enqueued, then out(s, d0, f0, nf) enqueues the caller's outputs of frames
+// [f0, f0 + nf) = device slots [d0, d0 + nf) on the chunk's stream s.  The right image may have its own row stride; frame
+// f starts at f * frame_stride on both sides.  Leaves the last pass over the slots resident; the caller synchronises.
+using ChunkOut = std::function<int(cudaStream_t s, int d0, int64_t f0, int nf)>;
+int run_stereo_chunks(orbx_ctx *c, int64_t n_frames, const uint8_t *left, size_t left_stride, const uint8_t *right, size_t right_stride, size_t frame_stride,
+                      bool on_device, bool piped, const ChunkOut &out);
 // per-frame records (orbx_record_layout) of device slots [d0, d0 + nf) assembled at d_rec; device staging for host outputs
 int pack_frame_records(orbx_ctx *c, cudaStream_t s, int d0, int nf, uint8_t *d_rec, size_t rec_stride);
 int ensure_record_staging(orbx_ctx *c, size_t rec_stride);

@@ -498,12 +498,6 @@ void launch_pyramid_levels(const Params &p, const LevelMaps &src_maps, int n_ima
   if (p.n_tiles > p.n_tiles0) pyramid_levels_kernel<<<dim3(p.n_tiles - p.n_tiles0, n_images), kPyrThreads, 0, s>>>(p, src_maps);
 }
 
-void launch_pyramid(const Params &p, const LevelMaps &src_maps, int n_images, cudaStream_t s)
-{
-  launch_pyramid_level0(p, n_images, s);
-  launch_pyramid_levels(p, src_maps, n_images, s);
-}
-
 // ------------------------------------------------------------------------------------------------------------------
 // K2: FAST-9/16 with non-max suppression per 30-px cell and the iniTh -> minTh fallback.  One warp per cell.
 //   arc value m(p) = max over the 16 arcs of 9 contiguous ring pixels of min(+-(I(p) - I(ring)));

@@ -521,9 +521,7 @@ extern "C"
       int rc = ensure_record_staging_impl(c, rs);
       if (rc) return rc;
     }
-    const size_t W = (size_t)c->cfg.width, H = (size_t)c->cfg.height, N = (size_t)c->cfg.n_features;
-    const size_t stride = io->stride, frame_stride = io->frame_stride;
-    if (stride < W || frame_stride < stride * (H - 1) + W) return fail(c, ORBX_ERR_INVALID_ARG, "stride / frame_stride smaller than the image");
+    const size_t N = (size_t)c->cfg.n_features;
     const bool kf_bow = kio && kio->vocab, kf_host = kio && !kio->on_device;
     if (kio)
     {
@@ -537,29 +535,18 @@ extern "C"
       if (rc) return rc;
     }
 
-    // inputs from the host are staged per slot exactly as in orbx_stereo_batch (one linear copy per side when rows are dense)
-    size_t fs = c->in_pitch * H, dstride = c->in_pitch;
-    uint8_t *dl = c->d_in, *dr = c->d_in + (size_t)c->cfg.max_batch * c->in_pitch * H;
-    const bool in_dev = io->input_on_device != 0;
-    const bool linear = !in_dev && frame_stride == stride * H && stride <= c->in_pitch;
-    if (linear) fs = frame_stride, dstride = stride;
-
-    const int chunk = std::min(c->kChunk, c->cfg.max_batch);
-    const int n_slots = std::max(1, c->cfg.max_batch / chunk);
-    ORBX_CUDA(c, cudaEventRecord(c->fork_ev, c->stream));
-    for (int i = 0; i < c->kPipe; ++i) ORBX_CUDA(c, cudaStreamWaitEvent(c->pipe[i], c->fork_ev, 0));
     const bool use_nccl = m->transport == ORBX_TRANSPORT_NCCL && R > 1;
-    if (m->comm_stream) ORBX_CUDA(c, cudaStreamWaitEvent(m->comm_stream, c->fork_ev, 0));
-    // padding rows of this rank's block (ragged last block) carry a zero count
+    // padding rows of this rank's block (ragged last block) carry a zero count; on the context's stream, so that the fork of
+    // the pipeline streams orders everything after it
     if (n_local < block)
     {
       if (m->transport == ORBX_TRANSPORT_PEER)
       {
         for (int r = 0; r < R; ++r)
-          ORBX_CUDA(c, cudaMemsetAsync(reinterpret_cast<int32_t *>(m->peer_base[r] + m->g.desc_bytes) + me * block + n_local, 0, (size_t)(block - n_local) * 4, c->pipe[0]));
+          ORBX_CUDA(c, cudaMemsetAsync(reinterpret_cast<int32_t *>(m->peer_base[r] + m->g.desc_bytes) + me * block + n_local, 0, (size_t)(block - n_local) * 4, c->stream));
       }
       else
-        ORBX_CUDA(c, cudaMemsetAsync(m->g.n() + me * block + n_local, 0, (size_t)(block - n_local) * 4, c->pipe[0]));
+        ORBX_CUDA(c, cudaMemsetAsync(m->g.n() + me * block + n_local, 0, (size_t)(block - n_local) * 4, c->stream));
     }
 
     PackArgs pa{};
@@ -584,7 +571,9 @@ extern "C"
 
     // NCCL: the block is exchanged in pieces of piece_frames frames (a multiple of the chunk) on the comm stream while later
     // chunks are still being computed; every rank runs the same number of pieces over the PADDED block so that the grouped
-    // send/recv calls match.  A piece is ready once everything enqueued so far on the pipeline streams has run.
+    // send/recv calls match.  A piece is ready once everything enqueued so far on the pipeline streams has run (which
+    // also orders the comm stream after the fork of the pipeline streams from the context's stream).
+    const int chunk = c->chunk();
     const int piece = std::max(chunk, (m->piece_frames / chunk) * chunk);
     const int64_t n_pieces = use_nccl ? (block + piece - 1) / piece : 0;
     int64_t next_piece = 0;
@@ -606,57 +595,33 @@ extern "C"
       return ORBX_OK;
     };
 
-    int k = 0;
-    for (int64_t f0 = 0; f0 < n_local; f0 += chunk, ++k)
-    {
-      const int nf = (int)std::min<int64_t>(chunk, n_local - f0);
-      const int slot = k % n_slots;
-      const size_t d0 = (size_t)slot * chunk;
-      cudaStream_t s = c->pipe[slot % c->kPipe];
-      const uint8_t *src_l = io->left + (size_t)f0 * frame_stride, *src_r = io->right + (size_t)f0 * frame_stride;
-      int rc;
-      if (in_dev)
-      { // kernels read the caller's device images in place; only the intermediate buffers cycle through the slots
-        rc = run_stereo_range(c, s, (int)d0, nf, src_l, src_r, stride, frame_stride);
-      }
-      else
-      {
-        if (linear)
-        {
-          ORBX_CUDA(c, cudaMemcpyAsync(dl + d0 * fs, src_l, fs * nf, cudaMemcpyHostToDevice, s));
-          ORBX_CUDA(c, cudaMemcpyAsync(dr + d0 * fs, src_r, fs * nf, cudaMemcpyHostToDevice, s));
-        }
-        else
-          for (int f = 0; f < nf; ++f)
-          {
-            ORBX_CUDA(c, cudaMemcpy2DAsync(dl + (d0 + f) * fs, c->in_pitch, src_l + (size_t)f * frame_stride, stride, W, H, cudaMemcpyHostToDevice, s));
-            ORBX_CUDA(c, cudaMemcpy2DAsync(dr + (d0 + f) * fs, c->in_pitch, src_r + (size_t)f * frame_stride, stride, W, H, cudaMemcpyHostToDevice, s));
-          }
-        rc = run_stereo_range(c, s, (int)d0, nf, dl + d0 * fs, dr + d0 * fs, dstride, fs);
-      }
-      if (rc) return rc;
-      const Params p = params_at(c, 2 * (int)d0, (int)d0);
-      pa.rec = rec_dev ? (uint8_t *)io->records + (size_t)f0 * rs : (rec_host ? c->rec_staging + d0 * rs : nullptr);
+    // per chunk on its pipeline stream: pack -> record copy -> keyframe records -> the NCCL pieces it completes
+    auto chunk_out = [&](cudaStream_t s, int d0, int64_t f0, int nf) -> int {
+      const Params p = params_at(c, 2 * d0, d0);
+      pa.rec = rec_dev ? (uint8_t *)io->records + (size_t)f0 * rs : (rec_host ? c->rec_staging + (size_t)d0 * rs : nullptr);
       pa.gframe0 = me * block + f0;
       pack_records_kernel<<<dim3(kPackBlocksPerFrame, nf), kPackThreads, 0, s>>>(p, pa);
       ++c->launches;
       ORBX_CUDA(c, cudaGetLastError());
-      if (rec_host) ORBX_CUDA(c, cudaMemcpyAsync((uint8_t *)io->records + (size_t)f0 * rs, c->rec_staging + d0 * rs, rs * nf, cudaMemcpyDeviceToHost, s));
+      if (rec_host) ORBX_CUDA(c, cudaMemcpyAsync((uint8_t *)io->records + (size_t)f0 * rs, c->rec_staging + (size_t)d0 * rs, rs * nf, cudaMemcpyDeviceToHost, s));
       if (kio)
       {
-        rc = keyframe_chunk(c, kio, p, s, d0, f0, nf, lo);
+        int rc = keyframe_chunk(c, kio, p, s, d0, f0, nf, lo);
         if (rc) return rc;
       }
       const int64_t done = f0 + nf;
       while (next_piece < n_pieces && done >= std::min<int64_t>(n_local, (next_piece + 1) * piece))
       {
-        rc = exchange_piece(next_piece++);
+        int rc = exchange_piece(next_piece++);
         if (rc) return rc;
       }
-    }
+      return ORBX_OK;
+    };
+    int rc = run_stereo_chunks(c, n_local, io->left, io->stride, io->right, io->stride, io->frame_stride, io->input_on_device != 0, true, chunk_out);
+    if (rc) return rc;
     while (next_piece < n_pieces)
     { // an empty block, or pieces that lie entirely in this rank's padding
-      int rc = exchange_piece(next_piece++);
+      rc = exchange_piece(next_piece++);
       if (rc) return rc;
     }
     for (int i = 0; i < c->kPipe; ++i) ORBX_CUDA(c, cudaStreamSynchronize(c->pipe[i]));
@@ -672,10 +637,6 @@ extern "C"
     if (io->gathered_desc_host) ORBX_CUDA(c, cudaMemcpy(io->gathered_desc_host, m->g.desc(), (size_t)F * N * 32, cudaMemcpyDeviceToHost));
     if (io->gathered_n_host) ORBX_CUDA(c, cudaMemcpy(io->gathered_n_host, m->g.n(), (size_t)F * 4, cudaMemcpyDeviceToHost));
 
-    c->last_frames = (int)std::min<int64_t>(n_local, (int64_t)n_slots * chunk);
-    c->last_images = 2 * c->last_frames;
-    ++c->frame_epoch;
-    c->last_stereo = 1;
     if (res)
     {
       res->frame_lo = lo;
