@@ -164,7 +164,11 @@ int orbx_stereo_batch_device(orbx_ctx *ctx, int n_frames, const uint8_t *d_left,
 /* mono extraction of n_images device-resident images (ORBExtractor only) */
 int orbx_extract_batch_device(orbx_ctx *ctx, int n_images, const uint8_t *d_images, size_t stride, size_t frame_stride,
                               orbx_device_results *out);
-/* RGB-D frames with device-resident gray + depth images */
+/* RGB-D frames with device-resident gray + depth images (up to 2 * max_batch frames).  Depth frame f, row y starts at
+ * d_depth + f * depth_frame_stride_bytes + y * depth_stride_bytes.  d_depth and both strides must be multiples of the
+ * element size (2 for ORBX_DEPTH_U16, 4 for ORBX_DEPTH_F32), depth_stride_bytes >= width * element size and, for more
+ * than one frame, depth_frame_stride_bytes >= depth_stride_bytes * (height - 1) + width * element size; otherwise
+ * ORBX_ERR_INVALID_ARG before anything is enqueued. */
 int orbx_rgbd_batch_device(orbx_ctx *ctx, int n_frames, const uint8_t *d_gray, size_t gray_stride,
                            size_t gray_frame_stride, const void *d_depth, size_t depth_stride_bytes,
                            size_t depth_frame_stride_bytes, int depth_type, orbx_device_results *out);

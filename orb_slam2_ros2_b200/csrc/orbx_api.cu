@@ -472,7 +472,8 @@ int fail(orbx_ctx *c, int code, const std::string &msg)
 int bow_buffers(orbx_ctx *c)
 {
   if (c->bow_ready) return ORBX_OK;
-  const size_t F = (size_t)c->cfg.max_batch, N = (size_t)c->cfg.n_features;
+  // one frame per image: a mono / RGB-D batch leaves up to n_img_max = 2 * max_batch frames resident
+  const size_t F = (size_t)c->n_img_max, N = (size_t)c->cfg.n_features;
   if (N > 65535) return fail(c, ORBX_ERR_CAPACITY, "the bag-of-words kernels index features with 16 bits");
   int rc;
   BowArgs &b = c->bow;
@@ -1129,6 +1130,12 @@ extern "C"
   {
     if (!c || !d_gray || !d_depth || n_frames < 1 || (depth_type != ORBX_DEPTH_U16 && depth_type != ORBX_DEPTH_F32)) return ORBX_ERR_INVALID_ARG;
     if (n_frames > c->n_img_max) return fail(c, ORBX_ERR_CAPACITY, "n_frames > 2 * max_batch");
+    // rgbd_kernel loads whole elements at depth + f * frame_stride + y * stride: a misaligned address would fault
+    const size_t esz = depth_type == ORBX_DEPTH_F32 ? 4 : 2, W = (size_t)c->cfg.width, H = (size_t)c->cfg.height;
+    if ((size_t)d_depth % esz || depth_stride_bytes % esz || depth_frame_stride_bytes % esz)
+      return fail(c, ORBX_ERR_INVALID_ARG, "depth pointer, stride and frame stride must be multiples of the depth element size");
+    if (depth_stride_bytes < W * esz || (n_frames > 1 && depth_frame_stride_bytes < depth_stride_bytes * (H - 1) + W * esz))
+      return fail(c, ORBX_ERR_INVALID_ARG, "depth stride / frame stride smaller than the depth image");
     ORBX_CUDA(c, cudaSetDevice(c->device));
     Params p = c->p;
     p.stereo = 0;

@@ -104,7 +104,7 @@ int pack_frame_records(orbx_ctx *c, cudaStream_t s, int d0, int nf, uint8_t *d_r
 int ensure_record_staging(orbx_ctx *c, size_t rec_stride);
 // frees the gathered arrays a context keeps for single-rank sequence calls
 void destroy_self_comm(orbx_ctx *c);
-// allocates the context's bag-of-words result buffers (max_batch frames) on first use
+// allocates the context's bag-of-words result buffers (n_img_max frames, as many as an RGB-D batch holds) on first use
 int bow_buffers(orbx_ctx *c);
 // c->bow with the vocabulary's tree, ready for launch_bow_descend / launch_bow_assemble
 BowArgs bow_args(const orbx_ctx *c, const orbx_vocab *v, int levelsup);

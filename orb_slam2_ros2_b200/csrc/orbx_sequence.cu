@@ -273,7 +273,7 @@ int keyframe_chunk(orbx_ctx *c, const orbx_keyframe_io *kio, const Params &p, cu
   {
     BowArgs ba = bow_args(c, kio->vocab, kio->levelsup);
     ba.image_stride = 2;
-    ba.f_word += d0 * N, ba.f_nid += d0 * N, ba.f_weight += d0 * N; // the slots' own frames of the max_batch-frame buffers
+    ba.f_word += d0 * N, ba.f_nid += d0 * N, ba.f_weight += d0 * N; // the slots' own frames of the n_img_max-frame buffers
     ba.bow_ids += d0 * N, ba.bow_vals += d0 * N, ba.n_bow += d0;
     ba.fv_nodes += d0 * N, ba.fv_start += d0 * (N + 1), ba.fv_feats += d0 * N, ba.n_fv += d0;
     launch_bow_descend(p, ba, nf, s);
