@@ -492,12 +492,41 @@ int bow_buffers(orbx_ctx *c)
   return ORBX_OK;
 }
 
-BowArgs bow_args(const orbx_ctx *c, const orbx_vocab *v, int levelsup)
+BowArgs bow_args(const orbx_ctx *c, const orbx_vocab *v, int levelsup, int image_stride)
 {
   BowArgs a = c->bow;
   a.child_start = v->child_start, a.child_ids = v->child_ids, a.v_desc = v->desc, a.v_weight = v->weight, a.v_word = v->word;
-  a.L = v->L, a.levelsup = levelsup, a.image_stride = c->last_stereo ? 2 : 1;
+  a.L = v->L, a.levelsup = levelsup, a.image_stride = image_stride;
   return a;
+}
+
+BowArgs bow_at(const BowArgs &b, size_t frame0, size_t N)
+{
+  BowArgs a = b;
+  a.f_word += frame0 * N, a.f_nid += frame0 * N, a.f_weight += frame0 * N;
+  a.bow_ids += frame0 * N, a.bow_vals += frame0 * N, a.n_bow += frame0;
+  a.fv_nodes += frame0 * N, a.fv_start += frame0 * (N + 1), a.fv_feats += frame0 * N, a.n_fv += frame0;
+  return a;
+}
+
+SerArgs ser_args(const orbx_ctx *c, int image_stride, uint8_t *out, size_t stride, int64_t *sizes, uint64_t id0, const float *pose, int with_map_points)
+{
+  SerArgs a{};
+  a.out = out, a.stride = stride, a.sizes = (long long *)sizes, a.id0 = id0, a.pose = pose, a.with_map_points = with_map_points;
+  a.image_stride = image_stride;
+  a.max_u = c->max_u, a.max_v = c->max_v, a.min_u = c->min_u, a.min_v = c->min_v;
+  return a;
+}
+
+int DeviceBuffer::reserve(orbx_ctx *c, size_t want)
+{
+  if (want <= bytes) return ORBX_OK;
+  if (p) ORBX_CUDA(c, cudaDeviceSynchronize());
+  cudaFree(p);
+  p = nullptr, bytes = 0;
+  ORBX_CUDA(c, cudaMalloc((void **)&p, want));
+  bytes = want;
+  return ORBX_OK;
 }
 
 // Params whose per-image buffers start at image `img0` (and per-frame buffers at frame `frame0`)
@@ -535,6 +564,28 @@ static void set_resident(orbx_ctx *c, int images, int frames, int stereo)
   c->last_frames = frames;
   c->last_stereo = stereo;
   ++c->frame_epoch;
+}
+
+// frame f of the resident frames reads image f * image_stride(c)
+static int image_stride(const orbx_ctx *c) { return c->last_stereo ? 2 : 1; }
+
+// The residency rule of the frame-level consumers: ORBX_OK when the images / frames / BoW of [0, end) are resident (one index
+// i: end = i + 1LL), ORBX_ERR_STATE otherwise.  A BoW is resident from the orbx_bow_transform* call that covered its frame
+// until the next call that produces frames.
+static int require_images(orbx_ctx *c, int64_t end)
+{
+  if (end <= c->last_images) return ORBX_OK;
+  return fail(c, ORBX_ERR_STATE, "no image with that index has been processed");
+}
+static int require_frames(orbx_ctx *c, int64_t end)
+{
+  if (end <= c->last_frames) return ORBX_OK;
+  return fail(c, ORBX_ERR_STATE, "no frame with that index has been processed by the most recent stereo / RGB-D call");
+}
+static int require_bow(orbx_ctx *c, int64_t end)
+{
+  if (c->bow_epoch == c->frame_epoch && end <= c->bow_frames) return ORBX_OK;
+  return fail(c, ORBX_ERR_STATE, "the bag of words of that frame is not resident: call orbx_bow_transform* on the most recent call's frames first");
 }
 
 // the pipeline streams wait for the work enqueued so far on the context's stream
@@ -982,14 +1033,10 @@ extern "C"
     for (auto &je : c->join_ev)
       if (je) cudaEventDestroy(je);
     for (void *q : c->allocs) cudaFree(q);
-    if (c->match_scratch) cudaFree(c->match_scratch);
     drop_graph(c);
     destroy_self_comm(c);
-    if (c->rec_staging) cudaFree(c->rec_staging);
     if (c->h_rec1) cudaFreeHost(c->h_rec1);
-    if (c->kf_staging) cudaFree(c->kf_staging);
-    if (c->kf_sizes) cudaFree(c->kf_sizes);
-    delete c;
+    delete c; // frees the DeviceBuffers
   }
 
   const char *orbx_last_error(const orbx_ctx *c) { return c ? c->last_error.c_str() : ""; }
@@ -1170,13 +1217,13 @@ extern "C"
     orbx_record_layout lay;
     orbx_record_layout_get(c, &lay);
     const size_t rs = (size_t)lay.record_bytes;
-    int rc = ensure_record_staging(c, rs);
+    int rc = c->rec_staging.reserve(c, (size_t)c->cfg.max_batch * rs);
     if (rc) return rc;
     if (!c->h_rec1) ORBX_CUDA(c, cudaHostAlloc((void **)&c->h_rec1, rs, cudaHostAllocDefault));
     rc = run_stereo_chunks(c, 1, left, left_stride, right, right_stride, frame_stride, false, false, [&](cudaStream_t s, int, int64_t, int) -> int {
-      const int prc = pack_frame_records(c, s, 0, 1, c->rec_staging, rs);
+      const int prc = pack_frame_records(c, s, 0, 1, c->rec_staging.p, rs);
       if (prc) return prc;
-      ORBX_CUDA(c, cudaMemcpyAsync(c->h_rec1, c->rec_staging, rs, cudaMemcpyDeviceToHost, s));
+      ORBX_CUDA(c, cudaMemcpyAsync(c->h_rec1, c->rec_staging.p, rs, cudaMemcpyDeviceToHost, s));
       return ORBX_OK;
     });
     if (rc) return rc;
@@ -1280,7 +1327,7 @@ extern "C"
   int orbx_get_pyramid(orbx_ctx *c, int side, int level, int blurred, uint8_t *dst, size_t dst_stride)
   {
     if (!c || !dst || level < 0 || level >= c->cfg.n_levels || side < 0) return ORBX_ERR_INVALID_ARG;
-    if (side >= c->last_images) return fail(c, ORBX_ERR_STATE, "no image with that index has been processed");
+    if (int rc = require_images(c, side + 1LL)) return rc;
     ORBX_CUDA(c, cudaSetDevice(c->device));
     const Level &L = c->levels[level];
     const uint8_t *src = (blurred ? c->p.blur : c->p.pyr) + (size_t)side * c->p.pyr_img_stride + L.pyr_off;
@@ -1304,7 +1351,7 @@ extern "C"
   int orbx_get_grid(orbx_ctx *c, int frame, int32_t *cell_start, int32_t *entries)
   {
     if (!c || frame < 0 || !cell_start || !entries) return ORBX_ERR_INVALID_ARG;
-    if (frame >= c->last_frames) return fail(c, ORBX_ERR_STATE, "no frame with that index has a grid (stereo / RGB-D calls build it)");
+    if (int rc = require_frames(c, frame + 1LL)) return rc;
     ORBX_CUDA(c, cudaSetDevice(c->device));
     ORBX_CUDA(c, cudaStreamSynchronize(c->stream));
     const size_t nc = (size_t)c->p.grid_rows * c->p.grid_cols, N = (size_t)c->cfg.n_features;
@@ -1318,23 +1365,29 @@ extern "C"
 
   // ---------------------------------------------------------------------------------------------------------------
   // tracking-side matchers (SURVEY.md section 8(f) rank 2)
-  static int match_scratch(orbx_ctx *c, size_t bytes, uint8_t **out)
+  // the matcher staging grows with 50 % + 4 KiB of headroom, so that slowly rising input sizes do not reallocate every call
+  static int reserve_match_scratch(orbx_ctx *c, size_t bytes)
   {
-    if (bytes > c->match_scratch_bytes)
-    {
-      ORBX_CUDA(c, cudaStreamSynchronize(c->stream));
-      if (c->match_scratch) cudaFree(c->match_scratch);
-      c->match_scratch = nullptr;
-      c->match_scratch_bytes = 0;
-      const size_t want = bytes + bytes / 2 + 4096;
-      ORBX_CUDA(c, cudaMalloc((void **)&c->match_scratch, want));
-      c->match_scratch_bytes = want;
-    }
-    *out = c->match_scratch;
-    return ORBX_OK;
+    return bytes <= c->match_scratch.bytes ? ORBX_OK : c->match_scratch.reserve(c, bytes + bytes / 2 + 4096);
   }
 
   static inline size_t up256(size_t v) { return (v + 255) & ~(size_t)255; }
+
+  // orbx_search_in_area_batch_device on the resident frames [frame0, frame0 + n_frames), on the context's stream
+  static int search_in_area_device(orbx_ctx *c, int frame0, int n_frames, int query_stride, const orbx_area_query *d_queries, const uint8_t *d_query_desc,
+                                   const int32_t *d_n_queries, const uint8_t *d_exclude, int32_t *d_best_idx, int32_t *d_best_dist, float *d_ratio,
+                                   int32_t *d_n_candidates)
+  {
+    AreaArgs a{};
+    a.image_stride = image_stride(c), a.max_u = c->max_u, a.max_v = c->max_v;
+    a.q = d_queries, a.q_desc = d_query_desc, a.n_q = d_n_queries, a.n_q_all = query_stride, a.q_stride = query_stride;
+    a.exclude = d_exclude;
+    a.best_idx = d_best_idx, a.best_dist = d_best_dist, a.ratio = d_ratio, a.n_cand = d_n_candidates;
+    launch_area_match(params_at(c, frame0 * a.image_stride, frame0), a, n_frames, c->stream);
+    ++c->launches;
+    ORBX_CUDA(c, cudaGetLastError());
+    return ORBX_OK;
+  }
 
   int orbx_search_in_area_batch_device(orbx_ctx *c, int n_frames, int query_stride, const orbx_area_query *d_queries, const uint8_t *d_query_desc,
                                        const int32_t *d_n_queries, const uint8_t *d_exclude, int32_t *d_best_idx, int32_t *d_best_dist, float *d_ratio,
@@ -1342,48 +1395,33 @@ extern "C"
   {
     if (!c || n_frames < 1 || query_stride < 1 || !d_queries || !d_query_desc || !d_best_idx || !d_best_dist || !d_ratio || !d_n_candidates)
       return ORBX_ERR_INVALID_ARG;
-    if (n_frames > c->last_frames) return fail(c, ORBX_ERR_STATE, "more frames than the last stereo / RGB-D call processed (they own the grids)");
+    if (int rc = require_frames(c, n_frames)) return rc;
     ORBX_CUDA(c, cudaSetDevice(c->device));
-    AreaArgs a{};
-    a.q = d_queries, a.q_desc = d_query_desc, a.n_q = d_n_queries, a.n_q_all = query_stride, a.q_stride = query_stride;
-    a.exclude = d_exclude;
-    a.best_idx = d_best_idx, a.best_dist = d_best_dist, a.ratio = d_ratio, a.n_cand = d_n_candidates;
-    a.image_stride = c->last_stereo ? 2 : 1;
-    a.max_u = c->max_u, a.max_v = c->max_v;
-    launch_area_match(c->p, a, n_frames, c->stream);
-    ++c->launches;
-    ORBX_CUDA(c, cudaGetLastError());
-    return ORBX_OK;
+    return search_in_area_device(c, 0, n_frames, query_stride, d_queries, d_query_desc, d_n_queries, d_exclude, d_best_idx, d_best_dist, d_ratio,
+                                 d_n_candidates);
   }
 
   int orbx_search_in_area(orbx_ctx *c, int frame, int n_queries, const orbx_area_query *queries, const uint8_t *query_desc, const uint8_t *exclude,
                           int32_t *best_idx, int32_t *best_dist, float *ratio, int32_t *n_candidates)
   {
     if (!c || frame < 0 || n_queries < 0 || (n_queries && (!queries || !query_desc))) return ORBX_ERR_INVALID_ARG;
-    if (frame >= c->last_frames) return fail(c, ORBX_ERR_STATE, "no frame with that index has a grid (stereo / RGB-D calls build it)");
+    if (int rc = require_frames(c, frame + 1LL)) return rc;
     if (n_queries == 0) return ORBX_OK;
     ORBX_CUDA(c, cudaSetDevice(c->device));
     const size_t n = (size_t)n_queries, N = (size_t)c->cfg.n_features;
     const size_t o_q = 0, o_d = o_q + up256(n * sizeof(orbx_area_query)), o_x = o_d + up256(n * 32), o_out = o_x + up256(N), total = o_out + up256(n * 16);
-    uint8_t *base = nullptr;
-    int rc = match_scratch(c, total, &base);
+    int rc = reserve_match_scratch(c, total);
     if (rc) return rc;
+    uint8_t *base = c->match_scratch.p;
     cudaStream_t s = c->stream;
     ORBX_CUDA(c, cudaMemcpyAsync(base + o_q, queries, n * sizeof(orbx_area_query), cudaMemcpyHostToDevice, s));
     ORBX_CUDA(c, cudaMemcpyAsync(base + o_d, query_desc, n * 32, cudaMemcpyHostToDevice, s));
     if (exclude) ORBX_CUDA(c, cudaMemcpyAsync(base + o_x, exclude, N, cudaMemcpyHostToDevice, s));
     int32_t *d_idx = (int32_t *)(base + o_out), *d_dist = d_idx + n, *d_nc = d_dist + n;
     float *d_ratio = (float *)(d_nc + n);
-    AreaArgs a{};
-    a.q = (const orbx_area_query *)(base + o_q), a.q_desc = base + o_d, a.n_q = nullptr, a.n_q_all = n_queries, a.q_stride = n_queries;
-    a.exclude = exclude ? base + o_x : nullptr;
-    a.best_idx = d_idx, a.best_dist = d_dist, a.ratio = d_ratio, a.n_cand = d_nc;
-    a.image_stride = c->last_stereo ? 2 : 1;
-    a.max_u = c->max_u, a.max_v = c->max_v;
-    const Params p = params_at(c, frame * a.image_stride, frame);
-    launch_area_match(p, a, 1, s);
-    ++c->launches;
-    ORBX_CUDA(c, cudaGetLastError());
+    rc = search_in_area_device(c, frame, 1, n_queries, (const orbx_area_query *)(base + o_q), base + o_d, nullptr, exclude ? base + o_x : nullptr, d_idx,
+                               d_dist, d_ratio, d_nc);
+    if (rc) return rc;
     if (best_idx) ORBX_CUDA(c, cudaMemcpyAsync(best_idx, d_idx, n * 4, cudaMemcpyDeviceToHost, s));
     if (best_dist) ORBX_CUDA(c, cudaMemcpyAsync(best_dist, d_dist, n * 4, cudaMemcpyDeviceToHost, s));
     if (n_candidates) ORBX_CUDA(c, cudaMemcpyAsync(n_candidates, d_nc, n * 4, cudaMemcpyDeviceToHost, s));
@@ -1406,9 +1444,9 @@ extern "C"
     const size_t n = (size_t)n_matches;
     const size_t o_in = 0, o_k1 = o_in + up256(n * 12), o_k2 = o_k1 + up256((size_t)n1 * sizeof(orbx_keypoint)),
                  o_out = o_k2 + up256((size_t)n2 * sizeof(orbx_keypoint)), total = o_out + up256(n * 12 + 4);
-    uint8_t *base = nullptr;
-    int rc = match_scratch(c, total, &base);
+    int rc = reserve_match_scratch(c, total);
     if (rc) return rc;
+    uint8_t *base = c->match_scratch.p;
     cudaStream_t s = c->stream;
     int32_t *d_q = (int32_t *)(base + o_in), *d_t = d_q + n;
     float *d_d = (float *)(d_t + n);
@@ -1455,7 +1493,19 @@ extern "C"
     return (int64_t)((128 + 12 + (size_t)c->cfg.n_features * (28 + 4 + 4 + 36 + 10 + 17 + 13 + 3) + 15) & ~(size_t)15);
   }
 
-  static bool bow_resident(const orbx_ctx *c, int n_frames) { return c->bow_epoch == c->frame_epoch && n_frames <= c->bow_frames; }
+  // the serialiser on the resident frames [frame0, frame0 + n_frames) into device memory, on the context's stream; with `bow`,
+  // from their resident BoW
+  static int serialize_device(orbx_ctx *c, int frame0, int n_frames, uint64_t id0, const float *d_pose_rt, int with_map_points, uint8_t *d_out,
+                              size_t frame_stride, int64_t *d_sizes, bool bow)
+  {
+    const int is = image_stride(c);
+    SerArgs a = ser_args(c, is, d_out, frame_stride, d_sizes, id0, d_pose_rt, with_map_points);
+    if (bow) ser_bow_inputs(a, bow_at(c->bow, (size_t)frame0, (size_t)c->cfg.n_features));
+    launch_serialize(params_at(c, frame0 * is, frame0), a, n_frames, c->stream);
+    ++c->launches;
+    ORBX_CUDA(c, cudaGetLastError());
+    return ORBX_OK;
+  }
 
   static int serialize_frames_device(orbx_ctx *c, int n_frames, uint64_t id0, const float *d_pose_rt, int with_map_points, uint8_t *d_out,
                                      size_t frame_stride, int64_t *d_sizes, bool bow)
@@ -1465,18 +1515,10 @@ extern "C"
     if (bow && (int64_t)frame_stride < orbx_serialized_capacity_bow(c))
       return fail(c, ORBX_ERR_CAPACITY, "frame_stride is smaller than orbx_serialized_capacity_bow()");
     if ((int64_t)frame_stride < orbx_serialized_capacity(c)) return fail(c, ORBX_ERR_CAPACITY, "frame_stride is smaller than orbx_serialized_capacity()");
-    if (n_frames > c->last_frames) return fail(c, ORBX_ERR_STATE, "more frames than the last stereo / RGB-D call processed");
-    if (bow && !bow_resident(c, n_frames)) return fail(c, ORBX_ERR_STATE, "call orbx_bow_transform* for these frames first (their BoW must be resident)");
+    if (int rc = require_frames(c, n_frames)) return rc;
+    if (int rc = bow ? require_bow(c, n_frames) : ORBX_OK) return rc;
     ORBX_CUDA(c, cudaSetDevice(c->device));
-    SerArgs a{};
-    a.out = d_out, a.stride = frame_stride, a.sizes = (long long *)d_sizes, a.id0 = id0, a.pose = d_pose_rt, a.with_map_points = with_map_points;
-    a.image_stride = c->last_stereo ? 2 : 1;
-    a.max_u = c->max_u, a.max_v = c->max_v, a.min_u = c->min_u, a.min_v = c->min_v;
-    if (bow) ser_bow_inputs(a, c->bow, 0, (size_t)c->cfg.n_features);
-    launch_serialize(c->p, a, n_frames, c->stream);
-    ++c->launches;
-    ORBX_CUDA(c, cudaGetLastError());
-    return ORBX_OK;
+    return serialize_device(c, 0, n_frames, id0, d_pose_rt, with_map_points, d_out, frame_stride, d_sizes, bow);
   }
 
   int orbx_serialize_keyframes_device(orbx_ctx *c, int n_frames, uint64_t id0, const float *d_pose_rt, int with_map_points, uint8_t *d_out,
@@ -1495,27 +1537,19 @@ extern "C"
                              bool bow)
   {
     if (!c || frame < 0 || !out || !n_bytes) return ORBX_ERR_INVALID_ARG;
-    if (frame >= c->last_frames) return fail(c, ORBX_ERR_STATE, "no frame with that index has been processed by a stereo / RGB-D call");
-    if (bow && !bow_resident(c, frame + 1)) return fail(c, ORBX_ERR_STATE, "call orbx_bow_transform for this frame first (its BoW must be resident)");
+    if (int rc = require_frames(c, frame + 1LL)) return rc;
+    if (int rc = bow ? require_bow(c, frame + 1LL) : ORBX_OK) return rc;
     ORBX_CUDA(c, cudaSetDevice(c->device));
     const size_t rec = (size_t)(bow ? orbx_serialized_capacity_bow(c) : orbx_serialized_capacity(c));
-    uint8_t *base = nullptr;
-    int rc = match_scratch(c, rec + 256, &base);
+    int rc = reserve_match_scratch(c, rec + 256);
     if (rc) return rc;
+    uint8_t *base = c->match_scratch.p;
     cudaStream_t s = c->stream;
     float *d_pose = (float *)(base + rec);
     int64_t *d_size = (int64_t *)(base + rec + 64);
     if (pose_rt) ORBX_CUDA(c, cudaMemcpyAsync(d_pose, pose_rt, 12 * sizeof(float), cudaMemcpyHostToDevice, s));
-    SerArgs a{};
-    a.out = base, a.stride = rec, a.sizes = (long long *)d_size, a.id0 = id, a.pose = pose_rt ? d_pose : nullptr;
-    a.with_map_points = with_map_points;
-    a.image_stride = c->last_stereo ? 2 : 1;
-    a.max_u = c->max_u, a.max_v = c->max_v, a.min_u = c->min_u, a.min_v = c->min_v;
-    const Params p = params_at(c, frame * a.image_stride, frame); // the single CTA (block 0) works on `frame`
-    if (bow) ser_bow_inputs(a, c->bow, (size_t)frame, (size_t)c->cfg.n_features);
-    launch_serialize(p, a, 1, s);
-    ++c->launches;
-    ORBX_CUDA(c, cudaGetLastError());
+    rc = serialize_device(c, frame, 1, id, pose_rt ? d_pose : nullptr, with_map_points, base, rec, d_size, bow);
+    if (rc) return rc;
     int64_t sz = 0;
     ORBX_CUDA(c, cudaMemcpyAsync(&sz, d_size, sizeof(sz), cudaMemcpyDeviceToHost, s));
     ORBX_CUDA(c, cudaStreamSynchronize(s));
@@ -1570,10 +1604,10 @@ extern "C"
                                    char *out, size_t cap, int64_t *n_bytes)
   {
     if (!c || frame < 0 || !out || !n_bytes) return ORBX_ERR_INVALID_ARG;
-    if (frame >= c->last_frames) return fail(c, ORBX_ERR_STATE, "no frame with that index has been processed by a stereo / RGB-D call");
+    if (int rc = require_frames(c, frame + 1LL)) return rc;
     ORBX_CUDA(c, cudaSetDevice(c->device));
     ORBX_CUDA(c, cudaStreamSynchronize(c->stream));
-    const int img = frame * (c->last_stereo ? 2 : 1);
+    const int img = frame * image_stride(c);
     const size_t N = (size_t)c->cfg.n_features;
     int n = 0;
     ORBX_CUDA(c, cudaMemcpy(&n, c->p.n_kps + img, sizeof(int), cudaMemcpyDeviceToHost));
@@ -1754,11 +1788,11 @@ extern "C"
   {
     if (!c || !v || n_frames < 1 || !out) return ORBX_ERR_INVALID_ARG;
     if (v->device != c->device) return fail(c, ORBX_ERR_INVALID_ARG, "vocabulary lives on another device");
-    if (n_frames > c->last_frames) return fail(c, ORBX_ERR_STATE, "more frames than the last stereo / RGB-D call processed");
+    if (int rc = require_frames(c, n_frames)) return rc;
     ORBX_CUDA(c, cudaSetDevice(c->device));
     int rc = bow_buffers(c);
     if (rc) return rc;
-    const BowArgs a = bow_args(c, v, levelsup);
+    const BowArgs a = bow_args(c, v, levelsup, image_stride(c));
     launch_bow_descend(c->p, a, n_frames, c->stream);
     launch_bow_assemble(c->p, a, n_frames, c->stream);
     c->launches += 2;
@@ -1775,23 +1809,23 @@ extern "C"
                          int32_t *fv_start, int32_t *fv_feats, int32_t *n_fv_nodes)
   {
     if (!c || !v || frame < 0 || !n_bow || !n_fv_nodes) return ORBX_ERR_INVALID_ARG;
-    if (frame >= c->last_frames) return fail(c, ORBX_ERR_STATE, "no frame with that index has been processed by a stereo / RGB-D call");
+    if (int rc = require_frames(c, frame + 1LL)) return rc;
     orbx_device_bow d{};
     const int rc = orbx_bow_transform_batch_device(c, v, frame + 1, levelsup, &d); // frames 0..frame (single-frame calls: frame == 0)
     if (rc) return rc;
     ORBX_CUDA(c, cudaStreamSynchronize(c->stream));
-    const size_t N = (size_t)c->cfg.n_features, f = (size_t)frame;
-    ORBX_CUDA(c, cudaMemcpy(n_bow, d.n_bow + f, 4, cudaMemcpyDeviceToHost));
-    ORBX_CUDA(c, cudaMemcpy(n_fv_nodes, d.n_fv_nodes + f, 4, cudaMemcpyDeviceToHost));
-    if (bow_ids) ORBX_CUDA(c, cudaMemcpy(bow_ids, d.bow_ids + f * N, (size_t)*n_bow * 4, cudaMemcpyDeviceToHost));
-    if (bow_vals) ORBX_CUDA(c, cudaMemcpy(bow_vals, d.bow_vals + f * N, (size_t)*n_bow * 8, cudaMemcpyDeviceToHost));
-    if (fv_nodes) ORBX_CUDA(c, cudaMemcpy(fv_nodes, d.fv_nodes + f * N, (size_t)*n_fv_nodes * 4, cudaMemcpyDeviceToHost));
-    if (fv_start) ORBX_CUDA(c, cudaMemcpy(fv_start, d.fv_start + f * (N + 1), ((size_t)*n_fv_nodes + 1) * 4, cudaMemcpyDeviceToHost));
+    const BowArgs b = bow_at(c->bow, (size_t)frame, (size_t)c->cfg.n_features);
+    ORBX_CUDA(c, cudaMemcpy(n_bow, b.n_bow, 4, cudaMemcpyDeviceToHost));
+    ORBX_CUDA(c, cudaMemcpy(n_fv_nodes, b.n_fv, 4, cudaMemcpyDeviceToHost));
+    if (bow_ids) ORBX_CUDA(c, cudaMemcpy(bow_ids, b.bow_ids, (size_t)*n_bow * 4, cudaMemcpyDeviceToHost));
+    if (bow_vals) ORBX_CUDA(c, cudaMemcpy(bow_vals, b.bow_vals, (size_t)*n_bow * 8, cudaMemcpyDeviceToHost));
+    if (fv_nodes) ORBX_CUDA(c, cudaMemcpy(fv_nodes, b.fv_nodes, (size_t)*n_fv_nodes * 4, cudaMemcpyDeviceToHost));
+    if (fv_start) ORBX_CUDA(c, cudaMemcpy(fv_start, b.fv_start, ((size_t)*n_fv_nodes + 1) * 4, cudaMemcpyDeviceToHost));
     if (fv_feats)
     {
       int32_t n_listed = 0; // == fv_start[n_fv_nodes]: only that many entries were written
-      ORBX_CUDA(c, cudaMemcpy(&n_listed, d.fv_start + f * (N + 1) + (size_t)*n_fv_nodes, 4, cudaMemcpyDeviceToHost));
-      if (n_listed > 0) ORBX_CUDA(c, cudaMemcpy(fv_feats, d.fv_feats + f * N, (size_t)n_listed * 4, cudaMemcpyDeviceToHost));
+      ORBX_CUDA(c, cudaMemcpy(&n_listed, b.fv_start + *n_fv_nodes, 4, cudaMemcpyDeviceToHost));
+      if (n_listed > 0) ORBX_CUDA(c, cudaMemcpy(fv_feats, b.fv_feats, (size_t)n_listed * 4, cudaMemcpyDeviceToHost));
     }
     return ORBX_OK;
   }
@@ -1803,8 +1837,7 @@ extern "C"
     if (!c || frame < 0 || n_kf_nodes < 0 || n_kf < 0) return ORBX_ERR_INVALID_ARG;
     if (n_kf_nodes == 0) return ORBX_OK;
     if (!kf_fv_nodes || !kf_fv_start || !kf_fv_feats || !kf_desc) return ORBX_ERR_INVALID_ARG;
-    if (c->bow_epoch != c->frame_epoch || frame >= c->bow_frames)
-      return fail(c, ORBX_ERR_STATE, "call orbx_bow_transform for this frame first (its FeatureVector must be resident)");
+    if (int rc = require_bow(c, frame + 1LL)) return rc;
     const int n_listed = kf_fv_start[n_kf_nodes];
     if (n_listed <= 0) return ORBX_OK;
     for (int i = 0; i < n_listed; ++i)
@@ -1813,9 +1846,9 @@ extern "C"
     const size_t N = (size_t)c->cfg.n_features, nl = (size_t)n_listed, nn = (size_t)n_kf_nodes;
     const size_t o_nodes = 0, o_start = o_nodes + up256(nn * 4), o_feats = o_start + up256((nn + 1) * 4), o_desc = o_feats + up256(nl * 4),
                  o_qok = o_desc + up256((size_t)n_kf * 32), o_cok = o_qok + up256((size_t)n_kf), o_out = o_cok + up256(N), total = o_out + up256(nl * 16);
-    uint8_t *base = nullptr;
-    int rc = match_scratch(c, total, &base);
+    int rc = reserve_match_scratch(c, total);
     if (rc) return rc;
+    uint8_t *base = c->match_scratch.p;
     cudaStream_t s = c->stream;
     ORBX_CUDA(c, cudaMemcpyAsync(base + o_nodes, kf_fv_nodes, nn * 4, cudaMemcpyHostToDevice, s));
     ORBX_CUDA(c, cudaMemcpyAsync(base + o_start, kf_fv_start, (nn + 1) * 4, cudaMemcpyHostToDevice, s));
@@ -1823,11 +1856,10 @@ extern "C"
     ORBX_CUDA(c, cudaMemcpyAsync(base + o_desc, kf_desc, (size_t)n_kf * 32, cudaMemcpyHostToDevice, s));
     if (kf_query_ok) ORBX_CUDA(c, cudaMemcpyAsync(base + o_qok, kf_query_ok, (size_t)n_kf, cudaMemcpyHostToDevice, s));
     if (frame_cand_ok) ORBX_CUDA(c, cudaMemcpyAsync(base + o_cok, frame_cand_ok, N, cudaMemcpyHostToDevice, s));
-    const size_t f = (size_t)frame;
-    const int img = frame * (c->last_stereo ? 2 : 1);
+    const BowArgs b = bow_at(c->bow, (size_t)frame, N);
     BowMatchArgs a{};
-    a.f_nodes = c->bow.fv_nodes + f * N, a.f_start = c->bow.fv_start + f * (N + 1), a.f_feats = c->bow.fv_feats + f * N, a.f_n_nodes = c->bow.n_fv + f;
-    a.f_desc = c->p.desc + (size_t)img * N * 32, a.frame_cand_ok = frame_cand_ok ? base + o_cok : nullptr;
+    a.f_nodes = b.fv_nodes, a.f_start = b.fv_start, a.f_feats = b.fv_feats, a.f_n_nodes = b.n_fv;
+    a.f_desc = c->p.desc + (size_t)frame * image_stride(c) * N * 32, a.frame_cand_ok = frame_cand_ok ? base + o_cok : nullptr;
     a.k_nodes = (const int *)(base + o_nodes), a.k_start = (const int *)(base + o_start), a.k_feats = (const int *)(base + o_feats);
     a.k_n_nodes = n_kf_nodes, a.k_n_listed = n_listed;
     a.k_desc = base + o_desc, a.kf_query_ok = kf_query_ok ? base + o_qok : nullptr;
@@ -1848,7 +1880,7 @@ extern "C"
   int orbx_debug_level_corners(orbx_ctx *c, int image, int level, int32_t *xs, int32_t *ys, int32_t *scores, int cap, int32_t *n)
   {
     if (!c || !n || level < 0 || level >= c->cfg.n_levels || image < 0) return ORBX_ERR_INVALID_ARG;
-    if (image >= c->last_images) return fail(c, ORBX_ERR_STATE, "no image with that index has been processed");
+    if (int rc = require_images(c, image + 1LL)) return rc;
     ORBX_CUDA(c, cudaSetDevice(c->device));
     ORBX_CUDA(c, cudaStreamSynchronize(c->stream));
     const Level &L = c->levels[level];
@@ -1878,7 +1910,7 @@ extern "C"
   int orbx_debug_level_selected(orbx_ctx *c, int image, int level, int32_t *xs, int32_t *ys, int32_t *scores, int cap, int32_t *n)
   {
     if (!c || !n || level < 0 || level >= c->cfg.n_levels || image < 0) return ORBX_ERR_INVALID_ARG;
-    if (image >= c->last_images) return fail(c, ORBX_ERR_STATE, "no image with that index has been processed");
+    if (int rc = require_images(c, image + 1LL)) return rc;
     ORBX_CUDA(c, cudaSetDevice(c->device));
     ORBX_CUDA(c, cudaStreamSynchronize(c->stream));
     const Level &L = c->levels[level];

@@ -223,12 +223,11 @@ struct BowArgs
   int *fv_nodes, *fv_start /* [frame][n_features + 1] */, *fv_feats, *n_fv;
 };
 
-// the BoW results of frame `frame0` onwards as serialiser inputs
-inline void ser_bow_inputs(SerArgs &s, const BowArgs &b, size_t frame0, size_t n_features)
+// the BoW results of b's frames as serialiser inputs (frame f of the launch = frame f of b)
+inline void ser_bow_inputs(SerArgs &s, const BowArgs &b)
 {
-  s.bow_ids = b.bow_ids + frame0 * n_features, s.bow_vals = b.bow_vals + frame0 * n_features, s.n_bow = b.n_bow + frame0;
-  s.fv_nodes = b.fv_nodes + frame0 * n_features, s.fv_start = b.fv_start + frame0 * (n_features + 1), s.fv_feats = b.fv_feats + frame0 * n_features;
-  s.n_fv = b.n_fv + frame0;
+  s.bow_ids = b.bow_ids, s.bow_vals = b.bow_vals, s.n_bow = b.n_bow;
+  s.fv_nodes = b.fv_nodes, s.fv_start = b.fv_start, s.fv_feats = b.fv_feats, s.n_fv = b.n_fv;
 }
 
 // launchers (orbx_kernels.cu / orbx_match.cu / orbx_serialize.cu / orbx_bow.cu); every call enqueues exactly one kernel on `s`

@@ -7,6 +7,22 @@
 
 #include "orbx_device.cuh"
 
+namespace orbx
+{
+// Device memory that grows on demand and is freed with its context.  reserve(c, want) makes `p` hold at least `want` bytes;
+// a buffer that has to grow is freed after a device synchronisation (work on any of the context's streams may still use it).
+struct DeviceBuffer
+{
+  uint8_t *p = nullptr;
+  size_t bytes = 0;
+  DeviceBuffer() = default;
+  DeviceBuffer(const DeviceBuffer &) = delete;
+  DeviceBuffer &operator=(const DeviceBuffer &) = delete;
+  ~DeviceBuffer() { if (p) cudaFree(p); }
+  int reserve(orbx_ctx *c, size_t want);
+};
+} // namespace orbx
+
 struct orbx_ctx
 {
   orbx_config cfg;
@@ -42,15 +58,13 @@ struct orbx_ctx
   cudaStream_t pipe[kPipeMax] = {};
   cudaEvent_t fork_ev = nullptr;
   cudaEvent_t join_ev[kPipeMax] = {};
-  // staging for the host-side matcher calls (orbx_search_in_area / orbx_verify_angle), grown on demand
-  uint8_t *match_scratch = nullptr;
-  size_t match_scratch_bytes = 0;
+  // staging for the host-side matcher and serialiser calls (orbx_search_in_area, orbx_serialize_keyframe, ...)
+  orbx::DeviceBuffer match_scratch;
   // bag-of-words transform: per-feature and per-frame result buffers, allocated on first use
   orbx::BowArgs bow{};
   bool bow_ready = false;
   // sequences (orbx_sequence.cu): per-slot record staging for host outputs, gathered arrays of single-rank calls
-  uint8_t *rec_staging = nullptr;
-  size_t rec_staging_bytes = 0;
+  orbx::DeviceBuffer rec_staging;
   struct orbx_comm *self_comm = nullptr;
   uint8_t *h_rec1 = nullptr; // pinned host record of the single-frame calls (one D2H copy instead of nine)
   // single-pair latency path: the launch sequence of one stereo frame captured once as a CUDA graph (orbx_set_graph)
@@ -65,11 +79,8 @@ struct orbx_ctx
   uint64_t bow_epoch = ~0ull; // frame_epoch at the last bag-of-words call
   int bow_frames = 0;         // frames covered by that call
   // keyframe records of sequences (orbx_sequence_stereo_keyframes): per-slot staging of records + poses for host outputs,
-  // and the sizes of a whole block (copied to the host once at the end)
-  uint8_t *kf_staging = nullptr;
-  size_t kf_staging_bytes = 0;
-  int64_t *kf_sizes = nullptr;
-  size_t kf_sizes_count = 0;
+  // and the int64 sizes of a whole block (copied to the host once at the end)
+  orbx::DeviceBuffer kf_staging, kf_sizes;
 };
 
 // DBoW3 vocabulary tree resident on one device
@@ -90,6 +101,10 @@ namespace orbx
 int fail(orbx_ctx *c, int code, const std::string &msg);
 // Params whose per-image buffers start at image `img0` (and per-frame buffers at frame `frame0`)
 Params params_at(const orbx_ctx *c, int img0, int frame0);
+// the same BowArgs with every per-frame buffer starting at frame `frame0` (N = n_features)
+BowArgs bow_at(const BowArgs &b, size_t frame0, size_t N);
+// SerArgs of a serialiser launch over device slots whose frame f reads image f * image_stride; no BoW inputs (ser_bow_inputs)
+SerArgs ser_args(const orbx_ctx *c, int image_stride, uint8_t *out, size_t stride, int64_t *sizes, uint64_t id0, const float *pose, int with_map_points);
 // Stereo input of n_frames frames (host memory, or device memory with `on_device`) streamed through the device slots in
 // chunks of c->chunk() frames.  Chunk k lives in slot k % n_slots and, with `piped`, runs on stream pipe[slot % kPipe]
 // after a fork from the context's stream; otherwise everything runs on the context's stream.  Per chunk: host frames are
@@ -99,15 +114,15 @@ Params params_at(const orbx_ctx *c, int img0, int frame0);
 using ChunkOut = std::function<int(cudaStream_t s, int d0, int64_t f0, int nf)>;
 int run_stereo_chunks(orbx_ctx *c, int64_t n_frames, const uint8_t *left, size_t left_stride, const uint8_t *right, size_t right_stride, size_t frame_stride,
                       bool on_device, bool piped, const ChunkOut &out);
-// per-frame records (orbx_record_layout) of device slots [d0, d0 + nf) assembled at d_rec; device staging for host outputs
+// per-frame records (orbx_record_layout) of device slots [d0, d0 + nf) assembled at d_rec
 int pack_frame_records(orbx_ctx *c, cudaStream_t s, int d0, int nf, uint8_t *d_rec, size_t rec_stride);
-int ensure_record_staging(orbx_ctx *c, size_t rec_stride);
 // frees the gathered arrays a context keeps for single-rank sequence calls
 void destroy_self_comm(orbx_ctx *c);
 // allocates the context's bag-of-words result buffers (n_img_max frames, as many as an RGB-D batch holds) on first use
 int bow_buffers(orbx_ctx *c);
-// c->bow with the vocabulary's tree, ready for launch_bow_descend / launch_bow_assemble
-BowArgs bow_args(const orbx_ctx *c, const orbx_vocab *v, int levelsup);
+// c->bow with the vocabulary's tree, ready for launch_bow_descend / launch_bow_assemble over device slots whose frame f
+// reads image f * image_stride
+BowArgs bow_args(const orbx_ctx *c, const orbx_vocab *v, int levelsup, int image_stride);
 
 } // namespace orbx
 

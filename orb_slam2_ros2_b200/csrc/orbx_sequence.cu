@@ -203,83 +203,31 @@ __global__ void __launch_bounds__(kPackThreads) pack_records_kernel(const Params
   }
 }
 
-int ensure_record_staging_impl(orbx_ctx *c, size_t rec_stride)
-{
-  const size_t want = (size_t)c->cfg.max_batch * rec_stride;
-  if (c->rec_staging && c->rec_staging_bytes >= want) return ORBX_OK;
-  if (c->rec_staging)
-  {
-    ORBX_CUDA(c, cudaDeviceSynchronize());
-    cudaFree(c->rec_staging);
-    c->rec_staging = nullptr;
-  }
-  ORBX_CUDA(c, cudaMalloc((void **)&c->rec_staging, want));
-  c->rec_staging_bytes = want;
-  return ORBX_OK;
-}
-
-// host-side keyframe outputs: per slot `stride` bytes of record + 12 floats of pose; the sizes of a whole block
-int ensure_keyframe_staging(orbx_ctx *c, size_t stride, int64_t n_local)
-{
-  const size_t want = (size_t)c->cfg.max_batch * (stride + 12 * sizeof(float));
-  const size_t n_sizes = (size_t)std::max<int64_t>(1, n_local);
-  if ((c->kf_staging && c->kf_staging_bytes < want) || (c->kf_sizes && c->kf_sizes_count < n_sizes)) ORBX_CUDA(c, cudaDeviceSynchronize());
-  if (c->kf_staging && c->kf_staging_bytes < want)
-  {
-    cudaFree(c->kf_staging);
-    c->kf_staging = nullptr;
-  }
-  if (!c->kf_staging)
-  {
-    ORBX_CUDA(c, cudaMalloc((void **)&c->kf_staging, want));
-    c->kf_staging_bytes = want;
-  }
-  if (c->kf_sizes && c->kf_sizes_count < n_sizes)
-  {
-    cudaFree(c->kf_sizes);
-    c->kf_sizes = nullptr;
-  }
-  if (!c->kf_sizes)
-  {
-    ORBX_CUDA(c, cudaMalloc((void **)&c->kf_sizes, n_sizes * sizeof(int64_t)));
-    c->kf_sizes_count = n_sizes;
-  }
-  return ORBX_OK;
-}
-
 // keyframe records of the chunk in device slots [d0, d0 + nf) = local frames [f0, f0 + nf), on the chunk's stream after its
-// pack kernel: bag-of-words descent + assembly into the slots' BoW buffers (with a vocabulary), then the serialiser
+// pack kernel: bag-of-words descent + assembly into the slots' BoW buffers (with a vocabulary), then the serialiser.  The
+// slots hold stereo frames (image stride 2) whatever the context's previous call left resident.
 int keyframe_chunk(orbx_ctx *c, const orbx_keyframe_io *kio, const Params &p, cudaStream_t s, size_t d0, int64_t f0, int nf, int64_t lo)
 {
-  const size_t N = (size_t)c->cfg.n_features, ks = kio->stride;
+  const size_t ks = kio->stride;
   const bool host = !kio->on_device;
-  uint8_t *stage = host ? c->kf_staging + d0 * ks : nullptr;
-  float *stage_pose = host ? reinterpret_cast<float *>(c->kf_staging + (size_t)c->cfg.max_batch * ks) + d0 * 12 : nullptr;
-  SerArgs sa{};
-  sa.out = host ? stage : kio->out + (size_t)f0 * ks;
-  sa.stride = ks;
-  sa.sizes = (long long *)(host ? c->kf_sizes : kio->sizes) + f0;
-  sa.id0 = kio->id0 + (uint64_t)(lo + f0);
-  sa.pose = nullptr;
+  // host outputs: per slot `ks` bytes of record, then per slot 12 floats of pose; the sizes of the whole block
+  uint8_t *stage = host ? c->kf_staging.p + d0 * ks : nullptr;
+  float *stage_pose = host ? reinterpret_cast<float *>(c->kf_staging.p + (size_t)c->cfg.max_batch * ks) + d0 * 12 : nullptr;
+  const float *pose = nullptr;
   if (kio->pose_rt)
   {
     if (host) ORBX_CUDA(c, cudaMemcpyAsync(stage_pose, kio->pose_rt + (size_t)f0 * 12, (size_t)nf * 12 * sizeof(float), cudaMemcpyHostToDevice, s));
-    sa.pose = host ? stage_pose : kio->pose_rt + (size_t)f0 * 12;
+    pose = host ? stage_pose : kio->pose_rt + (size_t)f0 * 12;
   }
-  sa.with_map_points = kio->with_map_points;
-  sa.image_stride = 2;
-  sa.max_u = c->max_u, sa.max_v = c->max_v, sa.min_u = c->min_u, sa.min_v = c->min_v;
+  SerArgs sa = ser_args(c, 2, host ? stage : kio->out + (size_t)f0 * ks, ks, (host ? reinterpret_cast<int64_t *>(c->kf_sizes.p) : kio->sizes) + f0,
+                        kio->id0 + (uint64_t)(lo + f0), pose, kio->with_map_points);
   if (kio->vocab)
   {
-    BowArgs ba = bow_args(c, kio->vocab, kio->levelsup);
-    ba.image_stride = 2;
-    ba.f_word += d0 * N, ba.f_nid += d0 * N, ba.f_weight += d0 * N; // the slots' own frames of the n_img_max-frame buffers
-    ba.bow_ids += d0 * N, ba.bow_vals += d0 * N, ba.n_bow += d0;
-    ba.fv_nodes += d0 * N, ba.fv_start += d0 * (N + 1), ba.fv_feats += d0 * N, ba.n_fv += d0;
+    const BowArgs ba = bow_at(bow_args(c, kio->vocab, kio->levelsup, 2), d0, (size_t)c->cfg.n_features);
     launch_bow_descend(p, ba, nf, s);
     launch_bow_assemble(p, ba, nf, s);
     c->launches += 2;
-    ser_bow_inputs(sa, ba, 0, N);
+    ser_bow_inputs(sa, ba);
   }
   launch_serialize(p, sa, nf, s);
   ++c->launches;
@@ -518,7 +466,7 @@ extern "C"
     const bool rec_dev = io->records && io->records_on_device, rec_host = io->records && !io->records_on_device;
     if (rec_host)
     {
-      int rc = ensure_record_staging_impl(c, rs);
+      int rc = c->rec_staging.reserve(c, (size_t)c->cfg.max_batch * rs);
       if (rc) return rc;
     }
     const size_t N = (size_t)c->cfg.n_features;
@@ -531,7 +479,8 @@ extern "C"
       if ((int64_t)kio->stride < (kf_bow ? orbx_serialized_capacity_bow(c) : orbx_serialized_capacity(c)))
         return fail(c, ORBX_ERR_CAPACITY, kf_bow ? "keyframe stride is smaller than orbx_serialized_capacity_bow()" : "keyframe stride is smaller than orbx_serialized_capacity()");
       int rc = kf_bow ? bow_buffers(c) : ORBX_OK;
-      if (!rc && kf_host) rc = ensure_keyframe_staging(c, kio->stride, n_local);
+      if (!rc && kf_host) rc = c->kf_staging.reserve(c, (size_t)c->cfg.max_batch * (kio->stride + 12 * sizeof(float)));
+      if (!rc && kf_host) rc = c->kf_sizes.reserve(c, (size_t)std::max<int64_t>(1, n_local) * sizeof(int64_t));
       if (rc) return rc;
     }
 
@@ -598,12 +547,12 @@ extern "C"
     // per chunk on its pipeline stream: pack -> record copy -> keyframe records -> the NCCL pieces it completes
     auto chunk_out = [&](cudaStream_t s, int d0, int64_t f0, int nf) -> int {
       const Params p = params_at(c, 2 * d0, d0);
-      pa.rec = rec_dev ? (uint8_t *)io->records + (size_t)f0 * rs : (rec_host ? c->rec_staging + (size_t)d0 * rs : nullptr);
+      pa.rec = rec_dev ? (uint8_t *)io->records + (size_t)f0 * rs : (rec_host ? c->rec_staging.p + (size_t)d0 * rs : nullptr);
       pa.gframe0 = me * block + f0;
       pack_records_kernel<<<dim3(kPackBlocksPerFrame, nf), kPackThreads, 0, s>>>(p, pa);
       ++c->launches;
       ORBX_CUDA(c, cudaGetLastError());
-      if (rec_host) ORBX_CUDA(c, cudaMemcpyAsync((uint8_t *)io->records + (size_t)f0 * rs, c->rec_staging + (size_t)d0 * rs, rs * nf, cudaMemcpyDeviceToHost, s));
+      if (rec_host) ORBX_CUDA(c, cudaMemcpyAsync((uint8_t *)io->records + (size_t)f0 * rs, c->rec_staging.p + (size_t)d0 * rs, rs * nf, cudaMemcpyDeviceToHost, s));
       if (kio)
       {
         int rc = keyframe_chunk(c, kio, p, s, d0, f0, nf, lo);
@@ -633,7 +582,7 @@ extern "C"
         ORBX_NCCL(c, nccl().AllReduce(m->d_flag, m->d_flag + 1, 1, kNcclInt32, kNcclSum, m->nccl_comm, m->comm_stream));
       ORBX_CUDA(c, cudaStreamSynchronize(m->comm_stream));
     }
-    if (kf_host && n_local > 0) ORBX_CUDA(c, cudaMemcpy(kio->sizes, c->kf_sizes, (size_t)n_local * sizeof(int64_t), cudaMemcpyDeviceToHost));
+    if (kf_host && n_local > 0) ORBX_CUDA(c, cudaMemcpy(kio->sizes, c->kf_sizes.p, (size_t)n_local * sizeof(int64_t), cudaMemcpyDeviceToHost));
     if (io->gathered_desc_host) ORBX_CUDA(c, cudaMemcpy(io->gathered_desc_host, m->g.desc(), (size_t)F * N * 32, cudaMemcpyDeviceToHost));
     if (io->gathered_n_host) ORBX_CUDA(c, cudaMemcpy(io->gathered_n_host, m->g.n(), (size_t)F * 4, cudaMemcpyDeviceToHost));
 
@@ -668,8 +617,6 @@ int pack_frame_records(orbx_ctx *c, cudaStream_t s, int d0, int nf, uint8_t *d_r
   ORBX_CUDA(c, cudaGetLastError());
   return ORBX_OK;
 }
-
-int ensure_record_staging(orbx_ctx *c, size_t rec_stride) { return ensure_record_staging_impl(c, rec_stride); }
 
 void destroy_self_comm(orbx_ctx *c)
 {
