@@ -652,6 +652,17 @@ int oracle_search_by_stereo(const oracle_pyramid *left, const oracle_pyramid *ri
     if (best_d > 75) continue; /* mnMeanThreshold :1088 */
     const oracle_keypoint *rk = &kr[best_j];
     if (lk->octave > rk->octave + 1 || lk->octave < rk->octave - 1) continue;
+    /* Drop the match when the left 11x11 window or the right 11x21 window (11 shifts of 11 columns) leaves its level
+     * image, as stereo_kernel does: the reference throws in cv::Mat::rowRange there (DESIGN section 2).  Only undistorted
+     * left keypoints can get that close to the border. */
+    {
+      int lo = lk->octave, ro = rk->octave;
+      int lx = cv_floor_f(lk->x / left->sf[lo]), ly = cv_floor_f(lk->y / left->sf[lo]);
+      int rx = cv_floor_f(rk->x / right->sf[ro]), ry = cv_floor_f(rk->y / right->sf[ro]);
+      if (lx - 5 < 0 || ly - 5 < 0 || lx + 5 >= left->w[lo] || ly + 5 >= left->h[lo] || rx - 10 < 0 || ry - 5 < 0 || rx + 10 >= right->w[ro] ||
+          ry + 5 >= right->h[ro])
+        continue;
+    }
     float dU = pixel_sad_match(left, right, lk, rk);
     float rightU = rk->x + dU;
     rightU = rightU > 0.f ? rightU : 0.f;

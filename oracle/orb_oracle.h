@@ -88,7 +88,8 @@ int oracle_extract(const oracle_pyramid *p, int ini_th, int min_th, const float 
                    uint8_t *desc, double *angles_rad, int *level_counts /*[n_levels] optional*/);
 
 /* ---- stereo / RGB-D association ---- */
-/* src/ORBMatcher.cc:18-81 (+ :841-1011). kps_left are the (undistorted) left keypoints. Returns nMatches. */
+/* src/ORBMatcher.cc:18-81 (+ :841-1011). kps_left are the (undistorted) left keypoints. Returns nMatches.  A match whose
+ * SAD window leaves its level image is dropped, where the reference throws (DESIGN section 2). */
 int oracle_search_by_stereo(const oracle_pyramid *left, const oracle_pyramid *right, const oracle_keypoint *kl,
                             const uint8_t *dl, int nl, const oracle_keypoint *kr, const uint8_t *dr, int nr, float fx,
                             float bf, double *u_right, double *depth, int *match_idx /*optional [nl]*/);
