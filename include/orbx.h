@@ -374,6 +374,52 @@ int orbx_vocab_load_text(orbx_ctx *ctx, const char *path, orbx_vocab **out);
 void orbx_vocab_destroy(orbx_vocab *vocab);
 int orbx_vocab_info(const orbx_vocab *vocab, int32_t *k, int32_t *L, int32_t *n_nodes, int32_t *n_words);
 
+/* The nodes as text-format records (record i = node i + 1; n_nodes - 1 of them, orbx_vocab_info): parent, is_leaf, desc [32]
+ * and weight.  Any array may be NULL. */
+int orbx_vocab_arrays(const orbx_vocab *vocab, int32_t *parent, uint8_t *is_leaf, uint8_t *desc, double *weight);
+/* writes what ORB-SLAM2's TemplatedVocabulary::saveToTextFile writes and orbx_vocab_load_text reads: "k L  scoring weighting",
+ * then per node "parent isLeaf d0 .. d31  weight" (FORB::toString puts a blank after every byte; the weight as the stream's
+ * default "%g", 6 significant digits, as in orbx_serialize_keyframe_text).  ORBX_ERR_FILE_NOT_OPEN if it cannot be written. */
+int orbx_vocab_save_text(const orbx_vocab *vocab, const char *path);
+
+/* ---- vocabulary construction on the device ------------------------------------------------------------------- */
+/* replaces: DBoW2 / DBoW3 TemplatedVocabulary::create (HKmeansStep, initiateClustersKMpp, FORB::meanValue, createWords,
+ * setNodeWeights), the step that makes the ORBvoc.txt the reference loads (src/System.cc:93), from the training set
+ * desc[f][i] (i < n_kps[f]) -- the layout of orbx_sequence_result.gathered_desc / gathered_n and orbx_device_results.desc /
+ * n_kps.  Parity unpinned (DBoW is not vendored); the rules, which tests/vocab_build_oracle.c restates:
+ *   recursion  from the root with every training descriptor; a node of n <= k descriptors gets one child per descriptor,
+ *              otherwise k-means; children in cluster order, a child's members in their order in the parent's list; a
+ *              child is split again when its level < L and it holds more than one descriptor (else it is a leaf)
+ *   seeding    k-means++ with integer distances: first centre = descriptor r_0 % n; after every centre min_dist[i] drops
+ *              to the Hamming distance to it, S = sum min_dist; S == 0 stops with fewer than k centres, else the next
+ *              centre is the first i whose running sum reaches 1 + r_j % S
+ *   randomness counter-based, independent of the order nodes are processed in: root key = splitmix64(seed), child c of a
+ *              node with key K gets splitmix64(K + c + 1), draw j of a node is splitmix64(K ^ (j * 0x9E3779B97F4A7C15))
+ *   assignment nearest centre by Hamming distance, the first among equals
+ *   mean       bit b set iff at least ceil(m/2) of the m members have it; an empty cluster keeps its centre
+ *   stop       when no assignment changes, or after ORBX_VOCAB_MAX_ITERS assignment passes (the node is "capped")
+ *   ids        DBoW's creation order: a node's children get consecutive ids, nodes are split depth first; word ids go to the
+ *              leaves in id order
+ *   weights    TF_IDF: N = n_frames, N_i = frames with a descriptor whose descent (orbx_bow_transform's) ends at word i,
+ *              weight = log(N / N_i) in double, 0 when N_i = 0
+ * The result lives on ctx like a loaded vocabulary.  Blocks until it is built. */
+#define ORBX_VOCAB_MAX_ITERS 100 /* DBoW2 iterates without a bound; a cycle of assignments cannot spin here */
+#define ORBX_VOCAB_MAX_K 32      /* branching factors up to this (ORBvoc.txt: 10) */
+typedef struct orbx_vocab_train {
+  const uint8_t *desc;    /* [n_frames][stride][32] */
+  const int32_t *n_kps;   /* [n_frames], each 0..stride */
+  int32_t n_frames;       /* the N of TF_IDF: pass F, not the padded row count of a gather */
+  int32_t stride;         /* descriptors per frame row (1..65535) */
+  int32_t on_device;      /* 1: desc / n_kps are device memory of ctx's device (e.g. the gathered arrays), 0: host */
+  int32_t k, L;           /* branching factor (2..ORBX_VOCAB_MAX_K) and depth levels (>= 1; at most INT32_MAX nodes) */
+  uint64_t seed;
+  int32_t *iters;         /* optional host [L]: the most assignment passes a k-means node of each level took */
+  int32_t *n_capped;      /* optional host: nodes that stopped at ORBX_VOCAB_MAX_ITERS */
+  float *level_ms;        /* optional host [L + 1]: CUDA-event time of each level, then of the TF_IDF step */
+} orbx_vocab_train;
+/* ORBX_ERR_INVALID_ARG for bad k / L / sizes (before anything is enqueued), counts outside 0..stride or no descriptor at all */
+int orbx_vocab_build(orbx_ctx *ctx, const orbx_vocab_train *in, orbx_vocab **out);
+
 /* replaces: VirtualFrame::computeBow (include/ORB_SLAM2/Frame.h:224-231) = DBoW3::Vocabulary::transform(mvLeftDescriptor,
  * mBowVec, mFeatVec, levelsup = 4) for frame `frame` of the most recent stereo / RGB-D call.
  * BowVector (std::map<WordId, WordValue>): bow_ids ascending with their L1-normalised weights, *n_bow entries.

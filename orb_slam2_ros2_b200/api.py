@@ -82,7 +82,7 @@ EXPORTS = [
     "orbx_frame_epoch", "orbx_set_graph", "orbx_debug_quadtree_stats", "orbx_frame_range", "orbx_comm_unique_id", "orbx_comm_create", "orbx_comm_ipc_handle", "orbx_comm_open_peers",
     "orbx_comm_create_local", "orbx_comm_destroy", "orbx_comm_info", "orbx_record_layout_get", "orbx_sequence_stereo",
     "orbx_serialized_capacity_bow", "orbx_serialize_keyframe_bow", "orbx_serialize_keyframes_bow_device", "orbx_keyframe_list_head",
-    "orbx_keyframe_list_entry_prefix", "orbx_sequence_stereo_keyframes",
+    "orbx_keyframe_list_entry_prefix", "orbx_sequence_stereo_keyframes", "orbx_vocab_build", "orbx_vocab_save_text", "orbx_vocab_arrays",
 ]
 
 class OrbxRecordLayout(C.Structure):
@@ -104,6 +104,14 @@ class OrbxSequenceResult(C.Structure):
 class OrbxKeyframeIO(C.Structure):
     _fields_ = [("vocab", C.c_void_p), ("levelsup", C.c_int32), ("with_map_points", C.c_int32), ("id0", C.c_uint64), ("pose_rt", C.c_void_p),
                 ("on_device", C.c_int32), ("out", C.c_void_p), ("stride", C.c_size_t), ("sizes", C.c_void_p)]
+
+
+VOCAB_MAX_ITERS, VOCAB_MAX_K = 100, 32  # ORBX_VOCAB_MAX_ITERS / ORBX_VOCAB_MAX_K
+
+
+class OrbxVocabTrain(C.Structure):
+    _fields_ = [("desc", C.c_void_p), ("n_kps", C.c_void_p), ("n_frames", C.c_int32), ("stride", C.c_int32), ("on_device", C.c_int32), ("k", C.c_int32),
+                ("L", C.c_int32), ("seed", C.c_uint64), ("iters", C.c_void_p), ("n_capped", C.c_void_p), ("level_ms", C.c_void_p)]
 
 
 class OrbxDeviceBow(C.Structure):
@@ -201,6 +209,9 @@ def load_library(build_if_missing: bool = True):
     L.orbx_keyframe_list_head.argtypes = [vp, C.c_uint64, vp, sz, C.POINTER(C.c_int64)]
     L.orbx_keyframe_list_entry_prefix.argtypes = [C.c_int64, vp]
     L.orbx_sequence_stereo_keyframes.argtypes = [vp, vp, C.c_int64, C.POINTER(OrbxSequenceIO), C.POINTER(OrbxKeyframeIO), C.POINTER(OrbxSequenceResult)]
+    L.orbx_vocab_build.argtypes = [vp, C.POINTER(OrbxVocabTrain), C.POINTER(vp)]
+    L.orbx_vocab_save_text.argtypes = [vp, C.c_char_p]
+    L.orbx_vocab_arrays.argtypes = [vp, vp, vp, vp, vp]
     _lib = L
     return L
 
@@ -1015,6 +1026,48 @@ class Vocabulary:
         self._h = C.c_void_p()
         _check(ctx._h, self._L.orbx_vocab_load_text(ctx._h, path.encode(), C.byref(self._h)), "orbx_vocab_load_text")
         return self
+
+    @classmethod
+    def build(cls, ctx: Context, desc, counts, n_frames: int | None = None, k: int = 10, L: int = 6, seed: int = 0, stride: int | None = None,
+              stats: dict | None = None) -> "Vocabulary":
+        """DBoW TemplatedVocabulary::create on the device (orbx_vocab_build) from the training set desc[f][i], i < counts[f].
+        desc / counts: numpy arrays ((F, stride, 32) uint8 and (F,) int32), or device pointers (ints) of ctx's device, e.g.
+        OrbxSequenceResult.gathered_desc / gathered_n, which then need n_frames (the sequence's F: padding rows are not
+        frames) and stride (its n_features).  stats, if given, receives iters (per level), n_capped and level_ms (device time
+        per level, then of the TF_IDF step)."""
+        self = cls.__new__(cls)
+        self._L = ctx._L
+        self._h = C.c_void_p()
+        on_device = isinstance(desc, int)
+        if on_device:
+            assert isinstance(counts, int) and n_frames is not None and stride is not None, "device pointers need n_frames and stride"
+            F, S, dp, cp = int(n_frames), int(stride), desc, counts
+        else:
+            d = np.ascontiguousarray(desc, np.uint8)
+            assert d.ndim == 3 and d.shape[2] == 32
+            F = d.shape[0] if n_frames is None else int(n_frames)
+            S = d.shape[1]
+            d = np.ascontiguousarray(d[:F])
+            cnt = np.ascontiguousarray(np.asarray(counts)[:F], np.int32)
+            assert len(cnt) == F
+            dp, cp = d.ctypes.data, cnt.ctypes.data
+        iters, capped, ms = np.zeros(max(int(L), 1), np.int32), C.c_int32(0), np.zeros(max(int(L), 1) + 1, np.float32)
+        tr = OrbxVocabTrain(dp, cp, F, S, int(on_device), int(k), int(L), int(seed) & (2**64 - 1), iters.ctypes.data, C.addressof(capped), ms.ctypes.data)
+        _check(ctx._h, self._L.orbx_vocab_build(ctx._h, C.byref(tr), C.byref(self._h)), "orbx_vocab_build")
+        if stats is not None:
+            stats.update(iters=iters[: int(L)].tolist(), n_capped=int(capped.value), level_ms=ms[: int(L) + 1].tolist())
+        return self
+
+    def save_text(self, path: str):
+        """ORBvoc.txt text format (TemplatedVocabulary::saveToTextFile), readable by load_text"""
+        _check(None, self._L.orbx_vocab_save_text(self._h, path.encode()), f"orbx_vocab_save_text {path!r}")
+
+    def arrays(self) -> dict:
+        """the nodes as text-format records (record i = node i + 1): parent, is_leaf, desc (n, 32), weight"""
+        n = self.info()["n_nodes"] - 1
+        par, leaf, desc, w = np.zeros(n, np.int32), np.zeros(n, np.uint8), np.zeros((n, 32), np.uint8), np.zeros(n, np.float64)
+        _check(None, self._L.orbx_vocab_arrays(self._h, par.ctypes.data, leaf.ctypes.data, desc.ctypes.data, w.ctypes.data), "orbx_vocab_arrays")
+        return dict(parent=par, is_leaf=leaf, desc=desc, weight=w)
 
     def info(self):
         v = [C.c_int32() for _ in range(4)]

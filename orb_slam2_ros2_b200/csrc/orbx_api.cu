@@ -500,6 +500,13 @@ BowArgs bow_args(const orbx_ctx *c, const orbx_vocab *v, int levelsup, int image
   return a;
 }
 
+void append_g(std::string &t, double v)
+{
+  char buf[64];
+  t.append(buf, (size_t)std::snprintf(buf, sizeof(buf), "%g", v));
+  t.push_back(' ');
+}
+
 BowArgs bow_at(const BowArgs &b, size_t frame0, size_t N)
 {
   BowArgs a = b;
@@ -1625,10 +1632,7 @@ extern "C"
     std::string t;
     t.reserve((size_t)n * 200 + 256);
     char buf[64];
-    auto num = [&](double v) { // std::ostream << float / double: "%g", 6 significant digits
-      t.append(buf, (size_t)std::snprintf(buf, sizeof(buf), "%g", v));
-      t.push_back(' ');
-    };
+    auto num = [&](double v) { append_g(t, v); };
     auto integer = [&](long long v) {
       t.append(buf, (size_t)std::snprintf(buf, sizeof(buf), "%lld", v));
       t.push_back(' ');
@@ -1712,6 +1716,11 @@ extern "C"
     ORBX_CUDA(c, cudaSetDevice(c->device));
     orbx_vocab *v = new orbx_vocab();
     v->ctx = c, v->device = c->device, v->k = k, v->L = L, v->n_nodes = n, v->n_words = n_words;
+    v->rec_parent.assign(parent, parent + n_records);
+    v->rec_leaf.resize((size_t)n_records);
+    for (int i = 0; i < n_records; ++i) v->rec_leaf[(size_t)i] = is_leaf[i] != 0;
+    v->rec_desc.assign(desc, desc + (size_t)n_records * 32);
+    v->rec_weight.assign(weight, weight + n_records);
     auto up = [&](auto **dst, const auto &src) -> cudaError_t {
       cudaError_t e = cudaMalloc((void **)dst, src.size() * sizeof(src[0]) + 64);
       if (e != cudaSuccess) return e;
@@ -1771,7 +1780,47 @@ extern "C"
       weight.push_back(w);
     }
     if (parent.empty()) return fail(c, ORBX_ERR_INVALID_ARG, "vocabulary holds no nodes");
-    return orbx_vocab_create(c, k, L, (int)parent.size(), parent.data(), leaf.data(), desc.data(), weight.data(), out);
+    const int rc = orbx_vocab_create(c, k, L, (int)parent.size(), parent.data(), leaf.data(), desc.data(), weight.data(), out);
+    if (rc == ORBX_OK) (*out)->scoring = scoring, (*out)->weighting = weighting;
+    return rc;
+  }
+
+  int orbx_vocab_arrays(const orbx_vocab *v, int32_t *parent, uint8_t *is_leaf, uint8_t *desc, double *weight)
+  {
+    if (!v) return ORBX_ERR_INVALID_ARG;
+    const size_t n = v->rec_parent.size();
+    if (parent) std::memcpy(parent, v->rec_parent.data(), n * sizeof(int32_t));
+    if (is_leaf) std::memcpy(is_leaf, v->rec_leaf.data(), n);
+    if (desc) std::memcpy(desc, v->rec_desc.data(), n * 32);
+    if (weight) std::memcpy(weight, v->rec_weight.data(), n * sizeof(double));
+    return ORBX_OK;
+  }
+
+  int orbx_vocab_save_text(const orbx_vocab *v, const char *path)
+  {
+    if (!v || !path) return ORBX_ERR_INVALID_ARG;
+    // TemplatedVocabulary::saveToTextFile of ORB-SLAM2: "k L  scoring weighting", then per node
+    // "parent isLeaf " + FORB::toString (every byte followed by a blank) + " " + weight
+    std::string t;
+    t.reserve(v->rec_parent.size() * 140 + 32);
+    t += std::to_string(v->k) + " " + std::to_string(v->L) + "  " + std::to_string(v->scoring) + " " + std::to_string(v->weighting) + "\n";
+    for (size_t i = 0; i < v->rec_parent.size(); ++i)
+    {
+      t += std::to_string(v->rec_parent[i]);
+      t += v->rec_leaf[i] ? " 1 " : " 0 ";
+      for (int b = 0; b < 32; ++b)
+      {
+        t += std::to_string((int)v->rec_desc[i * 32 + (size_t)b]);
+        t.push_back(' ');
+      }
+      t.push_back(' ');
+      append_g(t, v->rec_weight[i]);
+      t.back() = '\n';
+    }
+    FILE *f = std::fopen(path, "wb");
+    if (!f) return ORBX_ERR_FILE_NOT_OPEN;
+    const bool ok = std::fwrite(t.data(), 1, t.size(), f) == t.size();
+    return (std::fclose(f) == 0 && ok) ? ORBX_OK : ORBX_ERR_FILE_NOT_OPEN;
   }
 
   int orbx_vocab_info(const orbx_vocab *v, int32_t *k, int32_t *L, int32_t *n_nodes, int32_t *n_words)

@@ -8,6 +8,8 @@
 //   bow_assemble_kernel  one CTA per frame: BowVector (std::map<WordId, double>: ids ascending, weights accumulated in
 //                        feature order, then L1-normalised with the sum taken in id order) and FeatureVector
 //                        (std::map<NodeId, vector<unsigned>>) from two stable sorts of (key << 16 | feature index)
+//   bow_word_frames_kernel  one CTA per frame: the frame's distinct words (the same sort), one integer atomic per word;
+//                        N_i of TF_IDF for orbx_vocab_build (setNodeWeights)
 #include "orbx_device.cuh"
 
 namespace orbx
@@ -205,6 +207,21 @@ __global__ void __launch_bounds__(kAsmThreads) bow_assemble_kernel(const Params 
   }
 }
 
+// N_i of setNodeWeights: n_frames_of_word[w] += 1 for every distinct word w among the frame's descents (f_word)
+__global__ void __launch_bounds__(kAsmThreads) bow_word_frames_kernel(const Params p, const BowArgs a, int P, int *n_frames_of_word)
+{
+  extern __shared__ unsigned long long s_key[]; // [P]
+  __shared__ int s_warp[kAsmThreads / 32];
+  const int frame = blockIdx.x;
+  const int n = min(p.n_kps[frame * a.image_stride], P);
+  const int *f_word = a.f_word + (size_t)frame * p.n_features;
+  for (int i = threadIdx.x; i < P; i += kAsmThreads)
+    s_key[i] = i < n ? ((unsigned long long)(unsigned)f_word[i] << 16) | (unsigned long long)i : ~0ull;
+  __syncthreads();
+  bitonic_sort(s_key, P);
+  for_each_head(s_key, n, P, s_warp, [&](int, int j) { atomicAdd(&n_frames_of_word[s_key[j] >> 16], 1); });
+}
+
 } // namespace
 
 void launch_bow_descend(const Params &p, const BowArgs &a, int n_frames, cudaStream_t s)
@@ -226,12 +243,19 @@ void launch_bow_assemble(const Params &p, const BowArgs &a, int n_frames, cudaSt
   bow_assemble_kernel<<<n_frames, kAsmThreads, (size_t)P * sizeof(unsigned long long), s>>>(p, a, P);
 }
 
+void launch_bow_word_frames(const Params &p, const BowArgs &a, int n_frames, int *n_frames_of_word, cudaStream_t s)
+{
+  const int P = bow_sort_size(p.n_features);
+  bow_word_frames_kernel<<<n_frames, kAsmThreads, (size_t)P * sizeof(unsigned long long), s>>>(p, a, P, n_frames_of_word);
+}
+
 int bow_configure(int n_features)
 {
   const size_t bytes = (size_t)bow_sort_size(n_features) * sizeof(unsigned long long);
   if (bytes <= 48 * 1024) return 0;
-  static SmemOptIn state;
-  return raise_dynamic_smem(bow_assemble_kernel, state, bytes);
+  static SmemOptIn state, state_words;
+  if (raise_dynamic_smem(bow_assemble_kernel, state, bytes)) return -1;
+  return raise_dynamic_smem(bow_word_frames_kernel, state_words, bytes);
 }
 
 } // namespace orbx

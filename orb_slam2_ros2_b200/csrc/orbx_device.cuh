@@ -249,7 +249,8 @@ void launch_bow_match(const BowMatchArgs &a, cudaStream_t s);
 void launch_serialize(const Params &p, const SerArgs &a, int n_frames, cudaStream_t s);
 void launch_bow_descend(const Params &p, const BowArgs &a, int n_frames, cudaStream_t s);
 void launch_bow_assemble(const Params &p, const BowArgs &a, int n_frames, cudaStream_t s);
-int bow_configure(int n_features); // opt in to the dynamic shared memory of the assemble kernel
+void launch_bow_word_frames(const Params &p, const BowArgs &a, int n_frames, int *n_frames_of_word, cudaStream_t s);
+int bow_configure(int n_features); // opt in to the dynamic shared memory of the assemble and word-frame kernels
 size_t quadtree_smem_bytes(int list_cap, int node_cap, int big_cap, int max_level_cells);
 int quadtree_configure(size_t smem_bytes); // opt in to large dynamic shared memory
 

@@ -89,9 +89,14 @@ struct orbx_vocab
   const orbx_ctx *ctx = nullptr; // the context that created it
   int device = 0;
   int k = 0, L = 0, n_nodes = 0, n_words = 0;
+  int scoring = 0, weighting = 0; // DBoW3 ScoringType / WeightingType of the text header (0 = L1_NORM / TF_IDF)
   int *child_start = nullptr, *child_ids = nullptr, *word = nullptr;
   uint8_t *desc = nullptr;
   double *weight = nullptr;
+  // the text format's records (record i = node i + 1), kept on the host for orbx_vocab_save_text / orbx_vocab_arrays
+  std::vector<int32_t> rec_parent;
+  std::vector<uint8_t> rec_leaf, rec_desc;
+  std::vector<double> rec_weight;
 };
 
 namespace orbx
@@ -123,6 +128,8 @@ int bow_buffers(orbx_ctx *c);
 // c->bow with the vocabulary's tree, ready for launch_bow_descend / launch_bow_assemble over device slots whose frame f
 // reads image f * image_stride
 BowArgs bow_args(const orbx_ctx *c, const orbx_vocab *v, int levelsup, int image_stride);
+// appends `v` as std::ostream << double prints it by default ("%g": 6 significant digits) and a blank
+void append_g(std::string &t, double v);
 
 } // namespace orbx
 
