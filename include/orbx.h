@@ -456,6 +456,51 @@ int orbx_search_by_bow(orbx_ctx *ctx, int frame, int n_kf_nodes, const int32_t *
                        const uint8_t *frame_cand_ok, int32_t *best_idx, int32_t *best_dist, float *ratio,
                        int32_t *n_candidates);
 
+/* ---- keyframe database: loop / relocalisation candidates over a sequence ----------------------------------------- */
+/* replaces: the first stage of KeyFrameDatabase::DetectLoopCandidates / DetectRelocalizationCandidates (ORB-SLAM2
+ * KeyFrameDatabase.cc): the BoW inverted file and DBoW's L1 score, for a database built once from the descriptors of a
+ * sequence desc[f][i] (i < n_kps[f]) -- the layout of orbx_sequence_result.gathered_desc / gathered_n, orbx_device_results.desc
+ * / n_kps and orbx_vocab_train.  Parity unpinned (DBoW3 and the reference's KeyFrameDatabase are not vendored); the rules,
+ * which tests/bowdb_oracle.c restates:
+ *   database   frame f's BowVector is orbx_bow_transform's for its descriptors with `vocab` (ascending word ids, L1-normalised,
+ *              stopped words left out); the inverted file lists, per word, the frames whose BowVector holds it
+ *   connected  a range query q excludes itself and every g with |g - q| <= exclude_window (standing in for the covisibility
+ *              set); the resident-frame query excludes nothing
+ *   sharing    the other frames that share at least one word with the query; common = number of shared words;
+ *              min_common = (int)((float)max_common * 0.8f); frames with common > min_common are scored (n_scored)
+ *   score      DBoW3 L1Scoring::score(v1 = query, v2 = candidate): over the shared words in ascending id, the double chain
+ *              score += fabs(vi - wi) - fabs(vi) - fabs(wi), then si = (float)(-score / 2.0)
+ *   kept       si >= min_score (n_kept); the output is the first top_k of them by score descending, then frame ascending,
+ *              each with (frame, si, common); slots past n_kept get frame -1, score 0, common 0.  No sharing frame: every
+ *              count is 0.
+ * The covisibility accumulation that follows in the reference needs the map graph and is not part of this stage. */
+#define ORBX_BOWDB_MAX_FRAMES 98304 /* 16-bit shared-word counters of every frame in the query kernel's shared memory: 192 KB */
+typedef struct orbx_bowdb orbx_bowdb;
+/* n_frames: the sequence's F (not the padded row count of a gather), 1..ORBX_BOWDB_MAX_FRAMES (ORBX_ERR_CAPACITY above);
+ * stride: descriptors per frame row (1..65535); counts 0..stride; on_device: desc / n_kps are device memory of ctx's device.
+ * vocab must belong to ctx.  Blocks until the database is built; leaves the context's resident frames, their bag of words and
+ * the frame epoch untouched. */
+int orbx_bowdb_build(orbx_ctx *ctx, const orbx_vocab *vocab, const uint8_t *desc /* [n_frames][stride][32] */, const int32_t *n_kps /* [n_frames] */,
+                     int32_t n_frames, int32_t stride, int32_t on_device, orbx_bowdb **out);
+void orbx_bowdb_destroy(orbx_bowdb *db);
+int orbx_bowdb_info(const orbx_bowdb *db, int32_t *n_frames, int32_t *n_words, int64_t *n_postings);
+typedef struct orbx_bowdb_io {
+  int32_t exclude_window; /* >= 0 for range queries; -1 for the resident-frame query */
+  float min_score;        /* not NaN */
+  int32_t top_k;          /* 1 .. n_frames */
+  int32_t on_device;      /* where the outputs live: device = asynchronous on ctx's stream, host = the call blocks */
+  int32_t *cand_frame;    /* [n_queries][top_k]; any output may be NULL */
+  float *cand_score;
+  int32_t *cand_common;
+  int32_t *n_sharing, *max_common, *n_scored, *n_kept; /* [n_queries] */
+} orbx_bowdb_io;
+/* queries q_lo .. q_hi - 1 (0 <= q_lo <= q_hi <= n_frames) with their own BowVectors.  Sharded: every rank builds the whole
+ * database from its gathered arrays and queries its block orbx_frame_range(F, rank, world). */
+int orbx_bowdb_query_range(orbx_ctx *ctx, const orbx_bowdb *db, int64_t q_lo, int64_t q_hi, const orbx_bowdb_io *io);
+/* relocalisation: the query is frame `frame` of the context's most recent call, whose BowVector must be resident from
+ * orbx_bow_transform* with the database's vocabulary (ORBX_ERR_STATE otherwise, or once the frame epoch has moved on) */
+int orbx_bowdb_query_frame(orbx_ctx *ctx, const orbx_bowdb *db, int frame, const orbx_bowdb_io *io);
+
 /* ---- introspection for benchmarks / profiles ----------------------------------------------------------- */
 #define ORBX_N_STAGES 7
 /* Same work as orbx_stereo_batch_device, with a CUDA event recorded on the stream after every kernel; blocks until

@@ -83,6 +83,7 @@ EXPORTS = [
     "orbx_comm_create_local", "orbx_comm_destroy", "orbx_comm_info", "orbx_record_layout_get", "orbx_sequence_stereo",
     "orbx_serialized_capacity_bow", "orbx_serialize_keyframe_bow", "orbx_serialize_keyframes_bow_device", "orbx_keyframe_list_head",
     "orbx_keyframe_list_entry_prefix", "orbx_sequence_stereo_keyframes", "orbx_vocab_build", "orbx_vocab_save_text", "orbx_vocab_arrays",
+    "orbx_bowdb_build", "orbx_bowdb_destroy", "orbx_bowdb_info", "orbx_bowdb_query_range", "orbx_bowdb_query_frame",
 ]
 
 class OrbxRecordLayout(C.Structure):
@@ -117,6 +118,15 @@ class OrbxVocabTrain(C.Structure):
 class OrbxDeviceBow(C.Structure):
     _fields_ = [("bow_ids", C.c_void_p), ("bow_vals", C.c_void_p), ("n_bow", C.c_void_p), ("fv_nodes", C.c_void_p), ("fv_start", C.c_void_p),
                 ("fv_feats", C.c_void_p), ("n_fv_nodes", C.c_void_p), ("stride", C.c_int32)]
+
+
+BOWDB_MAX_FRAMES = 98304  # ORBX_BOWDB_MAX_FRAMES
+
+
+class OrbxBowdbIO(C.Structure):
+    _fields_ = [("exclude_window", C.c_int32), ("min_score", C.c_float), ("top_k", C.c_int32), ("on_device", C.c_int32), ("cand_frame", C.c_void_p),
+                ("cand_score", C.c_void_p), ("cand_common", C.c_void_p), ("n_sharing", C.c_void_p), ("max_common", C.c_void_p), ("n_scored", C.c_void_p),
+                ("n_kept", C.c_void_p)]
 
 
 _lib = None
@@ -212,6 +222,12 @@ def load_library(build_if_missing: bool = True):
     L.orbx_vocab_build.argtypes = [vp, C.POINTER(OrbxVocabTrain), C.POINTER(vp)]
     L.orbx_vocab_save_text.argtypes = [vp, C.c_char_p]
     L.orbx_vocab_arrays.argtypes = [vp, vp, vp, vp, vp]
+    L.orbx_bowdb_build.argtypes = [vp, vp, vp, vp, C.c_int32, C.c_int32, C.c_int32, C.POINTER(vp)]
+    L.orbx_bowdb_destroy.argtypes = [vp]
+    L.orbx_bowdb_destroy.restype = None
+    L.orbx_bowdb_info.argtypes = [vp, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int64)]
+    L.orbx_bowdb_query_range.argtypes = [vp, vp, C.c_int64, C.c_int64, C.POINTER(OrbxBowdbIO)]
+    L.orbx_bowdb_query_frame.argtypes = [vp, vp, C.c_int, C.POINTER(OrbxBowdbIO)]
     _lib = L
     return L
 
@@ -1077,6 +1093,87 @@ class Vocabulary:
     def close(self):
         if getattr(self, "_h", None):
             self._L.orbx_vocab_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+BOWDB_OUTPUTS = ("cand_frame", "cand_score", "cand_common", "n_sharing", "max_common", "n_scored", "n_kept")
+
+
+class BowDatabase:
+    """Keyframe database over a sequence (orbx_bowdb_*): the BoW inverted file and the first stage of ORB-SLAM2's
+    KeyFrameDatabase::DetectLoopCandidates / DetectRelocalizationCandidates, built once on a context's device."""
+
+    @classmethod
+    def build(cls, ctx: Context, vocab: Vocabulary, desc, counts, n_frames: int | None = None, stride: int | None = None) -> "BowDatabase":
+        """from the descriptors desc[f][i], i < counts[f]: numpy arrays ((F, stride, 32) uint8 and (F,) int32), or device
+        pointers (ints) of ctx's device such as OrbxSequenceResult.gathered_desc / gathered_n, which then need n_frames (the
+        sequence's F) and stride (its n_features)"""
+        self = cls.__new__(cls)
+        self._L, self.ctx = ctx._L, ctx
+        self._h = C.c_void_p()
+        on_device = isinstance(desc, int)
+        if on_device:
+            assert isinstance(counts, int) and n_frames is not None and stride is not None, "device pointers need n_frames and stride"
+            F, S, dp, cp = int(n_frames), int(stride), desc, counts
+        else:
+            d = np.ascontiguousarray(desc, np.uint8)
+            assert d.ndim == 3 and d.shape[2] == 32
+            F = d.shape[0] if n_frames is None else int(n_frames)
+            S = d.shape[1]
+            d = np.ascontiguousarray(d[:F])
+            cnt = np.ascontiguousarray(np.asarray(counts)[:F], np.int32)
+            assert len(cnt) == F
+            dp, cp = d.ctypes.data, cnt.ctypes.data
+        _check(ctx._h, self._L.orbx_bowdb_build(ctx._h, vocab._h, dp, cp, F, S, int(on_device), C.byref(self._h)), "orbx_bowdb_build")
+        return self
+
+    def info(self) -> dict:
+        f, w, p = C.c_int32(), C.c_int32(), C.c_int64()
+        _check(None, self._L.orbx_bowdb_info(self._h, C.byref(f), C.byref(w), C.byref(p)), "orbx_bowdb_info")
+        return dict(n_frames=f.value, n_words=w.value, n_postings=p.value)
+
+    def _io(self, window, min_score, top_k, on_device, ptrs) -> OrbxBowdbIO:
+        return OrbxBowdbIO(int(window), float(min_score), int(top_k), int(on_device), *[p or None for p in ptrs])
+
+    def query_ptr(self, q_lo: int, q_hi: int, top_k: int, exclude_window: int, min_score: float, ptrs, on_device: bool = True):
+        """orbx_bowdb_query_range with raw output pointers, in BOWDB_OUTPUTS order (0 = not wanted)"""
+        io = self._io(exclude_window, min_score, top_k, on_device, ptrs)
+        _check(self.ctx._h, self._L.orbx_bowdb_query_range(self.ctx._h, self._h, int(q_lo), int(q_hi), C.byref(io)), "orbx_bowdb_query_range")
+
+    def query_frame_ptr(self, frame: int, top_k: int, min_score: float, ptrs, on_device: bool = True):
+        """orbx_bowdb_query_frame with raw output pointers, in BOWDB_OUTPUTS order (0 = not wanted)"""
+        io = self._io(-1, min_score, top_k, on_device, ptrs)
+        _check(self.ctx._h, self._L.orbx_bowdb_query_frame(self.ctx._h, self._h, int(frame), C.byref(io)), "orbx_bowdb_query_frame")
+
+    @staticmethod
+    def _outputs(nq: int, top_k: int) -> dict:
+        k = max(int(top_k), 0)
+        return dict(cand_frame=np.zeros((nq, k), np.int32), cand_score=np.zeros((nq, k), np.float32), cand_common=np.zeros((nq, k), np.int32),
+                    **{n: np.zeros(nq, np.int32) for n in BOWDB_OUTPUTS[3:]})
+
+    def query(self, q_lo: int, q_hi: int, top_k: int, exclude_window: int = 0, min_score: float = 0.0) -> dict:
+        """loop candidates of frames q_lo .. q_hi - 1 (each excludes the frames within exclude_window of itself) -> dict of
+        cand_frame / cand_score / cand_common [n][top_k] and n_sharing / max_common / n_scored / n_kept [n]"""
+        out = self._outputs(max(int(q_hi) - int(q_lo), 0), top_k)
+        self.query_ptr(q_lo, q_hi, top_k, exclude_window, min_score, [out[n].ctypes.data for n in BOWDB_OUTPUTS], on_device=False)
+        return out
+
+    def query_frame(self, frame: int = 0, top_k: int = 10, min_score: float = 0.0) -> dict:
+        """relocalisation candidates of frame `frame` of the context's most recent call, whose bow_transform() with this
+        database's vocabulary is resident; nothing is excluded.  -> the dict of query() with one row"""
+        out = self._outputs(1, top_k)
+        self.query_frame_ptr(frame, top_k, min_score, [out[n].ctypes.data for n in BOWDB_OUTPUTS], on_device=False)
+        return out
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._L.orbx_bowdb_destroy(self._h)
             self._h = None
 
     def __del__(self):

@@ -589,7 +589,7 @@ static int require_frames(orbx_ctx *c, int64_t end)
   if (end <= c->last_frames) return ORBX_OK;
   return fail(c, ORBX_ERR_STATE, "no frame with that index has been processed by the most recent stereo / RGB-D call");
 }
-static int require_bow(orbx_ctx *c, int64_t end)
+int require_bow(orbx_ctx *c, int64_t end)
 {
   if (c->bow_epoch == c->frame_epoch && end <= c->bow_frames) return ORBX_OK;
   return fail(c, ORBX_ERR_STATE, "the bag of words of that frame is not resident: call orbx_bow_transform* on the most recent call's frames first");
@@ -1847,6 +1847,7 @@ extern "C"
     c->launches += 2;
     c->bow_epoch = c->frame_epoch;
     c->bow_frames = n_frames;
+    c->bow_vocab = v;
     ORBX_CUDA(c, cudaGetLastError());
     out->bow_ids = a.bow_ids, out->bow_vals = a.bow_vals, out->n_bow = a.n_bow;
     out->fv_nodes = a.fv_nodes, out->fv_start = a.fv_start, out->fv_feats = a.fv_feats, out->n_fv_nodes = a.n_fv;

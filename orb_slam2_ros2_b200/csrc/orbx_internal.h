@@ -78,6 +78,7 @@ struct orbx_ctx
   uint64_t frame_epoch = 0;   // bumped by every call that produces frames
   uint64_t bow_epoch = ~0ull; // frame_epoch at the last bag-of-words call
   int bow_frames = 0;         // frames covered by that call
+  const orbx_vocab *bow_vocab = nullptr; // the vocabulary of that call
   // keyframe records of sequences (orbx_sequence_stereo_keyframes): per-slot staging of records + poses for host outputs,
   // and the int64 sizes of a whole block (copied to the host once at the end)
   orbx::DeviceBuffer kf_staging, kf_sizes;
@@ -123,6 +124,9 @@ int run_stereo_chunks(orbx_ctx *c, int64_t n_frames, const uint8_t *left, size_t
 int pack_frame_records(orbx_ctx *c, cudaStream_t s, int d0, int nf, uint8_t *d_rec, size_t rec_stride);
 // frees the gathered arrays a context keeps for single-rank sequence calls
 void destroy_self_comm(orbx_ctx *c);
+// ORBX_OK when the bag of words of frames [0, end) is resident from the orbx_bow_transform* call on the most recent call's
+// frames, ORBX_ERR_STATE otherwise
+int require_bow(orbx_ctx *c, int64_t end);
 // allocates the context's bag-of-words result buffers (n_img_max frames, as many as an RGB-D batch holds) on first use
 int bow_buffers(orbx_ctx *c);
 // c->bow with the vocabulary's tree, ready for launch_bow_descend / launch_bow_assemble over device slots whose frame f
