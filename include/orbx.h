@@ -501,6 +501,78 @@ int orbx_bowdb_query_range(orbx_ctx *ctx, const orbx_bowdb *db, int64_t q_lo, in
  * orbx_bow_transform* with the database's vocabulary (ORBX_ERR_STATE otherwise, or once the frame epoch has moved on) */
 int orbx_bowdb_query_frame(orbx_ctx *ctx, const orbx_bowdb *db, int frame, const orbx_bowdb_io *io);
 
+/* ---- loop verification: matching, rotation check and a fixed-scale RANSAC per (query, candidate) pair ------------- */
+/* replaces: the geometric check of LoopClosing::ComputeSim3 (ORB-SLAM2 LoopClosing.cc) -- ORBmatcher::SearchByBoW between the
+ * query keyframe and each loop candidate, the rotation check, and Sim3Solver (Horn's closed form, fixed scale for stereo) in
+ * RANSAC -- for many pairs at once over the frames of a stereo sequence.  Parity unpinned (the reference's LoopClosing /
+ * Sim3Solver and ORB-SLAM2 are not vendored); the rules, which tests/loopver_oracle.c restates:
+ *   frames     frame f's keypoints (kps_left: x, y, angle, octave), descriptors and depth come from its orbx_record_layout
+ *              record (n_left of them); its FeatureVector is orbx_bow_transform's at `levelsup`
+ *   matching   orbx_search_by_bow with the candidate as the keyframe and the query as the frame, no masks: rows in the
+ *              candidate's FeatureVector order, candidates = the query's features under the same node, getBestMatch; a row is
+ *              kept iff dist <= 50 && !(ratio > params.ratio) (n_bow), then orbx_verify_angle with kps1 = the query's,
+ *              kps2 = the candidate's keypoints (n_matches; `match` holds the result); n_matches < min_matches stops the pair
+ *   points     the surviving matches whose features both have depth > 0, in match order (n_corr); in double, each operation
+ *              rounded: z = depth, x = ((u - cx) * z) / fx, y = ((v - cy) * z) / fy with the context's camera
+ *   sums       every sum over a point list x_0 .. x_{m-1} with slots s_k: 32 partials p_l = 0.0, p_{s_k mod 32} += x_k in list
+ *              order, then p_l += p_{l+16} (l < 16), p_l += p_{l+8} (l < 8), .. 4, 2, 1; the sum is p_0
+ *   Horn       centroids cc / cq = sum / m; M_ab = sum (c_a - cc_a) (q_b - cq_b); N from M as Sim3Solver::ComputeSim3 (candidate =
+ *              its set 2, query = set 1); cyclic Jacobi on N: pairs (0,1) (0,2) (0,3) (1,2) (1,3) (2,3), a zero off-diagonal
+ *              skipped, theta = (a_qq - a_pp) / (2 a_pq), t = sign(theta) / (|theta| + sqrt(theta^2 + 1)), c = 1 / sqrt(t^2 + 1),
+ *              s = t c, columns then rows then a_pq = a_qp = 0, then the eigenvectors; stop when every off-diagonal is 0 or after
+ *              ORBX_LOOPVER_JACOBI_SWEEPS sweeps; q = eigenvector of the largest diagonal entry, the first among equals;
+ *              R = the quaternion's homogeneous rotation divided by |q|^2 (ORB-SLAM2: atan2 + Rodrigues); t = cq - R cc
+ *   hypothesis h draws 3 points without replacement: avail = 0 .. n-1, for j = 0..2: r = draw(h, j) % (n - j), idx_j = avail[r],
+ *              avail[r] = avail[n-1-j]; draw(h, j) = splitmix64(K ^ ((3h + j) * 0x9E3779B97F4A7C15)) with the pair key
+ *              K = splitmix64(splitmix64(splitmix64(seed) + query + 1) + candidate + 1) (orbx_vocab_build's generator);
+ *              Horn over the samples in draw order (slots 0, 1, 2)
+ *   inliers    candidate points go into the query camera with T (R X + t), query points into the candidate camera with
+ *              R^T X - R^T t, projected as (fx (X / Z) + cx, fy (Y / Z) + cy) in double; a point is an inlier iff both squared
+ *              pixel errors to its keypoints are < 9.210 * sigma2 of the keypoint's octave, sigma2 = (float)(sf * sf) of the
+ *              level scale factor (ORB-SLAM2 truncates this bound to an integer); NaN and infinity are outliers
+ *   iterations SetRansacParameters on the host: 0 when n_corr < min_inliers, else 1 when n_corr == min_inliers, else
+ *              ceil(log(1 - probability) / log(1 - pow(eps, 3))) with eps = (float)min_inliers / n_corr, clamped to
+ *              [1, max_iterations]
+ *   accepted   Sim3Solver::iterate: the first h whose inlier count is > min_inliers; otherwise the last among the maxima (>=)
+ *              and accepted = 0.  n_iters = accepted h + 1, or the table value.  T = Horn over the inliers of the reported
+ *              hypothesis in correspondence order (slot = correspondence index), or over its samples when it has fewer than 3
+ *   loop_frame the accepted candidate with the smallest (hypothesis / 5, table position) -- ComputeSim3 gives every candidate
+ *              iterate(5) per round -- or -1
+ * A pair that stops early reports 0 for the counts it did not reach, hypothesis -1 and T = 0; an empty slot (-1) also has
+ * n_bow = n_matches = 0 and match = -1.  Out of scope: SearchBySim3, OptimizeSim3 and the map-point projection check (they need
+ * g2o and map points), the covisibility accumulation, and RGB-D inputs (records exist for stereo sequences only). */
+#define ORBX_LOOPVER_JACOBI_SWEEPS 16
+typedef struct orbx_loopver orbx_loopver;
+/* records: the F frames' orbx_record_layout records, [F][record_stride] (>= record_bytes, multiple of 16), host or device memory
+ * of ctx's device; device records must be 16-byte aligned (they are read in place), else ORBX_ERR_INVALID_ARG.  The verifier copies what it needs into arrays it owns; `records` may be freed afterwards.  vocab must
+ * belong to ctx; levelsup >= 0 (>= L: the FeatureVector node is the root, as in orbx_bow_transform).  Blocks until the verifier is built; leaves the context's resident frames and their bag of words untouched. */
+int orbx_loopver_build(orbx_ctx *ctx, const orbx_vocab *vocab, int32_t levelsup, const void *records, size_t record_stride,
+                       int32_t n_frames, int32_t on_device, orbx_loopver **out);
+void orbx_loopver_destroy(orbx_loopver *lv);
+typedef struct orbx_loopver_params {
+  float ratio;            /* searchByBow's mfRatio (not NaN); ORB-SLAM2's loop matcher uses 0.75 */
+  int32_t min_matches;    /* ORB-SLAM2: 20 */
+  int32_t min_inliers;    /* >= 3; ORB-SLAM2: 20 */
+  int32_t max_iterations; /* >= 1; ORB-SLAM2: 300 */
+  double probability;     /* 0 < p < 1; ORB-SLAM2: 0.99 */
+  uint64_t seed;
+} orbx_loopver_params;
+typedef struct orbx_loopver_io {
+  int32_t on_device;      /* table + outputs: device = asynchronous on ctx's stream, host = the call blocks */
+  const int32_t *cand_frame; /* [n_queries][top_k], the layout orbx_bowdb_query_range writes; -1 = empty slot.  A host entry
+                                outside [-1, n_frames) is ORBX_ERR_INVALID_ARG; a device one is an empty slot */
+  int32_t top_k;
+  /* outputs, [n_queries][top_k] unless noted; any may be NULL */
+  int32_t *n_bow, *n_matches, *n_corr, *n_iters, *hypothesis, *n_inliers, *accepted;
+  double *T;              /* [n_queries][top_k][12]: R row-major then t, candidate camera -> query camera */
+  int32_t *match;         /* [n_queries][top_k][n_features]: query feature of each candidate feature after verifyAngle, or -1 */
+  int32_t *loop_frame;    /* [n_queries] */
+} orbx_loopver_io;
+/* verifies queries q_lo .. q_lo + n_queries - 1 (frames of the verifier) against their rows of the table.  Sharded: every rank
+ * builds the verifier from the whole record set and verifies its block orbx_frame_range(F, rank, world). */
+int orbx_loopver_verify(orbx_ctx *ctx, const orbx_loopver *lv, int64_t q_lo, int64_t n_queries, const orbx_loopver_params *prm,
+                        const orbx_loopver_io *io);
+
 /* ---- introspection for benchmarks / profiles ----------------------------------------------------------- */
 #define ORBX_N_STAGES 7
 /* Same work as orbx_stereo_batch_device, with a CUDA event recorded on the stream after every kernel; blocks until

@@ -84,6 +84,7 @@ EXPORTS = [
     "orbx_serialized_capacity_bow", "orbx_serialize_keyframe_bow", "orbx_serialize_keyframes_bow_device", "orbx_keyframe_list_head",
     "orbx_keyframe_list_entry_prefix", "orbx_sequence_stereo_keyframes", "orbx_vocab_build", "orbx_vocab_save_text", "orbx_vocab_arrays",
     "orbx_bowdb_build", "orbx_bowdb_destroy", "orbx_bowdb_info", "orbx_bowdb_query_range", "orbx_bowdb_query_frame",
+    "orbx_loopver_build", "orbx_loopver_destroy", "orbx_loopver_verify",
 ]
 
 class OrbxRecordLayout(C.Structure):
@@ -127,6 +128,20 @@ class OrbxBowdbIO(C.Structure):
     _fields_ = [("exclude_window", C.c_int32), ("min_score", C.c_float), ("top_k", C.c_int32), ("on_device", C.c_int32), ("cand_frame", C.c_void_p),
                 ("cand_score", C.c_void_p), ("cand_common", C.c_void_p), ("n_sharing", C.c_void_p), ("max_common", C.c_void_p), ("n_scored", C.c_void_p),
                 ("n_kept", C.c_void_p)]
+
+
+LOOPVER_JACOBI_SWEEPS = 16  # ORBX_LOOPVER_JACOBI_SWEEPS
+
+
+class OrbxLoopverParams(C.Structure):
+    _fields_ = [("ratio", C.c_float), ("min_matches", C.c_int32), ("min_inliers", C.c_int32), ("max_iterations", C.c_int32), ("probability", C.c_double),
+                ("seed", C.c_uint64)]
+
+
+class OrbxLoopverIO(C.Structure):
+    _fields_ = [("on_device", C.c_int32), ("cand_frame", C.c_void_p), ("top_k", C.c_int32), ("n_bow", C.c_void_p), ("n_matches", C.c_void_p),
+                ("n_corr", C.c_void_p), ("n_iters", C.c_void_p), ("hypothesis", C.c_void_p), ("n_inliers", C.c_void_p), ("accepted", C.c_void_p),
+                ("T", C.c_void_p), ("match", C.c_void_p), ("loop_frame", C.c_void_p)]
 
 
 _lib = None
@@ -228,6 +243,10 @@ def load_library(build_if_missing: bool = True):
     L.orbx_bowdb_info.argtypes = [vp, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int64)]
     L.orbx_bowdb_query_range.argtypes = [vp, vp, C.c_int64, C.c_int64, C.POINTER(OrbxBowdbIO)]
     L.orbx_bowdb_query_frame.argtypes = [vp, vp, C.c_int, C.POINTER(OrbxBowdbIO)]
+    L.orbx_loopver_build.argtypes = [vp, vp, C.c_int32, vp, sz, C.c_int32, C.c_int32, C.POINTER(vp)]
+    L.orbx_loopver_destroy.argtypes = [vp]
+    L.orbx_loopver_destroy.restype = None
+    L.orbx_loopver_verify.argtypes = [vp, vp, C.c_int64, C.c_int64, C.POINTER(OrbxLoopverParams), C.POINTER(OrbxLoopverIO)]
     _lib = L
     return L
 
@@ -1174,6 +1193,66 @@ class BowDatabase:
     def close(self):
         if getattr(self, "_h", None):
             self._L.orbx_bowdb_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+LOOPVER_OUTPUTS = ("n_bow", "n_matches", "n_corr", "n_iters", "hypothesis", "n_inliers", "accepted", "T", "match", "loop_frame")
+
+
+class LoopVerifier:
+    """Loop verification over the frames of a stereo sequence (orbx_loopver_*): ORB-SLAM2's LoopClosing::ComputeSim3 check --
+    searchByBow between a query and each of its loop candidates, the rotation check, and a fixed-scale Horn RANSAC --
+    for every (query, candidate) pair of a table such as BowDatabase.query's cand_frame, built once on a context's device."""
+
+    @classmethod
+    def build(cls, ctx: Context, vocab: Vocabulary, records, n_frames: int, levelsup: int = 4, record_stride: int | None = None) -> "LoopVerifier":
+        """from the frames' records (the layout of ctx.record_dtype(), e.g. sequence_stereo's): a host array of n_frames
+        records, or a device pointer (int) of ctx's device, which then needs record_stride when it is not record_bytes"""
+        self = cls.__new__(cls)
+        self._L, self.ctx, self.n_frames = ctx._L, ctx, int(n_frames)
+        self._h = C.c_void_p()
+        if isinstance(records, int):
+            ptr, stride, on_device = records, int(record_stride or ctx.record_layout().record_bytes), 1
+        else:
+            rec = np.ascontiguousarray(records).view(np.uint8).reshape(len(records), -1)[: int(n_frames)]
+            assert len(rec) == int(n_frames)
+            ptr, stride, on_device = rec.ctypes.data, rec.shape[1], 0
+        _check(ctx._h, self._L.orbx_loopver_build(ctx._h, vocab._h, int(levelsup), ptr, stride, int(n_frames), on_device, C.byref(self._h)),
+               "orbx_loopver_build")
+        return self
+
+    @staticmethod
+    def params(ratio=0.75, min_matches=20, min_inliers=20, max_iterations=300, probability=0.99, seed=0) -> OrbxLoopverParams:
+        return OrbxLoopverParams(float(ratio), int(min_matches), int(min_inliers), int(max_iterations), float(probability), int(seed) & (2**64 - 1))
+
+    def verify_ptr(self, q_lo: int, n_queries: int, cand_ptr: int, top_k: int, ptrs, on_device: bool = True, **params):
+        """orbx_loopver_verify with a raw table pointer and raw output pointers in LOOPVER_OUTPUTS order (0 = not wanted)"""
+        io = OrbxLoopverIO(int(on_device), cand_ptr or None, int(top_k), *[p or None for p in ptrs])
+        prm = self.params(**params)
+        _check(self.ctx._h, self._L.orbx_loopver_verify(self.ctx._h, self._h, int(q_lo), int(n_queries), C.byref(prm), C.byref(io)), "orbx_loopver_verify")
+
+    def verify(self, q_lo: int, cand_frame, ratio=0.75, min_matches=20, min_inliers=20, max_iterations=300, probability=0.99, seed=0) -> dict:
+        """verifies queries q_lo .. q_lo + len(cand_frame) - 1 against their rows of cand_frame ([n][top_k], -1 = empty slot)
+        -> dict of n_bow / n_matches / n_corr / n_iters / hypothesis / n_inliers / accepted [n][top_k], T [n][top_k][12],
+        match [n][top_k][n_features] and loop_frame [n]"""
+        tab = np.ascontiguousarray(cand_frame, np.int32)
+        assert tab.ndim == 2
+        nq, k, N = tab.shape[0], tab.shape[1], self.ctx.n_features
+        out = {n: np.zeros((nq, k), np.int32) for n in LOOPVER_OUTPUTS[:7]}
+        out.update(T=np.zeros((nq, k, 12), np.float64), match=np.zeros((nq, k, N), np.int32), loop_frame=np.zeros(nq, np.int32))
+        self.verify_ptr(q_lo, nq, tab.ctypes.data, k, [out[n].ctypes.data for n in LOOPVER_OUTPUTS], on_device=False, ratio=ratio,
+                        min_matches=min_matches, min_inliers=min_inliers, max_iterations=max_iterations, probability=probability, seed=seed)
+        return out
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._L.orbx_loopver_destroy(self._h)
             self._h = None
 
     def __del__(self):

@@ -13,8 +13,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "liborbx.so")
-SOURCES = ["orbx_kernels.cu", "orbx_match.cu", "orbx_serialize.cu", "orbx_bow.cu", "orbx_vocab.cu", "orbx_bowdb.cu", "orbx_sequence.cu", "orbx_api.cu"]
-HEADERS = [os.path.join(CSRC, "orbx_device.cuh"), os.path.join(CSRC, "orbx_internal.h"), os.path.join(HERE, "..", "include", "orbx.h"), os.path.join(HERE, "..", "include", "orbx_pattern.h")]
+SOURCES = ["orbx_kernels.cu", "orbx_match.cu", "orbx_serialize.cu", "orbx_bow.cu", "orbx_vocab.cu", "orbx_bowdb.cu", "orbx_loop.cu", "orbx_sequence.cu", "orbx_api.cu"]
+HEADERS = [os.path.join(CSRC, "orbx_device.cuh"), os.path.join(CSRC, "orbx_match.cuh"), os.path.join(CSRC, "orbx_internal.h"), os.path.join(HERE, "..", "include", "orbx.h"), os.path.join(HERE, "..", "include", "orbx_pattern.h")]
 
 
 def nvcc_cmd(extra=()):

@@ -24,6 +24,7 @@
 #include <vector>
 
 #include "orbx_internal.h"
+#include "orbx_match.cuh"
 
 struct orbx_bowdb
 {
@@ -53,7 +54,6 @@ namespace
 {
 
 constexpr int kQT = 256; // threads of the query CTA
-constexpr int kBuildChunk = 1024; // frames per transform launch: bounds the per-feature scratch at 28 B x stride x 1024
 constexpr unsigned kFull = 0xffffffffu;
 constexpr unsigned long long kNone = ~0ull; // a list slot holding no kept candidate (sorts last)
 constexpr size_t kSmemOptIn = 227 * 1024;  // shared memory one CTA may opt in to on sm_100
@@ -143,32 +143,6 @@ __device__ __forceinline__ float key_float(unsigned k) { return __uint_as_float(
 
 __device__ __forceinline__ int counter_of(const unsigned *cnt, int f) { return (int)((cnt[f >> 1] >> (16 * (f & 1))) & 0xffffu); }
 
-// block-wide inclusive-exclusive scan of one int per thread; *total = the block's sum
-__device__ __forceinline__ int block_exscan(int v, int *total, int *s_warp)
-{
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  int inc = v;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1)
-  {
-    const int t = __shfl_up_sync(kFull, inc, o);
-    if (lane >= o) inc += t;
-  }
-  if (lane == 31) s_warp[wid] = inc;
-  __syncthreads();
-  int base = 0, tot = 0;
-#pragma unroll
-  for (int w = 0; w < kQT / 32; ++w)
-  {
-    const int t = s_warp[w];
-    if (w < wid) base += t;
-    tot += t;
-  }
-  __syncthreads();
-  *total = tot;
-  return base + inc - v;
-}
-
 __global__ void __launch_bounds__(kQT) bowdb_query_kernel(const QueryArgs a)
 {
   extern __shared__ __align__(16) unsigned char smem[];
@@ -228,7 +202,7 @@ __global__ void __launch_bounds__(kQT) bowdb_query_kernel(const QueryArgs a)
     if (sharing > 0)
       for (int f = f0; f < f1; ++f) mine += common_of(f) > min_common;
     int n_sc;
-    int pos = block_exscan(mine, &n_sc, s_warp);
+    int pos = block_exscan<kQT>(mine, &n_sc, s_warp);
     if (sharing > 0)
       for (int f = f0; f < f1; ++f)
         if (common_of(f) > min_common) list[pos++] = (unsigned long long)f;
@@ -343,6 +317,45 @@ __global__ void __launch_bounds__(kQT) bowdb_query_kernel(const QueryArgs a)
 size_t up16(size_t v) { return (v + 15) & ~(size_t)15; }
 
 } // namespace
+
+int bow_frames(orbx_ctx *c, const orbx_vocab *v, int levelsup, const uint8_t *d_desc, const int *d_n, int F, int stride, const BowArgs &out)
+{
+  constexpr int kChunk = 1024; // frames per transform launch: bounds the per-feature scratch at 28 B x stride x 1024
+  cudaStream_t s = c->stream;
+  const size_t ch = (size_t)std::min(F, kChunk) * stride;
+  auto sc = [](const void *mine, size_t bytes) { return mine ? 0 : up16(bytes); }; // scratch only for the outputs left null
+  const size_t o_word = 0, o_nid = o_word + up16(ch * 4), o_w = o_nid + up16(ch * 4), o_ids = o_w + up16(ch * 8), o_vals = o_ids + sc(out.bow_ids, ch * 4),
+               o_nb = o_vals + sc(out.bow_vals, ch * 8), o_fvn = o_nb + sc(out.n_bow, (size_t)kChunk * 4), o_fvs = o_fvn + sc(out.fv_nodes, ch * 4),
+               o_fvf = o_fvs + sc(out.fv_start, ch * 4 + (size_t)kChunk * 4), o_nfv = o_fvf + sc(out.fv_feats, ch * 4),
+               sc_total = o_nfv + sc(out.n_fv, (size_t)kChunk * 4);
+  DeviceBuffer scratch;
+  if (int rc = scratch.reserve(c, sc_total)) return rc;
+  BowArgs b{};
+  b.child_start = v->child_start, b.child_ids = v->child_ids, b.v_desc = v->desc, b.v_weight = v->weight, b.v_word = v->word;
+  b.L = v->L, b.levelsup = levelsup, b.image_stride = 1;
+  b.f_word = (int *)(scratch.p + o_word), b.f_nid = (int *)(scratch.p + o_nid), b.f_weight = (double *)(scratch.p + o_w);
+  for (int f0 = 0; f0 < F; f0 += kChunk)
+  {
+    const int nf = std::min(kChunk, F - f0);
+    const size_t e0 = (size_t)f0 * stride;
+    auto at = [&](auto *mine, size_t off, size_t per_frame) { return mine ? mine + (size_t)f0 * per_frame : (decltype(mine))(scratch.p + off); };
+    Params p{};
+    p.n_features = stride;
+    p.desc = const_cast<uint8_t *>(d_desc) + e0 * 32;
+    p.n_kps = const_cast<int *>(d_n) + f0;
+    BowArgs bb = b;
+    bb.bow_ids = at(out.bow_ids, o_ids, stride), bb.bow_vals = at(out.bow_vals, o_vals, stride), bb.n_bow = at(out.n_bow, o_nb, 1);
+    bb.fv_nodes = at(out.fv_nodes, o_fvn, stride), bb.fv_start = at(out.fv_start, o_fvs, (size_t)stride + 1), bb.fv_feats = at(out.fv_feats, o_fvf, stride);
+    bb.n_fv = at(out.n_fv, o_nfv, 1);
+    launch_bow_descend(p, bb, nf, s);
+    launch_bow_assemble(p, bb, nf, s);
+    c->launches += 2;
+  }
+  ORBX_CUDA(c, cudaGetLastError());
+  // the scratch is freed on return: the work that reads it has to finish first
+  ORBX_CUDA(c, cudaStreamSynchronize(s));
+  return ORBX_OK;
+}
 
 } // namespace orbx
 
@@ -477,7 +490,7 @@ extern "C"
     ORBX_CUDA(c, cudaMalloc((void **)&db->n, (size_t)F * 4));
     ORBX_CUDA(c, cudaMalloc((void **)&db->word_start, ((size_t)v->n_words + 1) * 8));
     // inputs in device memory; the transform's per-feature and FeatureVector outputs in chunk scratch
-    DeviceBuffer in_desc, in_n, scratch, cursor;
+    DeviceBuffer in_desc, in_n, cursor;
     const uint8_t *d_desc = desc;
     const int *d_n = n_kps;
     if (!on_device)
@@ -488,28 +501,9 @@ extern "C"
       ORBX_CUDA(c, cudaMemcpyAsync(in_n.p, n_kps, (size_t)F * 4, cudaMemcpyHostToDevice, s));
       d_desc = in_desc.p, d_n = (const int *)in_n.p;
     }
-    const size_t ch = (size_t)std::min(F, kBuildChunk) * stride;
-    const size_t o_word = 0, o_nid = o_word + up16(ch * 4), o_w = o_nid + up16(ch * 4), o_fvn = o_w + up16(ch * 8), o_fvs = o_fvn + up16(ch * 4),
-                 o_fvf = o_fvs + up16(ch * 4 + (size_t)kBuildChunk * 4), o_nfv = o_fvf + up16(ch * 4), sc_total = o_nfv + up16((size_t)kBuildChunk * 4);
-    if (int rc = scratch.reserve(c, sc_total)) return rc;
-    BowArgs b{};
-    b.child_start = v->child_start, b.child_ids = v->child_ids, b.v_desc = v->desc, b.v_weight = v->weight, b.v_word = v->word;
-    b.L = v->L, b.levelsup = 0, b.image_stride = 1;
-    b.f_word = (int *)(scratch.p + o_word), b.f_nid = (int *)(scratch.p + o_nid), b.f_weight = (double *)(scratch.p + o_w);
-    b.fv_nodes = (int *)(scratch.p + o_fvn), b.fv_start = (int *)(scratch.p + o_fvs), b.fv_feats = (int *)(scratch.p + o_fvf), b.n_fv = (int *)(scratch.p + o_nfv);
-    for (int f0 = 0; f0 < F; f0 += kBuildChunk)
-    {
-      const int nf = std::min(kBuildChunk, F - f0);
-      Params p{};
-      p.n_features = stride;
-      p.desc = const_cast<uint8_t *>(d_desc) + (size_t)f0 * stride * 32;
-      p.n_kps = const_cast<int *>(d_n) + f0;
-      BowArgs bb = b;
-      bb.bow_ids = db->ids + (size_t)f0 * stride, bb.bow_vals = db->vals + (size_t)f0 * stride, bb.n_bow = db->n + f0;
-      launch_bow_descend(p, bb, nf, s);
-      launch_bow_assemble(p, bb, nf, s);
-      c->launches += 2;
-    }
+    BowArgs bow{};
+    bow.bow_ids = db->ids, bow.bow_vals = db->vals, bow.n_bow = db->n;
+    if (int rc = bow_frames(c, v, 0, d_desc, d_n, F, stride, bow)) return rc;
     ORBX_CUDA(c, cudaGetLastError());
     // inverted file: postings per word, exclusive scan, fill
     const unsigned blocks = (unsigned)((rows + 255) / 256);

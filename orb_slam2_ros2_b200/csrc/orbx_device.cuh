@@ -254,6 +254,16 @@ int bow_configure(int n_features); // opt in to the dynamic shared memory of the
 size_t quadtree_smem_bytes(int list_cap, int node_cap, int big_cap, int max_level_cells);
 int quadtree_configure(size_t smem_bytes); // opt in to large dynamic shared memory
 
+// the counter-based generator of orbx_vocab_build and orbx_loopver_verify (include/orbx.h)
+constexpr unsigned long long kGolden = 0x9E3779B97F4A7C15ull;
+__host__ __device__ __forceinline__ unsigned long long splitmix64(unsigned long long x)
+{
+  unsigned long long z = x + kGolden;
+  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+  z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+  return z ^ (z >> 31);
+}
+
 // cudaFuncAttributeMaxDynamicSharedMemorySize belongs to the kernel (per device), not to a context: it is only ever RAISED, so a
 // second context with a smaller configuration cannot shrink the limit under a live one (launches of the larger context would
 // fail with "invalid argument").  `state` = the caller's per-kernel high-water marks, one per device.

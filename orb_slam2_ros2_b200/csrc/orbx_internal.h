@@ -132,6 +132,10 @@ int bow_buffers(orbx_ctx *c);
 // c->bow with the vocabulary's tree, ready for launch_bow_descend / launch_bow_assemble over device slots whose frame f
 // reads image f * image_stride
 BowArgs bow_args(const orbx_ctx *c, const orbx_vocab *v, int levelsup, int image_stride);
+// BowVectors and FeatureVectors (orbx_bow_transform's, at `levelsup`) of F frames of device descriptors d_desc[f][stride][32],
+// d_n[f] each, in chunks of frames: frame f's results go to out.bow_ids / bow_vals / fv_nodes / fv_feats + f * stride,
+// out.fv_start + f * (stride + 1), out.n_bow / n_fv + f; the arrays left null in `out` get per-chunk scratch.  Synchronises.
+int bow_frames(orbx_ctx *c, const orbx_vocab *v, int levelsup, const uint8_t *d_desc, const int *d_n, int F, int stride, const BowArgs &out);
 // appends `v` as std::ostream << double prints it by default ("%g": 6 significant digits) and a blank
 void append_g(std::string &t, double v);
 

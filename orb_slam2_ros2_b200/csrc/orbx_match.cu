@@ -9,7 +9,7 @@
 //
 // Both reproduce the reference's candidate ORDER (grid cells row-major, ascending keypoint index inside a cell), which
 // decides ties of the best match and the value of the reference's order-dependent "second best".
-#include "orbx_device.cuh"
+#include "orbx_match.cuh"
 
 namespace orbx
 {
@@ -18,48 +18,6 @@ namespace
 {
 
 constexpr int kAreaWarps = 8;
-constexpr unsigned kFull = 0xffffffffu;
-
-__device__ __forceinline__ int hamming256(const uint4 &a0, const uint4 &a1, const uint4 &b0, const uint4 &b1)
-{
-  return __popc(a0.x ^ b0.x) + __popc(a0.y ^ b0.y) + __popc(a0.z ^ b0.z) + __popc(a0.w ^ b0.w) + __popc(a1.x ^ b1.x) + __popc(a1.y ^ b1.y) +
-         __popc(a1.z ^ b1.z) + __popc(a1.w ^ b1.w);
-}
-
-// One chunk of up to 32 candidates (lane order == the reference's candidate order; id < 0: no candidate on this lane) of
-// ORBMatcher::getBestMatch (src/ORBMatcher.cc:967-990).  The sequential rule
-//   if (d < min) { min = d; idx = i; } else if (d < second) second = d;
-// is evaluated with an exclusive prefix-minimum over the lanes: a candidate is a "new minimum" iff its distance is below
-// every earlier one (the running minimum included); `second` is the minimum over all the others.
-__device__ __forceinline__ void best_match_chunk(int id, int d, int lane, int &n_cand, int &min_d, int &second_d, int &min_idx)
-{
-  const unsigned valid = __ballot_sync(kFull, id >= 0);
-  if (!valid) return;
-  n_cand += __popc(valid);
-  int pm = d; // exclusive prefix minimum over the lanes, seeded with the running minimum
-#pragma unroll
-  for (int s = 1; s < 32; s <<= 1)
-  {
-    const int t = __shfl_up_sync(kFull, pm, s);
-    if (lane >= s) pm = min(pm, t);
-  }
-  int ex = __shfl_up_sync(kFull, pm, 1);
-  if (lane == 0) ex = 0x7fffffff;
-  ex = min(ex, min_d);
-  const bool is_new = id >= 0 && d < ex;
-  int sec = (id >= 0 && !is_new) ? d : 0x7fffffff;
-#pragma unroll
-  for (int s = 16; s; s >>= 1) sec = min(sec, __shfl_xor_sync(kFull, sec, s));
-  second_d = min(second_d, sec);
-  // the last "new minimum" lane of the chunk holds the chunk's minimum at its first occurrence
-  const unsigned news = __ballot_sync(kFull, is_new);
-  if (news)
-  {
-    const int src = 31 - __clz(news);
-    min_d = __shfl_sync(kFull, d, src);
-    min_idx = __shfl_sync(kFull, id, src);
-  }
-}
 
 // One warp per query.  Candidates are visited 32 at a time in the reference's order; getBestMatch's sequential rule
 //   if (d < min) { min = d; idx = i; } else if (d < second) second = d;
@@ -126,56 +84,14 @@ __global__ void __launch_bounds__(kAreaWarps * 32, 8) area_match_kernel(const Pa
 }
 
 // The matching loop of ORBMatcher::searchByBow (src/ORBMatcher.cc:170-255): one warp per entry of the keyframe's
-// FeatureVector.  The entry's vocabulary node is looked up in the frame's FeatureVector (both sorted by node id: binary
-// searches replace the reference's merge-join); candidates = the frame's features of that node that pass the mask.
+// FeatureVector (bow_match_row).
 __global__ void __launch_bounds__(kAreaWarps * 32) bow_match_kernel(const BowMatchArgs a)
 {
   const int lane = threadIdx.x & 31;
   const int e = blockIdx.x * kAreaWarps + (threadIdx.x >> 5);
   if (e >= a.k_n_listed) return;
-  int n_cand = 0, min_d = 0x7fffffff, second_d = 0x7fffffff, min_idx = -1;
-  const int pk = a.k_feats[e];
-  if (!a.kf_query_ok || a.kf_query_ok[pk])
-  {
-    // keyframe node segment containing entry e: last j with k_start[j] <= e
-    int lo = 0, hi = a.k_n_nodes;
-    while (hi - lo > 1)
-    {
-      const int mid = (lo + hi) >> 1;
-      if (a.k_start[mid] <= e) lo = mid; else hi = mid;
-    }
-    const int node = a.k_nodes[lo];
-    const int f_n = *a.f_n_nodes;
-    int l2 = 0, h2 = f_n; // first frame node >= node
-    while (l2 < h2)
-    {
-      const int mid = (l2 + h2) >> 1;
-      if (a.f_nodes[mid] < node) l2 = mid + 1; else h2 = mid;
-    }
-    if (l2 < f_n && a.f_nodes[l2] == node)
-    {
-      const uint4 *qd = reinterpret_cast<const uint4 *>(a.k_desc + (size_t)pk * 32);
-      const uint4 q0 = __ldg(qd), q1 = __ldg(qd + 1);
-      const uint4 *fd = reinterpret_cast<const uint4 *>(a.f_desc);
-      const int t0 = a.f_start[l2], t1 = a.f_start[l2 + 1];
-      for (int t = t0; t < t1; t += 32)
-      {
-        int id = -1, d = 0x7fffffff;
-        if (t + lane < t1)
-        {
-          id = a.f_feats[t + lane];
-          if (a.frame_cand_ok && !a.frame_cand_ok[id]) id = -1;
-        }
-        if (id >= 0)
-        {
-          const uint4 b0 = __ldg(fd + 2 * id), b1 = __ldg(fd + 2 * id + 1);
-          d = __popc(q0.x ^ b0.x) + __popc(q0.y ^ b0.y) + __popc(q0.z ^ b0.z) + __popc(q0.w ^ b0.w) + __popc(q1.x ^ b1.x) + __popc(q1.y ^ b1.y) +
-              __popc(q1.z ^ b1.z) + __popc(q1.w ^ b1.w);
-        }
-        best_match_chunk(id, d, lane, n_cand, min_d, second_d, min_idx);
-      }
-    }
-  }
+  int n_cand, min_d, second_d, min_idx;
+  bow_match_row(a, e, lane, n_cand, min_d, second_d, min_idx);
   if (lane == 0)
   {
     a.n_cand[e] = n_cand;
@@ -185,78 +101,16 @@ __global__ void __launch_bounds__(kAreaWarps * 32) bow_match_kernel(const BowMat
   }
 }
 
-constexpr int kVaThreads = 256;
-constexpr int kVaBins = 30;   // ORBMatcher::mnBinNum   (src/ORBMatcher.cc:1091)
-constexpr int kVaChoose = 3;  // ORBMatcher::mnBinChoose (src/ORBMatcher.cc:1092)
-
 __global__ void __launch_bounds__(kVaThreads) verify_angle_kernel(const VerifyArgs a)
 {
-  __shared__ int s_count[kVaBins], s_base[kVaBins], s_wcount[kVaThreads / 32][kVaBins];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int n = a.n;
-  auto bin_of = [&](int i) -> int {
-    float diff = __fsub_rn(a.kps1[a.query_idx[i]].angle, a.kps2[a.train_idx[i]].angle);
-    diff = diff >= 0.f ? diff : __fadd_rn(360.f, diff);
-    int b = (int)__fdiv_rn(diff, 12.f); // 360 / mnBinNum is an integer division in the reference
-    if (b == 30) b = 0;
-    return min(max(b, 0), kVaBins - 1);
-  };
-  if (tid < kVaBins) s_count[tid] = 0;
-  __syncthreads();
-  for (int i = tid; i < n; i += kVaThreads) atomicAdd(&s_count[bin_of(i)], 1);
-  __syncthreads();
-  if (tid == 0)
-  {
-    bool good[kVaBins];
-    for (int b = 0; b < kVaBins; ++b) good[b] = false;
-    for (int k = 0; k < kVaChoose; ++k)
-    {
-      int max_size = 0, max_id = 0;
-      bool init = false;
-      for (int b = 0; b < kVaBins; ++b)
-      {
-        if (good[b]) continue;
-        if (s_count[b] > max_size) max_id = b, max_size = s_count[b], init = true;
-      }
-      if (init) good[max_id] = true;
-    }
-    int off = 0;
-    for (int b = 0; b < kVaBins; ++b) // std::set iteration: ascending bin id
-    {
-      s_base[b] = good[b] ? off : -1;
-      if (good[b]) off += s_count[b];
-    }
-    *a.n_out = off;
-  }
-  __syncthreads();
-  // stable scatter: chunks of kVaThreads matches in order; rank inside a chunk from warp match masks + per-warp counts
-  for (int i0 = 0; i0 < n; i0 += kVaThreads)
-  {
-    for (int k = tid; k < (kVaThreads / 32) * kVaBins; k += kVaThreads) (&s_wcount[0][0])[k] = 0;
-    __syncthreads();
-    const int i = i0 + tid;
-    const int b = i < n ? bin_of(i) : -1;
-    const unsigned same = __match_any_sync(kFull, b);
-    const int rank = __popc(same & ((1u << lane) - 1));
-    if (b >= 0 && rank == 0) s_wcount[warp][b] = __popc(same);
-    __syncthreads();
-    if (b >= 0 && s_base[b] >= 0)
-    {
-      int off = s_base[b] + rank;
-      for (int w = 0; w < warp; ++w) off += s_wcount[w][b];
-      a.out_query[off] = a.query_idx[i];
-      a.out_train[off] = a.train_idx[i];
-      a.out_dist[off] = a.distance[i];
-    }
-    __syncthreads();
-    if (tid < kVaBins && s_base[tid] >= 0)
-    {
-      int add = 0;
-      for (int w = 0; w < kVaThreads / 32; ++w) add += s_wcount[w][tid];
-      s_base[tid] += add;
-    }
-    __syncthreads();
-  }
+  const int n_out = verify_angle_block(
+      a.n, [&](int i) { return angle_bin(a.kps1[a.query_idx[i]].angle, a.kps2[a.train_idx[i]].angle); },
+      [&](int off, int i) {
+        a.out_query[off] = a.query_idx[i];
+        a.out_train[off] = a.train_idx[i];
+        a.out_dist[off] = a.distance[i];
+      });
+  if (threadIdx.x == 0) *a.n_out = n_out;
 }
 
 } // namespace

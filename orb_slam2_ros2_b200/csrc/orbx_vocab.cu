@@ -34,15 +34,6 @@ namespace
 constexpr int kVT = 256;     // threads per CTA
 constexpr int kTile = 4096;  // descriptors per tile
 constexpr unsigned kFull = 0xffffffffu;
-constexpr unsigned long long kGolden = 0x9E3779B97F4A7C15ull;
-
-__host__ __device__ __forceinline__ unsigned long long splitmix64(unsigned long long x)
-{
-  unsigned long long z = x + kGolden;
-  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-  z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-  return z ^ (z >> 31);
-}
 
 struct VbArgs
 {
