@@ -47,10 +47,11 @@ def pose(i: int, n: int = N_LOOP):
     return R_wc.T, C
 
 
-def render(walls: list, R_cw: np.ndarray, C: np.ndarray) -> np.ndarray:
-    """one 8-bit view: every pixel centre's ray from C hits the box from inside"""
-    u, v = np.meshgrid(np.arange(W, dtype=np.float64), np.arange(H, dtype=np.float64))
-    d = np.stack([(u - CX) / FX, (v - CY) / FY, np.ones_like(u)], -1) @ R_cw  # world directions R_wc d, as rows
+def render(walls: list, R_cw: np.ndarray, C: np.ndarray, w: int = W, h: int = H, fx: float = FX, fy: float = FY, cx: float = CX,
+           cy: float = CY) -> np.ndarray:
+    """one 8-bit w x h view through intrinsics fx fy cx cy: every pixel centre's ray from C hits the box from inside"""
+    u, v = np.meshgrid(np.arange(w, dtype=np.float64), np.arange(h, dtype=np.float64))
+    d = np.stack([(u - cx) / fx, (v - cy) / fy, np.ones_like(u)], -1) @ R_cw  # world directions R_wc d, as rows
     t_best = np.full(u.shape, np.inf)
     img = np.zeros(u.shape, np.float32)
     hit_axis = np.full(u.shape, -1)
@@ -74,9 +75,10 @@ def render(walls: list, R_cw: np.ndarray, C: np.ndarray) -> np.ndarray:
     return np.clip(np.rint(img), 0, 255).astype(np.uint8)
 
 
-def stereo(walls, R_cw, C):
+def stereo(walls, R_cw, C, bl: float = BL, **cam):
+    """(left, right) views of a rectified pair with baseline bl; cam: render's image size and intrinsics"""
     R_wc = R_cw.T
-    return render(walls, R_cw, C), render(walls, R_cw, C + R_wc[:, 0] * BL)
+    return render(walls, R_cw, C, **cam), render(walls, R_cw, C + R_wc[:, 0] * bl, **cam)
 
 
 def relative_pose(seq: dict, q: int, c: int):

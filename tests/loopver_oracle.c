@@ -9,8 +9,10 @@
  *                  fx, fy, cx, cy, sf, n_levels,                camera and level scale factors
  *                  q_lo, n_queries, table, top_k,               query i is frame q_lo + i, its candidates table[i][0 .. top_k)
  *                  ratio, min_matches, min_inliers, max_iterations, probability, seed,
- *                  counts, T, match, loop_frame)                [nq][top_k][7]: n_bow n_matches n_corr n_iters hypothesis
+ *                  counts, T, match, loop_frame,                [nq][top_k][7]: n_bow n_matches n_corr n_iters hypothesis
  *                                                               n_inliers accepted; [nq][top_k][12]; [nq][top_k][N]; [nq]
+ *                  first_best)                                  NULL or [nq][top_k]: the first hypothesis that reached the
+ *                                                               reported one's inlier count (-1 without one)
  * The sums follow the rule of include/orbx.h: 32 slot partials, then the tree; the sweep bound is ORBX_LOOPVER_JACOBI_SWEEPS.
  */
 #include <math.h>
@@ -154,7 +156,8 @@ static int is_inlier(const corr_t *k, const double *T, double fx, double fy, dou
 int oracle_loopver(const oracle_vocab *v, int levelsup, int32_t F, int32_t N, const oracle_keypoint *kps, const uint8_t *desc, const double *depth,
                    const int32_t *n, float fx_, float fy_, float cx_, float cy_, const float *sf, int n_levels, int64_t q_lo, int32_t n_queries,
                    const int32_t *table, int32_t top_k, float ratio, int32_t min_matches, int32_t min_inliers, int32_t max_iterations,
-                   double probability, uint64_t seed, int32_t *counts, double *T_out, int32_t *match, int32_t *loop_frame)
+                   double probability, uint64_t seed, int32_t *counts, double *T_out, int32_t *match, int32_t *loop_frame,
+                   int32_t *first_best)
 {
   const double fx = fx_, fy = fy_, cx = cx_, cy = cy_;
   const size_t NN = (size_t)N;
@@ -217,6 +220,7 @@ int oracle_loopver(const oracle_vocab *v, int levelsup, int32_t F, int32_t N, co
       cnt[4] = -1;
       for (int j = 0; j < 12; ++j) T[j] = 0.0;
       for (int j = 0; j < N; ++j) mrow[j] = -1;
+      if (first_best) first_best[o] = -1;
       const int cf = table[o];
       if (cf < 0 || cf >= F) continue;
       const oracle_keypoint *kq = kps + (size_t)qf * NN, *kc = kps + (size_t)cf * NN;
@@ -257,7 +261,7 @@ int oracle_loopver(const oracle_vocab *v, int levelsup, int32_t F, int32_t N, co
       /* Sim3Solver::iterate, one hypothesis after another */
       const int nit = iters[m];
       const uint64_t K = splitmix64(splitmix64(seed_key + (uint64_t)qf + 1) + (uint64_t)cf + 1);
-      int best_h = -1, best_n = 0, acc = 0;
+      int best_h = -1, best_n = 0, acc = 0, first_h = -1;
       double bestT[15], Th[15];
       int *avail = malloc(sizeof(int) * (size_t)(m > 0 ? m : 1));
       for (int h = 0; h < nit; ++h)
@@ -276,6 +280,7 @@ int oracle_loopver(const oracle_vocab *v, int levelsup, int32_t F, int32_t N, co
         for (int i = 0; i < m; ++i) ninl += is_inlier(&corr[i], Th, fx, fy, cx, cy);
         if (ninl >= best_n)
         {
+          if (ninl > best_n || best_h < 0) first_h = h;
           best_n = ninl, best_h = h;
           memcpy(bestT, Th, sizeof(Th));
           if (ninl > min_inliers)
@@ -290,6 +295,7 @@ int oracle_loopver(const oracle_vocab *v, int levelsup, int32_t F, int32_t N, co
       cnt[4] = best_h;
       cnt[5] = best_h >= 0 ? best_n : 0;
       cnt[6] = acc;
+      if (first_best) first_best[o] = first_h;
       if (best_h < 0) continue;
       /* the refit over the inliers of the reported hypothesis (slot = correspondence index) */
       double Tf[15];

@@ -267,13 +267,14 @@ def _oracle_lib():
             shutil.rmtree(tmp, ignore_errors=True)
         lib.oracle_loopver.restype = C.c_int
         lib.oracle_loopver.argtypes = ([C.c_void_p, C.c_int, C.c_int32, C.c_int32] + [C.c_void_p] * 4 + [C.c_float] * 4 + [C.c_void_p, C.c_int, C.c_int64, C.c_int32,
-                                       C.c_void_p, C.c_int32, C.c_float, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_uint64] + [C.c_void_p] * 4)
+                                       C.c_void_p, C.c_int32, C.c_float, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_uint64] + [C.c_void_p] * 5)
         _lib = lib
     return _lib
 
 
 def oracle_verify(O, levelsup: int, fr: dict, cam, sf, q_lo: int, table, prm: dict) -> dict:
-    """oracle_loopver -> dict of LOOPVER_OUTPUTS"""
+    """oracle_loopver -> dict of LOOPVER_OUTPUTS, and first_best [nq][top_k]: the first hypothesis that reached the
+    reported hypothesis's inlier count (-1 without one)"""
     kps = np.ascontiguousarray(fr["kps"])
     desc, depth, n = (np.ascontiguousarray(fr[k], t) for k, t in (("desc", np.uint8), ("depth", np.float64), ("n", np.int32)))
     F, N = kps.shape
@@ -281,13 +282,14 @@ def oracle_verify(O, levelsup: int, fr: dict, cam, sf, q_lo: int, table, prm: di
     nq, top_k = tab.shape
     sfa = np.ascontiguousarray(sf, np.float32)
     counts, T, match, lf = np.zeros((nq, top_k, 7), np.int32), np.zeros((nq, top_k, 12)), np.zeros((nq, top_k, N), np.int32), np.zeros(nq, np.int32)
+    first = np.zeros((nq, top_k), np.int32)
     rc = _oracle_lib().oracle_loopver(C.addressof(O._c), levelsup, F, N, kps.ctypes.data, desc.ctypes.data, depth.ctypes.data, n.ctypes.data, cam[0], cam[1],
                                       cam[2], cam[3], sfa.ctypes.data, len(sfa), q_lo, nq, tab.ctypes.data, top_k, prm["ratio"], prm["min_matches"],
                                       prm["min_inliers"], prm["max_iterations"], prm["probability"], prm["seed"] & M64, counts.ctypes.data, T.ctypes.data,
-                                      match.ctypes.data, lf.ctypes.data)
+                                      match.ctypes.data, lf.ctypes.data, first.ctypes.data)
     assert rc == 0
     out = {k: counts[:, :, i].copy() for i, k in enumerate(COUNTS)}
-    out.update(T=T, match=match, loop_frame=lf)
+    out.update(T=T, match=match, loop_frame=lf, first_best=first)
     return out
 
 
@@ -310,9 +312,16 @@ def rot(axis, deg) -> np.ndarray:
 class _Builder:
     """frames of landmarks (3-D point + descriptor + base angle) seen from known poses X_cam = R X_world + t"""
 
-    def __init__(self, seed: int, kp_dtype):
+    def __init__(self, seed: int, kp_dtype, n_features: int = N_FEATURES, n_levels: int = N_LEVELS, voc=None, levelsup: int = 0):
+        """voc, levelsup: when given, a landmark's copy with flipped bits keeps its landmark's FeatureVector node and a word
+        that is not stopped"""
         self.rng = np.random.default_rng(seed)
         self.kp_dtype = kp_dtype
+        self.N, self.n_levels = n_features, n_levels
+        self.voc, self.levelsup = voc, levelsup
+        if voc is not None:
+            self.bits = np.unpackbits(voc["desc"], axis=1)
+            self.children = [np.flatnonzero(voc["parent"] == p) for p in range(len(voc["parent"]) + 1)]
         self.frames = []
 
     def landmarks(self, P) -> list:
@@ -322,9 +331,30 @@ class _Builder:
     def box(self, n, z=(3.0, 7.0)) -> list:
         return self.landmarks(np.stack([self.rng.uniform(-2, 2, n), self.rng.uniform(-1.5, 1.5, n), self.rng.uniform(*z, n)], 1))
 
-    def frame(self, lms, R=np.eye(3), t=(0, 0, 0), spin=0.0, no_depth=(), wrong=(), bad_angle=(), extra=20) -> int:
+    def node(self, d) -> int:
+        """the FeatureVector node descriptor d descends to (oracle_bow_descend), or -1 for a stopped word"""
+        b, node, at, level = np.unpackbits(d), 0, 0, 0
+        while len(self.children[node]):
+            level += 1
+            c = self.children[node]
+            node = int(c[(self.bits[c] != b).sum(1).argmin()]) + 1  # record i is node i + 1
+            if level == self.voc["L"] - self.levelsup:
+                at = node
+        return at if self.voc["weight"][node - 1] > 0 else -1
+
+    def copy_desc(self, d, flip: int):
+        """d with `flip` random bits flipped, in d's node"""
+        while True:
+            c = d.copy()
+            for b in self.rng.choice(256, flip, replace=False):
+                c[b // 8] ^= np.uint8(1 << (b % 8))
+            if self.voc is None or self.node(c) == self.node(d):
+                return c
+
+    def frame(self, lms, R=np.eye(3), t=(0, 0, 0), spin=0.0, no_depth=(), wrong=(), bad_angle=(), extra=20, turn=None, flip=0) -> int:
         """features: every landmark (those in `wrong` at a random point instead), `extra` distractors; no_depth: landmark
-        positions in `lms` whose feature has no depth; bad_angle: positions whose angle breaks the rotation check"""
+        positions in `lms` whose feature has no depth; bad_angle: positions whose angle breaks the rotation check; turn:
+        {position: degrees} added to those landmarks' angles as given; flip: bits flipped in each landmark's descriptor"""
         feats = []
         bad = sorted(bad_angle)
         for i, lm in enumerate(lms):
@@ -332,20 +362,22 @@ class _Builder:
             if i in wrong:
                 X = np.array([self.rng.uniform(-3, 3), self.rng.uniform(-2, 2), self.rng.uniform(2, 9)])
             ang = lm["a"] - spin + (60.0 + 40.0 * bad.index(i) if i in bad_angle else 0.0)  # one rotation bin each
+            if turn is not None:
+                ang += turn.get(i, 0.0)
             ang = (ang + 180.0) % 360.0 - 180.0
-            feats.append((X, lm["d"], ang, -1.0 if i in no_depth else X[2]))
+            feats.append((X, self.copy_desc(lm["d"], flip) if flip else lm["d"], ang, -1.0 if i in no_depth else X[2]))
         for _ in range(extra):
             X = np.array([self.rng.uniform(-2, 2), self.rng.uniform(-1.5, 1.5), self.rng.uniform(3, 7)])
             feats.append((X, self.rng.integers(0, 256, 32, dtype=np.uint8), float(self.rng.uniform(-170, 170)), X[2]))
-        assert len(feats) <= N_FEATURES
+        assert len(feats) <= self.N
         order = self.rng.permutation(len(feats))
-        kps = np.zeros(N_FEATURES, self.kp_dtype)
-        desc = np.zeros((N_FEATURES, 32), np.uint8)
-        depth = np.zeros(N_FEATURES)
+        kps = np.zeros(self.N, self.kp_dtype)
+        desc = np.zeros((self.N, 32), np.uint8)
+        depth = np.zeros(self.N)
         for j, k in enumerate(order):
             X, d, ang, z = feats[k]
             kps[j]["x"], kps[j]["y"] = np.float32(CAM[0] * X[0] / X[2] + CAM[2]), np.float32(CAM[1] * X[1] / X[2] + CAM[3])
-            kps[j]["angle"], kps[j]["octave"], kps[j]["size"] = ang, int(self.rng.integers(0, N_LEVELS)), 7.0
+            kps[j]["angle"], kps[j]["octave"], kps[j]["size"] = ang, int(self.rng.integers(0, self.n_levels)), 7.0
             desc[j], depth[j] = d, z
         self.frames.append((kps, desc, depth, len(feats)))
         return len(self.frames) - 1
@@ -396,6 +428,74 @@ def crafted(kp_dtype, seed: int = 3) -> dict:
     configs = [params(), params(seed=7), params(min_inliers=8, min_matches=12, seed=11), params(ratio=0.6, max_iterations=4, seed=5),
                params(min_inliers=3, min_matches=3, max_iterations=40, probability=0.5, seed=2)]
     return dict(frames=fr, table=table, configs=configs, truth=truth, levelsup=2, voc=synth.synth_vocabulary(10, 3, 21))
+
+
+def crafted_large(kp_dtype, N: int = 2000, n_levels: int = 8, seed: int = 1, param_seeds=(0, 0, 0)) -> dict:
+    """record sets at the benchmark's frame size that reach the verifier's block structure -> the dict of crafted() (no truth).
+
+    Scene A: a query of N features (1400 landmarks, five of them twice, 595 distractors) and ten candidates of
+    0 / 255 / 256 / 257 / 512 / 513 / N features, and three whose rotation check keeps 256 and 257 of 296 and 297 kept rows
+    (bins 10, 15 and 20 tie behind bin 0: bin 20 is dropped) or whose depths leave 256 and 257 correspondences.  With
+    levelsup 2 the FeatureVector node is one of the root's 10 children, so a row's candidates span several 32-lane chunks,
+    and the landmark copies differ by 3 bits from their originals.  Angles are multiples of 0.5 degrees, so angle
+    differences fall on bin edges; a few lie 2^-24 and 0.5 degrees below 360.
+    Scene R: eight queries of 200 features, each with six candidates of 25-40 % inliers in shuffled slots (accepted at a
+    hypothesis spread over many rounds of eight), one with exactly min_inliers = 20 inliers of 60 (never accepted: the
+    maxima tie across rounds), one with 20 inliers of 150 (runs to max_iterations), and itself.
+    configs: max_iterations 300, 157 and 299 (ratio 1.0: the rows whose two best distances tie are kept), seeds param_seeds."""
+    voc = synth.synth_vocabulary(10, 3, 21)
+    B = _Builder(seed, kp_dtype, N, n_levels, voc=voc, levelsup=2)
+    rows = []
+    Rc, tc = rot([0.2, 1, 0.1], 8.0), np.array([0.25, -0.05, 0.1])
+
+    def lms(n):
+        L = B.box(n)
+        for lm in L:
+            lm["a"] = round(2.0 * lm["a"]) / 2.0
+            while B.node(lm["d"]) < 0:  # a stopped word has no FeatureVector entry
+                lm["d"] = B.rng.integers(0, 256, 32, dtype=np.uint8)
+        return L
+
+    def cand(L, **kw):
+        return B.frame(L, Rc, tc, flip=3, **kw)
+
+    # scene A
+    LA = lms(1400)
+    for lm in LA[5:10]:
+        lm["a"] = 0.5
+    qa = B.frame(LA + LA[:5], no_depth=set(range(1300, 1310)), extra=N - 1405)
+    empty = B.frame([], extra=0)
+    sizes = [cand(LA[10 : 10 + n], extra=0) for n in (255, 256, 257, 512, 513)]
+    edge = {i: 2.0**-24 for i in (5, 6, 7)} | {8: 0.5, 9: 0.5}
+    full = cand(LA, extra=N - 1400, turn=edge, no_depth=set(range(1200, 1260)))
+
+    def tied(main, no_depth=()):
+        g = {main + i: -120.0 for i in range(40)} | {main + 40 + i: -180.0 for i in range(40)} | {main + 80 + i: -240.0 for i in range(40)}
+        return cand(LA[10 : 10 + main + 120], extra=0, turn=g, no_depth=no_depth)
+
+    rows.append((qa, [empty] + sizes + [full, tied(176), tied(177, no_depth={0}), cand(LA[10:310], extra=0, no_depth=set(range(43)))]))
+    # scene R
+    for _ in range(8):
+        L = lms(160)
+        q = B.frame(L, extra=40)
+        cs = []
+        for _ in range(6):
+            n_in = int(B.rng.integers(26, 41))
+            n = min(int(B.rng.integers(int(n_in / 0.4), int(n_in / 0.25) + 1)), 120)
+            cs.append(cand(L[:n], spin=12.0, wrong=set(B.rng.choice(n, n - n_in, replace=False).tolist())))
+        cs.append(cand(L[:60], spin=12.0, wrong=set(range(20, 60))))
+        cs.append(cand(L[:150], spin=12.0, wrong=set(range(20, 150))))
+        order = B.rng.permutation(len(cs))
+        rows.append((q, [cs[i] for i in order] + [q, -1]))
+    fr = B.arrays()
+    F = len(fr["n"])
+    table = np.full((F, 10), -1, np.int32)
+    for q, cands in rows:
+        table[q, : len(cands)] = cands
+    table[empty, :2] = [qa, sizes[0]]  # a query without features
+    s0, s1, s2 = param_seeds
+    configs = [params(seed=s0), params(max_iterations=157, seed=s1), params(ratio=1.0, max_iterations=299, seed=s2)]
+    return dict(frames=fr, table=table, configs=configs, levelsup=2, voc=voc)
 
 
 def to_records(ctx, fr: dict) -> np.ndarray:
