@@ -382,6 +382,14 @@ int orbx_vocab_arrays(const orbx_vocab *vocab, int32_t *parent, uint8_t *is_leaf
  * default "%g", 6 significant digits, as in orbx_serialize_keyframe_text).  ORBX_ERR_FILE_NOT_OPEN if it cannot be written. */
 int orbx_vocab_save_text(const orbx_vocab *vocab, const char *path);
 
+/* Most descriptors per frame any bag-of-words entry point takes: the transform, the vocabulary build's TF_IDF step and the
+ * keyframe database sort a frame's (id << 16 | feature) keys as one power-of-two array of 8-byte keys in one CTA's shared
+ * memory, and 16384 keys (128 KB) is the largest such sort that fits the 227 KB a block may have; 16385 would need 32768
+ * keys (256 KB).  orbx_vocab_build / orbx_bowdb_build return ORBX_ERR_INVALID_ARG for a larger stride, and
+ * orbx_bow_transform* / orbx_loopver_build ORBX_ERR_CAPACITY on a context with more n_features, before anything is
+ * enqueued.  Extraction and stereo keep the 65535 of orbx_config.n_features. */
+#define ORBX_BOW_MAX_STRIDE 16384
+
 /* ---- vocabulary construction on the device ------------------------------------------------------------------- */
 /* replaces: DBoW2 / DBoW3 TemplatedVocabulary::create (HKmeansStep, initiateClustersKMpp, FORB::meanValue, createWords,
  * setNodeWeights), the step that makes the ORBvoc.txt the reference loads (src/System.cc:93), from the training set
@@ -409,7 +417,7 @@ typedef struct orbx_vocab_train {
   const uint8_t *desc;    /* [n_frames][stride][32] */
   const int32_t *n_kps;   /* [n_frames], each 0..stride */
   int32_t n_frames;       /* the N of TF_IDF: pass F, not the padded row count of a gather */
-  int32_t stride;         /* descriptors per frame row (1..65535) */
+  int32_t stride;         /* descriptors per frame row (1..ORBX_BOW_MAX_STRIDE) */
   int32_t on_device;      /* 1: desc / n_kps are device memory of ctx's device (e.g. the gathered arrays), 0: host */
   int32_t k, L;           /* branching factor (2..ORBX_VOCAB_MAX_K) and depth levels (>= 1; at most INT32_MAX nodes) */
   uint64_t seed;
@@ -417,7 +425,8 @@ typedef struct orbx_vocab_train {
   int32_t *n_capped;      /* optional host: nodes that stopped at ORBX_VOCAB_MAX_ITERS */
   float *level_ms;        /* optional host [L + 1]: CUDA-event time of each level, then of the TF_IDF step */
 } orbx_vocab_train;
-/* ORBX_ERR_INVALID_ARG for bad k / L / sizes (before anything is enqueued), counts outside 0..stride or no descriptor at all */
+/* ORBX_ERR_INVALID_ARG for bad k / L / sizes, a stride above ORBX_BOW_MAX_STRIDE (before anything is enqueued), counts
+ * outside 0..stride or no descriptor at all */
 int orbx_vocab_build(orbx_ctx *ctx, const orbx_vocab_train *in, orbx_vocab **out);
 
 /* replaces: VirtualFrame::computeBow (include/ORB_SLAM2/Frame.h:224-231) = DBoW3::Vocabulary::transform(mvLeftDescriptor,
@@ -477,7 +486,7 @@ int orbx_search_by_bow(orbx_ctx *ctx, int frame, int n_kf_nodes, const int32_t *
 #define ORBX_BOWDB_MAX_FRAMES 98304 /* 16-bit shared-word counters of every frame in the query kernel's shared memory: 192 KB */
 typedef struct orbx_bowdb orbx_bowdb;
 /* n_frames: the sequence's F (not the padded row count of a gather), 1..ORBX_BOWDB_MAX_FRAMES (ORBX_ERR_CAPACITY above);
- * stride: descriptors per frame row (1..65535); counts 0..stride; on_device: desc / n_kps are device memory of ctx's device.
+ * stride: descriptors per frame row (1..ORBX_BOW_MAX_STRIDE, else ORBX_ERR_INVALID_ARG); counts 0..stride; on_device: desc / n_kps are device memory of ctx's device.
  * vocab must belong to ctx.  Blocks until the database is built; leaves the context's resident frames, their bag of words and
  * the frame epoch untouched. */
 int orbx_bowdb_build(orbx_ctx *ctx, const orbx_vocab *vocab, const uint8_t *desc /* [n_frames][stride][32] */, const int32_t *n_kps /* [n_frames] */,
@@ -545,7 +554,8 @@ int orbx_bowdb_query_frame(orbx_ctx *ctx, const orbx_bowdb *db, int frame, const
 typedef struct orbx_loopver orbx_loopver;
 /* records: the F frames' orbx_record_layout records, [F][record_stride] (>= record_bytes, multiple of 16), host or device memory
  * of ctx's device; device records must be 16-byte aligned (they are read in place), else ORBX_ERR_INVALID_ARG.  The verifier copies what it needs into arrays it owns; `records` may be freed afterwards.  vocab must
- * belong to ctx; levelsup >= 0 (>= L: the FeatureVector node is the root, as in orbx_bow_transform).  Blocks until the verifier is built; leaves the context's resident frames and their bag of words untouched. */
+ * belong to ctx; levelsup >= 0 (>= L: the FeatureVector node is the root, as in orbx_bow_transform); ORBX_ERR_CAPACITY when the
+ * context's n_features exceeds ORBX_BOW_MAX_STRIDE.  Blocks until the verifier is built; leaves the context's resident frames and their bag of words untouched. */
 int orbx_loopver_build(orbx_ctx *ctx, const orbx_vocab *vocab, int32_t levelsup, const void *records, size_t record_stride,
                        int32_t n_frames, int32_t on_device, orbx_loopver **out);
 void orbx_loopver_destroy(orbx_loopver *lv);

@@ -109,6 +109,7 @@ class OrbxKeyframeIO(C.Structure):
 
 
 VOCAB_MAX_ITERS, VOCAB_MAX_K = 100, 32  # ORBX_VOCAB_MAX_ITERS / ORBX_VOCAB_MAX_K
+BOW_MAX_STRIDE = 16384  # ORBX_BOW_MAX_STRIDE: most descriptors per frame of the bag-of-words entry points
 
 
 class OrbxVocabTrain(C.Structure):

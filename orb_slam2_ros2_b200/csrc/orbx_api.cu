@@ -474,8 +474,8 @@ int bow_buffers(orbx_ctx *c)
   if (c->bow_ready) return ORBX_OK;
   // one frame per image: a mono / RGB-D batch leaves up to n_img_max = 2 * max_batch frames resident
   const size_t F = (size_t)c->n_img_max, N = (size_t)c->cfg.n_features;
-  if (N > 65535) return fail(c, ORBX_ERR_CAPACITY, "the bag-of-words kernels index features with 16 bits");
   int rc;
+  if ((rc = bow_configure(c, (int)N, ORBX_ERR_CAPACITY))) return rc;
   BowArgs &b = c->bow;
   if ((rc = dev_alloc(c, &b.f_word, F * N))) return rc;
   if ((rc = dev_alloc(c, &b.f_nid, F * N))) return rc;
@@ -487,7 +487,6 @@ int bow_buffers(orbx_ctx *c)
   if ((rc = dev_alloc(c, &b.fv_start, F * (N + 1)))) return rc;
   if ((rc = dev_alloc(c, &b.fv_feats, F * N))) return rc;
   if ((rc = dev_alloc(c, &b.n_fv, F))) return rc;
-  if (bow_configure((int)N) != 0) return fail(c, ORBX_ERR_CUDA, "cannot reserve shared memory for the bag-of-words sort");
   c->bow_ready = true;
   return ORBX_OK;
 }

@@ -10,7 +10,7 @@
 //                        (std::map<NodeId, vector<unsigned>>) from two stable sorts of (key << 16 | feature index)
 //   bow_word_frames_kernel  one CTA per frame: the frame's distinct words (the same sort), one integer atomic per word;
 //                        N_i of TF_IDF for orbx_vocab_build (setNodeWeights)
-#include "orbx_device.cuh"
+#include "orbx_internal.h"
 
 namespace orbx
 {
@@ -249,13 +249,15 @@ void launch_bow_word_frames(const Params &p, const BowArgs &a, int n_frames, int
   bow_word_frames_kernel<<<n_frames, kAsmThreads, (size_t)P * sizeof(unsigned long long), s>>>(p, a, P, n_frames_of_word);
 }
 
-int bow_configure(int n_features)
+int bow_configure(orbx_ctx *c, int n_features, int too_large)
 {
+  if (n_features > ORBX_BOW_MAX_STRIDE) return fail(c, too_large, "the bag-of-words sort holds at most ORBX_BOW_MAX_STRIDE (16384) features per frame");
   const size_t bytes = (size_t)bow_sort_size(n_features) * sizeof(unsigned long long);
-  if (bytes <= 48 * 1024) return 0;
+  if (bytes <= 48 * 1024) return ORBX_OK;
   static SmemOptIn state, state_words;
-  if (raise_dynamic_smem(bow_assemble_kernel, state, bytes)) return -1;
-  return raise_dynamic_smem(bow_word_frames_kernel, state_words, bytes);
+  if (raise_dynamic_smem(bow_assemble_kernel, state, bytes) || raise_dynamic_smem(bow_word_frames_kernel, state_words, bytes))
+    return fail(c, ORBX_ERR_CUDA, "cannot reserve shared memory for the bag-of-words sort");
+  return ORBX_OK;
 }
 
 } // namespace orbx

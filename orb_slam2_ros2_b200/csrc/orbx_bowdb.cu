@@ -466,9 +466,10 @@ extern "C"
     if (v->ctx != c || v->device != c->device) return fail(c, ORBX_ERR_INVALID_ARG, "the vocabulary belongs to another context");
     if (F < 1) return fail(c, ORBX_ERR_INVALID_ARG, "keyframe database: n_frames < 1");
     if (F > ORBX_BOWDB_MAX_FRAMES) return fail(c, ORBX_ERR_CAPACITY, "keyframe database: more than ORBX_BOWDB_MAX_FRAMES frames");
-    if (stride < 1 || stride > 65535) return fail(c, ORBX_ERR_INVALID_ARG, "keyframe database: stride outside 1..65535");
+    if (stride < 1) return fail(c, ORBX_ERR_INVALID_ARG, "keyframe database: stride < 1");
     cudaStream_t s = c->stream;
     ORBX_CUDA(c, cudaSetDevice(c->device));
+    if (int rc = bow_configure(c, stride, ORBX_ERR_INVALID_ARG)) return rc;
     std::vector<int32_t> h_n((size_t)F);
     if (on_device)
     {
@@ -479,7 +480,6 @@ extern "C"
       std::memcpy(h_n.data(), n_kps, (size_t)F * 4);
     for (int f = 0; f < F; ++f)
       if (h_n[(size_t)f] < 0 || h_n[(size_t)f] > stride) return fail(c, ORBX_ERR_INVALID_ARG, "keyframe database: a count lies outside 0..stride");
-    if (bow_configure(stride) != 0) return fail(c, ORBX_ERR_CUDA, "cannot reserve shared memory for the bag-of-words sort");
 
     orbx_bowdb *db = new orbx_bowdb();
     DbGuard guard{db};

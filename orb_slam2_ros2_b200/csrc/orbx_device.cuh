@@ -250,7 +250,6 @@ void launch_serialize(const Params &p, const SerArgs &a, int n_frames, cudaStrea
 void launch_bow_descend(const Params &p, const BowArgs &a, int n_frames, cudaStream_t s);
 void launch_bow_assemble(const Params &p, const BowArgs &a, int n_frames, cudaStream_t s);
 void launch_bow_word_frames(const Params &p, const BowArgs &a, int n_frames, int *n_frames_of_word, cudaStream_t s);
-int bow_configure(int n_features); // opt in to the dynamic shared memory of the assemble and word-frame kernels
 size_t quadtree_smem_bytes(int list_cap, int node_cap, int big_cap, int max_level_cells);
 int quadtree_configure(size_t smem_bytes); // opt in to large dynamic shared memory
 
@@ -266,7 +265,8 @@ __host__ __device__ __forceinline__ unsigned long long splitmix64(unsigned long 
 
 // cudaFuncAttributeMaxDynamicSharedMemorySize belongs to the kernel (per device), not to a context: it is only ever RAISED, so a
 // second context with a smaller configuration cannot shrink the limit under a live one (launches of the larger context would
-// fail with "invalid argument").  `state` = the caller's per-kernel high-water marks, one per device.
+// fail with "invalid argument").  `state` = the caller's per-kernel high-water marks, one per device.  A refused size is
+// cleared from the runtime's last error, so that it is not reported again by an unrelated call's cudaGetLastError.
 struct SmemOptIn
 {
   std::mutex mu;
@@ -278,7 +278,11 @@ template <class Kernel> int raise_dynamic_smem(Kernel kernel, SmemOptIn &state, 
   if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return -1;
   std::lock_guard<std::mutex> lock(state.mu);
   if ((size_t)state.high[dev] >= bytes) return 0;
-  if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) != cudaSuccess) return -1;
+  if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) != cudaSuccess)
+  {
+    cudaGetLastError();
+    return -1;
+  }
   state.high[dev] = (int)bytes;
   return 0;
 }

@@ -129,6 +129,10 @@ void destroy_self_comm(orbx_ctx *c);
 int require_bow(orbx_ctx *c, int64_t end);
 // allocates the context's bag-of-words result buffers (n_img_max frames, as many as an RGB-D batch holds) on first use
 int bow_buffers(orbx_ctx *c);
+// every bag-of-words entry point's check before it enqueues anything: `too_large` (the caller's error code) for more than
+// ORBX_BOW_MAX_STRIDE features per frame, else opts the assemble and word-frame kernels in to the sort's shared memory
+// (ORBX_ERR_CUDA if that fails).  Needs the context's device current.
+int bow_configure(orbx_ctx *c, int n_features, int too_large);
 // c->bow with the vocabulary's tree, ready for launch_bow_descend / launch_bow_assemble over device slots whose frame f
 // reads image f * image_stride
 BowArgs bow_args(const orbx_ctx *c, const orbx_vocab *v, int levelsup, int image_stride);

@@ -513,7 +513,7 @@ extern "C"
     const int N = c->cfg.n_features;
     cudaStream_t s = c->stream;
     ORBX_CUDA(c, cudaSetDevice(c->device));
-    if (bow_configure(N) != 0) return fail(c, ORBX_ERR_CUDA, "cannot reserve shared memory for the bag-of-words sort");
+    if (int rc = bow_configure(c, N, ORBX_ERR_CAPACITY)) return rc;
     orbx_loopver *lv = new orbx_loopver();
     LvGuard guard{lv};
     lv->ctx = c, lv->vocab = v, lv->device = c->device, lv->F = F, lv->N = N;

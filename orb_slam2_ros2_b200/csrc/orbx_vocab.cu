@@ -437,8 +437,7 @@ extern "C" int orbx_vocab_build(orbx_ctx *c, const orbx_vocab_train *in, orbx_vo
   if (!c || !in || !out) return ORBX_ERR_INVALID_ARG;
   *out = nullptr;
   const int k = in->k, L = in->L, F = in->n_frames, stride = in->stride;
-  if (!in->desc || !in->n_kps || F < 1 || stride < 1 || stride > 65535)
-    return fail(c, ORBX_ERR_INVALID_ARG, "vocabulary training set: desc / n_kps missing, n_frames < 1 or stride outside 1..65535");
+  if (!in->desc || !in->n_kps || F < 1 || stride < 1) return fail(c, ORBX_ERR_INVALID_ARG, "vocabulary training set: desc / n_kps missing, n_frames < 1 or stride < 1");
   if (k < 2 || k > ORBX_VOCAB_MAX_K || L < 1) return fail(c, ORBX_ERR_INVALID_ARG, "vocabulary build: k must be 2..ORBX_VOCAB_MAX_K and L >= 1");
   {
     // a full tree of k^1 + .. + k^L nodes (+ the root) must fit int32 node ids
@@ -448,6 +447,7 @@ extern "C" int orbx_vocab_build(orbx_ctx *c, const orbx_vocab_train *in, orbx_vo
   }
   cudaStream_t s = c->stream;
   ORBX_CUDA(c, cudaSetDevice(c->device));
+  if (int rc = bow_configure(c, stride, ORBX_ERR_INVALID_ARG)) return rc; // the TF_IDF step sorts a frame row in shared memory
   Scratch sc;
   sc.dev = c->device;
   // counts on the host: row offsets of the gather, validation
@@ -735,7 +735,6 @@ extern "C" int orbx_vocab_build(orbx_ctx *c, const orbx_vocab_train *in, orbx_vo
   if (e == cudaSuccess) e = sc.get(&ni, (size_t)v->n_words);
   if (e == cudaSuccess) e = cudaMemsetAsync(ni, 0, (size_t)v->n_words * 4, s);
   if (e != cudaSuccess) return fail_v(ORBX_ERR_CUDA, std::string("vocabulary IDF buffers: ") + cudaGetErrorString(e));
-  if (bow_configure(stride) != 0) return fail_v(ORBX_ERR_CUDA, "cannot reserve shared memory for the bag-of-words sort");
   BowArgs b{};
   b.child_start = v->child_start, b.child_ids = v->child_ids, b.v_desc = v->desc, b.v_weight = v->weight, b.v_word = v->word;
   b.L = L, b.levelsup = 0, b.image_stride = 1;

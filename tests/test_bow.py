@@ -112,6 +112,20 @@ def test_cuda_bow_equals_oracle(oracle, tmp_path):
     ctx.close()
 
 
+def _read_device_bow(ctx, d, n):
+    """the n frames of a bow_transform_batch_device result as bow_transform dicts"""
+    N = d.stride
+    nb = ctx.read_device(d.n_bow, (n,), np.int32)
+    nf = ctx.read_device(d.n_fv_nodes, (n,), np.int32)
+    ids = ctx.read_device(d.bow_ids, (n, N), np.int32)
+    vals = ctx.read_device(d.bow_vals, (n, N), np.float64)
+    fnodes = ctx.read_device(d.fv_nodes, (n, N), np.int32)
+    fstart = ctx.read_device(d.fv_start, (n, N + 1), np.int32)
+    ffeats = ctx.read_device(d.fv_feats, (n, N), np.int32)
+    return [dict(bow_ids=ids[f, : nb[f]], bow_vals=vals[f, : nb[f]], fv_nodes=fnodes[f, : nf[f]], fv_start=fstart[f, : nf[f] + 1],
+                 fv_feats=ffeats[f, : fstart[f, nf[f]]]) for f in range(n)]
+
+
 @pytest.mark.gpu
 def test_cuda_bow_batch_device_rgbd_and_empty(oracle):
     import torch
@@ -130,19 +144,8 @@ def test_cuda_bow_batch_device_rgbd_and_empty(oracle):
     before = ctx.launch_count
     d = ctx.bow_transform_batch_device(V, n, 4)
     assert ctx.launch_count - before == 2
-    N = d.stride
-    nb = ctx.read_device(d.n_bow, (n,), np.int32)
-    nf = ctx.read_device(d.n_fv_nodes, (n,), np.int32)
-    ids = ctx.read_device(d.bow_ids, (n, N), np.int32)
-    vals = ctx.read_device(d.bow_vals, (n, N), np.float64)
-    fnodes = ctx.read_device(d.fv_nodes, (n, N), np.int32)
-    fstart = ctx.read_device(d.fv_start, (n, N + 1), np.int32)
-    ffeats = ctx.read_device(d.fv_feats, (n, N), np.int32)
-    for f in range(n):
-        e = oracle.bow_transform(O, host.desc_left[f][: host.n_left[f]], 4)
-        got = dict(bow_ids=ids[f, : nb[f]], bow_vals=vals[f, : nb[f]], fv_nodes=fnodes[f, : nf[f]], fv_start=fstart[f, : nf[f] + 1],
-                   fv_feats=ffeats[f, : fstart[f, nf[f]]])
-        _same(got, e, f"frame {f}")
+    for f, got in enumerate(_read_device_bow(ctx, d, n)):
+        _same(got, oracle.bow_transform(O, host.desc_left[f][: host.n_left[f]], 4), f"frame {f}")
     # searchByBow against a frame of the batch other than frame 0 (frame 2 vs frame 0's features as the "keyframe")
     e2, e0 = oracle.bow_transform(O, host.desc_left[2][: host.n_left[2]], 4), oracle.bow_transform(O, host.desc_left[0][: host.n_left[0]], 4)
     got = ctx.search_by_bow(e0, host.desc_left[0][: host.n_left[0]], frame=2)
@@ -162,6 +165,116 @@ def test_cuda_bow_batch_device_rgbd_and_empty(oracle):
     ctx.stereo_frame(np.full((c["height"], c["width"]), 80, np.uint8), np.full((c["height"], c["width"]), 80, np.uint8))
     got = ctx.bow_transform(V)
     assert len(got["bow_ids"]) == 0 and len(got["fv_nodes"]) == 0 and len(got["fv_feats"]) == 0
+    V.close()
+    ctx.close()
+
+
+_POP = np.array([bin(i).count("1") for i in range(256)], np.uint8)
+
+
+def _shared_minima(O, desc) -> int:
+    """descriptors whose descent meets, at some level, the smallest distance at two children (where the first among equals
+    decides), found by a numpy descent of all of them at once"""
+    node = np.zeros(len(desc), np.int64)
+    tie = np.zeros(len(desc), bool)
+    live = np.ones(len(desc), bool)
+    kmax = int(np.diff(O.child_start).max())
+    while live.any():
+        i = np.nonzero(live)[0]
+        c0, c1 = O.child_start[node[i]], O.child_start[node[i] + 1]
+        j = c0[:, None] + np.arange(kmax)
+        ok = j < c1[:, None]
+        ids = O.child_ids[np.where(ok, j, c0[:, None])]
+        d = _POP[O.desc[ids] ^ desc[i][:, None]].sum(-1, dtype=np.int32)
+        d[~ok] = 1 << 20
+        tie[i] |= (d == d.min(1)[:, None]).sum(1) > 1
+        node[i] = ids[np.arange(len(i)), d.argmin(1)]
+        live[i] = O.child_start[node[i]] != O.child_start[node[i] + 1]
+    return int(tie.sum())
+
+
+@pytest.mark.gpu
+def test_cuda_bow_at_the_bench_shape(oracle):
+    """bench.py's transform: 64 KITTI stereo frames of up to 2000 features in one bow_transform_batch_device call, on the
+    k = 10, L = 6 synthetic vocabulary of about a million nodes"""
+    import torch
+
+    c = synth.KITTI
+    n = 64
+    lefts, rights = synth.synth_stereo_pool(c["height"], c["width"], n, seed0=0)
+    ctx = api.Context(c["width"], c["height"], 2000, 8, 1.2, camera=api.Camera(c["fx"], c["fy"], c["cx"], c["cy"], c["bl"]), max_batch=n)
+    voc = synth.synth_vocabulary(10, 6, 0)
+    O, V = oracle.Vocabulary(**voc), api.Vocabulary(ctx, **voc)
+    assert O.n_nodes > 900000
+    dl, dr = torch.from_numpy(lefts).cuda(), torch.from_numpy(rights).cuda()
+    torch.cuda.synchronize()
+    res = ctx.stereo_batch_device(n, dl.data_ptr(), dr.data_ptr(), c["width"], c["width"] * c["height"])
+    N = ctx.n_features
+    desc = ctx.read_device(res.desc, (2 * n, N, 32), np.uint8)[0::2]  # image 2f = frame f's left image
+    nk = ctx.read_device(res.n_kps, (2 * n,), np.int32)[0::2]
+    assert nk.min() > 1000
+    got = _read_device_bow(ctx, ctx.bow_transform_batch_device(V, n, 4), n)
+    for f in range(n):
+        _same(got[f], oracle.bow_transform(O, desc[f][: nk[f]], 4), f"frame {f}")
+    assert sum(len(g["bow_ids"]) for g in got) > 50000
+    for up in (0, 6):
+        f = 37
+        _same(ctx.bow_transform(V, frame=f, levelsup=up), oracle.bow_transform(O, desc[f][: nk[f]], up), f"frame {f} levelsup {up}")
+    assert _shared_minima(O, np.concatenate([desc[f][: nk[f]] for f in range(n)])) > 0
+    V.close()
+    ctx.close()
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("n_features", [4097, 5000, 16384])
+def test_cuda_bow_past_4096_features(oracle, n_features):
+    """frames of more than 4096 keypoints: bow_assemble_kernel sorts 8192 or 16384 keys in shared memory opted in past 48 KB"""
+    h, w = 1200, 1600
+    rng = np.random.default_rng(n_features)
+    img = rng.integers(0, 256, (h, w), dtype=np.uint8)
+    ctx = api.Context(w, h, n_features, 8, 1.2, camera=api.Camera(1000.0, 1000.0, w / 2, h / 2, 0.1))
+    r = ctx.stereo_frame(img, np.ascontiguousarray(np.roll(img, -4, axis=1)))
+    n = len(r.desc_left)
+    assert n > 4096 and (n_features < 16384 or n > 8192), n
+    voc = synth.synth_vocabulary(10, 4, 5)
+    O0 = oracle.Vocabulary(**voc)
+    leaves = np.nonzero(O0.word_id >= 0)[0]
+    voc["desc"][leaves[:3000] - 1] = r.desc_left[rng.choice(n, 3000, replace=False)]  # leaves that the frame's features reach
+    O, V = oracle.Vocabulary(**voc), api.Vocabulary(ctx, **voc)
+    for up in (4, 0):
+        _same(ctx.bow_transform(V, levelsup=up), oracle.bow_transform(O, r.desc_left, up), f"levelsup {up}")
+    V.close()
+    ctx.close()
+
+
+@pytest.mark.gpu
+def test_cuda_database_at_stride_8193(oracle):
+    """a keyframe database from host rows of 8193 descriptors, one frame full: the transform's sort of 16384 keys"""
+    import bowdb_restatement as BR
+
+    stride = 8193
+    voc = synth.synth_vocabulary(10, 3, 6)
+    O = oracle.Vocabulary(**voc)
+    leaves = np.nonzero(O.word_id >= 0)[0]
+    rng = np.random.default_rng(8193)
+    pool = voc["desc"][rng.choice(leaves, 600, replace=False) - 1]
+    counts = np.array([stride, 0, 3000, stride - 1, 40, 5000, 700], np.int32)
+    desc = rng.integers(0, 256, (len(counts), stride, 32), dtype=np.uint8)
+    for f, m in enumerate(counts):  # each frame from its own window of the pool: neighbours share words, far frames fewer
+        desc[f, :m] = pool[(f * 60 + rng.integers(0, 200, m)) % len(pool)]
+    ctx = api.Context(320, 240, 500, 4, 1.2, camera=api.Camera(300.0, 300.0, 160.0, 120.0, 0.1))
+    V = api.Vocabulary(ctx, **voc)
+    D = api.BowDatabase.build(ctx, V, desc, counts)
+    db = BR.bow_arrays(oracle, O, desc, counts)
+    assert D.info() == dict(n_frames=len(counts), n_words=db["n_words"], n_postings=int(db["n"].sum()))
+    for window, min_score, top_k in [(0, 0.0, 6), (1, 0.0, 3), (0, 0.05, 2)]:
+        exp = BR.oracle_query(db, db, 0, window, min_score, top_k)
+        got = D.query(0, len(counts), top_k, window, min_score)
+        for k in api.BOWDB_OUTPUTS:
+            g, e = np.asarray(got[k]), exp[k]
+            assert np.array_equal(g.view(np.uint32) if k == "cand_score" else g, e.view(np.uint32) if k == "cand_score" else e), (window, k)
+    assert exp["n_scored"].max() > 0 and db["n"].max() > 150
+    D.close()
     V.close()
     ctx.close()
 

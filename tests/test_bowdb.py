@@ -249,8 +249,8 @@ def test_cuda_database_rejects_bad_arguments(cases):
     bad[3] = -1
     with pytest.raises(ValueError, match="invalid argument"):
         api.BowDatabase.build(ctx, V, desc, bad)
-    with pytest.raises(ValueError, match="invalid argument"):  # stride outside 1..65535
-        api.BowDatabase.build(ctx, V, np.zeros((1, 65536, 32), np.uint8), np.zeros(1, np.int32))
+    with pytest.raises(ValueError, match="invalid argument"):  # stride outside 1..ORBX_BOW_MAX_STRIDE
+        api.BowDatabase.build(ctx, V, np.zeros((1, api.BOW_MAX_STRIDE + 1, 32), np.uint8), np.zeros(1, np.int32))
     D = api.BowDatabase.build(ctx, V, desc, counts)
     for args in [(0, F + 1, 3, 1), (-1, 2, 3, 1), (3, 2, 3, 1), (0, F, 0, 1), (0, F, F + 1, 1), (0, F, 3, -1), (0, F, 3, 1, float("nan"))]:
         with pytest.raises(ValueError, match="invalid argument"):

@@ -45,13 +45,20 @@ def test_oracle_equals_literal_restatement(cases, name):
 
 
 def test_cases_reach_every_rule(cases):
-    seen = Counter()
+    """every rule, over all cases and again over the cases with k > 10 alone (the k-wide paths of the kernels)"""
+    seen, wide = Counter(), Counter()
     for c in cases.values():
-        R.py_vocab_build(c["desc"], c["counts"], c["n_frames"], c["k"], c["L"], c["seed"], seen)
+        st = Counter()
+        R.py_vocab_build(c["desc"], c["counts"], c["n_frames"], c["k"], c["L"], c["seed"], st)
+        seen.update(st)
+        if c["k"] > 10:
+            wide.update(st)
     rules = {"node_n_le_k", "node_kmeans", "seeding_stopped_early", "assignment_tie", "converged", "empty_cluster_kept", "single_member_mean",
              "bit_majority_at_exactly_half", "early_leaf", "leaf_at_depth_L", "frame_without_keypoints", "padding_rows", "word_without_frames"}
     assert rules <= {b for b, n in seen.items() if n > 0}, dict(seen)
+    assert rules <= {b for b, n in wide.items() if n > 0}, dict(wide)
     assert seen["capped"] == 0  # the ORBX_VOCAB_MAX_ITERS cap is not reached by these sets
+    assert {c["k"] for c in cases.values()} >= {17, 32}
 
 
 @pytest.mark.parametrize("name", ["random_k10_L3", "duplicates", "random_k3_L6"])

@@ -37,6 +37,7 @@ typedef struct vb_state {
   int32_t *parent, *first_child, *n_child;
   uint8_t *desc, *capped;
   int32_t *iters, *leaf_of, n_capped;
+  int32_t *root_picks; /* optional [k]: the root's k-means++ picks, positions in its segment */
 } vb_state;
 
 static void vb_step(vb_state *s, int node, uint64_t key, const int32_t *idx, int n, int level) {
@@ -57,6 +58,7 @@ static void vb_step(vb_state *s, int node, uint64_t key, const int32_t *idx, int
     int pick = (int)(vb_splitmix64(key) % (uint64_t)n);
     for (;;) {
       memcpy(cent + 32 * (size_t)kk, s->d + 32 * (size_t)idx[pick], 32);
+      if (node == 0 && s->root_picks) s->root_picks[kk] = pick;
       ++kk;
       if (kk == k) break;
       uint64_t S = 0;
@@ -158,11 +160,13 @@ static void vb_step(vb_state *s, int node, uint64_t key, const int32_t *idx, int
  * descriptors each, under the rules include/orbx.h states for orbx_vocab_build.  Outputs in the text format's record order
  * (record i = node i + 1): parent, is_leaf, node_desc [cap][32], weight.  iters[L]: most assignment passes of a k-means
  * node per level; *n_capped: nodes stopped by ORBX_VOCAB_MAX_ITERS.  Optional (NULL): leaf_of[n_frames * stride] = node
- * id each training descriptor was trained into (-1 for padding), node_capped[n_records + 1] per node id.  Returns the
+ * id each training descriptor was trained into (-1 for padding), node_capped[n_records + 1] per node id, root_picks[k] =
+ * the root's k-means++ picks as positions among the training descriptors in frame order (-1 past the last pick, and all -1
+ * when the root has n <= k descriptors).  Returns the
  * number of records, or -1 (bad arguments, no descriptors, more than cap_records records). */
 int oracle_vocab_build(const uint8_t *desc, const int32_t *n_kps, int n_frames, int stride, int k, int L, uint64_t seed,
                        int cap_records, int32_t *parent, uint8_t *is_leaf, uint8_t *node_desc, double *weight,
-                       int32_t *iters, int32_t *n_capped, int32_t *leaf_of, uint8_t *node_capped) {
+                       int32_t *iters, int32_t *n_capped, int32_t *leaf_of, uint8_t *node_capped, int32_t *root_picks) {
   if (k < 2 || L < 1 || n_frames < 1 || stride < 1 || cap_records < 1) return -1;
   int n = 0;
   for (int f = 0; f < n_frames; ++f) {
@@ -188,6 +192,9 @@ int oracle_vocab_build(const uint8_t *desc, const int32_t *n_kps, int n_frames, 
   s.desc = (uint8_t *)calloc((size_t)cap, 32);
   s.capped = (uint8_t *)calloc((size_t)cap, 1);
   s.iters = iters;
+  s.root_picks = root_picks;
+  if (root_picks)
+    for (int c = 0; c < k; ++c) root_picks[c] = -1;
   s.leaf_of = (int32_t *)malloc(sizeof(int32_t) * (size_t)n);
   for (int l = 0; l < L; ++l) iters[l] = 0;
   s.parent[0] = -1, s.first_child[0] = -1, s.n_child[0] = 0;

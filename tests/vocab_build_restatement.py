@@ -185,14 +185,15 @@ def _oracle_lib():
         finally:
             shutil.rmtree(tmp, ignore_errors=True)
         lib.oracle_vocab_build.restype = C.c_int
-        lib.oracle_vocab_build.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint64, C.c_int] + [C.c_void_p] * 8
+        lib.oracle_vocab_build.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint64, C.c_int] + [C.c_void_p] * 9
         _lib = lib
     return _lib
 
 
 def oracle_vocab_build(desc, counts, n_frames: int, k: int, L: int, seed: int):
     """oracle_vocab_build (tests/vocab_build_oracle.c) -> the same dict as py_vocab_build, leaf_of as an (n_frames, stride)
-    array (-1 = padding), plus node_capped per node id"""
+    array (-1 = padding), plus node_capped per node id and root_picks (the root's k-means++ picks as positions among the
+    training descriptors in frame order, -1 past the last)"""
     f = _oracle_lib().oracle_vocab_build
     d = np.ascontiguousarray(desc, np.uint8)
     cnt = np.ascontiguousarray(counts, np.int32)
@@ -200,12 +201,12 @@ def oracle_vocab_build(desc, counts, n_frames: int, k: int, L: int, seed: int):
     cap = max(1, int(cnt[:n_frames].sum())) * L + 1
     par, leaf, nd, w = np.zeros(cap, np.int32), np.zeros(cap, np.uint8), np.zeros((cap, 32), np.uint8), np.zeros(cap, np.float64)
     iters, ncap = np.zeros(L, np.int32), np.zeros(1, np.int32)
-    leaf_of, node_capped = np.zeros((n_frames, stride), np.int32), np.zeros(cap + 1, np.uint8)
+    leaf_of, node_capped, picks = np.zeros((n_frames, stride), np.int32), np.zeros(cap + 1, np.uint8), np.zeros(k, np.int32)
     n = f(d.ctypes.data, cnt.ctypes.data, n_frames, stride, k, L, seed & M64, cap, par.ctypes.data, leaf.ctypes.data, nd.ctypes.data, w.ctypes.data,
-          iters.ctypes.data, ncap.ctypes.data, leaf_of.ctypes.data, node_capped.ctypes.data)
+          iters.ctypes.data, ncap.ctypes.data, leaf_of.ctypes.data, node_capped.ctypes.data, picks.ctypes.data)
     assert n > 0, "oracle_vocab_build refused the input"
     return dict(parent=par[:n].copy(), is_leaf=leaf[:n].copy(), desc=nd[:n].copy(), weight=w[:n].copy(), iters=iters.tolist(), n_capped=int(ncap[0]),
-                leaf_of=leaf_of, node_capped=node_capped[: n + 1].copy())
+                leaf_of=leaf_of, node_capped=node_capped[: n + 1].copy(), root_picks=picks)
 
 
 def write_text(k: int, L: int, rec: dict) -> bytes:
@@ -234,11 +235,8 @@ def _frames(feats: np.ndarray, counts, stride: int, pad_rows: int = 0, seed: int
     counts = np.asarray(counts, np.int32)
     F = len(counts)
     desc = rng.integers(0, 256, (F + pad_rows, stride, 32), dtype=np.uint8)
-    o = 0
-    for f, n in enumerate(counts):
-        desc[f, :n] = feats[o : o + n]
-        o += n
-    assert o == len(feats)
+    assert counts.sum() == len(feats)
+    desc[:F][np.arange(stride) < counts[:, None]] = feats
     full = np.concatenate([counts, rng.integers(1, stride + 1, pad_rows).astype(np.int32)])
     return desc, full
 
@@ -251,6 +249,38 @@ def _clustered(n: int, n_centres: int, flip: int, seed: int) -> np.ndarray:
     for i in range(n):
         bits[i, rng.choice(256, rng.integers(0, flip + 1), replace=False)] ^= 1
     return np.packbits(bits, axis=1, bitorder="little")
+
+
+def _flip(d: np.ndarray, flip: int, rng) -> np.ndarray:
+    """every row with up to `flip` bits flipped at random positions (a position drawn twice flips back), vectorised"""
+    d = d.copy()
+    m = rng.integers(0, flip + 1, len(d))
+    pos = rng.integers(0, 256, (len(d), max(flip, 1)))
+    rows = np.arange(len(d))
+    for j in range(flip):
+        on = m > j
+        d[rows[on], pos[on, j] >> 3] ^= (1 << (pos[on, j] & 7)).astype(np.uint8)
+    return d
+
+
+def _two_level(n: int, n_top: int, n_sub: int, seed: int, spread: int = 40, flip: int = 8, decay: float = 0.85):
+    """n descriptors around n_top groups of n_sub sub-centres each: sub-centres within `spread` bits of their group's centre,
+    descriptors within `flip` bits of a sub-centre.  Group sizes fall geometrically by `decay`, so that some groups hold
+    fewer than k descriptors and others more than k clusters.  -> (descriptors, group of each)"""
+    rng = np.random.default_rng(seed)
+    top = rng.integers(0, 256, (n_top, 32), dtype=np.uint8)
+    sub = _flip(np.repeat(top, n_sub, axis=0), spread, rng)
+    w = decay ** np.arange(n_top)
+    g = rng.choice(n_top, n, p=w / w.sum())
+    return _flip(sub[g * n_sub + rng.integers(0, n_sub, n)], flip, rng), g
+
+
+def _spread(n: int, n_frames: int, seed: int) -> np.ndarray:
+    """n descriptors over n_frames frames of uneven counts, frame 1 empty"""
+    rng = np.random.default_rng(seed)
+    cut = np.sort(rng.choice(np.arange(1, n), n_frames - 2, replace=False))
+    counts = np.diff(np.concatenate([[0], cut, [n]]))
+    return np.insert(counts, 1, 0).astype(np.int32)
 
 
 def case(name: str):
@@ -290,11 +320,68 @@ def case(name: str):
         feats = np.packbits(bits, axis=1, bitorder="little")
         desc, full = _frames(feats, [8, 8, 8], 8, seed=6)
         return dict(desc=desc, counts=full, n_frames=3, k=3, L=3, seed=8)
+    if name == "k32_root_eq_k":  # exactly k = 32 descriptors, two equal: the root's children are its descriptors, a full warp
+        rng = np.random.default_rng(40)
+        feats = rng.integers(0, 256, (32, 32), dtype=np.uint8)
+        feats[29] = feats[6]
+        desc, full = _frames(feats, [10, 0, 22], 24, pad_rows=1, seed=40)
+        return dict(desc=desc, counts=full, n_frames=3, k=32, L=2, seed=41)
+    if name == "k32_root_k_plus_1":  # k-means++ picks 32 centres from 33 descriptors
+        rng = np.random.default_rng(42)
+        feats = _flip(np.repeat(rng.integers(0, 256, (3, 32), dtype=np.uint8), 11, axis=0), 60, rng)
+        desc, full = _frames(feats, [16, 17], 20, pad_rows=2, seed=42)
+        return dict(desc=desc, counts=full, n_frames=2, k=32, L=2, seed=43)
+    if name in ("k32_L2", "k31_L3", "k17_L2"):
+        k, L = (int(x) for x in name[1:].split("_L"))
+        n, n_top, n_sub = {32: (2600, 20, 48), 31: (4000, 45, 40), 17: (2200, 12, 30)}[k]
+        feats, _ = _two_level(n, n_top, n_sub, seed=k)
+        # a group of 60 copies of 6 distinct descriptors: a node with more than k descriptors but fewer than k distinct ones
+        rng = np.random.default_rng(k + 1)
+        feats[rng.choice(n, 60, replace=False)] = rng.integers(0, 256, (6, 32), dtype=np.uint8)[np.arange(60) % 6]
+        counts = _spread(n, 9, seed=k)
+        desc, full = _frames(feats, counts, int(counts.max()) + 3, pad_rows=2, seed=k)
+        return dict(desc=desc, counts=full, n_frames=len(counts), k=k, L=L, seed=k * 7)
+    if name.startswith("tile_"):  # a root of exactly n descriptors: k-means tiles of kTile = 4096, the last one full / of one / three tiles
+        n = int(name[5:])
+        feats, _ = _two_level(n, 14, 12, seed=n)
+        counts = _spread(n, 11, seed=n)
+        desc, full = _frames(feats, counts, int(counts.max()), pad_rows=1, seed=n)
+        return dict(desc=desc, counts=full, n_frames=len(counts), k=10, L=2, seed=n)
+    if name.startswith("wide_stride_"):  # frame rows past 4096 descriptors: one full row, one empty, in the IDF step's sort
+        stride = int(name[len("wide_stride_") :])
+        counts = np.array([stride, 0, stride // 3, 1, stride - 5], np.int32)
+        feats, _ = _two_level(int(counts.sum()), 16, 10, seed=stride)
+        desc, full = _frames(feats, counts, stride, pad_rows=1, seed=stride)
+        return dict(desc=desc, counts=full, n_frames=len(counts), k=10, L=3, seed=stride)
+    if name == "many_frames":
+        # 70,500 frames of up to 16 descriptors, 1,065,000 in all: the root spans 261 k-means tiles (more than one per thread
+        # of the pick kernel's 256) and the IDF step runs a second chunk of frames (>= 65535).  Frames from 65535 on draw
+        # half their descriptors from 4 groups no earlier frame uses, so some words are reached from the second chunk only.
+        F, stride = 70500, 16
+        counts = np.full(F, stride, np.int32)
+        counts[::3] = 14
+        counts[::50] = 0
+        counts[65535] = stride
+        n = int(counts.sum())
+        feats, _ = _two_level(n, 12, 8, seed=70, decay=0.97)
+        late_lo = int(counts[:65535].sum())
+        rng = np.random.default_rng(71)
+        new, _ = _two_level(n - late_lo, 4, 3, seed=72, decay=1.0)
+        take = rng.random(n - late_lo) < 0.5
+        feats[late_lo:][take] = new[take]
+        desc, full = _frames(feats, counts, stride, pad_rows=1, seed=73)
+        return dict(desc=desc, counts=full, n_frames=F, k=10, L=2, seed=74)
     raise KeyError(name)
 
 
 RANDOM_CASES = [f"random_k{k}_L{L}" for k in (2, 3, 10) for L in (1, 2, 3, 6)]
-CASES = RANDOM_CASES + ["duplicates", "all_identical", "n_le_k_root", "even_members"]
+# branching factors above 10, small enough for the literal restatement
+WIDE_K_CASES = ["k32_root_eq_k", "k32_root_k_plus_1", "k32_L2", "k17_L2"]
+CASES = RANDOM_CASES + ["duplicates", "all_identical", "n_le_k_root", "even_members"] + WIDE_K_CASES
+# the size limits of the device build, checked against the C oracle only (the restatement would take minutes)
+TILE_CASES = ["tile_4096", "tile_4097", "tile_8193"]
+WIDE_STRIDE_CASES = [f"wide_stride_{s}" for s in (4096, 4097, 8193, 16384)]
+LIMIT_CASES = ["k31_L3"] + TILE_CASES + WIDE_STRIDE_CASES + ["many_frames"]
 
 # the branches each case must reach (beyond the ones every case reaches)
 EXPECT = {
@@ -304,6 +391,8 @@ EXPECT = {
     "even_members": {"bit_majority_at_exactly_half", "node_kmeans"},
     "random_k10_L2": {"empty_cluster_kept", "node_n_le_k", "early_leaf", "assignment_tie", "word_without_frames"},
     "random_k2_L6": {"empty_cluster_kept", "single_member_mean", "early_leaf", "leaf_at_depth_L"},
+    "k32_root_eq_k": {"node_n_le_k", "early_leaf", "padding_rows", "frame_without_keypoints"},
+    "k32_root_k_plus_1": {"node_kmeans", "node_n_le_k", "padding_rows"},
 }
 # No case reaches the ORBX_VOCAB_MAX_ITERS cap (the most passes any node takes here is 9); the tests assert that the cap
 # count the builds report matches the passes they count.
