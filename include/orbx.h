@@ -51,7 +51,7 @@ typedef struct orbx_keypoint {
 
 /* Everything the reference reads from its YAML for this path (src/System.cc:27-73): ORBExtractor.* and Camera.* */
 typedef struct orbx_config {
-  int32_t width, height;   /* input image size (8-bit, single channel) */
+  int32_t width, height;   /* input image size (8-bit; single channel unless orbx_set_input_format says otherwise) */
   int32_t n_features;      /* ORBExtractor.nFeatures (1..65535: keypoint indices travel as uint16 in the row index / grid) */
   int32_t n_levels;        /* ORBExtractor.nLevels (1..16) */
   float scale_factor;      /* ORBExtractor.scaleFactor (> 1) */
@@ -88,6 +88,22 @@ int orbx_set_stream(orbx_ctx *ctx, void *cuda_stream);
  * captured at the first call (on by default; the legacy default stream cannot be captured and always takes plain launches).
  * enable = 0 restores plain stream launches (bench.py reports the p50 latency both ways).  Environment: ORBX_GRAPH=0. */
 int orbx_set_graph(orbx_ctx *ctx, int enable);
+
+/* Pixel format of the IMAGE inputs of every entry point that takes images (orbx_extract, orbx_stereo_frame,
+ * orbx_rgbd_frame, orbx_stereo_batch*, orbx_extract_batch_device, orbx_rgbd_batch_device, orbx_sequence_stereo*,
+ * orbx_profile_stereo_batch_device); depth inputs are unchanged.  The names mirror the ROS image encodings (mono8, rgb8,
+ * bgr8, rgba8, bgra8).  Colour is converted to gray on the device inside the level-0 pyramid pass with cv::cvtColor's
+ * 8-bit rule, gray = (9798 R + 19235 G + 3735 B + 16384) >> 15 (alpha ignored), which replaces the cvtColor call of
+ * Tracking::grabFrame (src/Tracking.cc:55-68).  Strides stay in bytes: rows hold width * bpp bytes (bpp = 1, 3 or 4) and
+ * the stride checks read stride >= width * bpp, frame_stride >= stride * (height - 1) + width * bpp.
+ * ORBX_FORMAT_GRAY8 is the default.  An unknown format returns ORBX_ERR_INVALID_ARG.  Resident frames and the epoch are
+ * untouched; a captured single-pair graph is dropped when the format changes and re-captured by the next call. */
+#define ORBX_FORMAT_GRAY8 0
+#define ORBX_FORMAT_RGB8 1
+#define ORBX_FORMAT_BGR8 2
+#define ORBX_FORMAT_RGBA8 3
+#define ORBX_FORMAT_BGRA8 4
+int orbx_set_input_format(orbx_ctx *ctx, int format);
 
 /* ---- per-config tables ---------------------------------------------------------------------------------- */
 /* replaces: ORBExtractor::getScaledFactors() (include/ORB_SLAM2/ORBExtractor.h:116), ORBExtractor::mnLevels,
@@ -132,8 +148,8 @@ int orbx_get_grid(orbx_ctx *ctx, int frame, int32_t *cell_start, int32_t *entrie
 /* A sequence of n_frames stereo pairs (ANY length) from HOST memory; pinned memory makes the copies asynchronous.  The
  * frames stream through the context's max_batch device slots in chunks, so that the H2D copy of one chunk, the kernels of
  * another and the D2H copy of a third overlap.
- * left/right: frame f at base + f * frame_stride bytes, rows `stride` bytes apart (stride >= width and frame_stride >=
- * stride * (height - 1) + width, else ORBX_ERR_INVALID_ARG).  Outputs are fixed-stride arrays:
+ * left/right: frame f at base + f * frame_stride bytes, rows `stride` bytes apart (stride >= width * bpp and frame_stride >=
+ * stride * (height - 1) + width * bpp, bpp = bytes per pixel of orbx_set_input_format, else ORBX_ERR_INVALID_ARG).  Outputs are fixed-stride arrays:
  * kps_*[f * n_features + i], desc_*[(f * n_features + i) * 32], u_right/depth[f * n_features + i], n_*[f].
  * Returns after all results have landed in the output arrays. */
 int orbx_stereo_batch(orbx_ctx *ctx, int n_frames, const uint8_t *left, const uint8_t *right, size_t stride,

@@ -32,6 +32,14 @@
 
 #include "../orbx.h"
 
+// OpenCV's type codes of 8-bit 3- and 4-channel images (CV_MAKETYPE(CV_8U, n)), for cv:: headers that leave them out
+#ifndef CV_8UC3
+#define CV_8UC3 16
+#endif
+#ifndef CV_8UC4
+#define CV_8UC4 24
+#endif
+
 namespace ORB_SLAM2_ROS2_B200
 {
 
@@ -83,18 +91,32 @@ struct Camera
     mfBf = mfFx * mfBl;
     mDistCoeff = dist;
   }
+  // Camera.Color: colour frames (CV_8UC3 / CV_8UC4) arrive as RGB(A) when true, as BGR(A), OpenCV's order, when false.
+  // Set next to set(); the shim converts them to gray on the device instead of Tracking::grabFrame's cvtColor
+  // (src/Tracking.cc:55-68).
+  static inline bool mbRGB = false;
 };
 
 // ---- one CUDA context per distinct configuration (the reference keeps these tables in process-wide statics) ----
 namespace detail
 {
+// the ORBX_FORMAT_* of an image: CV_8UC1 gray, CV_8UC3 / CV_8UC4 colour in the order Camera::mbRGB names; other types throw
+inline int input_format(const cv::Mat &img)
+{
+  if (img.type() == CV_8U) return ORBX_FORMAT_GRAY8;
+  if (img.type() == CV_8UC3) return Camera::mbRGB ? ORBX_FORMAT_RGB8 : ORBX_FORMAT_BGR8;
+  if (img.type() == CV_8UC4) return Camera::mbRGB ? ORBX_FORMAT_RGBA8 : ORBX_FORMAT_BGRA8;
+  throw ORBSlam2Error("unsupported image type: expected CV_8UC1, CV_8UC3 or CV_8UC4");
+}
+
 struct CtxKey
 {
   int w, h, nFeatures, nLevels, iniTh, minTh;
   float scale, fx, fy, cx, cy, bf, dScale;
   std::array<float, 5> dist;
   std::string tmpl;
-  auto tie() const { return std::tie(w, h, nFeatures, nLevels, iniTh, minTh, scale, fx, fy, cx, cy, bf, dScale, dist, tmpl); }
+  int format;
+  auto tie() const { return std::tie(w, h, nFeatures, nLevels, iniTh, minTh, scale, fx, fy, cx, cy, bf, dScale, dist, tmpl, format); }
   bool operator<(const CtxKey &o) const { return tie() < o.tie(); }
 };
 
@@ -113,11 +135,13 @@ struct Context
 typedef std::shared_ptr<Context> ContextPtr;
 typedef std::lock_guard<std::mutex> Lock;
 
-inline ContextPtr context_for(int w, int h, int nFeatures, int nLevels, float scale, const std::string &tmpl, int iniTh, int minTh, float dScale)
+inline ContextPtr context_for(int w, int h, int nFeatures, int nLevels, float scale, const std::string &tmpl, int iniTh, int minTh, float dScale,
+                              int format = ORBX_FORMAT_GRAY8)
 {
   static std::mutex mtx;
   static std::map<std::pair<CtxKey, std::thread::id>, ContextPtr> cache;
-  CtxKey key{w, h, nFeatures, nLevels, iniTh, minTh, scale, Camera::mfFx, Camera::mfFy, Camera::mfCx, Camera::mfCy, Camera::mfBf, dScale, Camera::mDistCoeff, tmpl};
+  CtxKey key{w, h, nFeatures, nLevels, iniTh, minTh, scale, Camera::mfFx, Camera::mfFy, Camera::mfCx, Camera::mfCy, Camera::mfBf, dScale, Camera::mDistCoeff, tmpl,
+             format};
   const auto full = std::make_pair(key, std::this_thread::get_id());
   std::lock_guard<std::mutex> lock(mtx);
   auto it = cache.find(full);
@@ -145,6 +169,7 @@ inline ContextPtr context_for(int w, int h, int nFeatures, int nLevels, float sc
   orbx_ctx *raw = nullptr;
   check(nullptr, orbx_create(&cfg, &raw), "orbx_create"); // ImageSizeError (:310-314)
   ContextPtr sp = std::make_shared<Context>(raw);
+  check(raw, orbx_set_input_format(raw, format), "orbx_set_input_format");
   cache[full] = sp;
   return sp;
 }
@@ -244,7 +269,10 @@ private:
     static std::vector<float> v;
     return v;
   }
-  detail::ContextPtr context() const { return detail::context_for(mImage.cols, mImage.rows, mnFeats, mnPyrLevels, mfScale, mTmpl, mIniTh, mMinTh, 1.f); }
+  detail::ContextPtr context() const
+  {
+    return detail::context_for(mImage.cols, mImage.rows, mnFeats, mnPyrLevels, mfScale, mTmpl, mIniTh, mMinTh, 1.f, detail::input_format(mImage));
+  }
   void run(std::vector<cv::KeyPoint> *keyPoints, std::vector<cv::Mat> *descriptors, bool want_pyramid = false)
   {
     mCtx = context();
@@ -317,7 +345,7 @@ public:
     SharedPtr f(new Frame());
     f->mCapacity = nFeatures;
     f->mLeftIm = colorImg;
-    f->mCtx = detail::context_for(colorImg.cols, colorImg.rows, nFeatures, nLevels, scale, briefF, maxThresh, minThresh, dScale);
+    f->mCtx = detail::context_for(colorImg.cols, colorImg.rows, nFeatures, nLevels, scale, briefF, maxThresh, minThresh, dScale, detail::input_format(colorImg));
     if (depthImg.rows != colorImg.rows || depthImg.cols != colorImg.cols) throw ORBSlam2Error("createRGBD: depth image size differs from the colour image");
     if (depthImg.type() != CV_16U && depthImg.type() != CV_32F)
     { // any other depth type goes through the reference's own conversion (depthImg.convertTo(CV_32F), src/Frame.cc:130)
@@ -614,7 +642,9 @@ inline Frame::SharedPtr Frame::createStereo(cv::Mat leftImg, cv::Mat rightImg, i
   f->mCapacity = nFeatures;
   f->mLeftIm = leftImg;
   f->mRightIm = rightImg;
-  f->mCtx = detail::context_for(leftImg.cols, leftImg.rows, nFeatures, nLevels, scale, briefFp, maxThresh, minThresh, 1.f);
+  const int format = detail::input_format(leftImg);
+  if (detail::input_format(rightImg) != format) throw ORBSlam2Error("createStereo: the right image's type differs from the left one's");
+  f->mCtx = detail::context_for(leftImg.cols, leftImg.rows, nFeatures, nLevels, scale, briefFp, maxThresh, minThresh, 1.f, format);
   std::vector<orbx_keypoint> kl((size_t)nFeatures), kr((size_t)nFeatures);
   f->mDescLeft = cv::Mat(nFeatures, 32, CV_8U);
   f->mDescRight = cv::Mat(nFeatures, 32, CV_8U);

@@ -34,6 +34,9 @@ COMM_ID_BYTES, IPC_HANDLE_BYTES = 128, 64
 TRANSPORT_NONE, TRANSPORT_NCCL, TRANSPORT_PEER = 0, 1, 2
 DEPTH_U16, DEPTH_F32 = 0, 1
 N_STAGES = 7  # ORBX_N_STAGES
+# ORBX_FORMAT_*: pixel format of the image inputs (Context.set_input_format), named after the ROS image encodings
+FORMAT_GRAY8, FORMAT_RGB8, FORMAT_BGR8, FORMAT_RGBA8, FORMAT_BGRA8 = 0, 1, 2, 3, 4
+FORMAT_BPP = {FORMAT_GRAY8: 1, FORMAT_RGB8: 3, FORMAT_BGR8: 3, FORMAT_RGBA8: 4, FORMAT_BGRA8: 4}
 
 
 # the reference's exception types (include/ORB_SLAM2/Error.h:13-98)
@@ -84,7 +87,7 @@ EXPORTS = [
     "orbx_serialized_capacity_bow", "orbx_serialize_keyframe_bow", "orbx_serialize_keyframes_bow_device", "orbx_keyframe_list_head",
     "orbx_keyframe_list_entry_prefix", "orbx_sequence_stereo_keyframes", "orbx_vocab_build", "orbx_vocab_save_text", "orbx_vocab_arrays",
     "orbx_bowdb_build", "orbx_bowdb_destroy", "orbx_bowdb_info", "orbx_bowdb_query_range", "orbx_bowdb_query_frame",
-    "orbx_loopver_build", "orbx_loopver_destroy", "orbx_loopver_verify",
+    "orbx_loopver_build", "orbx_loopver_destroy", "orbx_loopver_verify", "orbx_set_input_format",
 ]
 
 class OrbxRecordLayout(C.Structure):
@@ -215,6 +218,7 @@ def load_library(build_if_missing: bool = True):
     L.orbx_frame_epoch.argtypes = [vp]
     L.orbx_debug_quadtree_stats.argtypes = [vp, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
     L.orbx_set_graph.argtypes = [vp, C.c_int]
+    L.orbx_set_input_format.argtypes = [vp, C.c_int]
     L.orbx_frame_epoch.restype = C.c_uint64
     L.orbx_frame_range.argtypes = [C.c_int64, C.c_int, C.c_int, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
     L.orbx_frame_range.restype = None
@@ -287,6 +291,7 @@ class Camera:
     bl: float = 0.537166
     dist: tuple = (0.0, 0.0, 0.0, 0.0, 0.0)
     depth_scale: float = 1.0
+    rgb: bool = False  # Camera.Color: colour images arrive as RGB (True) or as BGR, OpenCV's order (False)
 
     @property
     def bf(self) -> np.float32:
@@ -315,6 +320,7 @@ class Context:
         self._h = C.c_void_p()
         self.width, self.height, self.n_features, self.n_levels, self.max_batch = int(width), int(height), int(n_features), int(n_levels), int(max_batch)
         self.camera = cam
+        self.input_format, self.bpp = FORMAT_GRAY8, 1
         rc = L.orbx_create(C.byref(cfg), C.byref(self._h))
         if rc != ORBX_OK:
             self._h = C.c_void_p()
@@ -353,6 +359,14 @@ class Context:
         """single-pair calls as one CUDA graph launch (default) or as plain stream launches"""
         _check(self._h, self._L.orbx_set_graph(self._h, int(bool(enable))), "orbx_set_graph")
 
+    def set_input_format(self, fmt: int):
+        """pixel format (FORMAT_*) of the images every later call reads; colour is converted to gray on the device"""
+        _check(self._h, self._L.orbx_set_input_format(self._h, int(fmt)), "orbx_set_input_format")
+        self.input_format, self.bpp = int(fmt), FORMAT_BPP[int(fmt)]
+
+    def _image(self, a: np.ndarray) -> np.ndarray:
+        return _as_image(a, self.height, self.width, self.bpp)
+
     def synchronize(self):
         _check(self._h, self._L.orbx_synchronize(self._h), "orbx_synchronize")
 
@@ -371,7 +385,7 @@ class Context:
 
     # ---- single frame, host buffers -----------------------------------------------------------------------------
     def extract(self, image: np.ndarray):
-        img = _as_u8(image, self.height, self.width)
+        img = self._image(image)
         N = self.n_features
         kps, desc, n = np.zeros(N, KP_DTYPE), np.zeros((N, 32), np.uint8), C.c_int32(0)
         rc = self._L.orbx_extract(self._h, img.ctypes.data, img.strides[0], kps.ctypes.data, desc.ctypes.data, C.addressof(n))
@@ -388,7 +402,7 @@ class Context:
         return out
 
     def stereo_frame(self, left: np.ndarray, right: np.ndarray):
-        l, r = _as_u8(left, self.height, self.width), _as_u8(right, self.height, self.width)
+        l, r = self._image(left), self._image(right)
         N = self.n_features
         kl, kr = np.zeros(N, KP_DTYPE), np.zeros(N, KP_DTYPE)
         dl, dr = np.zeros((N, 32), np.uint8), np.zeros((N, 32), np.uint8)
@@ -401,7 +415,7 @@ class Context:
         return StereoResult(kl[:a], dl[:a], kr[:b], dr[:b], ur[:a], dp[:a], nm.value)
 
     def rgbd_frame(self, gray: np.ndarray, depth_image: np.ndarray):
-        g = _as_u8(gray, self.height, self.width)
+        g = self._image(gray)
         if depth_image.dtype == np.float32:
             d, dt = np.ascontiguousarray(depth_image), DEPTH_F32
         else:
@@ -598,15 +612,23 @@ class Context:
 
     # ---- batches ----------------------------------------------------------------------------------------------------
     def stereo_batch(self, left: np.ndarray, right: np.ndarray, out: "StereoBatchBuffers | None" = None):
-        """left/right: (n, H, W) uint8 host arrays (pinned memory makes the copies asynchronous)."""
+        """left/right: (n, H, W) uint8 host arrays, (n, H, W, bpp) for a colour format (pinned memory makes the copies
+        asynchronous)."""
         n = left.shape[0]
-        assert left.shape == right.shape == (n, self.height, self.width) and left.strides == right.strides and left.dtype == np.uint8
+        self._check_frames(left, right)
         ob = out or StereoBatchBuffers.numpy(n, self.n_features)
         rc = self._L.orbx_stereo_batch(self._h, n, left.ctypes.data, right.ctypes.data, left.strides[1], left.strides[0], ob.kps_left.ctypes.data,
                                        ob.desc_left.ctypes.data, ob.n_left.ctypes.data, ob.kps_right.ctypes.data, ob.desc_right.ctypes.data,
                                        ob.n_right.ctypes.data, ob.u_right.ctypes.data, ob.depth.ctypes.data, ob.n_matches.ctypes.data)
         _check(self._h, rc, "orbx_stereo_batch")
         return ob
+
+    def _check_frames(self, left: np.ndarray, right: np.ndarray):
+        """(n, H, W) or, for a colour format, (n, H, W, bpp) uint8 stacks with equal strides and packed pixels"""
+        n = left.shape[0]
+        shape = (n, self.height, self.width) + ((self.bpp,) if self.bpp > 1 else ())
+        assert left.shape == right.shape == shape and left.strides == right.strides and left.dtype == right.dtype == np.uint8
+        assert self.bpp == 1 or (left.strides[2] == self.bpp and left.strides[3] == 1)
 
     def stereo_batch_ptr(self, n_frames, left_ptr, right_ptr, stride, frame_stride, ptrs):
         """raw-pointer variant of stereo_batch (host pointers; ptrs = 9 output addresses or 0)."""
@@ -661,7 +683,7 @@ class Context:
         records = numpy structured array (record_dtype) of the block's frames; gathered_* cover the WHOLE sequence."""
         n = left.shape[0]
         F = n if n_frames_total is None else int(n_frames_total)
-        assert left.shape == right.shape == (n, self.height, self.width) and left.strides == right.strides and left.dtype == np.uint8
+        self._check_frames(left, right)
         rec = np.zeros(max(n, 1), self.record_dtype())
         gd = np.zeros((F, self.n_features, 32), np.uint8) if gather_to_host else None
         gn = np.zeros(F, np.int32) if gather_to_host else None
@@ -695,7 +717,7 @@ class Context:
         keyframes[i, :sizes[i]]; write_keyframe_list() frames them as a KeyFrameList."""
         n = left.shape[0]
         F = n if n_frames_total is None else int(n_frames_total)
-        assert left.shape == right.shape == (n, self.height, self.width) and left.strides == right.strides and left.dtype == np.uint8
+        self._check_frames(left, right)
         pose = None if poses is None else np.ascontiguousarray(poses, np.float32).reshape(n, 12)
         ks = self.serialized_capacity_bow() if vocab is not None else self.serialized_capacity()
         kf = _aligned_zeros((max(n, 1), ks))
@@ -817,12 +839,25 @@ class Communicator:
             pass
 
 
-def _as_u8(a: np.ndarray, h: int, w: int) -> np.ndarray:
-    if a.dtype != np.uint8 or a.ndim != 2 or a.shape != (h, w):
-        raise ValueError(f"expected a {h}x{w} uint8 image, got {a.shape} {a.dtype}")
-    if a.strides[1] != 1:
+def _as_image(a: np.ndarray, h: int, w: int, bpp: int = 1) -> np.ndarray:
+    """an (h, w) uint8 image, (h, w, bpp) for a colour format, with packed pixels (rows may keep any stride)"""
+    shape = (h, w) if bpp == 1 else (h, w, bpp)
+    if a.dtype != np.uint8 or a.shape != shape:
+        raise ValueError(f"expected a {'x'.join(map(str, shape))} uint8 image, got {a.shape} {a.dtype}")
+    if a.strides[1] != bpp or (bpp > 1 and a.strides[2] != 1):
         a = np.ascontiguousarray(a)
     return a
+
+
+def image_format(image: np.ndarray, rgb: bool = False) -> int:
+    """the FORMAT_* of an (H, W) gray or (H, W, 3 | 4) colour uint8 image; rgb = Camera.Color (False: BGR, OpenCV's order)"""
+    if image.ndim == 2:
+        return FORMAT_GRAY8
+    if image.ndim == 3 and image.shape[2] in (3, 4):
+        if image.shape[2] == 3:
+            return FORMAT_RGB8 if rgb else FORMAT_BGR8
+        return FORMAT_RGBA8 if rgb else FORMAT_BGRA8
+    raise ValueError(f"unsupported image shape {image.shape}: expected (H, W), (H, W, 3) or (H, W, 4)")
 
 
 @dataclass
@@ -871,12 +906,14 @@ class StereoBatchBuffers:
 _ctx_cache: dict = {}
 
 
-def _context_for(h, w, n_features, n_levels, scale, ini_th, min_th, camera: Camera, pattern_key, pattern) -> Context:
+def _context_for(h, w, n_features, n_levels, scale, ini_th, min_th, camera: Camera, pattern_key, pattern, fmt: int = FORMAT_GRAY8) -> Context:
     key = (h, w, n_features, n_levels, float(scale), ini_th, min_th, camera.fx, camera.fy, camera.cx, camera.cy, camera.bl, tuple(camera.dist),
-           camera.depth_scale, pattern_key)
+           camera.depth_scale, pattern_key, fmt)
     ctx = _ctx_cache.get(key)
     if ctx is None:
         ctx = Context(w, h, n_features, n_levels, scale, ini_th, min_th, camera, max_batch=1, pattern=pattern)
+        if fmt != FORMAT_GRAY8:
+            ctx.set_input_format(fmt)
         _ctx_cache[key] = ctx
     return ctx
 
@@ -894,8 +931,9 @@ class ORBExtractor:
                  minThreshold: int, camera: Camera | None = None):
         pattern = load_brief_template(bfTemFp) if bfTemFp else None  # FileNotOpenError like :247-250
         self._image = image
-        h, w = image.shape
-        self._ctx = _context_for(h, w, nFeatures, pyramidLevels, scaleFactor, maxThreshold, minThreshold, camera or Camera(), bfTemFp, pattern)
+        h, w = image.shape[:2]
+        cam = camera or Camera()
+        self._ctx = _context_for(h, w, nFeatures, pyramidLevels, scaleFactor, maxThreshold, minThreshold, cam, bfTemFp, pattern, image_format(image, cam.rgb))
         self._done = False
 
     def extract(self):
@@ -927,23 +965,25 @@ class Frame:
 
     @staticmethod
     def createStereo(leftImg, rightImg, nFeatures, briefFp, maxThresh, minThresh, pVoc=None, nLevels=8, scale=1.2, camera: Camera | None = None) -> "Frame":
-        """Frame::createStereo (include/ORB_SLAM2/Frame.h:313-322)."""
+        """Frame::createStereo (include/ORB_SLAM2/Frame.h:313-322).  Gray (H, W) or colour (H, W, 3 | 4) images, converted
+        on the device in the order camera.rgb names (Tracking::grabFrame's cvtColor, src/Tracking.cc:55-68)."""
         pattern = load_brief_template(briefFp) if briefFp else None
-        h, w = leftImg.shape
-        ctx = _context_for(h, w, nFeatures, nLevels, scale, maxThresh, minThresh, camera or Camera(), briefFp, pattern)
+        h, w = leftImg.shape[:2]
+        cam = camera or Camera()
+        ctx = _context_for(h, w, nFeatures, nLevels, scale, maxThresh, minThresh, cam, briefFp, pattern, image_format(leftImg, cam.rgb))
         r = ctx.stereo_frame(leftImg, rightImg)
         return Frame(r.kps_left, r.desc_left, r.kps_right, r.desc_right, r.u_right, r.depth, r.n_matches, {"ctx": ctx})
 
     @staticmethod
     def createRGBD(colorImg, depthImg, nFeatures, briefF, maxThresh, minThresh, pVoc=None, dScale=1.0, nLevels=8, scale=1.2,
                    camera: Camera | None = None) -> "Frame":
-        """Frame::createRGBD (include/ORB_SLAM2/Frame.h:325-331)."""
+        """Frame::createRGBD (include/ORB_SLAM2/Frame.h:325-331); colorImg may be gray or colour, as in createStereo."""
         import dataclasses
 
         cam = dataclasses.replace(camera or Camera(), depth_scale=float(dScale))
         pattern = load_brief_template(briefF) if briefF else None
-        h, w = colorImg.shape
-        ctx = _context_for(h, w, nFeatures, nLevels, scale, maxThresh, minThresh, cam, briefF, pattern)
+        h, w = colorImg.shape[:2]
+        ctx = _context_for(h, w, nFeatures, nLevels, scale, maxThresh, minThresh, cam, briefF, pattern, image_format(colorImg, cam.rgb))
         r = ctx.rgbd_frame(colorImg, depthImg)
         return Frame(r.kps, r.desc, None, None, r.u_right, r.depth, int((r.depth > 0).sum()), {"ctx": ctx, "kps_raw": r.kps_raw})
 

@@ -354,6 +354,7 @@ int build_tables(orbx_ctx *c)
   p.depth_scale_inv = (float)(1.0 / (double)(g.depth_scale != 0.f ? g.depth_scale : 1.f)); // Mat /= s == convertTo(.., 1./s)
   for (int i = 0; i < 5; ++i) p.dist[i] = g.dist[i];
   p.undistort = g.dist[0] != 0.f ? 1 : 0; // Camera::undistortPoints returns early when k1 == 0 (src/Camera.cc:31)
+  p.in_bpp = 1;
   {
     // VirtualFrame ctor (include/ORB_SLAM2/Frame.h:33-43): undistort (0,0) and (width,height); grid size (src/Frame.cc:55-56)
     float b[4] = {0.f, 0.f, (float)g.width, (float)g.height};
@@ -721,7 +722,7 @@ static int run_stereo_single(orbx_ctx *c, cudaStream_t s, const uint8_t *d_left,
       cudaGraphNodeType t;
       cudaKernelNodeParams kp;
       if (cudaGraphNodeGetType(nd, &t) == cudaSuccess && t == cudaGraphNodeTypeKernel && cudaGraphKernelNodeGetParams(nd, &kp) == cudaSuccess &&
-          kp.func == pyramid_kernel_symbol())
+          kp.func == pyramid_kernel_symbol(c->p.in_bpp))
         c->graph1_pyr = nd;
     }
     if (!c->graph1_pyr)
@@ -752,7 +753,7 @@ static int run_stereo_single(orbx_ctx *c, cudaStream_t s, const uint8_t *d_left,
 int run_stereo_chunks(orbx_ctx *c, int64_t n_frames, const uint8_t *left, size_t left_stride, const uint8_t *right, size_t right_stride, size_t frame_stride,
                       bool on_device, bool piped, const ChunkOut &out)
 {
-  const size_t W = (size_t)c->cfg.width, H = (size_t)c->cfg.height;
+  const size_t W = (size_t)c->cfg.width * (size_t)c->p.in_bpp, H = (size_t)c->cfg.height; // row bytes
   if (std::min(left_stride, right_stride) < W || frame_stride < std::max(left_stride, right_stride) * (H - 1) + W)
     return fail(c, ORBX_ERR_INVALID_ARG, "stride / frame_stride smaller than the image");
   // Densely stacked rows that fit the staging pitch are copied as ONE linear transfer per side and read on the device
@@ -1061,6 +1062,42 @@ extern "C"
     return ORBX_OK;
   }
 
+  int orbx_set_input_format(orbx_ctx *c, int format)
+  {
+    if (!c) return ORBX_ERR_INVALID_ARG;
+    // gray weights of bytes 0, 1, 2 of a pixel (cv::cvtColor, 8-bit: R 9798, G 19235, B 3735, 15 fractional bits)
+    int bpp = 0;
+    uint32_t w0 = 0, w2 = 0;
+    switch (format)
+    {
+    case ORBX_FORMAT_GRAY8: bpp = 1; break;
+    case ORBX_FORMAT_RGB8: bpp = 3, w0 = 9798, w2 = 3735; break;
+    case ORBX_FORMAT_BGR8: bpp = 3, w0 = 3735, w2 = 9798; break;
+    case ORBX_FORMAT_RGBA8: bpp = 4, w0 = 9798, w2 = 3735; break;
+    case ORBX_FORMAT_BGRA8: bpp = 4, w0 = 3735, w2 = 9798; break;
+    default: return fail(c, ORBX_ERR_INVALID_ARG, "unknown input format");
+    }
+    if (format == c->in_format) return ORBX_OK;
+    ORBX_CUDA(c, cudaSetDevice(c->device));
+    const size_t pitch = ((size_t)c->cfg.width * bpp + 15) & ~(size_t)15;
+    if (pitch > c->in_pitch)
+    { // the host staging grows; work of earlier calls may still read the old buffer
+      uint8_t *q = nullptr;
+      ORBX_CUDA(c, cudaDeviceSynchronize());
+      ORBX_CUDA(c, cudaMalloc((void **)&q, (size_t)c->n_img_max * pitch * (size_t)c->cfg.height + 256));
+      std::replace(c->allocs.begin(), c->allocs.end(), (void *)c->d_in, (void *)q);
+      cudaFree(c->d_in);
+      c->d_in = q;
+      c->in_pitch = pitch;
+    }
+    drop_graph(c); // the captured level-0 node is the kernel of the old format
+    c->in_format = format;
+    c->p.in_bpp = bpp;
+    c->p.cvt_w01 = w0 | (19235u << 16);
+    c->p.cvt_w2 = w2;
+    return ORBX_OK;
+  }
+
   int orbx_num_levels(const orbx_ctx *c) { return c ? c->cfg.n_levels : ORBX_ERR_INVALID_ARG; }
 
   int orbx_level_info(const orbx_ctx *c, int level, int32_t *width, int32_t *height, float *scale, int32_t *quota)
@@ -1092,7 +1129,13 @@ extern "C"
 
   int64_t orbx_launch_count(const orbx_ctx *c) { return c ? c->launches : 0; }
   uint64_t orbx_frame_epoch(const orbx_ctx *c) { return c ? c->frame_epoch : 0; }
-  int64_t orbx_algorithmic_bytes(const orbx_ctx *c, int stereo) { return c ? (stereo ? c->alg_bytes_stereo : c->alg_bytes_image) : 0; }
+  int64_t orbx_algorithmic_bytes(const orbx_ctx *c, int stereo)
+  {
+    if (!c) return 0;
+    // a colour context reads bpp bytes per level-0 pixel instead of one
+    const int64_t extra = (int64_t)(c->p.in_bpp - 1) * c->cfg.width * c->cfg.height * (stereo ? 2 : 1);
+    return (stereo ? c->alg_bytes_stereo : c->alg_bytes_image) + extra;
+  }
 
   // ---------------------------------------------------------------------------------------------------------------
   int orbx_extract_batch_device(orbx_ctx *c, int n_images, const uint8_t *d_images, size_t stride, size_t frame_stride, orbx_device_results *out)
@@ -1297,7 +1340,7 @@ extern "C"
     if (!c || !image) return ORBX_ERR_INVALID_ARG;
     ORBX_CUDA(c, cudaSetDevice(c->device));
     const size_t W = (size_t)c->cfg.width, H = (size_t)c->cfg.height, N = (size_t)c->cfg.n_features;
-    ORBX_CUDA(c, cudaMemcpy2DAsync(c->d_in, c->in_pitch, image, stride, W, H, cudaMemcpyHostToDevice, c->stream));
+    ORBX_CUDA(c, cudaMemcpy2DAsync(c->d_in, c->in_pitch, image, stride, W * c->p.in_bpp, H, cudaMemcpyHostToDevice, c->stream));
     int rc = orbx_extract_batch_device(c, 1, c->d_in, c->in_pitch, c->in_pitch * H, nullptr);
     if (rc) return rc;
     const Params &p = c->p;
@@ -1315,7 +1358,7 @@ extern "C"
     ORBX_CUDA(c, cudaSetDevice(c->device));
     const size_t W = (size_t)c->cfg.width, H = (size_t)c->cfg.height, N = (size_t)c->cfg.n_features;
     const size_t esz = depth_type == ORBX_DEPTH_F32 ? 4 : 2;
-    ORBX_CUDA(c, cudaMemcpy2DAsync(c->d_in, c->in_pitch, gray, gray_stride, W, H, cudaMemcpyHostToDevice, c->stream));
+    ORBX_CUDA(c, cudaMemcpy2DAsync(c->d_in, c->in_pitch, gray, gray_stride, W * c->p.in_bpp, H, cudaMemcpyHostToDevice, c->stream));
     ORBX_CUDA(c, cudaMemcpy2DAsync(c->d_depth_in, W * esz, depth_image, depth_stride_bytes, W * esz, H, cudaMemcpyHostToDevice, c->stream));
     int rc = orbx_rgbd_batch_device(c, 1, c->d_in, c->in_pitch, c->in_pitch * H, c->d_depth_in, W * esz, W * H * esz, depth_type, nullptr);
     if (rc) return rc;

@@ -148,6 +148,10 @@ struct Params
   float fx, fy, cx, cy, bf, depth_scale_inv;
   float dist[5];
   int undistort;
+  // input format (orbx_set_input_format): bytes per pixel of the caller's images (1, 3 or 4) and, for colour, the gray
+  // weights of the first three bytes of a pixel packed for DP2A: cvt_w01 = w0 | w1 << 16, cvt_w2 = w2 (the 4th byte weighs 0)
+  int in_bpp;
+  uint32_t cvt_w01, cvt_w2;
 };
 
 // tracking-side matchers (orbx_match.cu)
@@ -234,7 +238,7 @@ inline void ser_bow_inputs(SerArgs &s, const BowArgs &b)
 constexpr int kPyrBoxBytesHost = 18 * 1024; // = kPyrBoxBytes of orbx_kernels.cu: shared-memory bytes a level's source box may take
 void launch_pyramid_level0(const Params &p, int n_images, cudaStream_t s);
 void launch_pyramid_levels(const Params &p, const LevelMaps &src_maps, int n_images, cudaStream_t s);
-const void *pyramid_kernel_symbol(); // host handle of the level-0 pyramid kernel, the only reader of the caller's images (to find its node in a captured graph)
+const void *pyramid_kernel_symbol(int bpp); // host handle of the level-0 pyramid kernel for p.in_bpp == bpp, the only reader of the caller's images (to find its node in a captured graph)
 void launch_fast(const Params &p, const LevelMaps &maps, int n_images, cudaStream_t s);
 int fast_configure(const Params &p); // opt in to the dynamic shared memory of the FAST kernel
 void launch_quadtree(const Params &p, int n_images, size_t smem_bytes, cudaStream_t s);

@@ -41,7 +41,8 @@ struct orbx_ctx
   // device allocations
   std::vector<void *> allocs;
   uint8_t *d_in = nullptr;      // staging for host-side calls: [n_img_max][H][in_pitch]
-  size_t in_pitch = 0;
+  size_t in_pitch = 0;          // 16-byte multiple >= width * p.in_bpp (grows with orbx_set_input_format)
+  int in_format = ORBX_FORMAT_GRAY8;
   uint8_t *d_depth_in = nullptr; // [max_batch][H][W] float/uint16 (sized for float)
   int last_images = 0;          // images processed by the most recent call (for orbx_get_pyramid)
   int last_stereo = 0;

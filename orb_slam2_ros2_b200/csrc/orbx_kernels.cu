@@ -240,7 +240,36 @@ template <class S> __device__ __forceinline__ void pyr_blur_cols(const S &sm, co
   }
 }
 
-__global__ void __launch_bounds__(kPyrThreads) pyramid_level0_kernel(const Params p)
+// Colour input (orbx_set_input_format): cv::cvtColor's 8-bit RGB -> gray rule, gray = (w0 c0 + w1 c1 + w2 c2 + 16384) >> 15
+// with the weights of the channel order (9798 R, 19235 G, 3735 B; they sum to 32768, so the result is at most 255).  `px`
+// holds one pixel's first three bytes in bytes 0..2; byte 3 (alpha, or the next pixel's first byte) weighs 0.
+__device__ __forceinline__ uint32_t gray_of(uint32_t px, uint32_t w01, uint32_t w2) { return __dp2a_lo(w01, px, __dp2a_hi(w2, px, 16384u)) >> 15; }
+
+// one gray pixel of the caller's image: q = its first byte
+template <int kBpp> __device__ __forceinline__ uint32_t gray_at(const uint8_t *q, const Params &p)
+{
+  if constexpr (kBpp == 1)
+    return *q;
+  else
+    return gray_of((uint32_t)q[0] | ((uint32_t)q[1] << 8) | ((uint32_t)q[2] << 16), p.cvt_w01, p.cvt_w2);
+}
+
+// the 4 gray bytes of 4 consecutive pixels held in b[0 .. kBpp) (4 * kBpp bytes, pixel k at byte k * kBpp)
+template <int kBpp> __device__ __forceinline__ uint32_t gray4(const uint32_t (&b)[kBpp], uint32_t w01, uint32_t w2)
+{
+  uint32_t px[4];
+  if constexpr (kBpp == 4)
+    px[0] = b[0], px[1] = b[1], px[2] = b[2], px[3] = b[3];
+  else
+    px[0] = b[0], px[1] = __funnelshift_r(b[0], b[1], 24), px[2] = __funnelshift_r(b[1], b[2], 16), px[3] = b[2] >> 8;
+  uint32_t v = 0;
+#pragma unroll
+  for (int k = 0; k < 4; ++k) v |= gray_of(px[k], w01, w2) << (8 * k);
+  return v;
+}
+
+// kBpp = bytes per pixel of the caller's images (1 gray, 3 RGB / BGR, 4 RGBA / BGRA); the channel order travels as weights
+template <int kBpp> __global__ void __launch_bounds__(kPyrThreads) pyramid_level0_kernel(const Params p)
 {
   __shared__ PyrShared sm;
   const Tile t = p.tiles[blockIdx.x];
@@ -265,45 +294,81 @@ __global__ void __launch_bounds__(kPyrThreads) pyramid_level0_kernel(const Param
   // stage A: thread <-> word column j (source columns x0 - 4 + 4 j .. + 3), kWordRows rows per pass.  Word columns jl .. jh lie
   // completely inside the image: two aligned loads + a funnel shift per word, no per-row branch.  The others (the left / right
   // borders: REFLECT_101, zero beyond the level + halo) and the first / last image row are patched byte by byte afterwards.
+  // Colour: the 4 pixels of a word column are a 12- / 16-byte window at any alignment, read as 4 / 5 aligned words (at most
+  // 3 bytes before and 4 after the window, as for gray) and funnel-shifted into place, then converted to 4 gray bytes.
   const int jl = t.x0 == 0 ? 1 : 0, jh = min(kSrcWords - 1, (lw - t.x0) >> 2);
   {
     const int j = tid % kSrcWords, grp = tid / kSrcWords;
     if (grp < kWordRows && j >= jl && j <= jh)
     {
       uint32_t *dst = reinterpret_cast<uint32_t *>(sm.src) + kSrcWord0 + j + grp * (kSrcPitch / 4);
-      const uint8_t *col_src = src + (t.x0 - 4 + 4 * j);
+      const uint8_t *col_src = src + (t.x0 - 4 + 4 * j) * kBpp;
       asm volatile("" : "+l"(col_src)); // one register pair: a row address is one IMAD.WIDE.U32
       const uint4 *rp = sm.row + grp;
       constexpr int U = 5; // 70 rows = 14 rows per pass x 5: all loads of a tile are issued before the first use
       static_assert(kWordRows * U == kSrcH, "the row passes tile the buffer exactly");
-      uint32_t w0[U], w1[U], sh[U], ok[U];
-#pragma unroll
-      for (int u = 0; u < U; ++u)
+      if constexpr (kBpp == 1)
       {
-        const uint4 r = rp[u * kWordRows];
-        const uint8_t *a = col_src + r.x;
-        ok[u] = r.z;
-        w0[u] = w1[u] = 0u;
-        if (ok[u])
-        {
-          const uint32_t *al = reinterpret_cast<const uint32_t *>(reinterpret_cast<uintptr_t>(a) & ~(uintptr_t)3);
-          w0[u] = al[0], w1[u] = al[1];
-        }
-        sh[u] = (uint32_t)reinterpret_cast<uintptr_t>(a) << 3; // funnel shifts take the amount modulo 32
-      }
+        uint32_t w0[U], w1[U], sh[U], ok[U];
 #pragma unroll
-      for (int u = 0; u < U; ++u)
-        if (ok[u]) dst[u * kWordRows * (kSrcPitch / 4)] = __funnelshift_r(w0[u], w1[u], sh[u]);
+        for (int u = 0; u < U; ++u)
+        {
+          const uint4 r = rp[u * kWordRows];
+          const uint8_t *a = col_src + r.x;
+          ok[u] = r.z;
+          w0[u] = w1[u] = 0u;
+          if (ok[u])
+          {
+            const uint32_t *al = reinterpret_cast<const uint32_t *>(reinterpret_cast<uintptr_t>(a) & ~(uintptr_t)3);
+            w0[u] = al[0], w1[u] = al[1];
+          }
+          sh[u] = (uint32_t)reinterpret_cast<uintptr_t>(a) << 3; // funnel shifts take the amount modulo 32
+        }
+#pragma unroll
+        for (int u = 0; u < U; ++u)
+          if (ok[u]) dst[u * kWordRows * (kSrcPitch / 4)] = __funnelshift_r(w0[u], w1[u], sh[u]);
+      }
+      else
+      {
+        constexpr int NW = kBpp + 1; // aligned words that cover a window of kBpp words at any alignment
+        uint32_t w[U][NW], sh[U], ok[U];
+#pragma unroll
+        for (int u = 0; u < U; ++u)
+        {
+          const uint4 r = rp[u * kWordRows];
+          const uint8_t *a = col_src + r.x;
+          ok[u] = r.z;
+#pragma unroll
+          for (int k = 0; k < NW; ++k) w[u][k] = 0u;
+          if (ok[u])
+          {
+            const uint32_t *al = reinterpret_cast<const uint32_t *>(reinterpret_cast<uintptr_t>(a) & ~(uintptr_t)3);
+#pragma unroll
+            for (int k = 0; k < NW; ++k) w[u][k] = al[k];
+          }
+          sh[u] = (uint32_t)reinterpret_cast<uintptr_t>(a) << 3;
+        }
+        const uint32_t w01 = p.cvt_w01, w2 = p.cvt_w2;
+#pragma unroll
+        for (int u = 0; u < U; ++u)
+          if (ok[u])
+          {
+            uint32_t b[kBpp];
+#pragma unroll
+            for (int k = 0; k < kBpp; ++k) b[k] = __funnelshift_r(w[u][k], w[u][k + 1], sh[u]);
+            dst[u * kWordRows * (kSrcPitch / 4)] = gray4<kBpp>(b, w01, w2);
+          }
+      }
     }
   }
   {
-    auto gather_word = [&](int ty, int j) { // REFLECT_101 per byte; columns beyond the level + halo are zero
+    auto gather_word = [&](int ty, int j) { // REFLECT_101 per pixel; columns beyond the level + halo are zero
       const uint8_t *rowp = src + (size_t)sm.row[ty].x;
       const int rx = t.x0 - 4 + 4 * j;
       uint32_t v = 0;
 #pragma unroll
       for (int k = 0; k < 4; ++k)
-        if (rx + k < lw + kHalo) v |= (uint32_t)rowp[refl101(rx + k, lw)] << (8 * k);
+        if (rx + k < lw + kHalo) v |= gray_at<kBpp>(rowp + refl101(rx + k, lw) * kBpp, p) << (8 * k);
       reinterpret_cast<uint32_t *>(sm.src)[ty * (kSrcPitch / 4) + kSrcWord0 + j] = v;
     };
     // border word columns [0, jl) and (jh, kSrcWords), all rows
@@ -488,10 +553,23 @@ __global__ void __launch_bounds__(kPyrThreads) pyramid_levels_kernel(const Param
   pyr_blur_cols(sm, t, lh, pitch, p.blur + (size_t)img * p.pyr_img_stride + L.pyr_off);
 }
 
-const void *pyramid_kernel_symbol() { return reinterpret_cast<const void *>(&pyramid_level0_kernel); }
+const void *pyramid_kernel_symbol(int bpp)
+{
+  return bpp == 4 ? reinterpret_cast<const void *>(&pyramid_level0_kernel<4>)
+                  : (bpp == 3 ? reinterpret_cast<const void *>(&pyramid_level0_kernel<3>) : reinterpret_cast<const void *>(&pyramid_level0_kernel<1>));
+}
 
 // two launches: level 0 (reads the caller's images), then the resized levels (read level 0 from the pyramid buffer)
-void launch_pyramid_level0(const Params &p, int n_images, cudaStream_t s) { pyramid_level0_kernel<<<dim3(p.n_tiles0, n_images), kPyrThreads, 0, s>>>(p); }
+void launch_pyramid_level0(const Params &p, int n_images, cudaStream_t s)
+{
+  const dim3 grid(p.n_tiles0, n_images);
+  if (p.in_bpp == 4)
+    pyramid_level0_kernel<4><<<grid, kPyrThreads, 0, s>>>(p);
+  else if (p.in_bpp == 3)
+    pyramid_level0_kernel<3><<<grid, kPyrThreads, 0, s>>>(p);
+  else
+    pyramid_level0_kernel<1><<<grid, kPyrThreads, 0, s>>>(p);
+}
 
 void launch_pyramid_levels(const Params &p, const LevelMaps &src_maps, int n_images, cudaStream_t s)
 {
