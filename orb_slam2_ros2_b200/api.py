@@ -1079,6 +1079,22 @@ class ORBMatcher:
         return np.stack([qi, ti, di.astype(np.int32)], axis=1).astype(np.int32).reshape(-1, 3)
 
 
+def _training_set(desc, counts, n_frames, stride):
+    """(F, stride, desc pointer, counts pointer) of the descriptors desc[f][i], i < counts[f]: numpy arrays ((F, stride, 32)
+    uint8 and (F,) int32), or device pointers (ints), which then need n_frames and stride.  The pointers to host copies come
+    from ctypes.data_as, which keeps its array alive as long as the pointer is."""
+    if isinstance(desc, int):
+        assert isinstance(counts, int) and n_frames is not None and stride is not None, "device pointers need n_frames and stride"
+        return int(n_frames), int(stride), desc, counts
+    d = np.ascontiguousarray(desc, np.uint8)
+    assert d.ndim == 3 and d.shape[2] == 32
+    F = d.shape[0] if n_frames is None else int(n_frames)
+    d = np.ascontiguousarray(d[:F])
+    cnt = np.ascontiguousarray(np.asarray(counts)[:F], np.int32)
+    assert len(cnt) == F
+    return F, d.shape[1], d.ctypes.data_as(C.c_void_p), cnt.ctypes.data_as(C.c_void_p)
+
+
 class Vocabulary:
     """DBoW3::Vocabulary resident on a context's device (the reference loads it in src/System.cc:93)."""
 
@@ -1115,18 +1131,7 @@ class Vocabulary:
         self._L = ctx._L
         self._h = C.c_void_p()
         on_device = isinstance(desc, int)
-        if on_device:
-            assert isinstance(counts, int) and n_frames is not None and stride is not None, "device pointers need n_frames and stride"
-            F, S, dp, cp = int(n_frames), int(stride), desc, counts
-        else:
-            d = np.ascontiguousarray(desc, np.uint8)
-            assert d.ndim == 3 and d.shape[2] == 32
-            F = d.shape[0] if n_frames is None else int(n_frames)
-            S = d.shape[1]
-            d = np.ascontiguousarray(d[:F])
-            cnt = np.ascontiguousarray(np.asarray(counts)[:F], np.int32)
-            assert len(cnt) == F
-            dp, cp = d.ctypes.data, cnt.ctypes.data
+        F, S, dp, cp = _training_set(desc, counts, n_frames, stride)
         iters, capped, ms = np.zeros(max(int(L), 1), np.int32), C.c_int32(0), np.zeros(max(int(L), 1) + 1, np.float32)
         tr = OrbxVocabTrain(dp, cp, F, S, int(on_device), int(k), int(L), int(seed) & (2**64 - 1), iters.ctypes.data, C.addressof(capped), ms.ctypes.data)
         _check(ctx._h, self._L.orbx_vocab_build(ctx._h, C.byref(tr), C.byref(self._h)), "orbx_vocab_build")
@@ -1178,18 +1183,7 @@ class BowDatabase:
         self._L, self.ctx = ctx._L, ctx
         self._h = C.c_void_p()
         on_device = isinstance(desc, int)
-        if on_device:
-            assert isinstance(counts, int) and n_frames is not None and stride is not None, "device pointers need n_frames and stride"
-            F, S, dp, cp = int(n_frames), int(stride), desc, counts
-        else:
-            d = np.ascontiguousarray(desc, np.uint8)
-            assert d.ndim == 3 and d.shape[2] == 32
-            F = d.shape[0] if n_frames is None else int(n_frames)
-            S = d.shape[1]
-            d = np.ascontiguousarray(d[:F])
-            cnt = np.ascontiguousarray(np.asarray(counts)[:F], np.int32)
-            assert len(cnt) == F
-            dp, cp = d.ctypes.data, cnt.ctypes.data
+        F, S, dp, cp = _training_set(desc, counts, n_frames, stride)
         _check(ctx._h, self._L.orbx_bowdb_build(ctx._h, vocab._h, dp, cp, F, S, int(on_device), C.byref(self._h)), "orbx_bowdb_build")
         return self
 

@@ -470,6 +470,42 @@ int fail(orbx_ctx *c, int code, const std::string &msg)
   return code;
 }
 
+int require_owner(orbx_ctx *c, const orbx_ctx *owner_ctx, int owner_device, const char *what)
+{
+  if (owner_ctx != c || owner_device != c->device) return fail(c, ORBX_ERR_INVALID_ARG, std::string(what) + " belongs to another context");
+  return ORBX_OK;
+}
+
+int resident_ctas(orbx_ctx *c, const void *kernel, int threads, size_t smem, const char *what, int *n)
+{
+  int per_sm = 0, n_sm = 0;
+  ORBX_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
+  ORBX_CUDA(c, cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, c->device));
+  if (per_sm < 1) return fail(c, ORBX_ERR_CUDA, std::string(what) + " does not fit an SM");
+  *n = per_sm * n_sm;
+  return ORBX_OK;
+}
+
+int IoStaging::place()
+{
+  if (int rc = buf.reserve(c, total)) return rc;
+  for (const Slice &x : slices)
+  {
+    x.set(buf.p + x.off);
+    if (x.from) ORBX_CUDA(c, cudaMemcpyAsync(buf.p + x.off, x.from, x.bytes, cudaMemcpyHostToDevice, c->stream));
+  }
+  return ORBX_OK;
+}
+
+int IoStaging::finish()
+{
+  if (on_device) return ORBX_OK;
+  for (const Slice &x : slices)
+    if (x.to) ORBX_CUDA(c, cudaMemcpyAsync(x.to, buf.p + x.off, x.bytes, cudaMemcpyDeviceToHost, c->stream));
+  ORBX_CUDA(c, cudaStreamSynchronize(c->stream));
+  return ORBX_OK;
+}
+
 int bow_buffers(orbx_ctx *c)
 {
   if (c->bow_ready) return ORBX_OK;
@@ -490,14 +526,6 @@ int bow_buffers(orbx_ctx *c)
   if ((rc = dev_alloc(c, &b.n_fv, F))) return rc;
   c->bow_ready = true;
   return ORBX_OK;
-}
-
-BowArgs bow_args(const orbx_ctx *c, const orbx_vocab *v, int levelsup, int image_stride)
-{
-  BowArgs a = c->bow;
-  a.child_start = v->child_start, a.child_ids = v->child_ids, a.v_desc = v->desc, a.v_weight = v->weight, a.v_word = v->word;
-  a.L = v->L, a.levelsup = levelsup, a.image_stride = image_stride;
-  return a;
 }
 
 void append_g(std::string &t, double v)
@@ -1756,7 +1784,7 @@ extern "C"
     std::vector<double> w((size_t)n, 0.0);
     std::memcpy(w.data() + 1, weight, (size_t)n_records * sizeof(double));
     ORBX_CUDA(c, cudaSetDevice(c->device));
-    orbx_vocab *v = new orbx_vocab();
+    Building<orbx_vocab> v(new orbx_vocab(), orbx_vocab_destroy);
     v->ctx = c, v->device = c->device, v->k = k, v->L = L, v->n_nodes = n, v->n_words = n_words;
     v->rec_parent.assign(parent, parent + n_records);
     v->rec_leaf.resize((size_t)n_records);
@@ -1768,17 +1796,12 @@ extern "C"
       if (e != cudaSuccess) return e;
       return cudaMemcpy(*dst, src.data(), src.size() * sizeof(src[0]), cudaMemcpyHostToDevice);
     };
-    cudaError_t e = up(&v->child_start, start);
-    if (e == cudaSuccess) e = up(&v->child_ids, ids);
-    if (e == cudaSuccess) e = up(&v->word, word);
-    if (e == cudaSuccess) e = up(&v->desc, d);
-    if (e == cudaSuccess) e = up(&v->weight, w);
-    if (e != cudaSuccess)
-    {
-      orbx_vocab_destroy(v);
-      return fail(c, ORBX_ERR_CUDA, std::string("vocabulary upload: ") + cudaGetErrorString(e));
-    }
-    *out = v;
+    ORBX_CUDA(c, up(&v->child_start, start));
+    ORBX_CUDA(c, up(&v->child_ids, ids));
+    ORBX_CUDA(c, up(&v->word, word));
+    ORBX_CUDA(c, up(&v->desc, d));
+    ORBX_CUDA(c, up(&v->weight, w));
+    *out = v.release();
     return ORBX_OK;
   }
 
@@ -1883,10 +1906,8 @@ extern "C"
     ORBX_CUDA(c, cudaSetDevice(c->device));
     int rc = bow_buffers(c);
     if (rc) return rc;
-    const BowArgs a = bow_args(c, v, levelsup, image_stride(c));
-    launch_bow_descend(c->p, a, n_frames, c->stream);
-    launch_bow_assemble(c->p, a, n_frames, c->stream);
-    c->launches += 2;
+    const BowArgs a = bow_args(v, levelsup, image_stride(c), c->bow);
+    launch_bow_transform(c, c->p, a, n_frames, c->stream);
     c->bow_epoch = c->frame_epoch;
     c->bow_frames = n_frames;
     c->bow_vocab = v;

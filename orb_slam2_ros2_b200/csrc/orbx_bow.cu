@@ -10,6 +10,11 @@
 //                        (std::map<NodeId, vector<unsigned>>) from two stable sorts of (key << 16 | feature index)
 //   bow_word_frames_kernel  one CTA per frame: the frame's distinct words (the same sort), one integer atomic per word;
 //                        N_i of TF_IDF for orbx_vocab_build (setNodeWeights)
+// and the host code the bag-of-words entry points share: the tree arguments, the transform launch, the builders' training-set
+// intake and bow_frames, the chunked transform of the keyframe database and the loop verifier.
+#include <algorithm>
+#include <cstring>
+
 #include "orbx_internal.h"
 
 namespace orbx
@@ -257,6 +262,79 @@ int bow_configure(orbx_ctx *c, int n_features, int too_large)
   static SmemOptIn state, state_words;
   if (raise_dynamic_smem(bow_assemble_kernel, state, bytes) || raise_dynamic_smem(bow_word_frames_kernel, state_words, bytes))
     return fail(c, ORBX_ERR_CUDA, "cannot reserve shared memory for the bag-of-words sort");
+  return ORBX_OK;
+}
+
+BowArgs bow_args(const orbx_vocab *v, int levelsup, int image_stride, BowArgs b)
+{
+  b.child_start = v->child_start, b.child_ids = v->child_ids, b.v_desc = v->desc, b.v_weight = v->weight, b.v_word = v->word;
+  b.L = v->L, b.levelsup = levelsup, b.image_stride = image_stride;
+  return b;
+}
+
+void launch_bow_transform(orbx_ctx *c, const Params &p, const BowArgs &a, int n_frames, cudaStream_t s)
+{
+  launch_bow_descend(p, a, n_frames, s);
+  launch_bow_assemble(p, a, n_frames, s);
+  c->launches += 2;
+}
+
+int read_training_set(orbx_ctx *c, const uint8_t *desc, const int32_t *n_kps, int F, int stride, bool on_device, const char *what, TrainingSet &ts)
+{
+  cudaStream_t s = c->stream;
+  ts.n.resize((size_t)F);
+  if (on_device)
+  {
+    ORBX_CUDA(c, cudaMemcpyAsync(ts.n.data(), n_kps, (size_t)F * 4, cudaMemcpyDeviceToHost, s));
+    ORBX_CUDA(c, cudaStreamSynchronize(s));
+  }
+  else
+    std::memcpy(ts.n.data(), n_kps, (size_t)F * 4);
+  for (int32_t x : ts.n)
+    if (x < 0 || x > stride) return fail(c, ORBX_ERR_INVALID_ARG, std::string(what) + ": a count lies outside 0..stride");
+  ts.desc = desc, ts.d_n = n_kps;
+  if (on_device) return ORBX_OK;
+  // the kernels read no byte past rows * 32 of the descriptors and F * 4 of the counts
+  const size_t desc_bytes = up16((size_t)F * stride * 32);
+  if (int rc = ts.staged.reserve(c, desc_bytes + (size_t)F * 4)) return rc;
+  ORBX_CUDA(c, cudaMemcpyAsync(ts.staged.p, desc, (size_t)F * stride * 32, cudaMemcpyHostToDevice, s));
+  ORBX_CUDA(c, cudaMemcpyAsync(ts.staged.p + desc_bytes, n_kps, (size_t)F * 4, cudaMemcpyHostToDevice, s));
+  ts.desc = ts.staged.p, ts.d_n = (const int32_t *)(ts.staged.p + desc_bytes);
+  return ORBX_OK;
+}
+
+int bow_frames(orbx_ctx *c, const orbx_vocab *v, int levelsup, const uint8_t *d_desc, const int *d_n, int F, int stride, const BowArgs &out)
+{
+  constexpr int kChunk = 1024; // frames per transform launch: bounds the per-feature scratch at 28 B x stride x 1024
+  cudaStream_t s = c->stream;
+  const size_t ch = (size_t)std::min(F, kChunk) * stride;
+  auto sc = [](const void *mine, size_t bytes) { return mine ? 0 : up16(bytes); }; // scratch only for the outputs left null
+  const size_t o_word = 0, o_nid = o_word + up16(ch * 4), o_w = o_nid + up16(ch * 4), o_ids = o_w + up16(ch * 8), o_vals = o_ids + sc(out.bow_ids, ch * 4),
+               o_nb = o_vals + sc(out.bow_vals, ch * 8), o_fvn = o_nb + sc(out.n_bow, (size_t)kChunk * 4), o_fvs = o_fvn + sc(out.fv_nodes, ch * 4),
+               o_fvf = o_fvs + sc(out.fv_start, ch * 4 + (size_t)kChunk * 4), o_nfv = o_fvf + sc(out.fv_feats, ch * 4),
+               sc_total = o_nfv + sc(out.n_fv, (size_t)kChunk * 4);
+  DeviceBuffer scratch;
+  if (int rc = scratch.reserve(c, sc_total)) return rc;
+  BowArgs b = bow_args(v, levelsup, 1);
+  b.f_word = (int *)(scratch.p + o_word), b.f_nid = (int *)(scratch.p + o_nid), b.f_weight = (double *)(scratch.p + o_w);
+  for (int f0 = 0; f0 < F; f0 += kChunk)
+  {
+    const int nf = std::min(kChunk, F - f0);
+    const size_t e0 = (size_t)f0 * stride;
+    auto at = [&](auto *mine, size_t off, size_t per_frame) { return mine ? mine + (size_t)f0 * per_frame : (decltype(mine))(scratch.p + off); };
+    Params p{};
+    p.n_features = stride;
+    p.desc = const_cast<uint8_t *>(d_desc) + e0 * 32;
+    p.n_kps = const_cast<int *>(d_n) + f0;
+    BowArgs bb = b;
+    bb.bow_ids = at(out.bow_ids, o_ids, stride), bb.bow_vals = at(out.bow_vals, o_vals, stride), bb.n_bow = at(out.n_bow, o_nb, 1);
+    bb.fv_nodes = at(out.fv_nodes, o_fvn, stride), bb.fv_start = at(out.fv_start, o_fvs, (size_t)stride + 1), bb.fv_feats = at(out.fv_feats, o_fvf, stride);
+    bb.n_fv = at(out.n_fv, o_nfv, 1);
+    launch_bow_transform(c, p, bb, nf, s);
+  }
+  ORBX_CUDA(c, cudaGetLastError());
+  // the scratch is freed on return: the work that reads it has to finish first
+  ORBX_CUDA(c, cudaStreamSynchronize(s));
   return ORBX_OK;
 }
 

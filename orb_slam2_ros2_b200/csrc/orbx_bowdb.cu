@@ -3,8 +3,8 @@
 // Restates the first stage of ORB-SLAM2's KeyFrameDatabase::DetectLoopCandidates / DetectRelocalizationCandidates with
 // DBoW3's L1Scoring::score under the rules of include/orbx.h; tests/bowdb_oracle.c is the sequential restatement the kernels
 // are tested against bit for bit.
-//   build: the BowVectors of every frame come from bow_descend_kernel + bow_assemble_kernel (orbx_bow.cu) in chunks of
-//   frames; the inverted file is a CSR by word:
+//   build: the BowVectors of every frame come from bow_frames (orbx_bow.cu: bow_descend_kernel + bow_assemble_kernel in
+//   chunks of frames); the inverted file is a CSR by word:
 //     bowdb_word_count_kernel   postings per word (one integer atomic per BowVector entry)
 //     bowdb_scan_kernel         exclusive scan over the words (one CTA: a serial run per thread + a block scan)
 //     bowdb_fill_kernel         frame ids into the postings (order inside a word is not observable: counts are integers)
@@ -19,9 +19,6 @@
 //     output     (score desc, frame asc) packed into 64-bit keys, bitonic sort of the kept ones, the first top_k written
 #include <algorithm>
 #include <cmath>
-#include <cstring>
-#include <string>
-#include <vector>
 
 #include "orbx_internal.h"
 #include "orbx_match.cuh"
@@ -314,48 +311,7 @@ __global__ void __launch_bounds__(kQT) bowdb_query_kernel(const QueryArgs a)
   }
 }
 
-size_t up16(size_t v) { return (v + 15) & ~(size_t)15; }
-
 } // namespace
-
-int bow_frames(orbx_ctx *c, const orbx_vocab *v, int levelsup, const uint8_t *d_desc, const int *d_n, int F, int stride, const BowArgs &out)
-{
-  constexpr int kChunk = 1024; // frames per transform launch: bounds the per-feature scratch at 28 B x stride x 1024
-  cudaStream_t s = c->stream;
-  const size_t ch = (size_t)std::min(F, kChunk) * stride;
-  auto sc = [](const void *mine, size_t bytes) { return mine ? 0 : up16(bytes); }; // scratch only for the outputs left null
-  const size_t o_word = 0, o_nid = o_word + up16(ch * 4), o_w = o_nid + up16(ch * 4), o_ids = o_w + up16(ch * 8), o_vals = o_ids + sc(out.bow_ids, ch * 4),
-               o_nb = o_vals + sc(out.bow_vals, ch * 8), o_fvn = o_nb + sc(out.n_bow, (size_t)kChunk * 4), o_fvs = o_fvn + sc(out.fv_nodes, ch * 4),
-               o_fvf = o_fvs + sc(out.fv_start, ch * 4 + (size_t)kChunk * 4), o_nfv = o_fvf + sc(out.fv_feats, ch * 4),
-               sc_total = o_nfv + sc(out.n_fv, (size_t)kChunk * 4);
-  DeviceBuffer scratch;
-  if (int rc = scratch.reserve(c, sc_total)) return rc;
-  BowArgs b{};
-  b.child_start = v->child_start, b.child_ids = v->child_ids, b.v_desc = v->desc, b.v_weight = v->weight, b.v_word = v->word;
-  b.L = v->L, b.levelsup = levelsup, b.image_stride = 1;
-  b.f_word = (int *)(scratch.p + o_word), b.f_nid = (int *)(scratch.p + o_nid), b.f_weight = (double *)(scratch.p + o_w);
-  for (int f0 = 0; f0 < F; f0 += kChunk)
-  {
-    const int nf = std::min(kChunk, F - f0);
-    const size_t e0 = (size_t)f0 * stride;
-    auto at = [&](auto *mine, size_t off, size_t per_frame) { return mine ? mine + (size_t)f0 * per_frame : (decltype(mine))(scratch.p + off); };
-    Params p{};
-    p.n_features = stride;
-    p.desc = const_cast<uint8_t *>(d_desc) + e0 * 32;
-    p.n_kps = const_cast<int *>(d_n) + f0;
-    BowArgs bb = b;
-    bb.bow_ids = at(out.bow_ids, o_ids, stride), bb.bow_vals = at(out.bow_vals, o_vals, stride), bb.n_bow = at(out.n_bow, o_nb, 1);
-    bb.fv_nodes = at(out.fv_nodes, o_fvn, stride), bb.fv_start = at(out.fv_start, o_fvs, (size_t)stride + 1), bb.fv_feats = at(out.fv_feats, o_fvf, stride);
-    bb.n_fv = at(out.n_fv, o_nfv, 1);
-    launch_bow_descend(p, bb, nf, s);
-    launch_bow_assemble(p, bb, nf, s);
-    c->launches += 2;
-  }
-  ORBX_CUDA(c, cudaGetLastError());
-  // the scratch is freed on return: the work that reads it has to finish first
-  ORBX_CUDA(c, cudaStreamSynchronize(s));
-  return ORBX_OK;
-}
 
 } // namespace orbx
 
@@ -364,66 +320,31 @@ using namespace orbx;
 namespace
 {
 
-// frees a partly built database on the error paths of orbx_bowdb_build
-struct DbGuard
-{
-  orbx_bowdb *db;
-  ~DbGuard()
-  {
-    if (db) orbx_bowdb_destroy(db);
-  }
-};
-
 int run_query(orbx_ctx *c, const orbx_bowdb *db, QueryArgs a, const orbx_bowdb_io *io)
 {
   const size_t nq = (size_t)a.n_queries, nk = nq * (size_t)a.top_k;
-  cudaStream_t s = c->stream;
-  uint8_t *st = nullptr;
-  const size_t o_f = 0, o_s = o_f + up16(nk * 4), o_c = o_s + up16(nk * 4), o_n = o_c + up16(nk * 4), total = o_n + 4 * up16(nq * 4);
-  if (io->on_device)
-  {
-    a.cand_frame = io->cand_frame, a.cand_score = io->cand_score, a.cand_common = io->cand_common;
-    a.n_sharing = io->n_sharing, a.max_common = io->max_common, a.n_scored = io->n_scored, a.n_kept = io->n_kept;
-  }
-  else
-  {
-    if (int rc = const_cast<orbx_bowdb *>(db)->staging.reserve(c, total)) return rc;
-    st = db->staging.p;
-    a.cand_frame = io->cand_frame ? (int *)(st + o_f) : nullptr;
-    a.cand_score = io->cand_score ? (float *)(st + o_s) : nullptr;
-    a.cand_common = io->cand_common ? (int *)(st + o_c) : nullptr;
-    int *cnts = (int *)(st + o_n);
-    const size_t q4 = up16(nq * 4) / 4;
-    a.n_sharing = io->n_sharing ? cnts : nullptr;
-    a.max_common = io->max_common ? cnts + q4 : nullptr;
-    a.n_scored = io->n_scored ? cnts + 2 * q4 : nullptr;
-    a.n_kept = io->n_kept ? cnts + 3 * q4 : nullptr;
-  }
+  IoStaging st{c, const_cast<orbx_bowdb *>(db)->staging, io->on_device != 0};
+  st.out(a.cand_frame, io->cand_frame, nk * 4);
+  st.out(a.cand_score, io->cand_score, nk * 4);
+  st.out(a.cand_common, io->cand_common, nk * 4);
+  st.out(a.n_sharing, io->n_sharing, nq * 4);
+  st.out(a.max_common, io->max_common, nq * 4);
+  st.out(a.n_scored, io->n_scored, nq * 4);
+  st.out(a.n_kept, io->n_kept, nq * 4);
+  if (int rc = st.place()) return rc;
   a.ids = db->ids, a.n = db->n, a.vals = db->vals, a.stride = db->stride, a.word_start = db->word_start, a.post = db->post;
   a.F = db->F, a.P = db->P, a.list_in_smem = db->list_in_smem, a.g_list = db->g_list;
   const int grid = (int)std::min<size_t>(nq, (size_t)db->grid_max);
-  bowdb_query_kernel<<<grid, kQT, db->smem, s>>>(a);
+  bowdb_query_kernel<<<grid, kQT, db->smem, c->stream>>>(a);
   ++c->launches;
   ORBX_CUDA(c, cudaGetLastError());
-  if (io->on_device) return ORBX_OK;
-  auto back = [&](void *dst, const void *src, size_t bytes) -> cudaError_t {
-    return dst ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, s) : cudaSuccess;
-  };
-  ORBX_CUDA(c, back(io->cand_frame, a.cand_frame, nk * 4));
-  ORBX_CUDA(c, back(io->cand_score, a.cand_score, nk * 4));
-  ORBX_CUDA(c, back(io->cand_common, a.cand_common, nk * 4));
-  ORBX_CUDA(c, back(io->n_sharing, a.n_sharing, nq * 4));
-  ORBX_CUDA(c, back(io->max_common, a.max_common, nq * 4));
-  ORBX_CUDA(c, back(io->n_scored, a.n_scored, nq * 4));
-  ORBX_CUDA(c, back(io->n_kept, a.n_kept, nq * 4));
-  ORBX_CUDA(c, cudaStreamSynchronize(s));
-  return ORBX_OK;
+  return st.finish();
 }
 
 int check_io(orbx_ctx *c, const orbx_bowdb *db, const orbx_bowdb_io *io, bool range)
 {
   if (!io) return ORBX_ERR_INVALID_ARG;
-  if (db->ctx != c || db->device != c->device) return fail(c, ORBX_ERR_INVALID_ARG, "the database belongs to another context");
+  if (int rc = require_owner(c, db->ctx, db->device, "the database")) return rc;
   if (io->top_k < 1 || io->top_k > db->F) return fail(c, ORBX_ERR_INVALID_ARG, "top_k must be 1..n_frames");
   if (range ? io->exclude_window < 0 : io->exclude_window != -1)
     return fail(c, ORBX_ERR_INVALID_ARG, "exclude_window must be >= 0 for range queries and -1 for the resident-frame query");
@@ -463,47 +384,28 @@ extern "C"
   {
     if (!c || !v || !desc || !n_kps || !out) return ORBX_ERR_INVALID_ARG;
     *out = nullptr;
-    if (v->ctx != c || v->device != c->device) return fail(c, ORBX_ERR_INVALID_ARG, "the vocabulary belongs to another context");
+    if (int rc = require_owner(c, v->ctx, v->device, "the vocabulary")) return rc;
     if (F < 1) return fail(c, ORBX_ERR_INVALID_ARG, "keyframe database: n_frames < 1");
     if (F > ORBX_BOWDB_MAX_FRAMES) return fail(c, ORBX_ERR_CAPACITY, "keyframe database: more than ORBX_BOWDB_MAX_FRAMES frames");
     if (stride < 1) return fail(c, ORBX_ERR_INVALID_ARG, "keyframe database: stride < 1");
     cudaStream_t s = c->stream;
     ORBX_CUDA(c, cudaSetDevice(c->device));
     if (int rc = bow_configure(c, stride, ORBX_ERR_INVALID_ARG)) return rc;
-    std::vector<int32_t> h_n((size_t)F);
-    if (on_device)
-    {
-      ORBX_CUDA(c, cudaMemcpyAsync(h_n.data(), n_kps, (size_t)F * 4, cudaMemcpyDeviceToHost, s));
-      ORBX_CUDA(c, cudaStreamSynchronize(s));
-    }
-    else
-      std::memcpy(h_n.data(), n_kps, (size_t)F * 4);
-    for (int f = 0; f < F; ++f)
-      if (h_n[(size_t)f] < 0 || h_n[(size_t)f] > stride) return fail(c, ORBX_ERR_INVALID_ARG, "keyframe database: a count lies outside 0..stride");
+    TrainingSet in;
+    if (int rc = read_training_set(c, desc, n_kps, F, stride, on_device, "keyframe database", in)) return rc;
 
-    orbx_bowdb *db = new orbx_bowdb();
-    DbGuard guard{db};
+    Building<orbx_bowdb> db(new orbx_bowdb(), orbx_bowdb_destroy);
     db->ctx = c, db->vocab = v, db->device = c->device, db->F = F, db->stride = stride, db->n_words = v->n_words;
     const size_t rows = (size_t)F * stride;
     ORBX_CUDA(c, cudaMalloc((void **)&db->ids, rows * 4));
     ORBX_CUDA(c, cudaMalloc((void **)&db->vals, rows * 8));
     ORBX_CUDA(c, cudaMalloc((void **)&db->n, (size_t)F * 4));
     ORBX_CUDA(c, cudaMalloc((void **)&db->word_start, ((size_t)v->n_words + 1) * 8));
-    // inputs in device memory; the transform's per-feature and FeatureVector outputs in chunk scratch
-    DeviceBuffer in_desc, in_n, cursor;
-    const uint8_t *d_desc = desc;
-    const int *d_n = n_kps;
-    if (!on_device)
-    {
-      if (int rc = in_desc.reserve(c, rows * 32)) return rc;
-      if (int rc = in_n.reserve(c, (size_t)F * 4)) return rc;
-      ORBX_CUDA(c, cudaMemcpyAsync(in_desc.p, desc, rows * 32, cudaMemcpyHostToDevice, s));
-      ORBX_CUDA(c, cudaMemcpyAsync(in_n.p, n_kps, (size_t)F * 4, cudaMemcpyHostToDevice, s));
-      d_desc = in_desc.p, d_n = (const int *)in_n.p;
-    }
+    // the transform's per-feature and FeatureVector outputs in chunk scratch
+    DeviceBuffer cursor;
     BowArgs bow{};
     bow.bow_ids = db->ids, bow.bow_vals = db->vals, bow.n_bow = db->n;
-    if (int rc = bow_frames(c, v, 0, d_desc, d_n, F, stride, bow)) return rc;
+    if (int rc = bow_frames(c, v, 0, in.desc, in.d_n, F, stride, bow)) return rc;
     ORBX_CUDA(c, cudaGetLastError());
     // inverted file: postings per word, exclusive scan, fill
     const unsigned blocks = (unsigned)((rows + 255) / 256);
@@ -531,16 +433,11 @@ extern "C"
       static SmemOptIn state;
       if (raise_dynamic_smem(bowdb_query_kernel, state, db->smem)) return fail(c, ORBX_ERR_CUDA, "cannot reserve shared memory for the keyframe database query");
     }
-    int per_sm = 0, n_sm = 0;
-    ORBX_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, bowdb_query_kernel, kQT, db->smem));
-    ORBX_CUDA(c, cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, c->device));
-    if (per_sm < 1) return fail(c, ORBX_ERR_CUDA, "the keyframe database query kernel does not fit an SM");
-    db->grid_max = per_sm * n_sm;
+    if (int rc = resident_ctas(c, (const void *)bowdb_query_kernel, kQT, db->smem, "the keyframe database query kernel", &db->grid_max)) return rc;
     if (!db->list_in_smem) ORBX_CUDA(c, cudaMalloc((void **)&db->g_list, (size_t)db->grid_max * list_bytes));
     // the scratch buffers are freed on return: the work that reads them has to finish first
     ORBX_CUDA(c, cudaStreamSynchronize(s));
-    guard.db = nullptr;
-    *out = db;
+    *out = db.release();
     return ORBX_OK;
   }
 

@@ -2,6 +2,7 @@
 #pragma once
 
 #include <functional>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -21,6 +22,12 @@ struct DeviceBuffer
   ~DeviceBuffer() { if (p) cudaFree(p); }
   int reserve(orbx_ctx *c, size_t want);
 };
+
+// the next multiple of 16 bytes: offsets of arrays laid out one after another in one device buffer
+inline size_t up16(size_t v) { return (v + 15) & ~(size_t)15; }
+
+// an object a builder is making, freed by its public *_destroy on every error path; release() hands it to the caller
+template <class T> using Building = std::unique_ptr<T, void (*)(T *)>;
 } // namespace orbx
 
 struct orbx_ctx
@@ -106,6 +113,12 @@ namespace orbx
 
 // records `msg` as the context's last error and returns `code`
 int fail(orbx_ctx *c, int code, const std::string &msg);
+// ORBX_OK when an object that context `owner_ctx` made on device `owner_device` belongs to `c`, else ORBX_ERR_INVALID_ARG
+// with a message that names `what` as another context's
+int require_owner(orbx_ctx *c, const orbx_ctx *owner_ctx, int owner_device, const char *what);
+// resident CTAs of a grid-stride kernel on the context's device (CTAs per SM x SMs) in *n; ORBX_ERR_CUDA ("<what> does not
+// fit an SM") when not one CTA fits
+int resident_ctas(orbx_ctx *c, const void *kernel, int threads, size_t smem, const char *what, int *n);
 // Params whose per-image buffers start at image `img0` (and per-frame buffers at frame `frame0`)
 Params params_at(const orbx_ctx *c, int img0, int frame0);
 // the same BowArgs with every per-frame buffer starting at frame `frame0` (N = n_features)
@@ -134,15 +147,65 @@ int bow_buffers(orbx_ctx *c);
 // ORBX_BOW_MAX_STRIDE features per frame, else opts the assemble and word-frame kernels in to the sort's shared memory
 // (ORBX_ERR_CUDA if that fails).  Needs the context's device current.
 int bow_configure(orbx_ctx *c, int n_features, int too_large);
-// c->bow with the vocabulary's tree, ready for launch_bow_descend / launch_bow_assemble over device slots whose frame f
-// reads image f * image_stride
-BowArgs bow_args(const orbx_ctx *c, const orbx_vocab *v, int levelsup, int image_stride);
+// `b` with the vocabulary's tree, ready for launch_bow_descend / launch_bow_assemble over frames whose frame f reads image
+// f * image_stride (the context's slots: b = c->bow)
+BowArgs bow_args(const orbx_vocab *v, int levelsup, int image_stride, BowArgs b = {});
+// the transform of n_frames frames on `s`: launch_bow_descend, then launch_bow_assemble; counts both launches
+void launch_bow_transform(orbx_ctx *c, const Params &p, const BowArgs &a, int n_frames, cudaStream_t s);
+// A training set desc[F][stride][32] + n_kps[F] (host memory, or device memory with `on_device`) as the builders read it:
+// the counts on the host, each checked to lie in 0..stride (else ORBX_ERR_INVALID_ARG, "<what>: a count lies outside
+// 0..stride"), and device pointers to both arrays -- the caller's, or copies of host arrays staged on the context's stream
+// that live as long as the TrainingSet.
+struct TrainingSet
+{
+  std::vector<int32_t> n;
+  const uint8_t *desc = nullptr;
+  const int32_t *d_n = nullptr;
+  DeviceBuffer staged;
+};
+int read_training_set(orbx_ctx *c, const uint8_t *desc, const int32_t *n_kps, int F, int stride, bool on_device, const char *what, TrainingSet &ts);
 // BowVectors and FeatureVectors (orbx_bow_transform's, at `levelsup`) of F frames of device descriptors d_desc[f][stride][32],
 // d_n[f] each, in chunks of frames: frame f's results go to out.bow_ids / bow_vals / fv_nodes / fv_feats + f * stride,
 // out.fv_start + f * (stride + 1), out.n_bow / n_fv + f; the arrays left null in `out` get per-chunk scratch.  Synchronises.
 int bow_frames(orbx_ctx *c, const orbx_vocab *v, int levelsup, const uint8_t *d_desc, const int *d_n, int F, int stride, const BowArgs &out);
 // appends `v` as std::ostream << double prints it by default ("%g": 6 significant digits) and a blank
 void append_g(std::string &t, double v);
+
+// The arrays of one call of a query entry point whose io lives on the host or on the device, each stated once with the
+// kernel argument it sets:
+//   out(arg, user, bytes)      the caller's array (device io), a slice of `buf` that finish() copies back to `user` (host io,
+//                              array wanted) or null (not wanted)
+//   scratch(arg, bytes, host)  a slice of `buf` in either case, filled from `host` by place() when that is given
+// place() sizes `buf`, points every staged argument at its slice and enqueues the copies in; after the launch, finish()
+// enqueues the copies back and synchronises (host io only).  Everything runs on the context's stream.
+struct IoStaging
+{
+  struct Slice
+  {
+    std::function<void(uint8_t *)> set;
+    const void *from;
+    void *to;
+    size_t off, bytes;
+  };
+  orbx_ctx *c;
+  DeviceBuffer &buf;
+  bool on_device;
+  size_t total = 0;
+  std::vector<Slice> slices;
+  template <class T> void out(T *&arg, T *user, size_t bytes)
+  {
+    if (on_device || !user) arg = user;
+    else stage(arg, nullptr, user, bytes);
+  }
+  template <class T> void scratch(T *&arg, size_t bytes, const void *host = nullptr) { stage(arg, host, nullptr, bytes); }
+  template <class T> void stage(T *&arg, const void *from, void *to, size_t bytes)
+  {
+    slices.push_back({[&arg](uint8_t *p) { arg = reinterpret_cast<T *>(p); }, from, to, total, bytes});
+    total += up16(bytes);
+  }
+  int place();
+  int finish();
+};
 
 } // namespace orbx
 

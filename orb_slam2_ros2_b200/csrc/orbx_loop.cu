@@ -5,7 +5,7 @@
 // fixed scale) under the rules of include/orbx.h; tests/loopver_oracle.c is the sequential restatement the kernels are tested
 // against bit for bit.
 //   build: loopver_extract_kernel copies keypoints (x, y, angle, octave), descriptors and depth out of the records into
-//   arrays the verifier owns; the FeatureVectors come from bow_frames (bow_descend_kernel + bow_assemble_kernel, orbx_bow.cu).
+//   arrays the verifier owns; the FeatureVectors come from bow_frames (orbx_bow.cu: bow_descend_kernel + bow_assemble_kernel).
 //   verify: loopver_pair_kernel, one 256-thread CTA per pair (a grid-stride loop over the pairs), per-CTA scratch in global
 //   memory:
 //     rows          a warp per row of the candidate's FeatureVector (bow_match_row, orbx_match.cuh)
@@ -443,8 +443,6 @@ __global__ void __launch_bounds__(256) loopver_extract_kernel(const uint8_t *rec
   depth[o] = z;
 }
 
-size_t up16(size_t v) { return (v + 15) & ~(size_t)15; }
-
 size_t cta_bytes(int N) { return up16((size_t)N * sizeof(Corr) + (size_t)N * 5 * 4); }
 
 } // namespace
@@ -455,15 +453,6 @@ using namespace orbx;
 
 namespace
 {
-
-struct LvGuard
-{
-  orbx_loopver *lv;
-  ~LvGuard()
-  {
-    if (lv) orbx_loopver_destroy(lv);
-  }
-};
 
 // SetRansacParameters (include/orbx.h: iterations) for every n_corr in 0..N
 std::vector<int32_t> iteration_table(int N, const orbx_loopver_params *p)
@@ -502,7 +491,7 @@ extern "C"
   {
     if (!c || !v || !records || !out) return ORBX_ERR_INVALID_ARG;
     *out = nullptr;
-    if (v->ctx != c || v->device != c->device) return fail(c, ORBX_ERR_INVALID_ARG, "the vocabulary belongs to another context");
+    if (int rc = require_owner(c, v->ctx, v->device, "the vocabulary")) return rc;
     orbx_record_layout lay;
     orbx_record_layout_get(c, &lay);
     if (F < 1) return fail(c, ORBX_ERR_INVALID_ARG, "loop verifier: n_frames < 1");
@@ -514,8 +503,7 @@ extern "C"
     cudaStream_t s = c->stream;
     ORBX_CUDA(c, cudaSetDevice(c->device));
     if (int rc = bow_configure(c, N, ORBX_ERR_CAPACITY)) return rc;
-    orbx_loopver *lv = new orbx_loopver();
-    LvGuard guard{lv};
+    Building<orbx_loopver> lv(new orbx_loopver(), orbx_loopver_destroy);
     lv->ctx = c, lv->vocab = v, lv->device = c->device, lv->F = F, lv->N = N;
     const size_t e = (size_t)F * N;
     ORBX_CUDA(c, cudaMalloc((void **)&lv->kp, e * sizeof(float4)));
@@ -552,14 +540,9 @@ extern "C"
     BowArgs fv{};
     fv.fv_nodes = lv->fv_nodes, fv.fv_start = lv->fv_start, fv.fv_feats = lv->fv_feats, fv.n_fv = lv->n_fv;
     if (int rc = bow_frames(c, v, levelsup, lv->desc, lv->n, F, N, fv)) return rc;
-    int per_sm = 0, n_sm = 0;
-    ORBX_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, loopver_pair_kernel, kLT, 0));
-    ORBX_CUDA(c, cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, c->device));
-    if (per_sm < 1) return fail(c, ORBX_ERR_CUDA, "the loop verification kernel does not fit an SM");
-    lv->grid_max = per_sm * n_sm;
+    if (int rc = resident_ctas(c, (const void *)loopver_pair_kernel, kLT, 0, "the loop verification kernel", &lv->grid_max)) return rc;
     if (int rc = lv->scratch.reserve(c, (size_t)lv->grid_max * cta_bytes(N))) return rc;
-    guard.lv = nullptr;
-    *out = lv;
+    *out = lv.release();
     return ORBX_OK;
   }
 
@@ -567,7 +550,7 @@ extern "C"
   {
     if (!c || !lv_ || !prm || !io) return ORBX_ERR_INVALID_ARG;
     orbx_loopver *lv = const_cast<orbx_loopver *>(lv_);
-    if (lv->ctx != c || lv->device != c->device) return fail(c, ORBX_ERR_INVALID_ARG, "the verifier belongs to another context");
+    if (int rc = require_owner(c, lv->ctx, lv->device, "the verifier")) return rc;
     if (std::isnan(prm->ratio)) return fail(c, ORBX_ERR_INVALID_ARG, "ratio is NaN");
     if (!(prm->probability > 0.0 && prm->probability < 1.0)) return fail(c, ORBX_ERR_INVALID_ARG, "probability outside (0, 1)");
     if (prm->min_inliers < 3) return fail(c, ORBX_ERR_INVALID_ARG, "min_inliers < 3");
@@ -584,14 +567,6 @@ extern "C"
     cudaStream_t s = c->stream;
     const int N = lv->N;
     const std::vector<int32_t> iters = iteration_table(N, prm);
-    // staging: iteration table, loop keys, then (host io) the table and the outputs
-    const size_t o_it = 0, o_key = o_it + up16(((size_t)N + 1) * 4), o_tab = o_key + up16((size_t)nq * 8);
-    const size_t o_i32 = o_tab + (io->on_device ? 0 : up16(n_pairs * 4)), n_i32 = 7;
-    const size_t o_T = o_i32 + n_i32 * up16(n_pairs * 4), o_match = o_T + (io->on_device ? 0 : up16(n_pairs * 96));
-    const size_t o_lf = o_match + (io->on_device || !io->match ? 0 : up16(n_pairs * (size_t)N * 4)), total = o_lf + up16((size_t)nq * 4);
-    if (int rc = lv->staging.reserve(c, total)) return rc;
-    uint8_t *st = lv->staging.p;
-    ORBX_CUDA(c, cudaMemcpyAsync(st + o_it, iters.data(), iters.size() * 4, cudaMemcpyHostToDevice, s));
     LvArgs a{};
     a.kp = lv->kp, a.desc = lv->desc, a.depth = lv->depth, a.n = lv->n;
     a.fv_nodes = lv->fv_nodes, a.fv_start = lv->fv_start, a.fv_feats = lv->fv_feats, a.n_fv = lv->n_fv;
@@ -603,28 +578,27 @@ extern "C"
       const float s2 = sf * sf; // mvLevelSigma2: the float square of the level scale factor
       a.thr[l] = 9.210 * (double)s2;
     }
-    a.iters = (const int *)(st + o_it);
     a.top_k = io->top_k, a.n_queries = (int)nq, a.q_lo = q_lo;
     a.ratio = prm->ratio, a.min_matches = prm->min_matches, a.min_inliers = prm->min_inliers;
     a.seed_key = splitmix64(prm->seed);
     a.scratch = lv->scratch.p, a.cta_bytes = cta_bytes(N);
-    a.loop_key = (unsigned long long *)(st + o_key);
-    int *i32[7];
-    int *const user[7] = {io->n_bow, io->n_matches, io->n_corr, io->n_iters, io->hypothesis, io->n_inliers, io->accepted};
-    for (int j = 0; j < 7; ++j) i32[j] = io->on_device ? user[j] : (user[j] ? (int *)(st + o_i32 + j * up16(n_pairs * 4)) : nullptr);
-    a.n_bow = i32[0], a.n_matches = i32[1], a.n_corr = i32[2], a.n_iters = i32[3], a.hypothesis = i32[4], a.n_inliers = i32[5], a.accepted = i32[6];
-    int *loop_frame = io->loop_frame;
-    if (io->on_device)
-      a.table = io->cand_frame, a.T = io->T, a.match = io->match;
-    else
-    {
-      ORBX_CUDA(c, cudaMemcpyAsync(st + o_tab, io->cand_frame, n_pairs * 4, cudaMemcpyHostToDevice, s));
-      a.table = (const int *)(st + o_tab);
-      a.T = io->T ? (double *)(st + o_T) : nullptr;
-      a.match = io->match ? (int *)(st + o_match) : nullptr;
-      loop_frame = io->loop_frame ? (int *)(st + o_lf) : nullptr;
-    }
-    if (!loop_frame) a.loop_key = nullptr;
+    IoStaging st{c, lv->staging, io->on_device != 0};
+    st.scratch(a.iters, iters.size() * 4, iters.data());
+    if (io->on_device) a.table = io->cand_frame;
+    else st.scratch(a.table, n_pairs * 4, io->cand_frame);
+    st.out(a.n_bow, io->n_bow, n_pairs * 4);
+    st.out(a.n_matches, io->n_matches, n_pairs * 4);
+    st.out(a.n_corr, io->n_corr, n_pairs * 4);
+    st.out(a.n_iters, io->n_iters, n_pairs * 4);
+    st.out(a.hypothesis, io->hypothesis, n_pairs * 4);
+    st.out(a.n_inliers, io->n_inliers, n_pairs * 4);
+    st.out(a.accepted, io->accepted, n_pairs * 4);
+    st.out(a.T, io->T, n_pairs * 96);
+    st.out(a.match, io->match, n_pairs * (size_t)N * 4);
+    int *loop_frame = nullptr;
+    st.out(loop_frame, io->loop_frame, (size_t)nq * 4);
+    if (io->loop_frame) st.scratch(a.loop_key, (size_t)nq * 8); // no loop_frame, no loop keys
+    if (int rc = st.place()) return rc;
     if (a.loop_key) ORBX_CUDA(c, cudaMemsetAsync(a.loop_key, 0xff, (size_t)nq * 8, s));
     const int grid = (int)std::min<size_t>(n_pairs, (size_t)lv->grid_max);
     loopver_pair_kernel<<<grid, kLT, 0, s>>>(a);
@@ -635,16 +609,7 @@ extern "C"
       ++c->launches;
     }
     ORBX_CUDA(c, cudaGetLastError());
-    if (io->on_device) return ORBX_OK;
-    auto back = [&](void *dst, const void *src, size_t bytes) -> cudaError_t {
-      return dst ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, s) : cudaSuccess;
-    };
-    for (int j = 0; j < 7; ++j) ORBX_CUDA(c, back(user[j], i32[j], n_pairs * 4));
-    ORBX_CUDA(c, back(io->T, a.T, n_pairs * 96));
-    ORBX_CUDA(c, back(io->match, a.match, n_pairs * (size_t)N * 4));
-    ORBX_CUDA(c, back(io->loop_frame, loop_frame, (size_t)nq * 4));
-    ORBX_CUDA(c, cudaStreamSynchronize(s));
-    return ORBX_OK;
+    return st.finish();
   }
 
 } // extern "C"

@@ -87,8 +87,6 @@ NcclApi &nccl()
 constexpr int kMaxRanks = 16;
 constexpr int kPieceEvents = orbx_ctx::kPipeMax;
 
-inline size_t up16(size_t v) { return (v + 15) & ~(size_t)15; }
-
 // gathered arrays of one rank: [world * block][N][32] descriptors followed by [world * block] counts, ONE allocation so
 // that one IPC handle covers both
 struct Gathered
@@ -223,10 +221,8 @@ int keyframe_chunk(orbx_ctx *c, const orbx_keyframe_io *kio, const Params &p, cu
                         kio->id0 + (uint64_t)(lo + f0), pose, kio->with_map_points);
   if (kio->vocab)
   {
-    const BowArgs ba = bow_at(bow_args(c, kio->vocab, kio->levelsup, 2), d0, (size_t)c->cfg.n_features);
-    launch_bow_descend(p, ba, nf, s);
-    launch_bow_assemble(p, ba, nf, s);
-    c->launches += 2;
+    const BowArgs ba = bow_at(bow_args(kio->vocab, kio->levelsup, 2, c->bow), d0, (size_t)c->cfg.n_features);
+    launch_bow_transform(c, p, ba, nf, s);
     ser_bow_inputs(sa, ba);
   }
   launch_serialize(p, sa, nf, s);
@@ -428,8 +424,8 @@ extern "C"
                                      orbx_sequence_result *res)
   {
     if (!c || !io || n_frames_total < 0 || !io->left || !io->right) return ORBX_ERR_INVALID_ARG;
-    if (m && m->ctx != c) return fail(c, ORBX_ERR_INVALID_ARG, "communicator belongs to another context");
-    if (kio && kio->vocab && kio->vocab->ctx != c) return fail(c, ORBX_ERR_INVALID_ARG, "vocabulary belongs to another context");
+    if (int rc = m ? require_owner(c, m->ctx, c->device, "the communicator") : ORBX_OK) return rc; // a communicator lives on its context's device
+    if (int rc = kio && kio->vocab ? require_owner(c, kio->vocab->ctx, kio->vocab->device, "the vocabulary") : ORBX_OK) return rc;
     ORBX_CUDA(c, cudaSetDevice(c->device));
     if (!m)
     { // single rank: the context keeps its own gathered arrays

@@ -448,40 +448,21 @@ extern "C" int orbx_vocab_build(orbx_ctx *c, const orbx_vocab_train *in, orbx_vo
   cudaStream_t s = c->stream;
   ORBX_CUDA(c, cudaSetDevice(c->device));
   if (int rc = bow_configure(c, stride, ORBX_ERR_INVALID_ARG)) return rc; // the TF_IDF step sorts a frame row in shared memory
-  Scratch sc;
-  sc.dev = c->device;
-  // counts on the host: row offsets of the gather, validation
-  std::vector<int32_t> h_n((size_t)F);
-  if (in->on_device)
-  {
-    ORBX_CUDA(c, cudaMemcpyAsync(h_n.data(), in->n_kps, (size_t)F * 4, cudaMemcpyDeviceToHost, s));
-    ORBX_CUDA(c, cudaStreamSynchronize(s));
-  }
-  else
-    std::memcpy(h_n.data(), in->n_kps, (size_t)F * 4);
+  TrainingSet tr;
+  if (int rc = read_training_set(c, in->desc, in->n_kps, F, stride, in->on_device, "vocabulary training set", tr)) return rc;
+  // row offsets of the gather
   std::vector<long long> row_off((size_t)F);
   long long N = 0;
   for (int f = 0; f < F; ++f)
   {
-    if (h_n[(size_t)f] < 0 || h_n[(size_t)f] > stride) return fail(c, ORBX_ERR_INVALID_ARG, "vocabulary training set: a count lies outside 0..stride");
     row_off[(size_t)f] = N;
-    N += h_n[(size_t)f];
+    N += tr.n[(size_t)f];
   }
   if (N == 0) return fail(c, ORBX_ERR_INVALID_ARG, "vocabulary training set holds no descriptor");
   if (N > 2147483647LL) return fail(c, ORBX_ERR_INVALID_ARG, "vocabulary training set: more than INT32_MAX descriptors");
   const size_t rows = (size_t)F * stride;
-  const uint8_t *d_train = in->desc;
-  const int32_t *d_n = in->n_kps;
-  if (!in->on_device)
-  {
-    uint8_t *td;
-    int32_t *tn;
-    ORBX_CUDA(c, sc.get(&td, rows * 32));
-    ORBX_CUDA(c, sc.get(&tn, (size_t)F));
-    ORBX_CUDA(c, cudaMemcpyAsync(td, in->desc, rows * 32, cudaMemcpyHostToDevice, s));
-    ORBX_CUDA(c, cudaMemcpyAsync(tn, in->n_kps, (size_t)F * 4, cudaMemcpyHostToDevice, s));
-    d_train = td, d_n = tn;
-  }
+  Scratch sc;
+  sc.dev = c->device;
   uint4 *D, *Dn;
   uint16_t *md;
   uint8_t *asg;
@@ -492,7 +473,7 @@ extern "C" int orbx_vocab_build(orbx_ctx *c, const orbx_vocab_train *in, orbx_vo
   ORBX_CUDA(c, sc.get(&asg, (size_t)N));
   ORBX_CUDA(c, sc.get(&d_row_off, (size_t)F));
   ORBX_CUDA(c, cudaMemcpyAsync(d_row_off, row_off.data(), (size_t)F * 8, cudaMemcpyHostToDevice, s));
-  vocab_gather_kernel<<<(unsigned)((rows + kVT - 1) / kVT), kVT, 0, s>>>(reinterpret_cast<const uint4 *>(d_train), d_n, d_row_off, stride, (long long)rows, D);
+  vocab_gather_kernel<<<(unsigned)((rows + kVT - 1) / kVT), kVT, 0, s>>>(reinterpret_cast<const uint4 *>(tr.desc), tr.d_n, d_row_off, stride, (long long)rows, D);
   ++c->launches;
   ORBX_CUDA(c, cudaGetLastError());
 
@@ -719,33 +700,26 @@ extern "C" int orbx_vocab_build(orbx_ctx *c, const orbx_vocab_train *in, orbx_vo
     leaf[r] = nodes[v].n_child == 0;
     std::memcpy(rdesc.data() + r * 32, nodes[v].desc, 32);
   }
-  orbx_vocab *v = nullptr;
-  int rc = orbx_vocab_create(c, k, L, n_rec, parent.data(), leaf.data(), rdesc.data(), weight.data(), &v);
-  if (rc) return rc;
+  orbx_vocab *built = nullptr;
+  if (int rc = orbx_vocab_create(c, k, L, n_rec, parent.data(), leaf.data(), rdesc.data(), weight.data(), &built)) return rc;
+  Building<orbx_vocab> v(built, orbx_vocab_destroy);
   // TF_IDF: descend every training descriptor (the transform's descent), count each word once per frame
-  auto fail_v = [&](int code, const std::string &msg) {
-    orbx_vocab_destroy(v);
-    return fail(c, code, msg);
-  };
   int *f_word, *f_nid, *ni;
   double *f_weight;
-  cudaError_t e = sc.get(&f_word, rows);
-  if (e == cudaSuccess) e = sc.get(&f_nid, rows);
-  if (e == cudaSuccess) e = sc.get(&f_weight, rows);
-  if (e == cudaSuccess) e = sc.get(&ni, (size_t)v->n_words);
-  if (e == cudaSuccess) e = cudaMemsetAsync(ni, 0, (size_t)v->n_words * 4, s);
-  if (e != cudaSuccess) return fail_v(ORBX_ERR_CUDA, std::string("vocabulary IDF buffers: ") + cudaGetErrorString(e));
-  BowArgs b{};
-  b.child_start = v->child_start, b.child_ids = v->child_ids, b.v_desc = v->desc, b.v_weight = v->weight, b.v_word = v->word;
-  b.L = L, b.levelsup = 0, b.image_stride = 1;
-  e = cudaEventRecord(ev.a, s);
-  for (int f0 = 0; f0 < F && e == cudaSuccess; f0 += 65535) // grid.y of the descent carries the frame
+  ORBX_CUDA(c, sc.get(&f_word, rows));
+  ORBX_CUDA(c, sc.get(&f_nid, rows));
+  ORBX_CUDA(c, sc.get(&f_weight, rows));
+  ORBX_CUDA(c, sc.get(&ni, (size_t)v->n_words));
+  ORBX_CUDA(c, cudaMemsetAsync(ni, 0, (size_t)v->n_words * 4, s));
+  const BowArgs b = bow_args(v.get(), 0, 1);
+  ORBX_CUDA(c, cudaEventRecord(ev.a, s));
+  for (int f0 = 0; f0 < F; f0 += 65535) // grid.y of the descent carries the frame
   {
     const int nf = std::min(65535, F - f0);
     Params p{};
     p.n_features = stride;
-    p.desc = const_cast<uint8_t *>(d_train) + (size_t)f0 * stride * 32;
-    p.n_kps = const_cast<int *>(d_n) + f0;
+    p.desc = const_cast<uint8_t *>(tr.desc) + (size_t)f0 * stride * 32;
+    p.n_kps = const_cast<int *>(tr.d_n) + f0;
     BowArgs bb = b;
     bb.f_word = f_word + (size_t)f0 * stride, bb.f_nid = f_nid + (size_t)f0 * stride, bb.f_weight = f_weight + (size_t)f0 * stride;
     launch_bow_descend(p, bb, nf, s);
@@ -753,12 +727,11 @@ extern "C" int orbx_vocab_build(orbx_ctx *c, const orbx_vocab_train *in, orbx_vo
     c->launches += 2;
   }
   std::vector<int> h_ni((size_t)v->n_words);
-  if (e == cudaSuccess) e = cudaGetLastError();
-  if (e == cudaSuccess) e = cudaEventRecord(ev.b, s);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(h_ni.data(), ni, (size_t)v->n_words * 4, cudaMemcpyDeviceToHost, s);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-  if (e == cudaSuccess) e = cudaEventElapsedTime(&level_ms[(size_t)L], ev.a, ev.b);
-  if (e != cudaSuccess) return fail_v(ORBX_ERR_CUDA, std::string("vocabulary IDF: ") + cudaGetErrorString(e));
+  ORBX_CUDA(c, cudaGetLastError());
+  ORBX_CUDA(c, cudaEventRecord(ev.b, s));
+  ORBX_CUDA(c, cudaMemcpyAsync(h_ni.data(), ni, (size_t)v->n_words * 4, cudaMemcpyDeviceToHost, s));
+  ORBX_CUDA(c, cudaStreamSynchronize(s));
+  ORBX_CUDA(c, cudaEventElapsedTime(&level_ms[(size_t)L], ev.a, ev.b));
   // setNodeWeights: log(N / N_i) in double on the host, from the integer counts
   std::vector<double> node_w((size_t)v->n_nodes, 0.0);
   for (int r = 0, w = 0; r < n_rec; ++r)
@@ -769,12 +742,11 @@ extern "C" int orbx_vocab_build(orbx_ctx *c, const orbx_vocab_train *in, orbx_vo
       node_w[(size_t)r + 1] = weight[(size_t)r];
     }
   v->rec_weight = weight;
-  e = cudaMemcpyAsync(v->weight, node_w.data(), node_w.size() * sizeof(double), cudaMemcpyHostToDevice, s);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-  if (e != cudaSuccess) return fail_v(ORBX_ERR_CUDA, std::string("vocabulary weights: ") + cudaGetErrorString(e));
+  ORBX_CUDA(c, cudaMemcpyAsync(v->weight, node_w.data(), node_w.size() * sizeof(double), cudaMemcpyHostToDevice, s));
+  ORBX_CUDA(c, cudaStreamSynchronize(s));
   if (in->iters) std::memcpy(in->iters, level_iters.data(), (size_t)L * 4);
   if (in->n_capped) *in->n_capped = n_capped;
   if (in->level_ms) std::memcpy(in->level_ms, level_ms.data(), ((size_t)L + 1) * sizeof(float));
-  *out = v;
+  *out = v.release();
   return ORBX_OK;
 }

@@ -249,6 +249,12 @@ def test_cuda_database_rejects_bad_arguments(cases):
     bad[3] = -1
     with pytest.raises(ValueError, match="invalid argument"):
         api.BowDatabase.build(ctx, V, desc, bad)
+    import torch
+
+    d_desc, d_bad = torch.from_numpy(np.ascontiguousarray(desc)).cuda(), torch.from_numpy(np.ascontiguousarray(bad, np.int32)).cuda()
+    torch.cuda.synchronize()
+    with pytest.raises(ValueError, match=r"invalid argument \(keyframe database: a count lies outside 0\.\.stride"):  # the same counts in device memory
+        api.BowDatabase.build(ctx, V, d_desc.data_ptr(), d_bad.data_ptr(), n_frames=F, stride=desc.shape[1])
     with pytest.raises(ValueError, match="invalid argument"):  # stride outside 1..ORBX_BOW_MAX_STRIDE
         api.BowDatabase.build(ctx, V, np.zeros((1, api.BOW_MAX_STRIDE + 1, 32), np.uint8), np.zeros(1, np.int32))
     D = api.BowDatabase.build(ctx, V, desc, counts)

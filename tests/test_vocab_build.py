@@ -267,6 +267,12 @@ def test_cuda_build_rejects_bad_arguments(cases):
     bad[0] = c["desc"].shape[1] + 1
     with pytest.raises(ValueError, match="invalid argument"):
         api.Vocabulary.build(ctx, c["desc"], bad, n_frames=c["n_frames"], k=3, L=2)
+    import torch
+
+    d_desc, d_bad = torch.from_numpy(np.ascontiguousarray(c["desc"])).cuda(), torch.from_numpy(bad).cuda()
+    torch.cuda.synchronize()
+    with pytest.raises(ValueError, match=r"invalid argument \(vocabulary training set: a count lies outside 0\.\.stride"):  # the same counts in device memory
+        api.Vocabulary.build(ctx, d_desc.data_ptr(), d_bad.data_ptr(), n_frames=c["n_frames"], stride=c["desc"].shape[1], k=3, L=2)
     with pytest.raises(ValueError, match="invalid argument"):
         api.Vocabulary.build(ctx, c["desc"], np.zeros_like(bad), n_frames=c["n_frames"], k=3, L=2)  # no descriptor
     # a vocabulary built on another context is refused, as a created / loaded one is
