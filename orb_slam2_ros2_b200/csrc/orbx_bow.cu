@@ -25,7 +25,6 @@ namespace
 
 constexpr int kBowWarps = 8;
 constexpr int kAsmThreads = 256;
-constexpr unsigned kFullMask = 0xffffffffu;
 
 __global__ void __launch_bounds__(kBowWarps * 32) bow_descend_kernel(const Params p, const BowArgs a)
 {
@@ -52,8 +51,7 @@ __global__ void __launch_bounds__(kBowWarps * 32) bow_descend_kernel(const Param
       {
         const int id = a.child_ids[c];
         const uint4 g0 = __ldg(vdesc + 2 * (size_t)id), g1 = __ldg(vdesc + 2 * (size_t)id + 1);
-        const unsigned d = __popc(f0.x ^ g0.x) + __popc(f0.y ^ g0.y) + __popc(f0.z ^ g0.z) + __popc(f0.w ^ g0.w) + __popc(f1.x ^ g1.x) +
-                           __popc(f1.y ^ g1.y) + __popc(f1.z ^ g1.z) + __popc(f1.w ^ g1.w);
+        const unsigned d = (unsigned)hamming256(f0, f1, g0, g1);
         best = min(best, (d << 20) | (unsigned)(c - c0)); // strict < over children in id order == lexicographic minimum
       }
     }
@@ -71,55 +69,6 @@ __global__ void __launch_bounds__(kBowWarps * 32) bow_descend_kernel(const Param
   }
 }
 
-__device__ __forceinline__ int asm_block_scan(int v, int &total, int *s_warp)
-{
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  int inc = v;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1)
-  {
-    const int t = __shfl_up_sync(kFullMask, inc, o);
-    if (lane >= o) inc += t;
-  }
-  if (lane == 31) s_warp[wid] = inc;
-  __syncthreads();
-  int base = 0, tot = 0;
-#pragma unroll
-  for (int w = 0; w < kAsmThreads / 32; ++w)
-  {
-    const int t = s_warp[w];
-    if (w < wid) base += t;
-    tot += t;
-  }
-  __syncthreads();
-  total = tot;
-  return base + inc - v;
-}
-
-// ascending bitonic sort of P (power of two) 64-bit keys in shared memory
-__device__ void bitonic_sort(unsigned long long *key, int P)
-{
-  for (int k = 2; k <= P; k <<= 1)
-    for (int j = k >> 1; j > 0; j >>= 1)
-    {
-      for (int i = threadIdx.x; i < P; i += kAsmThreads)
-      {
-        const int x = i ^ j;
-        if (x > i)
-        {
-          const unsigned long long u = key[i], v = key[x];
-          const bool asc = (i & k) == 0;
-          if ((u > v) == asc)
-          {
-            key[i] = v;
-            key[x] = u;
-          }
-        }
-      }
-      __syncthreads();
-    }
-}
-
 // segments of equal (key >> 16) in the sorted prefix [0, nv): returns the number of segments; seg_of(j) via the scan
 template <typename HeadFn> __device__ int for_each_head(const unsigned long long *key, int nv, int P, int *s_warp, HeadFn fn)
 {
@@ -128,7 +77,7 @@ template <typename HeadFn> __device__ int for_each_head(const unsigned long long
   int mine = 0;
   for (int j = j0; j < j1; ++j) mine += (j == 0) || ((key[j] >> 16) != (key[j - 1] >> 16));
   int total;
-  int seg = asm_block_scan(mine, total, s_warp);
+  int seg = block_exclusive_scan<kAsmThreads>(mine, total, s_warp);
   for (int j = j0; j < j1; ++j)
     if ((j == 0) || ((key[j] >> 16) != (key[j - 1] >> 16))) fn(seg++, j);
   return total;
@@ -170,7 +119,7 @@ __global__ void __launch_bounds__(kAsmThreads) bow_assemble_kernel(const Params 
     atomicAdd(&s_nv, cnt);
     __syncthreads();
     const int nv = s_nv;
-    bitonic_sort(s_key, P);
+    bitonic_sort<kAsmThreads>(s_key, P);
     if (pass == 0)
     {
       // BowVector::addWeight in feature order: the first feature of a word inserts its weight, the others add to it
@@ -223,7 +172,7 @@ __global__ void __launch_bounds__(kAsmThreads) bow_word_frames_kernel(const Para
   for (int i = threadIdx.x; i < P; i += kAsmThreads)
     s_key[i] = i < n ? ((unsigned long long)(unsigned)f_word[i] << 16) | (unsigned long long)i : ~0ull;
   __syncthreads();
-  bitonic_sort(s_key, P);
+  bitonic_sort<kAsmThreads>(s_key, P);
   for_each_head(s_key, n, P, s_warp, [&](int, int j) { atomicAdd(&n_frames_of_word[s_key[j] >> 16], 1); });
 }
 

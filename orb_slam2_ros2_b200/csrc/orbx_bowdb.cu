@@ -21,7 +21,6 @@
 #include <cmath>
 
 #include "orbx_internal.h"
-#include "orbx_match.cuh"
 
 struct orbx_bowdb
 {
@@ -51,7 +50,6 @@ namespace
 {
 
 constexpr int kQT = 256; // threads of the query CTA
-constexpr unsigned kFull = 0xffffffffu;
 constexpr unsigned long long kNone = ~0ull; // a list slot holding no kept candidate (sorts last)
 constexpr size_t kSmemOptIn = 227 * 1024;  // shared memory one CTA may opt in to on sm_100
 constexpr size_t kCounterBytes = (size_t)(ORBX_BOWDB_MAX_FRAMES + 1) / 2 * 4;
@@ -69,26 +67,12 @@ __global__ void __launch_bounds__(256) bowdb_word_count_kernel(const int *ids, c
 __global__ void __launch_bounds__(1024) bowdb_scan_kernel(long long *cnt, int n)
 {
   __shared__ long long s_warp[32];
-  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+  const int tid = threadIdx.x;
   const int per = (n + 1023) / 1024, j0 = min(tid * per, n), j1 = min(j0 + per, n);
   long long mine = 0;
   for (int j = j0; j < j1; ++j) mine += cnt[j];
-  long long inc = mine;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1)
-  {
-    const long long t = __shfl_up_sync(kFull, inc, o);
-    if (lane >= o) inc += t;
-  }
-  if (lane == 31) s_warp[wid] = inc;
-  __syncthreads();
-  long long base = 0, tot = 0;
-  for (int w = 0; w < 32; ++w)
-  {
-    if (w < wid) base += s_warp[w];
-    tot += s_warp[w];
-  }
-  long long run = base + inc - mine;
+  long long tot;
+  long long run = block_exclusive_scan<1024>(mine, tot, s_warp);
   for (int j = j0; j < j1; ++j)
   {
     const long long c = cnt[j];
@@ -186,8 +170,8 @@ __global__ void __launch_bounds__(kQT) bowdb_query_kernel(const QueryArgs a)
     }
     for (int o = 16; o > 0; o >>= 1)
     {
-      sharing += __shfl_xor_sync(kFull, sharing, o);
-      mx = max(mx, __shfl_xor_sync(kFull, mx, o));
+      sharing += __shfl_xor_sync(kFullMask, sharing, o);
+      mx = max(mx, __shfl_xor_sync(kFullMask, mx, o));
     }
     if (lane == 0) s_red[0][wid] = sharing, s_red[1][wid] = mx;
     __syncthreads();
@@ -199,7 +183,7 @@ __global__ void __launch_bounds__(kQT) bowdb_query_kernel(const QueryArgs a)
     if (sharing > 0)
       for (int f = f0; f < f1; ++f) mine += common_of(f) > min_common;
     int n_sc;
-    int pos = block_exscan<kQT>(mine, &n_sc, s_warp);
+    int pos = block_exclusive_scan<kQT>(mine, n_sc, s_warp);
     if (sharing > 0)
       for (int f = f0; f < f1; ++f)
         if (common_of(f) > min_common) list[pos++] = (unsigned long long)f;
@@ -220,13 +204,7 @@ __global__ void __launch_bounds__(kQT) bowdb_query_kernel(const QueryArgs a)
         if (j < m)
         {
           const int w = g_ids[j];
-          int lo = 0, hi = nq; // lower_bound of w in the query's ids
-          while (lo < hi)
-          {
-            const int mid = (lo + hi) >> 1;
-            if (q_ids[mid] < w) lo = mid + 1;
-            else hi = mid;
-          }
+          const int lo = lower_bound(q_ids, 0, nq, w);
           if (lo < nq && q_ids[lo] == w)
           {
             hit = true;
@@ -234,12 +212,12 @@ __global__ void __launch_bounds__(kQT) bowdb_query_kernel(const QueryArgs a)
             t = __dsub_rn(__dsub_rn(fabs(__dsub_rn(vi, wi)), fabs(vi)), fabs(wi));
           }
         }
-        unsigned b = __ballot_sync(kFull, hit);
+        unsigned b = __ballot_sync(kFullMask, hit);
         while (b)
         {
           const int src = __ffs(b) - 1;
           b &= b - 1;
-          const double x = __shfl_sync(kFull, t, src);
+          const double x = __shfl_sync(kFullMask, t, src);
           score = __dadd_rn(score, x);
         }
       }
@@ -264,24 +242,7 @@ __global__ void __launch_bounds__(kQT) bowdb_query_kernel(const QueryArgs a)
     {
       for (int i = n_sc + tid; i < P2; i += kQT) list[i] = kNone;
       __syncthreads();
-      for (int k = 2; k <= P2; k <<= 1)
-        for (int j = k >> 1; j > 0; j >>= 1)
-        {
-          for (int i = tid; i < P2; i += kQT)
-          {
-            const int x = i ^ j;
-            if (x > i)
-            {
-              const unsigned long long u = list[i], v = list[x];
-              if ((u > v) == ((i & k) == 0))
-              {
-                list[i] = v;
-                list[x] = u;
-              }
-            }
-          }
-          __syncthreads();
-        }
+      bitonic_sort<kQT>(list, P2);
     }
     const size_t o = (size_t)qi * a.top_k;
     for (int t = tid; t < a.top_k; t += kQT)

@@ -1,4 +1,5 @@
-// orbx_device.cuh -- device-side data layout shared by the kernels (orbx_kernels.cu) and the host layer (orbx_api.cu).
+// orbx_device.cuh -- device-side data layout shared by the kernels (orbx_kernels.cu) and the host layer (orbx_api.cu), and
+// the device building blocks (scans, Hamming distance, sort, binary search) every kernel file uses.
 //
 // HBM layout (all buffers are per context, sized for n_img_max = 2 * max_batch images):
 //   pyr / blur     [image][pyr_img_stride]   every level stored with a 16-byte aligned pitch at Level::pyr_off
@@ -265,6 +266,88 @@ __host__ __device__ __forceinline__ unsigned long long splitmix64(unsigned long 
   z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
   z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
   return z ^ (z >> 31);
+}
+
+// ------------------------------------------------------------------------------------------------------------------
+// device building blocks of the kernels of every .cu file: one definition each, so that their tie rules and sum orders
+// (which the bit-exact tests depend on) cannot drift apart
+// ------------------------------------------------------------------------------------------------------------------
+constexpr unsigned kFullMask = 0xffffffffu;
+
+// Hamming distance of two 256-bit descriptors, each as two uint4
+__device__ __forceinline__ int hamming256(uint4 a0, uint4 a1, uint4 b0, uint4 b1)
+{
+  return __popc(a0.x ^ b0.x) + __popc(a0.y ^ b0.y) + __popc(a0.z ^ b0.z) + __popc(a0.w ^ b0.w) + __popc(a1.x ^ b1.x) + __popc(a1.y ^ b1.y) +
+         __popc(a1.z ^ b1.z) + __popc(a1.w ^ b1.w);
+}
+
+// inclusive prefix sum of v over the lanes of a full warp; lane = threadIdx.x & 31
+template <typename T> __device__ __forceinline__ T warp_inclusive_scan(T v, int lane)
+{
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1)
+  {
+    const T t = __shfl_up_sync(kFullMask, v, o);
+    if (lane >= o) v += t;
+  }
+  return v;
+}
+
+// exclusive prefix sum of one value per thread over a CTA of NT threads (NT a multiple of 32, <= 1024); total = the CTA's
+// sum.  Ends with a barrier, so s_warp [NT / 32] may be reused at once.
+template <int NT, typename T> __device__ __forceinline__ T block_exclusive_scan(T v, T &total, T *s_warp)
+{
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const T inc = warp_inclusive_scan(v, lane);
+  if (lane == 31) s_warp[wid] = inc;
+  __syncthreads();
+  T base = 0, tot = 0;
+#pragma unroll
+  for (int w = 0; w < NT / 32; ++w)
+  {
+    const T t = s_warp[w];
+    if (w < wid) base += t;
+    tot += t;
+  }
+  __syncthreads();
+  total = tot;
+  return base + inc - v;
+}
+
+// ascending bitonic sort of P (a power of two) 64-bit keys in shared memory by a CTA of NT threads; ends with a barrier
+template <int NT> __device__ __forceinline__ void bitonic_sort(unsigned long long *key, int P)
+{
+  for (int k = 2; k <= P; k <<= 1)
+    for (int j = k >> 1; j > 0; j >>= 1)
+    {
+      for (int i = threadIdx.x; i < P; i += NT)
+      {
+        const int x = i ^ j;
+        if (x > i)
+        {
+          const unsigned long long u = key[i], v = key[x];
+          const bool asc = (i & k) == 0;
+          if ((u > v) == asc)
+          {
+            key[i] = v;
+            key[x] = u;
+          }
+        }
+      }
+      __syncthreads();
+    }
+}
+
+// first index in the ascending a[lo, hi) whose value is >= v (hi if none)
+__device__ __forceinline__ int lower_bound(const int *a, int lo, int hi, int v)
+{
+  while (lo < hi)
+  {
+    const int mid = (lo + hi) >> 1;
+    if (a[mid] < v) lo = mid + 1;
+    else hi = mid;
+  }
+  return lo;
 }
 
 // cudaFuncAttributeMaxDynamicSharedMemorySize belongs to the kernel (per device), not to a context: it is only ever RAISED, so a

@@ -35,34 +35,8 @@ __device__ __forceinline__ const uint8_t *input_image(const Params &p, int img)
 __device__ __forceinline__ int warp_sum(int v)
 {
 #pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(kFullMask, v, o);
   return v;
-}
-
-// exclusive scan of one int per thread over a block of NT threads (NT multiple of 32, <= 1024); returns the block total
-template <int NT> __device__ __forceinline__ int block_exclusive_scan(int v, int &total, int *s_warp /* [NT/32] */)
-{
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  int inc = v;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1)
-  {
-    int t = __shfl_up_sync(0xffffffffu, inc, o);
-    if (lane >= o) inc += t;
-  }
-  if (lane == 31) s_warp[wid] = inc;
-  __syncthreads();
-  int base = 0, tot = 0;
-#pragma unroll
-  for (int w = 0; w < NT / 32; ++w)
-  {
-    int t = s_warp[w];
-    if (w < wid) base += t;
-    tot += t;
-  }
-  __syncthreads();
-  total = tot;
-  return base + inc - v;
 }
 
 // shared-memory accesses of the compaction lists by 32-bit shared address: one LDS / STS each, no generic-pointer arithmetic
@@ -666,7 +640,6 @@ __global__ void __launch_bounds__(kFastThreads) fast_cells_kernel(const Params p
   const Cell c = p.cells[cell];
   const int pw = c.pw, ph = c.ph;
   const int zw = pw - 6, zh = ph - 6; // detection zone: FAST looks at [3, w-3) x [3, h-3) of the patch
-  const unsigned FULL = 0xffffffffu;
   if (zw <= 0 || zh <= 0)
   {
     if (lane == 0) p.cell_cnt[(size_t)img * p.n_cells + cell] = 0;
@@ -759,15 +732,9 @@ __global__ void __launch_bounds__(kFastThreads) fast_cells_kernel(const Params p
         acc_a &= step_ok;
         acc_b &= step_ok;
         const int cnt = __popc(acc_a) + __popc(acc_b);
-        int inc = cnt;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1)
-        {
-          const int up = __shfl_up_sync(FULL, inc, o);
-          if (lane >= o) inc += up;
-        }
+        const int inc = warp_inclusive_scan(cnt, lane);
         uint32_t wa = cand_u32 + 2u * (uint32_t)(n_cand + inc - cnt);
-        n_cand += __shfl_sync(FULL, inc, 31);
+        n_cand += __shfl_sync(kFullMask, inc, 31);
         const uint32_t code0 = (uint32_t)(2 * yq * kZoneMax + zx0);
 #pragma unroll
         for (int h = 0; h < 2; ++h)
@@ -804,7 +771,7 @@ __global__ void __launch_bounds__(kFastThreads) fast_cells_kernel(const Params p
         if (corner) s_map[(zy + 1) * mp + zx + 1] = (uint8_t)m;
       }
       __syncwarp();
-      const unsigned m = __ballot_sync(FULL, corner);
+      const unsigned m = __ballot_sync(kFullMask, corner);
       sts_u16_if(cend + 2u * __popc(m & lt_mask), i, corner);
       cend += 2u * __popc(m);
     }
@@ -827,20 +794,14 @@ __global__ void __launch_bounds__(kFastThreads) fast_cells_kernel(const Params p
     __syncwarp();
     keep0 = lane < zh ? s_keep[lane] : 0ull;
     keep1 = lane + 32 < zh ? s_keep[lane + 32] : 0ull;
-    if (__any_sync(FULL, (keep0 | keep1) != 0ull)) break; // fallback iff the post-NMS list is empty (:366)
+    if (__any_sync(kFullMask, (keep0 | keep1) != 0ull)) break; // fallback iff the post-NMS list is empty (:366)
   }
 
   // lane <-> zone rows lane and lane + 32, row-major output order: exclusive scans of the rows' corner counts
   static_assert(kZoneMax <= 64, "the output scan covers two rows per lane");
   const int cnt0 = __popcll(keep0), cnt1 = __popcll(keep1);
-  int inc0 = cnt0, inc1 = cnt1;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1)
-  {
-    const int u0 = __shfl_up_sync(FULL, inc0, o), u1 = __shfl_up_sync(FULL, inc1, o);
-    if (lane >= o) inc0 += u0, inc1 += u1;
-  }
-  const int tot0 = __shfl_sync(FULL, inc0, 31), total = tot0 + __shfl_sync(FULL, inc1, 31);
+  const int inc0 = warp_inclusive_scan(cnt0, lane), inc1 = warp_inclusive_scan(cnt1, lane);
+  const int tot0 = __shfl_sync(kFullMask, inc0, 31), total = tot0 + __shfl_sync(kFullMask, inc1, 31);
   uint32_t *slot = p.cell_list + (size_t)img * p.cell_entries + c.slot;
 #pragma unroll
   for (int h = 0; h < 2; ++h)
@@ -1011,8 +972,8 @@ __device__ __forceinline__ int qt_big_extreme(const QtState &q, int lane, bool w
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1)
   {
-    const unsigned long long ok = __shfl_xor_sync(0xffffffffu, best, o);
-    const int op = __shfl_xor_sync(0xffffffffu, best_pos, o);
+    const unsigned long long ok = __shfl_xor_sync(kFullMask, best, o);
+    const int op = __shfl_xor_sync(kFullMask, best_pos, o);
     const bool take = op >= 0 && (best_pos < 0 || (want_max ? ok > best : ok < best));
     if (take)
     {
@@ -1101,7 +1062,6 @@ __device__ void qt_simulate(const Params &p, const Level &L, QtState &q, const u
                             IdxT *ia, IdxT *ib, int n, int need, int node_cap, int lane, int live, int n_alloc, bool root_pending, int &out_n_alloc,
                             int &out_take)
 {
-  const unsigned FULL = 0xffffffffu;
   const unsigned lt_mask = (1u << lane) - 1u;
   QtNodePool &np = q.np;
   int n_free = 0;
@@ -1129,7 +1089,7 @@ __device__ void qt_simulate(const Params &p, const Level &L, QtState &q, const u
       {
         const int b = cursor - lane;
         const bool hit = (b >= 0) && (q.bhead[b] != (uint16_t)kNil);
-        const unsigned m = __ballot_sync(FULL, hit);
+        const unsigned m = __ballot_sync(kFullMask, hit);
         if (m)
         {
           cursor -= __ffs(m) - 1;
@@ -1206,7 +1166,7 @@ __device__ void qt_simulate(const Params &p, const Level &L, QtState &q, const u
             const long long x = (long long)(e & 0xfffu) << kFixShift, y = (long long)((e >> 12) & 0xfffu) << kFixShift;
             f = x > cols[k] && x < cols[k + 1] && y > r0 && y < r1;
           }
-          const unsigned m = __ballot_sync(FULL, f);
+          const unsigned m = __ballot_sync(kFullMask, f);
           if (f) dst[base + run + __popc(m & lt_mask)] = (IdxT)idx;
           run += __popc(m);
         }
@@ -1294,8 +1254,8 @@ __device__ void qt_simulate(const Params &p, const Level &L, QtState &q, const u
           idx = src[lo + lane];
           d = digit_of(idx);
         }
-        const unsigned m0 = __ballot_sync(FULL, d == 0), m1 = __ballot_sync(FULL, d == 1);
-        const unsigned m2 = __ballot_sync(FULL, d == 2), m3 = __ballot_sync(FULL, d == 3);
+        const unsigned m0 = __ballot_sync(kFullMask, d == 0), m1 = __ballot_sync(kFullMask, d == 1);
+        const unsigned m2 = __ballot_sync(kFullMask, d == 2), m3 = __ballot_sync(kFullMask, d == 3);
         t0 = __popc(m0);
         t1 = __popc(m1);
         t2 = __popc(m2);
@@ -1320,10 +1280,10 @@ __device__ void qt_simulate(const Params &p, const Level &L, QtState &q, const u
 #pragma unroll
           for (int u = 0; u < 4; ++u)
           {
-            t0 += __popc(__ballot_sync(FULL, d[u] == 0));
-            t1 += __popc(__ballot_sync(FULL, d[u] == 1));
-            t2 += __popc(__ballot_sync(FULL, d[u] == 2));
-            t3 += __popc(__ballot_sync(FULL, d[u] == 3));
+            t0 += __popc(__ballot_sync(kFullMask, d[u] == 0));
+            t1 += __popc(__ballot_sync(kFullMask, d[u] == 1));
+            t2 += __popc(__ballot_sync(kFullMask, d[u] == 2));
+            t3 += __popc(__ballot_sync(kFullMask, d[u] == 3));
           }
         }
         const uint32_t b0 = lo, b1 = b0 + t0, b2 = b1 + t1, b3 = b2 + t2;
@@ -1347,8 +1307,8 @@ __device__ void qt_simulate(const Params &p, const Level &L, QtState &q, const u
 #pragma unroll
           for (int u = 0; u < 4; ++u)
           {
-            const unsigned m0 = __ballot_sync(FULL, d[u] == 0), m1 = __ballot_sync(FULL, d[u] == 1);
-            const unsigned m2 = __ballot_sync(FULL, d[u] == 2), m3 = __ballot_sync(FULL, d[u] == 3);
+            const unsigned m0 = __ballot_sync(kFullMask, d[u] == 0), m1 = __ballot_sync(kFullMask, d[u] == 1);
+            const unsigned m2 = __ballot_sync(kFullMask, d[u] == 2), m3 = __ballot_sync(kFullMask, d[u] == 3);
             if (d[u] == 0) dst[b0 + q0 + __popc(m0 & lt_mask)] = idx[u];
             if (d[u] == 1) dst[b1 + q1 + __popc(m1 & lt_mask)] = idx[u];
             if (d[u] == 2) dst[b2 + q2 + __popc(m2 & lt_mask)] = idx[u];
@@ -1629,7 +1589,6 @@ __device__ __noinline__ bool qt_fast_path(uint8_t *pool, uint8_t *lists, int *sc
   QtFast f;
   f.pool = pool, f.lists = lists, f.scr = scr, f.lf = lf, f.bin_best = bin_best, f.cap = cap, f.nc = nc;
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-  const unsigned FULL = 0xffffffffu;
   enum { kRun = 0, kEmpty = 1, kNoPop = 2, kBail = 3 };
   int *D = f.scr;
   long long t_prev = clock64();
@@ -1660,13 +1619,7 @@ __device__ __noinline__ bool qt_fast_path(uint8_t *pool, uint8_t *lists, int *sc
       d = D[c];
     else if (c >= 2)
       for (int w = 0; w < kFpWarps; ++w) d += s_small[w][c];
-    int inc = d;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1)
-    {
-      const int t = __shfl_up_sync(FULL, inc, o);
-      if (lane >= o) inc += t;
-    }
+    const int inc = warp_inclusive_scan(d, lane);
     if (tid == 0) s_first = 0x7fffffff;
     if (lane == 31) s_warp[wid] = inc;
     fp_sync();
@@ -1934,13 +1887,7 @@ __device__ __noinline__ bool qt_fast_path(uint8_t *pool, uint8_t *lists, int *sc
     {
       const int b = 255 - tid;
       const int h = cursor[b];
-      int inc = h;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1)
-      {
-        const int t = __shfl_up_sync(FULL, inc, o);
-        if (lane >= o) inc += t;
-      }
+      const int inc = warp_inclusive_scan(h, lane);
       if (lane == 31) s_warp[wid] = inc;
       fp_sync();
       int base = 0;
@@ -1979,18 +1926,12 @@ __device__ __noinline__ bool qt_fast_path(uint8_t *pool, uint8_t *lists, int *sc
       {
         const int j = j0 + lane;
         const int val = j < mb ? (int)dlt[j] : 0;
-        int inc = val;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1)
-        {
-          const int t = __shfl_up_sync(FULL, inc, o);
-          if (lane >= o) inc += t;
-        }
+        const int inc = warp_inclusive_scan(val, lane);
         const bool pops = j < mb && run + inc - val < need; // the loop tests the node count BEFORE every pop
-        const unsigned pm = __ballot_sync(FULL, pops);
+        const unsigned pm = __ballot_sync(kFullMask, pops);
         k += __popc(pm);
-        run += __shfl_sync(FULL, inc, 31);
-        if (pm != FULL) break;
+        run += __shfl_sync(kFullMask, inc, 31);
+        if (pm != kFullMask) break;
       }
       if (lane == 0) s_k = k;
     }
@@ -2544,19 +2485,12 @@ template <int kBriefGroup> __global__ void __launch_bounds__(kBriefWarps * 32, 5
   const int img = blockIdx.y;
   const int lane = threadIdx.x & 31;
   const int slot0 = (blockIdx.x * kBriefWarps + (threadIdx.x >> 5)) * kBriefGroup;
-  const unsigned FULL = 0xffffffffu;
 
   // which level does an output slot belong to? (level-major concatenation, src/ORBExtractor.cc:501-506)
   const int *sel_cnt = p.sel_cnt + (size_t)img * p.n_levels;
   const int my = lane < p.n_levels ? sel_cnt[lane] : 0;
-  int inc = my;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1)
-  {
-    int t = __shfl_up_sync(FULL, inc, o);
-    if (lane >= o) inc += t;
-  }
-  const int total = __shfl_sync(FULL, inc, 31);
+  const int inc = warp_inclusive_scan(my, lane);
+  const int total = __shfl_sync(kFullMask, inc, 31);
   if (slot0 == 0 && lane == 0) p.n_kps[img] = total;
   if (slot0 >= total) return;
   const int n_here = min(kBriefGroup, total - slot0);
@@ -2574,9 +2508,9 @@ template <int kBriefGroup> __global__ void __launch_bounds__(kBriefWarps * 32, 5
   for (int j = 0; j < n_here; ++j)
   {
     const int slot = slot0 + j;
-    const unsigned above = __ballot_sync(FULL, inc > slot); // first lane whose inclusive sum exceeds the slot
+    const unsigned above = __ballot_sync(kFullMask, inc > slot); // first lane whose inclusive sum exceeds the slot
     const int level = __ffs(above) - 1;
-    const int level_start = __shfl_sync(FULL, inc - my, level);
+    const int level_start = __shfl_sync(kFullMask, inc - my, level);
     const Level &L = p.levels[level];
     const uint32_t e = p.sel[(size_t)img * p.sel_entries + L.sel_off + (slot - level_start)];
     const int x = (int)(e & 0xfffu), y = (int)((e >> 12) & 0xfffu);
@@ -2594,13 +2528,13 @@ template <int kBriefGroup> __global__ void __launch_bounds__(kBriefWarps * 32, 5
 #pragma unroll
     for (int i = 0; i < 11; ++i)
     {
-      const uint32_t nxt = __shfl_down_sync(FULL, a[i], 1);
+      const uint32_t nxt = __shfl_down_sync(kFullMask, a[i], 1);
       const uint32_t v = __funnelshift_r(a[i], nxt, sh);
       m10 = dp4a_u8_s8(v, s_wx[i][lane], m10);
       m01 = dp4a_u8_s8(v, s_wy[i][lane], m01);
     }
-    m10 = __reduce_add_sync(FULL, m10);
-    m01 = __reduce_add_sync(FULL, m01);
+    m10 = __reduce_add_sync(kFullMask, m10);
+    m01 = __reduce_add_sync(kFullMask, m01);
     if (lane == j) my_e = e, my_level = level, my_m10 = m10, my_m01 = m01;
   }
 
@@ -2623,8 +2557,8 @@ template <int kBriefGroup> __global__ void __launch_bounds__(kBriefWarps * 32, 5
   }
   __syncwarp();
   auto request_patch = [&](int j) { // all lanes call; lane 0 issues the load of keypoint j's patch into buffer j & 1
-    const uint32_t e = __shfl_sync(FULL, my_e, j);
-    const int level = __shfl_sync(FULL, my_level, j);
+    const uint32_t e = __shfl_sync(kFullMask, my_e, j);
+    const int level = __shfl_sync(kFullMask, my_level, j);
     if (lane == 0)
     {
       const int kx_i = (int)(e & 0xfffu), ky_i = (int)((e >> 12) & 0xfffu);
@@ -2642,8 +2576,8 @@ template <int kBriefGroup> __global__ void __launch_bounds__(kBriefWarps * 32, 5
 #pragma unroll 1
   for (int j = 0; j < n_here; ++j)
   {
-    const uint32_t e = __shfl_sync(FULL, my_e, j);
-    const double sj = __shfl_sync(FULL, sn, j), cj = __shfl_sync(FULL, cs, j);
+    const uint32_t e = __shfl_sync(kFullMask, my_e, j);
+    const double sj = __shfl_sync(kFullMask, sn, j), cj = __shfl_sync(kFullMask, cs, j);
     const float fx = (float)(e & 0xfffu), fy = (float)((e >> 12) & 0xfffu);
     const int kx_i = (int)(e & 0xfffu), ky_i = (int)((e >> 12) & 0xfffu);
     __syncwarp(); // keypoint j - 1's gathers from the other buffer are done
@@ -2800,7 +2734,6 @@ __global__ void __launch_bounds__(kStereoWarps * 32, 8) stereo_kernel(const Para
   const int frame = blockIdx.y;
   const int lane = threadIdx.x & 31;
   const int li = blockIdx.x * kStereoWarps + (threadIdx.x >> 5);
-  const unsigned FULL = 0xffffffffu;
   const int imgL = 2 * frame, imgR = 2 * frame + 1;
   const int nL = p.n_kps[imgL];
   if (li >= p.n_features) return;
@@ -2837,14 +2770,13 @@ __global__ void __launch_bounds__(kStereoWarps * 32, 8) stereo_kernel(const Para
       {
         const uint4 *dr4 = reinterpret_cast<const uint4 *>(p.desc + (oR + j) * 32);
         const uint4 b0 = dr4[0], b1 = dr4[1];
-        const int d = __popc(a0.x ^ b0.x) + __popc(a0.y ^ b0.y) + __popc(a0.z ^ b0.z) + __popc(a0.w ^ b0.w) + __popc(a1.x ^ b1.x) +
-                      __popc(a1.y ^ b1.y) + __popc(a1.z ^ b1.z) + __popc(a1.w ^ b1.w);
+        const int d = hamming256(a0, a1, b0, b1);
         best = min(best, ((unsigned)d << 20) | (unsigned)j);
       }
     }
   }
 #pragma unroll
-  for (int o = 16; o > 0; o >>= 1) best = min(best, __shfl_xor_sync(FULL, best, o));
+  for (int o = 16; o > 0; o >>= 1) best = min(best, __shfl_xor_sync(kFullMask, best, o));
   if (best == 0xffffffffu) return;          // no candidates (:49-50)
   if ((int)(best >> 20) > 75) return;       // mnMeanThreshold (:53)
   const int rj = (int)(best & 0xfffffu);
@@ -2909,7 +2841,7 @@ __global__ void __launch_bounds__(kStereoWarps * 32, 8) stereo_kernel(const Para
   }
   int sad[11];
 #pragma unroll
-  for (int s = 0; s < 11; ++s) sad[s] = __reduce_add_sync(FULL, acc[s]);
+  for (int s = 0; s < 11; ++s) sad[s] = __reduce_add_sync(kFullMask, acc[s]);
   if (lane != 0) return;
   int bi = 0;
 #pragma unroll

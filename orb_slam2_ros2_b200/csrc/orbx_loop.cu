@@ -220,8 +220,8 @@ __device__ __noinline__ void hypothesis_solve(const Corr *corr, int n, unsigned 
 __device__ __forceinline__ double tree_sum(double p)
 {
 #pragma unroll
-  for (int s = 16; s; s >>= 1) p = dA(p, __shfl_down_sync(kMatchFull, p, s));
-  return __shfl_sync(kMatchFull, p, 0);
+  for (int s = 16; s; s >>= 1) p = dA(p, __shfl_down_sync(kFullMask, p, s));
+  return __shfl_sync(kFullMask, p, 0);
 }
 
 // Horn over the inliers of T0 in correspondence order, by one warp (lane l = the rule's partial of slot l)
@@ -304,7 +304,7 @@ __global__ void __launch_bounds__(kLT) loopver_pair_kernel(const LvArgs a)
         const int e = e0 + tid;
         const bool keep = e < n_rows && row[e] >= 0;
         int tot;
-        const int pos = nb + block_exscan<kLT>(keep, &tot, s_warp);
+        const int pos = nb + block_exclusive_scan<kLT>((int)keep, tot, s_warp);
         if (keep) kq[pos] = row[e], kc[pos] = m.k_feats[e];
         nb += tot;
       }
@@ -324,7 +324,7 @@ __global__ void __launch_bounds__(kLT) loopver_pair_kernel(const LvArgs a)
           const int i = i0 + tid;
           const bool ok = i < nm && dep_c[mc[i]] > 0.0 && dep_q[mq[i]] > 0.0;
           int tot;
-          const int pos = ncorr + block_exscan<kLT>(ok, &tot, s_warp);
+          const int pos = ncorr + block_exclusive_scan<kLT>((int)ok, tot, s_warp);
           if (ok)
           {
             Corr k;
@@ -353,7 +353,7 @@ __global__ void __launch_bounds__(kLT) loopver_pair_kernel(const LvArgs a)
             int cnt = 0;
             for (int i = lane; i < ncorr; i += 32) cnt += is_inlier(corr[i], s_T[warp], a);
 #pragma unroll
-            for (int o = 16; o; o >>= 1) cnt += __shfl_xor_sync(kMatchFull, cnt, o);
+            for (int o = 16; o; o >>= 1) cnt += __shfl_xor_sync(kFullMask, cnt, o);
             if (lane == 0) s_cnt[warp] = cnt;
           }
           __syncthreads();

@@ -1,19 +1,11 @@
-// orbx_match.cuh -- device building blocks of the Hamming matchers, shared by orbx_match.cu (one query per launch) and
-// orbx_loop.cu (every (query, candidate) pair of a loop-candidate table in one launch).
+// orbx_match.cuh -- device code of the Hamming matchers, shared by orbx_match.cu (one query per launch) and orbx_loop.cu
+// (every (query, candidate) pair of a loop-candidate table in one launch).
 #pragma once
 
 #include "orbx_device.cuh"
 
 namespace orbx
 {
-
-constexpr unsigned kMatchFull = 0xffffffffu;
-
-__device__ __forceinline__ int hamming256(const uint4 &a0, const uint4 &a1, const uint4 &b0, const uint4 &b1)
-{
-  return __popc(a0.x ^ b0.x) + __popc(a0.y ^ b0.y) + __popc(a0.z ^ b0.z) + __popc(a0.w ^ b0.w) + __popc(a1.x ^ b1.x) + __popc(a1.y ^ b1.y) +
-         __popc(a1.z ^ b1.z) + __popc(a1.w ^ b1.w);
-}
 
 // One chunk of up to 32 candidates (lane order == the reference's candidate order; id < 0: no candidate on this lane) of
 // ORBMatcher::getBestMatch (src/ORBMatcher.cc:967-990).  The sequential rule
@@ -22,31 +14,31 @@ __device__ __forceinline__ int hamming256(const uint4 &a0, const uint4 &a1, cons
 // every earlier one (the running minimum included); `second` is the minimum over all the others.
 __device__ __forceinline__ void best_match_chunk(int id, int d, int lane, int &n_cand, int &min_d, int &second_d, int &min_idx)
 {
-  const unsigned valid = __ballot_sync(kMatchFull, id >= 0);
+  const unsigned valid = __ballot_sync(kFullMask, id >= 0);
   if (!valid) return;
   n_cand += __popc(valid);
   int pm = d; // exclusive prefix minimum over the lanes, seeded with the running minimum
 #pragma unroll
   for (int s = 1; s < 32; s <<= 1)
   {
-    const int t = __shfl_up_sync(kMatchFull, pm, s);
+    const int t = __shfl_up_sync(kFullMask, pm, s);
     if (lane >= s) pm = min(pm, t);
   }
-  int ex = __shfl_up_sync(kMatchFull, pm, 1);
+  int ex = __shfl_up_sync(kFullMask, pm, 1);
   if (lane == 0) ex = 0x7fffffff;
   ex = min(ex, min_d);
   const bool is_new = id >= 0 && d < ex;
   int sec = (id >= 0 && !is_new) ? d : 0x7fffffff;
 #pragma unroll
-  for (int s = 16; s; s >>= 1) sec = min(sec, __shfl_xor_sync(kMatchFull, sec, s));
+  for (int s = 16; s; s >>= 1) sec = min(sec, __shfl_xor_sync(kFullMask, sec, s));
   second_d = min(second_d, sec);
   // the last "new minimum" lane of the chunk holds the chunk's minimum at its first occurrence
-  const unsigned news = __ballot_sync(kMatchFull, is_new);
+  const unsigned news = __ballot_sync(kFullMask, is_new);
   if (news)
   {
     const int src = 31 - __clz(news);
-    min_d = __shfl_sync(kMatchFull, d, src);
-    min_idx = __shfl_sync(kMatchFull, id, src);
+    min_d = __shfl_sync(kFullMask, d, src);
+    min_idx = __shfl_sync(kFullMask, id, src);
   }
 }
 
@@ -67,12 +59,7 @@ __device__ __forceinline__ void bow_match_row(const BowMatchArgs &a, int e, int 
   }
   const int node = a.k_nodes[lo];
   const int f_n = *a.f_n_nodes;
-  int l2 = 0, h2 = f_n; // first frame node >= node
-  while (l2 < h2)
-  {
-    const int mid = (l2 + h2) >> 1;
-    if (a.f_nodes[mid] < node) l2 = mid + 1; else h2 = mid;
-  }
+  const int l2 = lower_bound(a.f_nodes, 0, f_n, node);
   if (l2 >= f_n || a.f_nodes[l2] != node) return;
   const uint4 *qd = reinterpret_cast<const uint4 *>(a.k_desc + (size_t)pk * 32);
   const uint4 q0 = __ldg(qd), q1 = __ldg(qd + 1);
@@ -89,32 +76,6 @@ __device__ __forceinline__ void bow_match_row(const BowMatchArgs &a, int e, int 
     if (id >= 0) d = hamming256(q0, q1, __ldg(fd + 2 * id), __ldg(fd + 2 * id + 1));
     best_match_chunk(id, d, lane, n_cand, min_d, second_d, min_idx);
   }
-}
-
-// block-wide exclusive scan of one int per thread of a kThreads-thread CTA; *total = the block's sum
-template <int kThreads> __device__ __forceinline__ int block_exscan(int v, int *total, int *s_warp /* [kThreads / 32] */)
-{
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  int inc = v;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1)
-  {
-    const int t = __shfl_up_sync(kMatchFull, inc, o);
-    if (lane >= o) inc += t;
-  }
-  if (lane == 31) s_warp[wid] = inc;
-  __syncthreads();
-  int base = 0, tot = 0;
-#pragma unroll
-  for (int w = 0; w < kThreads / 32; ++w)
-  {
-    const int t = s_warp[w];
-    if (w < wid) base += t;
-    tot += t;
-  }
-  __syncthreads();
-  *total = tot;
-  return base + inc - v;
 }
 
 constexpr int kVaThreads = 256;
@@ -173,7 +134,7 @@ template <class BinOf, class Emit> __device__ __forceinline__ int verify_angle_b
     __syncthreads();
     const int i = i0 + tid;
     const int b = i < n ? bin_of(i) : -1;
-    const unsigned same = __match_any_sync(kMatchFull, b);
+    const unsigned same = __match_any_sync(kFullMask, b);
     const int rank = __popc(same & ((1u << lane) - 1));
     if (b >= 0 && rank == 0) s_wcount[warp][b] = __popc(same);
     __syncthreads();

@@ -21,32 +21,6 @@ namespace
 
 constexpr int kSerThreads = 256;
 
-// exclusive scan of one int per thread over the block; returns the block total in `total`
-__device__ __forceinline__ int block_exclusive_scan_ser(int v, int &total, int *s_warp /* [kSerThreads / 32] */)
-{
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  int inc = v;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1)
-  {
-    const int t = __shfl_up_sync(0xffffffffu, inc, o);
-    if (lane >= o) inc += t;
-  }
-  if (lane == 31) s_warp[wid] = inc;
-  __syncthreads();
-  int base = 0, tot = 0;
-#pragma unroll
-  for (int w = 0; w < kSerThreads / 32; ++w)
-  {
-    const int t = s_warp[w];
-    if (w < wid) base += t;
-    tot += t;
-  }
-  __syncthreads();
-  total = tot;
-  return base + inc - v;
-}
-
 __device__ __forceinline__ int put_varint(uint8_t *o, unsigned long long v)
 {
   int n = 0;
@@ -86,18 +60,6 @@ __device__ __forceinline__ int varint_len(unsigned long long v)
   return n;
 }
 
-// first index in the ascending a[lo, hi) whose value is >= v
-__device__ __forceinline__ int lower_bound_int(const int *a, int lo, int hi, int v)
-{
-  while (lo < hi)
-  {
-    const int mid = (lo + hi) >> 1;
-    if (a[mid] < v) lo = mid + 1;
-    else hi = mid;
-  }
-  return lo;
-}
-
 // FeatureVector.FeatureNode j: 0A len [08 node_id, left out when 0] 12 plen <packed varint feature ids>.  Feature ids
 // ascend inside a node and are < 2^16, so plen = count + (count >= 128) + (count >= 16384) from two binary searches.
 struct FvNode
@@ -109,8 +71,8 @@ __device__ __forceinline__ FvNode fv_node(const int *fv_nodes, const int *fv_sta
 {
   FvNode d;
   d.s = fv_start[j], d.e = fv_start[j + 1];
-  d.lb1 = lower_bound_int(fv_feats, d.s, d.e, 1 << 7);
-  d.lb2 = lower_bound_int(fv_feats, d.lb1, d.e, 1 << 14);
+  d.lb1 = lower_bound(fv_feats, d.s, d.e, 1 << 7);
+  d.lb2 = lower_bound(fv_feats, d.lb1, d.e, 1 << 14);
   d.node = fv_nodes[j];
   d.plen = (d.e - d.s) + (d.e - d.lb1) + (d.e - d.lb2);
   d.inner = (d.node ? 1 + varint_len((unsigned)d.node) : 0) + 1 + varint_len((unsigned)d.plen) + d.plen;
@@ -174,7 +136,7 @@ __global__ void __launch_bounds__(kSerThreads) serialize_kernel(const Params p, 
     int len = 0;
     if (i < n) len = keypoint_entry(kps[i], m);
     int total;
-    const int off = block_exclusive_scan_ser(len, total, s_warp);
+    const int off = block_exclusive_scan<kSerThreads>(len, total, s_warp);
     uint8_t *o = out + base + off;
     for (int k = 0; k < len; ++k) o[k] = m[k];
     base += total;
@@ -192,11 +154,11 @@ __global__ void __launch_bounds__(kSerThreads) serialize_kernel(const Params p, 
     n_bow = a.n_bow[frame], n_fv = a.n_fv[frame];
     // entry k = 0A len 08 <varint id> 11 <double>: 12 + varint_len(id) bytes; ids ascend, so the bytes before entry k are
     // 13 k + sum over t of max(0, k - s_lb[t])
-    if (tid < 4) s_lb[tid] = lower_bound_int(bow_ids, 0, n_bow, 1 << (7 * (tid + 1)));
+    if (tid < 4) s_lb[tid] = lower_bound(bow_ids, 0, n_bow, 1 << (7 * (tid + 1)));
     int mine = 0;
     for (int j = tid; j < n_fv; j += kSerThreads) mine += fv_node(fv_nodes, fv_start, fv_feats, j).len;
     int fv_total;
-    block_exclusive_scan_ser(mine, fv_total, s_warp); // its barriers also publish s_lb
+    block_exclusive_scan<kSerThreads>(mine, fv_total, s_warp); // its barriers also publish s_lb
     sz_bow = 13ll * n_bow;
     for (int t = 0; t < 4; ++t) sz_bow += n_bow - s_lb[t];
     sz_fv = fv_total;
@@ -294,7 +256,7 @@ __global__ void __launch_bounds__(kSerThreads) serialize_kernel(const Params p, 
     FvNode d{};
     if (j < n_fv) d = fv_node(fv_nodes, fv_start, fv_feats, j);
     int chunk_total;
-    const int off = block_exclusive_scan_ser(j < n_fv ? d.len : 0, chunk_total, s_warp);
+    const int off = block_exclusive_scan<kSerThreads>(j < n_fv ? d.len : 0, chunk_total, s_warp);
     if (j < n_fv)
     {
       uint8_t *o = out + fbase + off;

@@ -33,7 +33,6 @@ namespace
 
 constexpr int kVT = 256;     // threads per CTA
 constexpr int kTile = 4096;  // descriptors per tile
-constexpr unsigned kFull = 0xffffffffu;
 
 struct VbArgs
 {
@@ -57,38 +56,6 @@ struct VbArgs
   int *changed, *active, *iters, *capped; // [S]
   int *n_active;
 };
-
-__device__ __forceinline__ int hamming(uint4 a0, uint4 a1, uint4 b0, uint4 b1)
-{
-  return __popc(a0.x ^ b0.x) + __popc(a0.y ^ b0.y) + __popc(a0.z ^ b0.z) + __popc(a0.w ^ b0.w) + __popc(a1.x ^ b1.x) + __popc(a1.y ^ b1.y) +
-         __popc(a1.z ^ b1.z) + __popc(a1.w ^ b1.w);
-}
-
-// exclusive block scan of one 64-bit value per thread; *total = the block's sum
-__device__ unsigned long long block_exscan(unsigned long long v, unsigned long long *total, unsigned long long *s_warp)
-{
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  unsigned long long inc = v;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1)
-  {
-    const unsigned long long t = __shfl_up_sync(kFull, inc, o);
-    if (lane >= o) inc += t;
-  }
-  if (lane == 31) s_warp[wid] = inc;
-  __syncthreads();
-  unsigned long long base = 0, tot = 0;
-#pragma unroll
-  for (int w = 0; w < kVT / 32; ++w)
-  {
-    const unsigned long long t = s_warp[w];
-    if (w < wid) base += t;
-    tot += t;
-  }
-  __syncthreads();
-  *total = tot;
-  return base + inc - v;
-}
 
 __global__ void __launch_bounds__(kVT) vocab_gather_kernel(const uint4 *src, const int *n_kps, const long long *row_off, int stride, long long n_rows_x_stride,
                                                             uint4 *D)
@@ -119,13 +86,13 @@ __global__ void __launch_bounds__(kVT) vocab_kpp_dist_kernel(const VbArgs a, int
   for (int e = threadIdx.x; e < len; e += kVT)
   {
     const size_t g = (size_t)base + e;
-    int d = hamming(a.D[2 * g], a.D[2 * g + 1], c0, c1);
+    int d = hamming256(a.D[2 * g], a.D[2 * g + 1], c0, c1);
     if (round > 1) d = min(d, (int)a.md[g]);
     a.md[g] = (uint16_t)d;
     sum += (unsigned long long)d;
   }
   unsigned long long total;
-  block_exscan(sum, &total, s_warp);
+  block_exclusive_scan<kVT>(sum, total, s_warp);
   if (threadIdx.x == 0) a.tile_sum[t] = total;
 }
 
@@ -155,7 +122,7 @@ __global__ void __launch_bounds__(kVT) vocab_kpp_pick_kernel(const VbArgs a, int
   unsigned long long mine = 0;
   for (int j = j0; j < j1; ++j) mine += a.tile_sum[t0 + j];
   unsigned long long S;
-  const unsigned long long ex = block_exscan(mine, &S, s_warp);
+  const unsigned long long ex = block_exclusive_scan<kVT>(mine, S, s_warp);
   if (S == 0) return; // every descriptor equals a centre: fewer than k clusters
   const unsigned long long cut = 1 + splitmix64(K ^ ((unsigned long long)round * kGolden)) % S;
   if (ex < cut && cut <= ex + mine)
@@ -181,7 +148,7 @@ __global__ void __launch_bounds__(kVT) vocab_kpp_pick_kernel(const VbArgs a, int
   unsigned long long mine2 = 0;
   for (int e = e0; e < e1; ++e) mine2 += a.md[(size_t)base + e];
   unsigned long long tot2;
-  const unsigned long long ex2 = block_exscan(mine2, &tot2, s_warp);
+  const unsigned long long ex2 = block_exclusive_scan<kVT>(mine2, tot2, s_warp);
   if (ex2 < rem && rem <= ex2 + mine2)
   {
     unsigned long long run = ex2;
@@ -232,11 +199,11 @@ __global__ void __launch_bounds__(kVT) vocab_assign_kernel(const VbArgs a, int p
     {
       const size_t g = (size_t)base + e;
       x0 = a.D[2 * g], x1 = a.D[2 * g + 1];
-      int best = hamming(x0, x1, s_c[0][0], s_c[0][1]);
+      int best = hamming256(x0, x1, s_c[0][0], s_c[0][1]);
       bc = 0;
       for (int c = 1; c < nk; ++c)
       {
-        const int d = hamming(x0, x1, s_c[c][0], s_c[c][1]);
+        const int d = hamming256(x0, x1, s_c[c][0], s_c[c][1]);
         if (d < best) best = d, bc = c;
       }
       if (pass > 1 && a.asg[g] != bc) changed = true;
@@ -252,14 +219,14 @@ __global__ void __launch_bounds__(kVT) vocab_assign_kernel(const VbArgs a, int p
 #pragma unroll
       for (int b = 0; b < 32; ++b)
       {
-        const unsigned m = __ballot_sync(kFull, (xw[q] >> b) & 1u);
+        const unsigned m = __ballot_sync(kFullMask, (xw[q] >> b) & 1u);
         if (lane == b) mine = m;
       }
       col[q] = mine;
     }
     for (int c = 0; c < nk; ++c)
     {
-      const unsigned in_c = __ballot_sync(kFull, bc == c);
+      const unsigned in_c = __ballot_sync(kFullMask, bc == c);
       if (!in_c) continue;
       if (lane == 0) atomicAdd(&s_mem[c], (unsigned)__popc(in_c));
 #pragma unroll
@@ -298,7 +265,7 @@ __global__ void __launch_bounds__(kVT) vocab_update_kernel(const VbArgs a, int p
   {
     const unsigned m = a.members[(size_t)seg * a.k + c];
     if (m == 0) continue; // an empty cluster keeps its centre
-    const unsigned w = __ballot_sync(kFull, g_cnt[c * 256 + tid] >= (m + 1) / 2);
+    const unsigned w = __ballot_sync(kFullMask, g_cnt[c * 256 + tid] >= (m + 1) / 2);
     if ((tid & 31) == 0) cw[c * 8 + (tid >> 5)] = w;
   }
   __syncthreads();
@@ -339,7 +306,7 @@ __global__ void __launch_bounds__(kVT) vocab_scatter_kernel(const VbArgs a)
     const int bc = e < w1 ? (int)a.asg[(size_t)base + e] : -1;
     for (int c = 0; c < nk; ++c)
     {
-      const unsigned m = __ballot_sync(kFull, bc == c);
+      const unsigned m = __ballot_sync(kFullMask, bc == c);
       if (lane == c) cnt_c += __popc(m);
     }
   }
@@ -358,11 +325,11 @@ __global__ void __launch_bounds__(kVT) vocab_scatter_kernel(const VbArgs a)
     int add = 0;
     for (int c = 0; c < nk; ++c)
     {
-      const unsigned m = __ballot_sync(kFull, bc == c);
+      const unsigned m = __ballot_sync(kFullMask, bc == c);
       if (bc == c) mine = m;
       if (lane == c) add = __popc(m);
     }
-    const int before = __shfl_sync(kFull, run, valid ? bc : 0);
+    const int before = __shfl_sync(kFullMask, run, valid ? bc : 0);
     if (valid && dst[bc] >= 0)
     {
       const size_t o = (size_t)dst[bc] + before + __popc(mine & ((1u << lane) - 1u));
